@@ -15,6 +15,7 @@ reference on the host cores) and ``extra`` (BASELINE configs[0], [2], [4]: ESOL 
 screening at batch 4096, skewed-degree stress at batch 1024).
 
   python bench.py --gpus N --steps K --warmup W             (torchrun launches N ranks for N > 1)
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's results as DIR/*.npy
   python bench.py --impl reference ...                      the reference itself on the host cores, same metric
 """
 from __future__ import annotations
@@ -68,7 +69,15 @@ def parse():
     ap.add_argument("--no-plan-prefetch", action="store_true",
                     help="collate every batch at the head of its own step instead of underneath the previous one")
     ap.add_argument("--no-tf32", action="store_true", help="skip the second timed region (value_tf32)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of `value`, write what their last step returned to its caller (loss, "
+                         "updated parameters, their gradients) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is supported for --impl ours only")
+    return args
 
 
 def make_batches(shape, batch, rotate, pool, seed, pretrain=True):
@@ -449,9 +458,10 @@ def run_reference(args):
 
 # ------------------------------------------------------------------------------------------------
 def make_step(batch=1024, shape="unimol", rotate=4, pool=512, precision="fp32", rank=0, world=1, dev=None,
-              return_host=False, autograd_path=False, pack=False):
+              return_host=False, autograd_path=False, pack=False, return_model=False):
     """The timed unit: ``step(batch_dict)`` = on-device collate + forward + loss + backward + gradient all-reduce
-    (world > 1) + Adam on one batch.  Returns (step, device batches[, pinned host batches in the compact wire format])."""
+    (world > 1) + Adam on one batch.  Returns (step, device batches[, pinned host batches in the compact wire format]
+    [, the model the step trains])."""
     from fragnet.model.gat.gat2_pretrain import FragNetPreTrain
     from fragnet_b200 import config, ops
     from fragnet_b200.dataset.data import compact_batch, pack_batch
@@ -490,7 +500,8 @@ def make_step(batch=1024, shape="unimol", rotate=4, pool=512, precision="fp32", 
         from fragnet_b200.train.fused import FusedPretrainStep
         step = FusedPretrainStep(model, lr=LR).step
 
-    return (step, dev_batches, host_batches) if return_host else (step, dev_batches)
+    out = (step, dev_batches, host_batches) if return_host else (step, dev_batches)
+    return out + (model,) if return_model else out
 
 
 class Timer:
@@ -519,6 +530,22 @@ class Timer:
             import torch.distributed as dist
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms), self.lib.fnb_launch_count() - l0
+
+
+def dump_outputs(path, model, loss):
+    """``--dump-outputs``: what a training step hands its caller -- the loss, and the model's parameters after the
+    Adam update with the gradients they were updated from -- one float32 ``.npy`` per array (~6 MB in all at PT_KW),
+    so that two builds run with the same arguments can be compared array by array.  Returns the file names."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {"loss": loss}
+    for name, p in model.named_parameters():
+        arrays[f"param.{name}"] = p
+        if p.grad is not None:
+            arrays[f"grad.{name}"] = p.grad
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+    return sorted(arrays)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -611,8 +638,9 @@ def run_ours(args):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     lib = _abi.load()
-    step, dev_batches, host_batches = make_step(args.batch, args.shape, args.rotate, args.pool, args.precision, rank,
-                                                world, dev, return_host=True, autograd_path=args.autograd, pack=args.pack)
+    step, dev_batches, host_batches, model = make_step(args.batch, args.shape, args.rotate, args.pool, args.precision,
+                                                       rank, world, dev, return_host=True, autograd_path=args.autograd,
+                                                       pack=args.pack, return_model=True)
     timed = Timer(dev, world, lib)
     barrier = timed.barrier
     # a training loop knows its next batch: its on-device collate is queued underneath the running step
@@ -620,8 +648,10 @@ def run_ours(args):
     fs = getattr(step, "__self__", None)
     prefetch = fs.prefetch_plan if (fs is not None and hasattr(fs, "prefetch_plan") and not args.no_plan_prefetch) else None
 
+    last_loss = [None]
+
     def resident(i):
-        loss = step(dev_batches[i % args.rotate])
+        loss = last_loss[0] = step(dev_batches[i % args.rotate])
         if prefetch is not None:
             prefetch(dev_batches[(i + 1) % args.rotate])
         return loss
@@ -636,6 +666,9 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     mols = args.batch * world * args.steps
     value = mols / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # before the legs below take further steps on the same model
+        dump_outputs(args.dump_outputs, model, last_loss[0])
 
     # ---- the same step with single-TF32 products (stated tolerance 2e-3): value_tf32
     tf32 = None
@@ -770,7 +803,7 @@ def run_ours(args):
     # ---- BASELINE configs[4] and [2] on every rank (weak scaling / replicas), configs[0] on rank 0's host cores
     extra = {}
     if not args.no_extras and not args.autograd:
-        del step, dev_batches
+        del step, dev_batches, model
         torch.cuda.empty_cache()
         config.set_precision("fp32")
         for name, fn in (("stress_b1024", extra_stress), ("infer_b4096", extra_inference)):
