@@ -20,7 +20,6 @@ SIGNATURES = {
     "fnb_scratch_bytes": (_sz, []),
     "fnb_csr_workspace_bytes": (_sz, [_i64, _i64]),
     "fnb_csr_build": (C.c_int, [_vp, _vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp]),
-    "fnb_tile_ranges": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "fnb_gather_rows": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "fnb_segment_offsets": (C.c_int, [_vp, _i64, _i64, _vp, _vp]),
     "fnb_narrow_index": (C.c_int, [_vp, _i64, _vp, _vp]),
@@ -47,7 +46,6 @@ SIGNATURES = {
     "fnb_gat_fwd_tiled": (C.c_int, [_vp, _vp, _vp]),
     "fnb_gat_bwd_tiled": (C.c_int, [_vp, _vp, _vp]),
     "fnb_gat_bwd_tiled_marked": (C.c_int, [_vp, _vp, _vp, _vp]),
-    "fnb_debug_set_fused_bwd": (None, [C.c_int]),
     "fnb_edge_table_bwd_fused": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _f32, _vp, _vp, _vp, _vp]),
     "fnb_batch_plan_bytes": (_sz, [_vp]),
     "fnb_batch_plan_build": (C.c_int, [_vp, _vp, _sz, _vp, _vp]),
@@ -74,9 +72,7 @@ SIGNATURES = {
 class CGraph(C.Structure):
     _fields_ = [("n_nodes", _i64), ("n_edges", _i64), ("n_real_edges", _i64),
                 ("rowptr", _vp), ("col", _vp), ("row", _vp), ("eid", _vp), ("slot_of_eid", _vp),
-                ("rrowptr", _vp), ("rslot", _vp), ("rdst", _vp), ("tile_range", _vp), ("rtile_range", _vp),
-                ("edge_attr", _vp), ("comp_ptr", _vp), ("n_comps", _i64), ("comp_bucket", _vp),
-                ("comp_open", _vp)]
+                ("rrowptr", _vp), ("rslot", _vp), ("rdst", _vp), ("edge_attr", _vp)]
 
 
 class CPostAct(C.Structure):
@@ -116,7 +112,7 @@ class CWidenJob(C.Structure):
 WIDEN_U8_F32, WIDEN_I32_I64, WIDEN_MAX_JOBS = 0, 1, 16
 ARENA_COPY32, ARENA_INDEX, ARENA_FILL = 0, 1, 2
 ARENA_MAX_KINDS, ARENA_MAX_JOBS = 24, 32
-ABI_VERSION = 8
+ABI_VERSION = 9
 EDGE_NONE, EDGE_AFFINE1, EDGE_AFFINE6, EDGE_TABLE = 0, 1, 2, 3
 PRECISION_FP32, PRECISION_TF32, PRECISION_TF32X3 = 0, 1, 2
 

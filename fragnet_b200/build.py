@@ -48,7 +48,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
         raise RuntimeError("nvcc not found: cannot build libfragnet_b200.so")
     os.makedirs(LIB_DIR, exist_ok=True)
     tmp = f"{LIB_PATH}.{os.getpid()}.tmp"      # several ranks may build at once: private output, atomic rename
-    extra = os.environ.get("FNB_EXTRA_NVCC", "").split()      # experiments only (e.g. -DFNB_PDL_EARLY=1)
+    extra = os.environ.get("FNB_EXTRA_NVCC", "").split()      # experiments only (extra nvcc flags)
     cmd = [nvcc, *NVCC_FLAGS, *extra, "-I", INCLUDE, "-I", CSRC, "-o", tmp, *sources()]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")

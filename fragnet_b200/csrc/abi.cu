@@ -37,24 +37,9 @@ int fnb_aux_streams(FnbAux *out) {
     if (cudaEventCreateWithFlags(&a.fork, cudaEventDisableTiming) != cudaSuccess) return 1;
     if (cudaEventCreateWithFlags(&a.join, cudaEventDisableTiming) != cudaSuccess) return 1;
     if (cudaStreamCreateWithFlags(&a.wstream, cudaStreamNonBlocking) != cudaSuccess) return 1;
-    {
-      // Experiment switch FNB_PRIO=1: highest priority for the atom chain, whose short kernels otherwise wait for an
-      // SM slot behind the ~850 CTAs of a bond-graph launch.  Measured SLOWER (profiles/r3d_*: 1.370 vs 1.334 ms per
-      // step: the bond kernels it displaces are the critical path and the step is throughput-bound), hence off.
-      int least = 0, greatest = 0;
-      const char *e = getenv("FNB_PRIO");
-      const bool prio = e && e[0] == '1' && cudaDeviceGetStreamPriorityRange(&least, &greatest) == cudaSuccess;
-      if (cudaStreamCreateWithPriority(&a.astream, cudaStreamNonBlocking, prio ? greatest : 0) != cudaSuccess) return 1;
-    }
+    if (cudaStreamCreateWithFlags(&a.astream, cudaStreamNonBlocking) != cudaSuccess) return 1;
     if (cudaStreamCreateWithFlags(&a.estream, cudaStreamNonBlocking) != cudaSuccess) return 1;
-    {
-      // FNB_HEAD_PRIO=1 (measurement switch): highest priority for the energy head's stream.  No effect on the step
-      // (1.298 vs 1.296 ms, gpurun_out/r5n), hence off.
-      int least = 0, greatest = 0;
-      const char *e = getenv("FNB_HEAD_PRIO");
-      const bool prio = e && e[0] == '1' && cudaDeviceGetStreamPriorityRange(&least, &greatest) == cudaSuccess;
-      if (cudaStreamCreateWithPriority(&a.hstream, cudaStreamNonBlocking, prio ? greatest : 0) != cudaSuccess) return 1;
-    }
+    if (cudaStreamCreateWithFlags(&a.hstream, cudaStreamNonBlocking) != cudaSuccess) return 1;
     if (cudaEventCreateWithFlags(&a.h_done, cudaEventDisableTiming) != cudaSuccess) return 1;
     if (cudaStreamCreateWithFlags(&a.pstream, cudaStreamNonBlocking) != cudaSuccess) return 1;
     if (cudaStreamCreateWithFlags(&a.wstream2, cudaStreamNonBlocking) != cudaSuccess) return 1;
@@ -76,26 +61,3 @@ bool fnb_pdl_enabled() {
   static const bool on = [] { const char *e = getenv("FNB_PDL"); return !(e && e[0] == '0'); }();
   return on;
 }
-
-// FNB_STAGE=1: bulk-copy (TMA) staging of the gathered source rows in the attention forward (measured slower than the
-// gather path on B200, profiles/r1h_kbench_stage*.log); the plan computes the tile ranges it needs only then.
-bool fnb_use_staging() {
-  static const bool on = [] { const char *e = getenv("FNB_STAGE"); return e && e[0] == '1'; }();
-  return on;
-}
-
-// One-kernel attention backward for graphs with a component table (gat_tiled.cu: k_gat_bwd_fused).  Opt-in
-// (FNB_FUSED_BWD=1 or fnb_debug_set_fused_bwd(1)): measured no faster than the two-pass kernels on B200 in any of the
-// three forms tried (DESIGN.md section 3, gpurun_out/r5c..r5f_fused_bwd_bench.log); the batch plan builds the
-// component tables only while it is on.
-static int g_fused_bwd = -1;
-bool fnb_fused_bwd_enabled() {
-  int v = __atomic_load_n(&g_fused_bwd, __ATOMIC_RELAXED);
-  if (v < 0) {
-    const char *e = getenv("FNB_FUSED_BWD");
-    v = e && e[0] == '1';
-    __atomic_store_n(&g_fused_bwd, v, __ATOMIC_RELAXED);
-  }
-  return v != 0;
-}
-extern "C" void fnb_debug_set_fused_bwd(int on) { __atomic_store_n(&g_fused_bwd, on ? 1 : 0, __ATOMIC_RELAXED); }

@@ -75,19 +75,9 @@ __device__ __forceinline__ float leaky(float z) { return z > 0.f ? z : kNegSlope
 // previous grid has completed and flushed.  Every kernel launched through fnb_launch() calls pdl_wait() before its
 // first access to global memory and pdl_launch_dependents() once its main loop is done.  Both are no-ops for a
 // kernel launched without the attribute (FNB_PDL=0 in the environment turns the attribute off).
-#ifndef FNB_PDL_EARLY
-#define FNB_PDL_EARLY 0   // 1: signal the dependents right after pdl_wait() instead of after the main loop (experiment)
-#endif
-__device__ __forceinline__ void pdl_wait() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#if FNB_PDL_EARLY
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 bool fnb_pdl_enabled();
-bool fnb_use_staging();
-bool fnb_fused_bwd_enabled();   // FNB_FUSED_BWD=0 or fnb_debug_set_fused_bwd(0): two-pass attention backward only
 template <class... KArgs, class... Args>
 inline cudaError_t fnb_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                               Args... args) {
@@ -100,42 +90,6 @@ inline cudaError_t fnb_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   cfg.numAttrs = fnb_pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
-
-// ---- mbarrier + bulk asynchronous copy (TMA engine, 1-D): global -> shared memory ---------------------------------
-namespace bulk {
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.b32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-// Bounded spin: a protocol bug traps (reported as a launch failure) instead of hanging the GPU.
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  for (uint32_t spins = 0; !mbar_try_wait(bar, parity); ++spins)
-    if (spins > (1u << 26)) __trap();
-}
-// Orders this thread's earlier generic-proxy accesses to shared memory before later async-proxy (bulk copy) writes.
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// bytes: multiple of 16; src and dst 16-byte aligned.  Completion is signalled on `bar` (complete_tx).
-__device__ __forceinline__ void copy_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-}  // namespace bulk
 
 // ---- counter-based RNG for dropout masks (regenerated from (seed, counter), never stored) ------
 // Philox4x32-10 cost ~135 instructions per group of 4 elements and made the fused forward epilogue the largest single
@@ -260,19 +214,6 @@ int fnb_launch_reduce_segments(const float *partials, int n_blocks, int pstride,
 int fnb_launch_reduce_partials(const float *partials, int n_blocks, int pstride, int width, float *out, int row_len,
                                int out_stride, int accumulate, cudaStream_t stream);
 
-// Tile source ranges for the bulk-copy staging of gathered rows (csr.cu): up to 8 CSRs per launch.
-constexpr int kRangeTile = 64;
-struct RangeJobs {
-  const int *rowptr[8];
-  const int *col[8];
-  int n_nodes[8];
-  int *out[8];
-  int tile_base[8];   // first global tile index of job i; tile_base[n_jobs] = total
-  int n_jobs;
-  int total_tiles;
-};
-int fnb_launch_tile_ranges(const RangeJobs &jobs, cudaStream_t stream);
-
 // Auxiliary stream of the calling thread's current device (abi.cu); returns non-zero when only the caller's stream
 // should be used.
 struct FnbAux {
@@ -306,7 +247,6 @@ struct FnbDstFuse {
   float scale;
   const float *pool;         // [n_seg,128] gradient of sum-pooled rows to hand back to their members, or NULL
   const int *seg_of;         // [N]
-  int skip_dz;               // nobody reads args->dz after this call: the one-kernel backward keeps it in shared memory
 };
 int fnb_gat_bwd_tiled_fused(const fnb_graph *g, const fnb_gat_bwd_args *args, const FnbDstFuse *fuse,
                             cudaEvent_t after_dst, cudaEvent_t before_src, void *stream);
@@ -331,7 +271,6 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
 // x3 != 0: 3xTF32 (error-compensated, FP32-grade) instead of one TF32 product.
 int fnb_tc_proj_launch(const float *A, const float *B, const float *bias, int64_t M, int K, const float *alpha,
                        int alpha_stride, int off_t, int off_s, float *C, float *S, cudaStream_t stream, int x3);
-void fnb_tc_set_cta_cap(int cap);   // CTA cap of this thread's next projection launches (0 = none)
 int fnb_tc_transpose128_launch(const float *W, float *Wt, cudaStream_t stream);
 // Up to 16 [128,128] matrices transposed by one launch: Wt_base + i * 128 * 128 = Ws[i]^T.
 // zero[0..n_zero): scratch buffers whose arrival counters (first kScratchCounters floats) the launch clears on the way --

@@ -211,35 +211,6 @@ __global__ void k_narrow(const int64_t *__restrict__ in, int64_t n, int *__restr
     out[i] = (int)in[i];
 }
 
-// One warp per tile of kRangeTile consecutive rows: min / max column index over the tile's slots.
-__global__ void __launch_bounds__(256) k_tile_ranges(RangeJobs j) {
-  const int lane = threadIdx.x & 31;
-  const int w0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
-  for (int gt = w0; gt < j.total_tiles; gt += nw) {
-    int job = 0;
-#pragma unroll
-    for (int i = 1; i < 8; ++i) job += (i < j.n_jobs && gt >= j.tile_base[i]);
-    const int t = gt - j.tile_base[job];
-    const int n0 = t * kRangeTile, n1 = min(n0 + kRangeTile, j.n_nodes[job]);
-    const int beg = j.rowptr[job][n0], end = j.rowptr[job][n1];
-    int lo = INT32_MAX, hi = -1;
-    for (int s = beg + lane; s < end; s += 32) {
-      const int c = j.col[job][s];
-      lo = min(lo, c);
-      hi = max(hi, c);
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      lo = min(lo, __shfl_xor_sync(kFull, lo, o));
-      hi = max(hi, __shfl_xor_sync(kFull, hi, o));
-    }
-    if (lane == 0) {
-      j.out[job][2 * t] = hi >= 0 ? lo : 0;
-      j.out[job][2 * t + 1] = hi >= 0 ? hi + 1 : 0;
-    }
-  }
-}
-
 inline int grid_for(int64_t n, int block) {
   int64_t g = (n + block - 1) / block;
   const int64_t cap = (int64_t)kNumSMs * 16;
@@ -327,28 +298,6 @@ extern "C" int fnb_csr_build(const int64_t *dst, const int64_t *src, int64_t n_e
     }
   }
   return 0;
-}
-
-int fnb_launch_tile_ranges(const RangeJobs &jobs, cudaStream_t stream) {
-  if (jobs.total_tiles <= 0) return 0;
-  int64_t blocks = ((int64_t)jobs.total_tiles + 7) / 8;
-  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-  k_tile_ranges<<<(int)blocks, 256, 0, stream>>>(jobs);
-  FNB_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" int fnb_tile_ranges(const int32_t *rowptr, const int32_t *col, int64_t n_nodes, int32_t *ranges,
-                               void *stream) {
-  if (n_nodes < 0 || n_nodes >= (int64_t)INT32_MAX) return FNB_ERR_SIZE;
-  if (n_nodes == 0) return 0;
-  if (!rowptr || !col || !ranges) return FNB_ERR_NULL;
-  RangeJobs j{};
-  j.rowptr[0] = rowptr; j.col[0] = col; j.n_nodes[0] = (int)n_nodes; j.out[0] = ranges; j.tile_base[0] = 0;
-  j.n_jobs = 1;
-  j.total_tiles = (int)((n_nodes + kRangeTile - 1) / kRangeTile);
-  j.tile_base[1] = j.total_tiles;
-  return fnb_launch_tile_ranges(j, (cudaStream_t)stream);
 }
 
 extern "C" int fnb_gather_rows(const float *in, const int32_t *index, int64_t n_rows, int width, float *out,

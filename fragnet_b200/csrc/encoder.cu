@@ -13,8 +13,6 @@
 // ReLU(Dropout), the consumer graph's edge term, the fragment graph's node scalars.
 // Backward: per graph one destination pass + one source pass (parameter-gradient reductions inside), the edge-table
 // backward with the ReLU(Dropout) backward folded in, and the projection backward (dX, dW).
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace {
@@ -260,16 +258,6 @@ __global__ void __launch_bounds__(256) k_gather_rows4(const float *__restrict__ 
   if (e < n) st4(out + e * 4, ldg4(src + (int64_t)__ldg(index + e) * 4));
 }
 
-// CTA cap of the side chains' tcgen05 GEMMs (FNB_SIDE_CTAS, 0 = no cap), see fnb_tc_set_cta_cap.
-int side_ctas() {
-  static const int v = getenv("FNB_SIDE_CTAS") ? atoi(getenv("FNB_SIDE_CTAS")) : 0;
-  return v;
-}
-struct SideCap {     // scope guard
-  explicit SideCap(bool on) { if (on) fnb_tc_set_cta_cap(side_ctas()); }
-  ~SideCap() { fnb_tc_set_cta_cap(0); }
-};
-
 #define RC(expr)            \
   do {                      \
     const int rc__ = (expr); \
@@ -435,10 +423,7 @@ int fnb_encoder_forward_impl(const fnb_batch_plan *plan, const fnb_encoder_opts 
       RC((int)cudaEventRecord(aux.a_fork, stream));
       RC((int)cudaStreamWaitEvent(sA, aux.a_fork, 0));
     }
-    {
-      SideCap cap(two);
-      RC(fnb_proj_fwd(xa_in, Wa_in, P.ba, z.Na, Ka_in, P.a, A_STRIDE, A_T, A_S, b.ha, b.Sa, o->precision, sA_));
-    }
+    RC(fnb_proj_fwd(xa_in, Wa_in, P.ba, z.Na, Ka_in, P.a, A_STRIDE, A_T, A_S, b.ha, b.Sa, o->precision, sA_));
     // ---- bond graph (gat2.py:138-176); epilogue emits the atom graph's edge term <new_bond[e], a_e[h]>
     RC(fnb_proj_fwd(xb_in, Wb_in, P.bb, z.Nb, Kb_in, P.a_b, AB_STRIDE, AB_T, AB_S, b.hb, b.Sb, o->precision, stream_));
     {
@@ -479,11 +464,8 @@ int fnb_encoder_forward_impl(const fnb_batch_plan *plan, const fnb_encoder_opts 
       a_pending = true;
     }
     // ---- fragment-connection graph (gat2.py:239-278); epilogue emits the fragment graph's edge term
-    {
-      SideCap cap(two);
-      RC(fnb_proj_fwd(xfb_in, Wfb_in, P.bfb, z.Nfb, Kfb_in, P.f_a_b, AB_STRIDE, AB_T, AB_S, b.hfb, b.Sfb, o->precision,
-                      sB_));
-    }
+    RC(fnb_proj_fwd(xfb_in, Wfb_in, P.bfb, z.Nfb, Kfb_in, P.f_a_b, AB_STRIDE, AB_T, AB_S, b.hfb, b.Sfb, o->precision,
+                    sB_));
     pending = true;
     {
       fnb_gat_fwd_args f{};
@@ -705,17 +687,13 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
         FnbDstFuse fz{};
         fz.dz_up = frag_feeds_fbond ? W.dz_f : nullptr; fz.slot_of_eid = plan->frag.slot_of_eid; fz.alpha_up = P.f + A_E;
         fz.alpha_up_stride = A_STRIDE; fz.dy = dy_fbond; fz.y = dy_fbond ? y_fbond : nullptr; fz.scale = scale;
-        fz.skip_dz = 1;   // dz of this graph has no consumer
         RC(fnb_gat_bwd_tiled_fused(&plan->fbond, &a, &fz, nullptr, nullptr, sB_));
         float *dx = need_dx ? W.dx_fbond : (o->need_dx_fbond ? io->dx_fbond : nullptr);
         if (l == 0 && b.k_pad[2] && !dx)
           RC(fnb_tc_dw_launch(W.dh_fb, b.x_pad[2], z.Nfb, b.k_pad[2], P.K_fbond, D.Wfb, scratch_body(scratchB), sB, x3));
         else
-        {
-          SideCap cap(two);
           RC(fnb_proj_bwd_impl(xfb, P.Wfb, wt_of(l, 2), W.dh_fb, z.Nfb, P.K_fbond, dx, D.Wfb, nullptr, o->precision,
                                scratchB, sB_));
-        }
         dy_fbond = need_dx ? W.dx_fbond : nullptr;
       } else {
         dy_fbond = nullptr;
@@ -762,10 +740,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
         if (l == 0 && b.k_pad[1] && !dx) {
           RC(fnb_tc_dw_launch(dh_a, b.x_pad[1], z.Na, b.k_pad[1], P.K_atom, D.Wa, scratch_body(scratchWs[0]), sWs[0], x3));
         } else {
-          {
-            SideCap cap(two);
-            RC(fnb_proj_bwd_dx(P.Wa, wt_of(l, 1), dh_a, z.Na, P.K_atom, dx, o->precision, scratchA, sA_));
-          }
+          RC(fnb_proj_bwd_dx(P.Wa, wt_of(l, 1), dh_a, z.Na, P.K_atom, dx, o->precision, scratchA, sA_));
           RC(fnb_proj_bwd_dw(xa, dh_a, z.Na, P.K_atom, D.Wa, nullptr, o->precision, scratchWs[0], (void *)sWs[0]));
         }
         RC(w_end(0, par));
@@ -809,7 +784,6 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
         fz.dz_up = have ? dz_a : nullptr; fz.slot_of_eid = plan->atom.slot_of_eid; fz.alpha_up = P.a + A_E;
         fz.alpha_up_stride = A_STRIDE; fz.g_base = y_bond ? nullptr : dy_bond; fz.dy = y_bond ? dy_bond : nullptr;
         fz.y = y_bond && dy_bond ? y_bond : nullptr; fz.scale = scale;
-        fz.skip_dz = 1;   // dz of this graph has no consumer
         // (the weight-gradient GEMM two layers above read this dh buffer: only the source pass has to wait for it)
         const bool wait_w = two && w_pending[1][par];
         w_pending[1][par] = false;

@@ -18,9 +18,6 @@
 // The tiny edge-embedding algebra (App. A.5), the inter-layer ReLU(Dropout(.)) (gat2.py:414-418), the output masks
 // (gat2.py:173-176) and the consumer graph's edge term ride in the prologue/epilogue, and parameter-gradient partials
 // are reduced by the last CTA to finish (common.cuh: cta_finish) -- no floating-point atomics, no extra launches.
-#include <algorithm>
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace {
@@ -30,14 +27,7 @@ constexpr int T_THREADS = 256;
 constexpr int T_WARPS = T_THREADS / 32;
 constexpr int FWD_CAP = 1024;    // edge slots staged per sub-tile (forward)
 constexpr int BWD_CAP = 768;     // edge slots staged per sub-tile (backward kernels stage two float4 per slot)
-// Bulk-copy staging of the gathered rows.  Batched molecular graphs are block diagonal with consecutive node ids per
-// molecule, so the SOURCES of 64 consecutive destinations lie in a short contiguous id range (bond graph: ~105 rows,
-// atom graph: ~90): instead of E x 512-byte gathers through L1/L2, one cp.async.bulk (TMA) copies that row range
-// into shared memory while the logits are computed, and the aggregation reads it from there.  Tiles whose range
-// exceeds ROWS_CAP (or graphs without range hints) use the gather path.
-constexpr int ROWS_CAP = 160;
-constexpr size_t kStageRowsBytes = (size_t)ROWS_CAP * kD * 4;
-constexpr size_t kStageSBytes = (size_t)ROWS_CAP * 8 * 4;
+constexpr int kDeepDegree = 24;  // mean in-degree from which the DEEP instantiations pay
 
 // Largest le in (lb, nn] whose slots fit `cap`; returns lb when node lb alone exceeds it (hub path).
 __device__ __forceinline__ int subtile_end(const int *s_rowptr, int lb, int nn, int cap) {
@@ -63,18 +53,8 @@ struct FwdT {
   int next_stride;
   float *next_Se;
   int npc;
-  const int *tile_range;
   int deep;       // mean in-degree >= kDeepDegree: the DEEP instantiation
-  int prefetch;   // FNB_PREFETCH=1: phase 1 asks L2 for the source rows phase 3 will gather
 };
-
-__device__ __forceinline__ void prefetch_row_l2(const float *row) {
-  const char *p = reinterpret_cast<const char *>(row);
-  asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
-  asm volatile("prefetch.global.L2 [%0];" ::"l"(p + 128));
-  asm volatile("prefetch.global.L2 [%0];" ::"l"(p + 256));
-  asm volatile("prefetch.global.L2 [%0];" ::"l"(p + 384));
-}
 
 template <int MODE>
 __device__ __forceinline__ float4 edge_term_t(const FwdT &a, int slot, const float *coef) {
@@ -106,10 +86,9 @@ __device__ __forceinline__ float4 edge_term_t(const FwdT &a, int slot, const flo
 }
 
 template <int MODE>
-__device__ __forceinline__ float4 edge_logit(const FwdT &a, int slot, int t, int s, const float *coef,
-                                             const float *s_S = nullptr, int lo = 0) {
+__device__ __forceinline__ float4 edge_logit(const FwdT &a, int slot, int t, int s, const float *coef) {
   const float4 St = ldg4(a.S + (int64_t)t * 8);
-  const float4 Ss = s_S ? ld4(s_S + (s - lo) * 8 + 4) : ldg4(a.S + (int64_t)s * 8 + 4);
+  const float4 Ss = ldg4(a.S + (int64_t)s * 8 + 4);
   const float4 Se = edge_term_t<MODE>(a, slot, coef);
   return make_float4(leaky(St.x + Se.x + Ss.x), leaky(St.y + Se.y + Ss.y), leaky(St.z + Se.z + Ss.z),
                      leaky(St.w + Se.w + Ss.w));
@@ -203,11 +182,8 @@ __device__ void fwd_hub(const FwdT &a, int t, int beg, int end, const float *coe
 // WIDE: the same code compiled for 5 CTAs per SM (48 registers, no spills) instead of 6 (40 registers, 12 bytes
 // spilled).  Measured on the bond graph: batch 1 024 (843 tiles = one wave at 6 per SM) 38.6 us at 6 per SM vs 43.5 us
 // at 5; batch 4 096 (3 359 tiles) 127.6 us vs 119.7 us -- so graphs with more tiles than one 6-per-SM wave take WIDE.
-template <int MODE, bool STAGED, bool DEEP = false, bool WIDE = false>
-__global__ void __launch_bounds__(T_THREADS, STAGED ? 2 : (DEEP ? 4 : (WIDE ? 5 : 6))) k_gat_fwd_tiled(FwdT a) {
-  extern __shared__ __align__(128) float s_dyn[];   // STAGED: [ROWS_CAP][128] rows of h, then [ROWS_CAP][8] rows of S
-  __shared__ __align__(8) uint64_t s_bar[2];
-  __shared__ int s_stage[2];
+template <int MODE, bool DEEP = false, bool WIDE = false>
+__global__ void __launch_bounds__(T_THREADS, DEEP ? 4 : (WIDE ? 5 : 6)) k_gat_fwd_tiled(FwdT a) {
   __shared__ int s_rowptr[T_NPC + 1];
   constexpr int CAP = DEEP ? 2 * FWD_CAP : FWD_CAP;   // DEEP: longer sub-tiles, fewer phase barriers per node
   __shared__ int s_src[CAP];
@@ -220,37 +196,13 @@ __global__ void __launch_bounds__(T_THREADS, STAGED ? 2 : (DEEP ? 4 : (WIDE ? 5 
   if (MODE == FNB_EDGE_AFFINE6) edge_coef_prologue<6>(a.We, a.be, a.alpha_e, a.alpha_e_stride, s_coef);
   if (a.next_alpha)  // consumer graph's edge slice, 4 heads x 128 columns
     for (int i = tid; i < 4 * kD; i += T_THREADS) s_na[i] = __ldg(a.next_alpha + (int64_t)(i >> 7) * a.next_stride + (i & 127));
-  float *s_rows = s_dyn, *s_S = s_dyn + ROWS_CAP * kD;
-  const uint32_t bar_rows = bulk::smem_u32(&s_bar[0]), bar_S = bulk::smem_u32(&s_bar[1]);
-  uint32_t phase = 0;
-  if (STAGED && tid == 0) {
-    bulk::mbar_init(bar_rows, 1);
-    bulk::mbar_init(bar_S, 1);
-    bulk::mbar_init_fence();
-  }
 
   const int n_tiles = (a.n_nodes + a.npc - 1) / a.npc;
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const int n0 = tile * a.npc, nn = min(a.npc, a.n_nodes - n0);
-    __syncthreads();  // readers of the previous tile are done; also publishes s_coef and the barrier init
-    if (STAGED && tid == 0) {  // queue the bulk copies of this tile's source rows (S first: the logits need it first)
-      const int lo = __ldg(a.tile_range + 2 * tile), rows = __ldg(a.tile_range + 2 * tile + 1) - lo;
-      const int ok = rows > 0 && rows <= ROWS_CAP;
-      s_stage[0] = lo;
-      s_stage[1] = ok;
-      if (ok) {
-        bulk::fence_proxy_async();
-        bulk::mbar_expect_tx(bar_S, rows * 32);
-        bulk::copy_g2s(bulk::smem_u32(s_S), a.S + (int64_t)lo * 8, rows * 32, bar_S);
-        bulk::mbar_expect_tx(bar_rows, rows * kD * 4);
-        bulk::copy_g2s(bulk::smem_u32(s_rows), a.h + (int64_t)lo * kD, rows * kD * 4, bar_rows);
-      }
-    }
+    __syncthreads();  // readers of the previous tile are done; also publishes s_coef
     if (tid <= nn) s_rowptr[tid] = __ldg(a.rowptr + n0 + tid);
     __syncthreads();
-    const bool staged = STAGED && s_stage[1] != 0;
-    const int lo = STAGED ? s_stage[0] : 0;
-    if (staged) bulk::mbar_wait(bar_S, phase);
     int lb = 0;
     while (lb < nn) {
       const int le = subtile_end(s_rowptr, lb, nn, CAP);
@@ -264,8 +216,7 @@ __global__ void __launch_bounds__(T_THREADS, STAGED ? 2 : (DEEP ? 4 : (WIDE ? 5 
       for (int i = tid; i < cnt; i += T_THREADS) {
         const int slot = e0 + i;
         const int s = __ldg(a.col + slot), t = __ldg(a.row + slot);
-        if (a.prefetch) prefetch_row_l2(a.h + (int64_t)s * kD);
-        st4(s_l + i * 4, edge_logit<MODE>(a, slot, t, s, s_coef, staged ? s_S : nullptr, lo));
+        st4(s_l + i * 4, edge_logit<MODE>(a, slot, t, s, s_coef));
         s_src[i] = s;
       }
       __syncthreads();
@@ -311,21 +262,10 @@ __global__ void __launch_bounds__(T_THREADS, STAGED ? 2 : (DEEP ? 4 : (WIDE ? 5 
       // ---- phase 3: save p (coalesced), then one warp per node aggregates source rows
       if (a.p_saved)
         for (int i = tid; i < cnt; i += T_THREADS) st4(a.p_saved + (int64_t)(e0 + i) * 4, ld4(s_l + i * 4));
-      if (staged) bulk::mbar_wait(bar_rows, phase);
       for (int n = lb + warp; n < le; n += T_WARPS) {
         const int b = s_rowptr[n] - e0, e = s_rowptr[n + 1] - e0;
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
         int j = b;
-        if (staged) {  // rows come from the staged range in shared memory
-          for (; j < e; ++j) {
-            const float4 v = ld4(s_rows + (s_src[j] - lo) * kD + lane * 4);
-            const float pj = fabsf(s_l[j * 4 + head]);
-            acc.x = fmaf(pj, v.x, acc.x);
-            acc.y = fmaf(pj, v.y, acc.y);
-            acc.z = fmaf(pj, v.z, acc.z);
-            acc.w = fmaf(pj, v.w, acc.w);
-          }
-        }
         if (DEEP) {
           for (; j + 8 <= e; j += 8) {
             float4 v[8];
@@ -373,10 +313,6 @@ __global__ void __launch_bounds__(T_THREADS, STAGED ? 2 : (DEEP ? 4 : (WIDE ? 5 
       lb = le;
       if (lb < nn) __syncthreads();  // next sub-tile overwrites the staging arrays
     }
-    if (staged) {
-      bulk::mbar_wait(bar_rows, phase);   // (a tile made only of hub nodes never waited: consume the phase)
-      phase ^= 1;
-    }
   }
   pdl_launch_dependents();
 }
@@ -404,7 +340,6 @@ struct DstT {
   const float *f_pool;     // [n_seg,128] gradient of the pooled rows (atom -> fragment sum pooling), or NULL
   const int *f_seg;        // [N] segment of every row
   float *g_out;            // [N,128] assembled gradient, read by the source pass
-  const int *run_if_open;  // fnb_graph.comp_open when the fused kernel was launched ahead of this one: 0 = nothing to do
 };
 
 template <int MODE> struct CoefT { static constexpr int NC = 1, PARTS = 1, IN = 1; };
@@ -420,7 +355,7 @@ __device__ __forceinline__ float dz_of(float p, float dp, float delta) {
 // i.e. the edge-term backward of the consumer graph (gat2.py:203-208: this graph's output rows are the consumer's edge
 // vectors) plus the ReLU(Dropout) backward of gat2.py:414-418, in the summation order of k_edge_table_bwd_tiled, and
 // written once for the source pass -- a whole pass over [N,128] leaves the critical path of the backward.
-template <bool FUSE, bool STORE = true>
+template <bool FUSE>
 __device__ __forceinline__ float4 dst_grad_row(const DstT &a, int t, const float *s_ae) {
   const int lane = threadIdx.x & 31;
   const int64_t o = (int64_t)t * kD + lane * 4;
@@ -455,7 +390,7 @@ __device__ __forceinline__ float4 dst_grad_row(const DstT &a, int t, const float
     const float4 q = ldg4(a.f_pool + (int64_t)__ldg(a.f_seg + t) * kD + lane * 4);
     g.x += q.x; g.y += q.y; g.z += q.z; g.w += q.w;
   }
-  if (STORE) st4(a.g_out + o, g);
+  st4(a.g_out + o, g);
   return g;
 }
 
@@ -506,7 +441,6 @@ __global__ void __launch_bounds__(T_THREADS, 6) k_gat_bwd_dst_tiled(DstT a) {
   if (FUSE && a.f_dz)   // parameters, not produced by the preceding launch: staged before the dependency wait
     for (int i = tid; i < 4 * kD; i += T_THREADS) s_ae[i] = __ldg(a.f_alpha + (int64_t)(i >> 7) * a.f_stride + (i & 127));
   pdl_wait();
-  if (a.run_if_open && __ldg(a.run_if_open) == 0) return;   // the fused kernel has done this graph
 
   const int n_tiles = (a.n_nodes + a.npc - 1) / a.npc;
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -653,7 +587,6 @@ struct SrcT {
   float *scratch;
   int n_nodes;
   int npc;
-  const int *run_if_open;
 };
 
 template <bool DEEP>
@@ -667,7 +600,6 @@ __global__ void __launch_bounds__(T_THREADS, DEEP ? 3 : 4) k_gat_bwd_src_tiled(S
   static_assert(BWD_CAP * 4 >= T_WARPS * 384, "per-warp records must fit the staging array");
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, head = lane >> 3;
   pdl_wait();
-  if (a.run_if_open && __ldg(a.run_if_open) == 0) return;
   const float4 at = ldg4(a.alpha + (int64_t)head * a.alpha_stride + a.off_t + (lane & 7) * 4);
   const float4 as = ldg4(a.alpha + (int64_t)head * a.alpha_stride + a.off_s + (lane & 7) * 4);
   float pa[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -828,248 +760,6 @@ __global__ void __launch_bounds__(T_THREADS, DEEP ? 3 : 4) k_gat_bwd_src_tiled(S
 }
 
 // ================================================================================================
-// Backward, both sides in ONE kernel -- for graphs whose components (molecules) are closed and small
-// (fnb_graph.comp_ptr / comp_open, checked on the device by k_plan_comp_check).  A work unit is a run of consecutive
-// components; since no edge leaves it, every out-edge of a source node ends at a destination of the same unit, so the
-// source pass can read dz, p and the gradient rows of its destinations from the shared memory the destination pass
-// of the SAME CTA left them in: no dz / assembled-gradient round trip through L2, no second staging of p, no second
-// launch.  Per tile:  stage (col, p, reverse permutation) -> A: gradient row (assembled, stored) + dp per in-edge ->
-// B: softmax backward per (node, head) -> C: dz out (only if a consumer reads it), edge-term constants -> D: per
-// source node, sum_e p g[t_e] with p and dz from shared memory and the gradient rows this CTA stored in A, dh row out.
-// Arithmetic and summation order per row are those of the two-pass kernels (dh is bitwise equal); only the cross-CTA
-// trees of the parameter-gradient records see a different CTA partition.
-struct FusedT {
-  DstT d;
-  SrcT s;
-  const int *comp_ptr, *comp_bucket, *comp_open;
-  int n_b8;      // entries of comp_bucket - 1 = ceil(n_nodes / 8)
-  int bucket8;   // a work unit = the components whose first node lies in one bucket of 8 * bucket8 consecutive nodes
-  int write_dz;
-};
-
-constexpr int F_THREADS = 256, F_WARPS = F_THREADS / 32;
-constexpr int F_NODES = FNB_FUSED_NODES, F_SLOTS = FNB_FUSED_SLOTS, F_UNIT = 64;
-constexpr size_t kFusedSmem = (size_t)F_SLOTS * 8 * 4 + (size_t)F_SLOTS * 2 * 4;
-static_assert(F_SLOTS * 8 >= F_WARPS * 384, "per-warp records are parked in the probability staging arrays");
-static_assert(F_SLOTS < 65536 && F_NODES < 32768, "reverse entries pack (slot, node) into one word");
-
-template <int MODE, bool FUSE>
-__global__ void __launch_bounds__(F_THREADS, 4) k_gat_bwd_fused(FusedT a) {
-  constexpr int NC = CoefT<MODE>::NC, PARTS = CoefT<MODE>::PARTS, IN = CoefT<MODE>::IN;
-  extern __shared__ __align__(128) float s_dyn[];
-  float *s_p = s_dyn;                                        // [F_SLOTS][4] signed probabilities, slot order
-  float *s_dp = s_p + F_SLOTS * 4;                           // [F_SLOTS][4] dp, then dz
-  int *s_src = reinterpret_cast<int *>(s_dp + F_SLOTS * 4);  // [F_SLOTS] source node of every slot
-  int *s_rev = s_src + F_SLOTS;                              // [F_SLOTS] reverse order: local slot | local destination << 16
-  __shared__ int s_rowptr[F_NODES + 1], s_rrowptr[F_NODES + 1];
-  __shared__ int s_cn[F_UNIT + 1], s_ce[F_UNIT + 1];
-  __shared__ __align__(16) float s_dSt[F_NODES * 4];
-  __shared__ float s_red[PARTS * NC];
-  __shared__ float s_rec[416], s_fin[416];
-  __shared__ __align__(16) float s_ae[FUSE ? 4 * kD : 4];
-  const DstT &d = a.d;
-  const SrcT &sr = a.s;
-  // gradient rows: assembled and written by phase A of THIS CTA (FUSE) or given; phase D reads them back with plain
-  // (coherent) loads after the CTA barrier
-  const float *g_rows = FUSE ? d.g_out : d.dout;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, head = lane >> 3;
-  const bool coef_thread = NC > 1 && tid < NC * PARTS;
-  const int c = tid % NC, part = tid / NC;
-  const int c_head = (NC == 8) ? (c & 3) : (c < 24 ? c / 6 : c - 24);
-  const int c_k = (NC == 8) ? (c < 4 ? 0 : -1) : (c < 24 ? c % 6 : -1);
-  float cacc = 0.f;
-  if (FUSE && d.f_dz)
-    for (int i = tid; i < 4 * kD; i += F_THREADS) s_ae[i] = __ldg(d.f_alpha + (int64_t)(i >> 7) * d.f_stride + (i & 127));
-  pdl_wait();
-  if (__ldg(a.comp_open) != 0) return;   // the two-pass kernels behind this launch take over
-  const float4 at = ldg4(sr.alpha + (int64_t)head * sr.alpha_stride + sr.off_t + (lane & 7) * 4);
-  const float4 as = ldg4(sr.alpha + (int64_t)head * sr.alpha_stride + sr.off_s + (lane & 7) * 4);
-  float pa[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  float4 colsum = make_float4(0.f, 0.f, 0.f, 0.f);
-
-  const int n_units = (a.n_b8 + a.bucket8 - 1) / a.bucket8;
-  for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
-    const int c_lo = __ldg(a.comp_bucket + unit * a.bucket8);
-    const int c_hi = __ldg(a.comp_bucket + min((unit + 1) * a.bucket8, a.n_b8));
-   for (int c0 = c_lo; c0 < c_hi; c0 += F_UNIT) {   // (more than F_UNIT components per bucket only with runs of empty ones)
-    const int nc = min(F_UNIT, c_hi - c0);
-    __syncthreads();
-    if (tid <= nc) {
-      const int n = __ldg(a.comp_ptr + c0 + tid);
-      s_cn[tid] = n;
-      s_ce[tid] = __ldg(d.rowptr + n);
-    }
-    __syncthreads();
-    int cb = 0;
-    while (cb < nc) {
-      // the longest run of components that fits one tile (every single component does: k_plan_comp_check)
-      int ce = cb + 1;
-      while (ce < nc && s_cn[ce + 1] - s_cn[cb] <= F_NODES && s_ce[ce + 1] - s_ce[cb] <= F_SLOTS) ++ce;
-      const int n0 = s_cn[cb], nn = s_cn[ce] - n0, e0 = s_ce[cb], cnt = s_ce[ce] - e0;
-      cb = ce;
-      if (nn == 0) continue;
-      const int r0 = __ldg(sr.rrowptr + n0);
-      // ---- stage: CSR offsets, sources, probabilities, reverse permutation (all coalesced)
-      for (int i = tid; i <= nn; i += F_THREADS) {
-        s_rowptr[i] = __ldg(d.rowptr + n0 + i) - e0;
-        s_rrowptr[i] = __ldg(sr.rrowptr + n0 + i) - r0;
-      }
-      for (int i = tid; i < cnt; i += F_THREADS) {
-        s_src[i] = __ldg(d.col + e0 + i);
-        st4(s_p + i * 4, ldg4(d.p_saved + (int64_t)(e0 + i) * 4));
-        s_rev[i] = (__ldg(sr.rslot + r0 + i) - e0) | ((__ldg(sr.rdst + r0 + i) - n0) << 16);
-      }
-      __syncthreads();
-      // ---- A: gradient row (assembled and stored for phase D), dp per in-edge; one warp per destination node
-      for (int n = warp; n < nn; n += F_WARPS) {
-        const int b = s_rowptr[n], e = s_rowptr[n + 1];
-        const float4 g = dst_grad_row<FUSE, true>(d, n0 + n, s_ae);
-        int j = b;
-        for (; j + 4 <= e; j += 4) {
-          float4 v[4];
-#pragma unroll
-          for (int u = 0; u < 4; ++u) v[u] = ldg4(d.h + (int64_t)s_src[j + u] * kD + lane * 4);
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const float dd = head_sum(dot4(g, v[u]));
-            if ((lane & 7) == 0) s_dp[(j + u) * 4 + head] = dd;
-          }
-        }
-        for (; j < e; ++j) {
-          const float4 v = ldg4(d.h + (int64_t)s_src[j] * kD + lane * 4);
-          const float dd = head_sum(dot4(g, v));
-          if ((lane & 7) == 0) s_dp[j * 4 + head] = dd;
-        }
-      }
-      __syncthreads();
-      // ---- B: softmax backward per (node, head)
-      for (int q = tid; q < nn * 4; q += F_THREADS) {
-        const int n = q >> 2, hh = q & 3;
-        const int b = s_rowptr[n], e = s_rowptr[n + 1];
-        float delta = 0.f;
-        for (int j = b; j < e; ++j) delta = fmaf(fabsf(s_p[j * 4 + hh]), s_dp[j * 4 + hh], delta);
-        float dst = 0.f;
-        for (int j = b; j < e; ++j) {
-          const float v = dz_of(s_p[j * 4 + hh], s_dp[j * 4 + hh], delta);
-          s_dp[j * 4 + hh] = v;
-          dst += v;
-        }
-        s_dSt[q] = dst;
-      }
-      __syncthreads();
-      // ---- C: dz out (if a consumer graph reads it) and the edge-term constants
-      if (a.write_dz)
-        for (int i = tid; i < cnt; i += F_THREADS) st4(d.dz + (int64_t)(e0 + i) * 4, ld4(s_dp + i * 4));
-      if (coef_thread)
-        for (int i = part; i < cnt; i += PARTS) {
-          const float x = c_k < 0 ? 1.f : __ldg(d.edge_attr + (int64_t)(e0 + i) * IN + c_k);
-          cacc = fmaf(s_dp[i * 4 + c_head], x, cacc);
-        }
-      // ---- D: source side, one warp per node; destinations' gradient rows come from shared memory
-      for (int n = warp; n < nn; n += F_WARPS) {
-        const int b = s_rrowptr[n], e = s_rrowptr[n + 1];
-        const float gt = s_dSt[n * 4 + head];
-        const float4 hr = ldg4(d.h + (int64_t)(n0 + n) * kD + lane * 4);
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        float gs = 0.f;
-        int j = b;
-        for (; j + 4 <= e; j += 4) {
-          float4 v[4];
-          float pj[4];
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const int rv = s_rev[j + u], li = rv & 0xffff, ti = rv >> 16;
-            v[u] = ld4(g_rows + (int64_t)(n0 + ti) * kD + lane * 4);
-            pj[u] = fabsf(s_p[li * 4 + head]);
-            gs += s_dp[li * 4 + head];
-          }
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            acc.x = fmaf(pj[u], v[u].x, acc.x);
-            acc.y = fmaf(pj[u], v[u].y, acc.y);
-            acc.z = fmaf(pj[u], v[u].z, acc.z);
-            acc.w = fmaf(pj[u], v[u].w, acc.w);
-          }
-        }
-        for (; j < e; ++j) {
-          const int rv = s_rev[j], li = rv & 0xffff, ti = rv >> 16;
-          const float pj = fabsf(s_p[li * 4 + head]);
-          gs += s_dp[li * 4 + head];
-          const float4 v = ld4(g_rows + (int64_t)(n0 + ti) * kD + lane * 4);
-          acc.x = fmaf(pj, v.x, acc.x);
-          acc.y = fmaf(pj, v.y, acc.y);
-          acc.z = fmaf(pj, v.z, acc.z);
-          acc.w = fmaf(pj, v.w, acc.w);
-        }
-        acc.x += gt * at.x + gs * as.x;
-        acc.y += gt * at.y + gs * as.y;
-        acc.z += gt * at.z + gs * as.z;
-        acc.w += gt * at.w + gs * as.w;
-        st4(sr.dh + (int64_t)(n0 + n) * kD + lane * 4, acc);
-        colsum.x += acc.x; colsum.y += acc.y; colsum.z += acc.z; colsum.w += acc.w;
-        pa[0] = fmaf(gt, hr.x, pa[0]); pa[1] = fmaf(gt, hr.y, pa[1]); pa[2] = fmaf(gt, hr.z, pa[2]); pa[3] = fmaf(gt, hr.w, pa[3]);
-        pa[4] = fmaf(gs, hr.x, pa[4]); pa[5] = fmaf(gs, hr.y, pa[5]); pa[6] = fmaf(gs, hr.z, pa[6]); pa[7] = fmaf(gs, hr.w, pa[7]);
-      }
-      __syncthreads();   // the next tile overwrites the staging arrays
-    }
-   }
-  }
-
-  // CTA record: [0,128) d alpha_t, [128,256) d alpha_s, [256,384) colsum(dh), [384,416) edge-term constants
-  pdl_launch_dependents();
-  __syncthreads();
-  float *s_w = s_p;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    s_w[warp * 384 + lane * 4 + i] = pa[i];
-    s_w[warp * 384 + 128 + lane * 4 + i] = pa[4 + i];
-  }
-  st4(s_w + warp * 384 + 256 + lane * 4, colsum);
-  if (coef_thread) s_red[part * NC + c] = cacc;
-  __syncthreads();
-  for (int j = tid; j < 416; j += F_THREADS) {
-    float sum = 0.f;
-    if (j < 384) {
-#pragma unroll
-      for (int w = 0; w < F_WARPS; ++w) sum += s_w[w * 384 + j];
-    } else if (NC > 1 && j - 384 < NC) {
-      for (int k = 0; k < PARTS; ++k) sum += s_red[k * NC + (j - 384)];
-    }
-    s_rec[j] = sum;
-  }
-  __syncthreads();
-  if (!cta_finish<416>(s_rec, s_fin, d.scratch)) return;
-  for (int j = tid; j < 384; j += F_THREADS) {
-    const float v = s_fin[j];
-    if (j < 128) sr.d_alpha[(j >> 5) * sr.alpha_stride + sr.off_t + (j & 31)] = v;
-    else if (j < 256) sr.d_alpha[((j - 128) >> 5) * sr.alpha_stride + sr.off_s + (j & 31)] = v;
-    else if (sr.d_bias) sr.d_bias[j - 256] = v;
-  }
-  if (NC > 1) {   // App. A.5, as in the destination-pass kernel
-    const float *dcoef = s_fin + 384;
-    const int n_w = kHd * IN;
-    for (int o = tid; o < n_w + kHd + kH * kHd; o += F_THREADS) {
-      if (o < n_w) {
-        const int j = o / IN, k = o % IN;
-        float s = 0.f;
-        for (int hh = 0; hh < kH; ++hh) s = fmaf(dcoef[hh * IN + k], d.alpha_e[hh * d.alpha_e_stride + j], s);
-        d.dWe[o] = s;
-      } else if (o < n_w + kHd) {
-        const int j = o - n_w;
-        float s = 0.f;
-        for (int hh = 0; hh < kH; ++hh) s = fmaf(dcoef[4 * IN + hh], d.alpha_e[hh * d.alpha_e_stride + j], s);
-        d.dbe[j] = s;
-      } else {
-        const int r = o - n_w - kHd, hh = r / kHd, j = r % kHd;
-        float s = dcoef[4 * IN + hh] * d.be[j];
-        for (int k = 0; k < IN; ++k) s = fmaf(dcoef[hh * IN + k], d.We[j * IN + k], s);
-        d.d_alpha_e[hh * d.alpha_e_stride + j] = s;
-      }
-    }
-  }
-}
-
-// ================================================================================================
 // Edge-term backward for TABLE mode (atom graph <- bond features, fragment graph <- fragment-connection features):
 //   g_feat[e,:] = g_in[e,:] + sum_h dz[slot_of_eid[e],h] alpha_e[h,:],   d alpha_e[h,:] = sum_e dz[e,h] feat[e,:]
 // where g_in is either a plain gradient (g_base) or the ReLU(Dropout) backward of the gradient that arrived at the
@@ -1151,8 +841,6 @@ __global__ void __launch_bounds__(T_THREADS, 5) k_edge_table_bwd_tiled(TableT a)
 // small graphs (fragment / fragment-connection graphs have 5-10x fewer nodes than the bond graph) fill the machine
 // (measured sweep: profiles/r1f_kbench_npc*.log).
 inline int pick_npc(int64_t n_nodes) {
-  static const int forced = [] { const char *e = getenv("FNB_NPC"); return e ? atoi(e) : 0; }();
-  if (forced == 8 || forced == 16 || forced == 32 || forced == 64) return forced;
   for (int npc = T_NPC; npc > 8; npc >>= 1)
     if ((n_nodes + npc - 1) / npc >= (int64_t)kNumSMs * 2) return npc;
   return 8;
@@ -1166,48 +854,24 @@ inline int tile_grid(int64_t n_nodes, int npc, int ctas_per_sm) {
   return (int)tiles;
 }
 
-inline bool use_staging() { return fnb_use_staging(); }
-
-// Opt in to > 48 KB of dynamic shared memory once per device.
-template <class K>
-int allow_smem(K kernel, size_t bytes, bool (&done)[64]) {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) return FNB_ERR_SIZE;
-  if (!done[dev]) {
-    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e != cudaSuccess) return (int)e;
-    done[dev] = true;
-  }
-  return 0;
-}
-
 template <int MODE>
-int launch_fwd(const FwdT &a, bool staged, cudaStream_t stream) {
-  if (staged) {
-    static bool done[64] = {};
-    const size_t smem = kStageRowsBytes + kStageSBytes;
-    const int rc = allow_smem(k_gat_fwd_tiled<MODE, true>, smem, done);
-    if (rc) return rc;
-    k_gat_fwd_tiled<MODE, true><<<tile_grid(a.n_nodes, kRangeTile, 2), T_THREADS, smem, stream>>>(a);
-  } else if (a.deep) {
-    const cudaError_t le = fnb_launch(k_gat_fwd_tiled<MODE, false, true>, dim3(tile_grid(a.n_nodes, a.npc, 4)), dim3(T_THREADS), 0, stream, a);
+int launch_fwd(const FwdT &a, cudaStream_t stream) {
+  if (a.deep) {
+    const cudaError_t le = fnb_launch(k_gat_fwd_tiled<MODE, true>, dim3(tile_grid(a.n_nodes, a.npc, 4)), dim3(T_THREADS), 0, stream, a);
     if (le != cudaSuccess) return (int)le;
   } else if (((int64_t)a.n_nodes + a.npc - 1) / a.npc > (int64_t)kNumSMs * 6) {
-    const cudaError_t le = fnb_launch(k_gat_fwd_tiled<MODE, false, false, true>, dim3(tile_grid(a.n_nodes, a.npc, 5)), dim3(T_THREADS), 0, stream, a);
+    const cudaError_t le = fnb_launch(k_gat_fwd_tiled<MODE, false, true>, dim3(tile_grid(a.n_nodes, a.npc, 5)), dim3(T_THREADS), 0, stream, a);
     if (le != cudaSuccess) return (int)le;
   } else {
-    const cudaError_t le = fnb_launch(k_gat_fwd_tiled<MODE, false>, dim3(tile_grid(a.n_nodes, a.npc, 6)), dim3(T_THREADS), 0, stream, a);
+    const cudaError_t le = fnb_launch(k_gat_fwd_tiled<MODE>, dim3(tile_grid(a.n_nodes, a.npc, 6)), dim3(T_THREADS), 0, stream, a);
     if (le != cudaSuccess) return (int)le;
   }
   FNB_CHECK_LAUNCH();
   return 0;
 }
 
-// Mean in-degree from which the DEEP instantiations pay (FNB_DEEP=0 disables, FNB_DEEP=<degree> overrides).
 inline bool deep_graph(const fnb_graph *g) {
-  static const int thr = [] { const char *e = getenv("FNB_DEEP"); return e ? atoi(e) : 24; }();
-  return thr > 0 && g->n_nodes > 0 && g->n_edges >= (int64_t)thr * g->n_nodes;
+  return g->n_nodes > 0 && g->n_edges >= (int64_t)kDeepDegree * g->n_nodes;
 }
 
 inline bool graph_ok(const fnb_graph *g) {
@@ -1237,31 +901,25 @@ extern "C" int fnb_gat_fwd_tiled(const fnb_graph *g, const fnb_gat_fwd_args *f, 
   a.mask_lo = (int)f->mask_lo; a.mask_hi = (int)f->mask_hi;
   a.next_alpha = f->next_alpha_e; a.next_stride = f->next_alpha_stride; a.next_Se = f->next_Se;
   a.npc = pick_npc(g->n_nodes);
-  a.tile_range = g->tile_range;
-  {
-    static const int pf = [] { const char *e = getenv("FNB_PREFETCH"); return e && e[0] == '1' ? 1 : 0; }();
-    a.prefetch = pf;
-  }
   a.deep = deep_graph(g) ? 1 : 0;
-  const bool staged = use_staging() && g->tile_range != nullptr && a.npc == kRangeTile;
   cudaStream_t stream = (cudaStream_t)stream_;
   switch (f->edge_mode) {
     case FNB_EDGE_NONE:
-      return launch_fwd<FNB_EDGE_NONE>(a, staged, stream);
+      return launch_fwd<FNB_EDGE_NONE>(a, stream);
     case FNB_EDGE_AFFINE1:
       if (!g->edge_attr || !f->We || !f->be || !f->alpha_e) return FNB_ERR_NULL;
       a.edge_attr = g->edge_attr;
-      return launch_fwd<FNB_EDGE_AFFINE1>(a, staged, stream);
+      return launch_fwd<FNB_EDGE_AFFINE1>(a, stream);
     case FNB_EDGE_AFFINE6:
       if (!g->edge_attr || !f->We || !f->be || !f->alpha_e) return FNB_ERR_NULL;
       if (reinterpret_cast<uintptr_t>(g->edge_attr) & 7u) return FNB_ERR_ALIGN;
       a.edge_attr = g->edge_attr;
-      return launch_fwd<FNB_EDGE_AFFINE6>(a, staged, stream);
+      return launch_fwd<FNB_EDGE_AFFINE6>(a, stream);
     case FNB_EDGE_TABLE:
       if (!f->edge_table || !g->eid) return FNB_ERR_NULL;
       if (!fnb_aligned16(f->edge_table)) return FNB_ERR_ALIGN;
       a.edge_attr = f->edge_table;
-      return launch_fwd<FNB_EDGE_TABLE>(a, staged, stream);
+      return launch_fwd<FNB_EDGE_TABLE>(a, stream);
     default:
       return FNB_ERR_MODE;
   }
@@ -1316,48 +974,6 @@ int fnb_gat_bwd_tiled_fused(const fnb_graph *g, const fnb_gat_bwd_args *b, const
       b->edge_mode != FNB_EDGE_TABLE)
     return FNB_ERR_MODE;
   if (b->edge_mode == FNB_EDGE_AFFINE6 && (reinterpret_cast<uintptr_t>(g->edge_attr) & 7u)) return FNB_ERR_ALIGN;
-  d.run_if_open = nullptr;
-  // Graphs with a component table take the one-kernel backward; whether the table holds (closed, small components) is
-  // a device word, so the two-pass launches follow in any case and return at once when the fused kernel did the work.
-  const bool one_kernel = fnb_fused_bwd_enabled() && g->comp_ptr && g->comp_bucket && g->comp_open && !deep;
-  if (one_kernel) {
-    if (before_src)
-      if (cudaError_t ee = cudaStreamWaitEvent(stream, before_src, 0)) return (int)ee;
-    FusedT f;
-    f.d = d;
-    f.s.rrowptr = g->rrowptr; f.s.rslot = g->rslot; f.s.rdst = g->rdst; f.s.h = b->h; f.s.dout = b->dout;
-    f.s.p_saved = b->p_saved; f.s.dz = b->dz; f.s.dSt = b->dSt; f.s.alpha = b->alpha; f.s.alpha_stride = b->alpha_stride;
-    f.s.off_t = b->off_t; f.s.off_s = b->off_s; f.s.dh = b->dh; f.s.d_alpha = b->d_alpha; f.s.d_bias = b->d_bias;
-    f.s.scratch = (float *)b->scratch; f.s.n_nodes = (int)g->n_nodes; f.s.npc = d.npc; f.s.run_if_open = nullptr;
-    f.comp_ptr = g->comp_ptr; f.comp_bucket = g->comp_bucket; f.comp_open = g->comp_open;
-    f.write_dz = !(fz && fz->skip_dz);
-    // work unit = the components that start inside a bucket of up to 64 consecutive nodes (a multiple of 8), smaller
-    // for small graphs so that there are about two units per CTA slot
-    f.n_b8 = (int)((g->n_nodes + 7) / 8);
-    f.bucket8 = (int)std::max<int64_t>(1, std::min<int64_t>(8, g->n_nodes / (8 * (int64_t)kNumSMs * 4)));
-    const int64_t n_units = (f.n_b8 + f.bucket8 - 1) / f.bucket8;
-    const int fgrid = (int)std::min<int64_t>(n_units, (int64_t)kNumSMs * 4);
-#define FNB_LAUNCH_FUSED(MODE)                                                                                       \
-  do {                                                                                                               \
-    static bool done_f[64] = {}, done_n[64] = {};                                                                    \
-    cudaError_t le;                                                                                                  \
-    if (fuse) {                                                                                                      \
-      if (int rc = allow_smem(k_gat_bwd_fused<MODE, true>, kFusedSmem, done_f)) return rc;                           \
-      le = fnb_launch(k_gat_bwd_fused<MODE, true>, dim3(fgrid), dim3(F_THREADS), kFusedSmem, stream, f);             \
-    } else {                                                                                                         \
-      if (int rc = allow_smem(k_gat_bwd_fused<MODE, false>, kFusedSmem, done_n)) return rc;                          \
-      le = fnb_launch(k_gat_bwd_fused<MODE, false>, dim3(fgrid), dim3(F_THREADS), kFusedSmem, stream, f);            \
-    }                                                                                                                \
-    if (le != cudaSuccess) return (int)le;                                                                           \
-  } while (0)
-    if (b->edge_mode == FNB_EDGE_AFFINE1) FNB_LAUNCH_FUSED(FNB_EDGE_AFFINE1);
-    else if (b->edge_mode == FNB_EDGE_AFFINE6) FNB_LAUNCH_FUSED(FNB_EDGE_AFFINE6);
-    else FNB_LAUNCH_FUSED(FNB_EDGE_NONE);
-#undef FNB_LAUNCH_FUSED
-    FNB_CHECK_LAUNCH();
-    d.run_if_open = g->comp_open;
-    before_src = nullptr;
-  }
 #define FNB_LAUNCH_DST(MODE)                                                                                         \
   do {                                                                                                               \
     cudaError_t le;                                                                                                  \
@@ -1391,7 +1007,6 @@ int fnb_gat_bwd_tiled_fused(const fnb_graph *g, const fnb_gat_bwd_args *b, const
   s.off_s = b->off_s; s.dh = b->dh; s.d_alpha = b->d_alpha; s.d_bias = b->d_bias; s.scratch = (float *)b->scratch;
   s.n_nodes = (int)g->n_nodes;
   s.npc = d.npc;
-  s.run_if_open = d.run_if_open;
   if (deep) {
     if (cudaError_t le = fnb_launch(k_gat_bwd_src_tiled<true>, dim3(tile_grid(g->n_nodes, d.npc, 3)), dim3(T_THREADS), 0, stream, s)) return (int)le;
   } else {

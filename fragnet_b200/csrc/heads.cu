@@ -20,7 +20,6 @@
 //     from shared memory; the backward tail recomputes the hidden layer, and reduces the parameter gradients of the
 //     tail (dW1 [MID,IN], db1, dW2, db2, db0) over the rows of its tile out of shared memory into per-CTA records.
 // Parameter-gradient sums are fixed-order two-stage reductions: run-to-run deterministic, no atomics.
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -918,20 +917,6 @@ __global__ void __launch_bounds__(EH_THREADS) k_energy_head_fused(EnergyArgs a) 
   if (tid < EH_H) rec[EH_MID * EH_H + 2 * EH_MID + 1 + tid] = b0acc;
 }
 
-// FNB_ENERGY_EARLY=1 (measurement switch): fork the energy stream at the head of the forward program instead of at the
-// head of the backward program.  Earlier looks better on paper (everything the kernel reads is complete there) and
-// measured worse, 1.312 vs 1.299 ms per step on the same box (gpurun_out/r5n): its 128 CTAs then hold their SMs when
-// the per-atom / per-bond tail kernel -- the critical path -- launches, which gets one CTA per SM instead of three.
-bool energy_fork_early() {
-  static const bool on = [] { const char *e = getenv("FNB_ENERGY_EARLY"); return e && e[0] == '1'; }();
-  return on;
-}
-
-bool energy_fused_enabled() {
-  static const bool on = [] { const char *e = getenv("FNB_ENERGY_FUSED"); return !(e && e[0] == '0'); }();
-  return on;
-}
-
 template <int IN, int MID, int ROWS>
 constexpr size_t tail_bwd_smem() {
   return sizeof(float) * ((size_t)IN * MID + 2 * (size_t)ROWS * (IN + 4) + 2 * (size_t)ROWS * (MID + 1) + ROWS);
@@ -1059,17 +1044,11 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
   const bool want_bl = io->bond_length != nullptr && Ea > 0 && !skip_tails;
 
   // ---- energy head: ~1e3 rows, latency-bound kernels on an auxiliary stream underneath the per-atom / per-bond heads.
-  // Training step with the fused energy kernel: that kernel is launched by the backward program (see energy_fork_early
-  // for the variant that forks the stream here).
+  // Training step (skip_tails): the fused energy kernel is launched by the backward program.
   FnbAux aux{};
   const bool two = fnb_aux_streams(&aux) == 0;
   cudaStream_t sB = two ? aux.hstream : stream;
   void *sB_ = (void *)sB;
-  const bool energy_in_backward = skip_tails && energy_fused_enabled();
-  if (two && G > 0 && energy_in_backward && energy_fork_early()) {
-    RC((int)cudaEventRecord(aux.fork, stream));
-    RC((int)cudaStreamWaitEvent(sB, aux.fork, 0));
-  }
   {  // padded / split operands (one launch)
     PackJobs p{};
     p.W0[0] = P->ba.W0; p.b0[0] = P->ba.b0; p.Wpad[0] = B.W0pad_ba; p.WpadT[0] = B.W0padT_ba; p.bpad[0] = B.b0pad_ba;
@@ -1082,7 +1061,7 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
     FNB_CHECK_LAUNCH();
   }
   // ---- energy head (graph readout pretrain_heads.py:93-96, first layer, tail)
-  if (G > 0 && !energy_in_backward) {
+  if (G > 0 && !skip_tails) {
     if (two) {
       RC((int)cudaEventRecord(aux.fork, stream));
       RC((int)cudaStreamWaitEvent(sB, aux.fork, 0));
@@ -1090,14 +1069,12 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
     RC(fnb_segment_sum(io->mol_atom_ptr, nullptr, G, io->x_atoms, B.readout, 2 * kD, nullptr, 0, 0, 0, nullptr, sB_));
     RC(fnb_segment_sum(io->mol_frag_ptr, nullptr, G, io->x_frags, B.readout + kD, 2 * kD, nullptr, 0, 0, 0, nullptr, sB_));
     RC(fnb_proj_fwd(B.readout, P->fc.W0, P->fc.b0, G, 2 * kD, nullptr, 0, 0, 0, B.h0_fc, nullptr, precision, sB_));
-    if (!skip_tails) {
-      TailJobs F{};
-      F.n = 1;
-      TailJob &t = F.j[0];
-      t.h0 = B.h0_fc; t.n = G; t.W1 = P->fc.W1; t.b1 = P->fc.b1; t.W2 = P->fc.W2; t.b2 = P->fc.b2; t.out = io->energy;
-      if (cudaError_t le = fnb_launch(k_mlp_tail_fwd<128, 64>, dim3((unsigned)((G + 127) / 128), 1), dim3(128), 0, sB, F)) return (int)le;
-      FNB_CHECK_LAUNCH();
-    }
+    TailJobs F{};
+    F.n = 1;
+    TailJob &t = F.j[0];
+    t.h0 = B.h0_fc; t.n = G; t.W1 = P->fc.W1; t.b1 = P->fc.b1; t.W2 = P->fc.W2; t.b2 = P->fc.b2; t.out = io->energy;
+    if (cudaError_t le = fnb_launch(k_mlp_tail_fwd<128, 64>, dim3((unsigned)((G + 127) / 128), 1), dim3(128), 0, sB, F)) return (int)le;
+    FNB_CHECK_LAUNCH();
   }
   (void)Nf;
   // ---- first layers on the projection kernels
@@ -1195,15 +1172,12 @@ int fnb_pretrain_heads_backward_impl(const fnb_pretrain_head_params *P, const fn
   // ---- energy head on the auxiliary stream (its ~1e3-row kernels are latency-bound and hide under the other heads):
   // tail, dX / dW of its first layer, readout backward of the fragments
   if (G > 0) {
-    const bool one_kernel = fused && energy_fused_enabled();
     if (two) {
-      if (!one_kernel || !energy_fork_early()) {
-        RC((int)cudaEventRecord(aux.fork, stream));
-        RC((int)cudaStreamWaitEvent(sB, aux.fork, 0));
-      }
+      RC((int)cudaEventRecord(aux.fork, stream));
+      RC((int)cudaStreamWaitEvent(sB, aux.fork, 0));
       RC((int)cudaMemsetAsync(W.scratch2, 0, kScratchCounters * sizeof(float), sB));
     }
-    if (one_kernel) {
+    if (fused) {
       // training step: readout, first layer, tail forward + loss + backward, input gradient and the fragments' readout
       // backward in one kernel (the forward program skipped the energy head)
       EnergyArgs e{};
@@ -1221,7 +1195,6 @@ int fnb_pretrain_heads_backward_impl(const fnb_pretrain_head_params *P, const fn
     TailJob &t = F.j[0];
     t.h0 = B.h0_fc; t.n = G; t.W1 = P->fc.W1; t.b1 = P->fc.b1; t.W2 = P->fc.W2; t.b2 = P->fc.b2; t.gout = io->g_energy;
     t.dh0 = W.dh0_fc; t.rec = W.rec_fc;
-    if (fused) { t.target = fused[2].target; t.loss_coef = fused[2].weight / (float)G; }
     if (cudaError_t le = fnb_launch(k_mlp_tail_bwd<128, 64, 256, 32>, dim3(ctas_fc, 1), dim3(256), tail_bwd_smem<128, 64, 32>(), sB, F))
       return (int)le;
     FNB_CHECK_LAUNCH();

@@ -243,11 +243,6 @@ struct AuxArgs {
   const int64_t *a2f, *batch, *frag_batch;
   int *a2f32, *batch32, *frag_batch32, *atom_ptr, *frag_ptr;
   int n_atoms, n_frags, n_graphs;
-  // component tables of the bond / fragment-connection graphs: node e of those graphs is edge e of the atom /
-  // fragment graph and belongs to the molecule of that edge's source
-  const int64_t *bond_src, *fbond_src;
-  int n_bonds, n_fbond_nodes;
-  int *bond_ptr, *fbond_ptr;
 };
 __device__ __forceinline__ int lower_bound64(const int64_t *ids, int n, int64_t key) {
   int lo = 0, hi = n;
@@ -257,20 +252,8 @@ __device__ __forceinline__ int lower_bound64(const int64_t *ids, int n, int64_t 
   }
   return lo;
 }
-// first edge whose source node belongs to molecule >= key (edges are molecule-sorted in a collated batch; anything
-// else is caught by k_plan_comp_check, which then marks the graph open)
-__device__ __forceinline__ int lower_bound_via(const int64_t *src, int n, const int64_t *mol, int n_src, int64_t key) {
-  int lo = 0, hi = n;
-  while (lo < hi) {
-    const int mid = (lo + hi) >> 1;
-    const int64_t v = src[mid];
-    const int64_t m = (v >= 0 && v < n_src) ? mol[v] : INT64_MAX;
-    if (m < key) lo = mid + 1; else hi = mid;
-  }
-  return lo;
-}
 // int64 -> int32 narrowing of atom_to_frag_ids / batch / frag_batch, and the molecule boundaries of the sorted
-// batch vectors (data.py:896-901) for the readout (gat2.py:820-821) and the fused attention backward.
+// batch vectors (data.py:896-901) for the readout (gat2.py:820-821).
 __global__ void k_plan_aux(AuxArgs a) {
   pdl_wait();
   const int stride = gridDim.x * blockDim.x, t0 = blockIdx.x * blockDim.x + threadIdx.x;
@@ -284,77 +267,14 @@ __global__ void k_plan_aux(AuxArgs a) {
     for (int g = t0; g <= a.n_graphs; g += stride) {
       a.atom_ptr[g] = lower_bound64(a.batch, a.n_atoms, g);
       a.frag_ptr[g] = lower_bound64(a.frag_batch, a.n_frags, g);
-      if (a.bond_ptr) {
-        a.bond_ptr[g] = lower_bound_via(a.bond_src, a.n_bonds, a.batch, a.n_atoms, g);
-        a.fbond_ptr[g] = lower_bound_via(a.fbond_src, a.n_fbond_nodes, a.frag_batch, a.n_frags, g);
-      }
     }
-}
-
-// Is every component [comp_ptr[c], comp_ptr[c+1]) of a graph closed (all in-edge sources and out-edge destinations
-// inside it), small enough for one tile of the fused attention backward, and do the components tile the node range?
-// One warp per (graph, component); a violation sets the graph's open word, which the backward kernels read.
-struct CompJobs {
-  int n_jobs, n_comps;
-  const int *rowptr[4], *col[4], *rrowptr[4], *rdst[4], *comp_ptr[4];
-  int n_nodes[4];
-  int *open[4];
-  int *bucket[4];   // [ceil(n_nodes / 8) + 1]: first component whose first node is >= 8 k (work units of the fused backward)
-};
-__global__ void __launch_bounds__(256) k_plan_comp_check(CompJobs j) {
-  pdl_wait();
-  const int lane = threadIdx.x & 31;
-  const int w0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
-  const int total = j.n_jobs * (j.n_comps + 1);
-  for (int w = w0; w < total; w += nw) {
-    const int job = w / (j.n_comps + 1), c = w % (j.n_comps + 1);
-    const int *cp = j.comp_ptr[job];
-    bool bad = false;
-    if (c == j.n_comps) {   // the table covers [0, n_nodes)
-      bad = cp[0] != 0 || cp[j.n_comps] != j.n_nodes[job];
-    } else {
-      const int n0 = cp[c], n1 = cp[c + 1];
-      if (n0 < 0 || n1 < n0 || n1 > j.n_nodes[job] || n1 - n0 > FNB_FUSED_NODES) {
-        bad = true;
-      } else if (n1 > n0) {
-        const int e0 = j.rowptr[job][n0], e1 = j.rowptr[job][n1];
-        const int r0 = j.rrowptr[job][n0], r1 = j.rrowptr[job][n1];
-        bad = e1 - e0 > FNB_FUSED_SLOTS || e1 - e0 != r1 - r0;
-        if (!bad) {
-          for (int s = e0 + lane; s < e1; s += 32) {
-            const int v = j.col[job][s];
-            bad |= v < n0 || v >= n1;
-          }
-          for (int s = r0 + lane; s < r1; s += 32) {
-            const int v = j.rdst[job][s];
-            bad |= v < n0 || v >= n1;
-          }
-        }
-      }
-    }
-    if (__any_sync(kFull, bad) && lane == 0) atomicExch(j.open[job], 1);
-  }
-  for (int job = 0; job < j.n_jobs; ++job) {
-    const int nb = (j.n_nodes[job] + 7) / 8;
-    const int *cp = j.comp_ptr[job];
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k <= nb; k += gridDim.x * blockDim.x) {
-      const int key = min(8 * k, j.n_nodes[job]);
-      int lo = 0, hi = j.n_comps + 1;
-      while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (cp[mid] < key) lo = mid + 1; else hi = mid;
-      }
-      j.bucket[job][k] = min(lo, j.n_comps);
-    }
-  }
 }
 
 struct PlanLayout {
   // outputs
   int *rowptr[PG], *col[PG], *row[PG], *eid[PG], *slot_of_eid[PG], *rrowptr[PG], *rslot[PG], *rdst[PG];
-  int *tile_range[PG], *rtile_range[PG], *comp_bucket[PG];
   float *attr_bond, *attr_fbond;
-  int *a2f32, *batch32, *frag_batch32, *atom_ptr, *frag_ptr, *bond_ptr, *fbond_ptr, *status;
+  int *a2f32, *batch32, *frag_batch32, *atom_ptr, *frag_ptr, *status;
   // temporaries
   int *cnt_dst, *cnt_src, *x_dst, *x_src, *tmp_eid, *tmp_reid, *tiles0, *tiles1;
   size_t cnt_bytes;   // cnt_dst and cnt_src are adjacent: one memset
@@ -399,10 +319,6 @@ PlanLayout plan_layout(const fnb_batch_inputs *in, char *base) {
       L.rrowptr[i] = take<int>(base, off, (size_t)z.n_nodes[i] + 1);
       L.rslot[i] = take<int>(base, off, z.n_total[i]);
       L.rdst[i] = take<int>(base, off, z.n_total[i]);
-      const size_t nt = ((size_t)z.n_nodes[i] + kRangeTile - 1) / kRangeTile;
-      L.tile_range[i] = take<int>(base, off, 2 * nt);
-      L.rtile_range[i] = take<int>(base, off, 2 * nt);
-      L.comp_bucket[i] = take<int>(base, off, ((size_t)z.n_nodes[i] + 7) / 8 + 1);
     }
   }
   L.attr_bond = take<float>(base, off, in->n_bond_edges);
@@ -412,9 +328,7 @@ PlanLayout plan_layout(const fnb_batch_inputs *in, char *base) {
   L.frag_batch32 = take<int>(base, off, in->n_frags);
   L.atom_ptr = take<int>(base, off, (size_t)in->n_graphs + 1);
   L.frag_ptr = take<int>(base, off, (size_t)in->n_graphs + 1);
-  L.bond_ptr = take<int>(base, off, (size_t)in->n_graphs + 1);
-  L.fbond_ptr = take<int>(base, off, (size_t)in->n_graphs + 1);
-  L.status = take<int>(base, off, 64);   // [0] index error, [8..12) comp_open of the four graphs
+  L.status = take<int>(base, off, 1);    // index error
   L.cnt_dst = take<int>(base, off, (size_t)z.n_total_nodes);
   {
     char *before = reinterpret_cast<char *>(L.cnt_dst);
@@ -450,21 +364,16 @@ inline int grid_for(int64_t n) {
   return (int)g;
 }
 
-// The plan struct over a laid-out arena (pure function of the inputs' sizes and the two build options).
-void fill_plan(const fnb_batch_inputs *in, const PlanLayout &L, const Sz &z, bool staging, bool comps, fnb_batch_plan *out) {
+// The plan struct over a laid-out arena (pure function of the inputs' sizes).
+void fill_plan(const fnb_batch_inputs *in, const PlanLayout &L, const Sz &z, fnb_batch_plan *out) {
   const int n_real[PG] = {(int)in->n_bond_edges, (int)in->n_bonds, (int)in->n_fbond_edges, (int)in->n_fbond_nodes,
                           (int)in->n_atoms};
-  int *comp_ptr[4] = {L.bond_ptr, L.atom_ptr, L.fbond_ptr, L.frag_ptr};
   fnb_graph *gs[4] = {&out->bond, &out->atom, &out->fbond, &out->frag};
   for (int i = 0; i < 4; ++i) {
     fnb_graph &g = *gs[i];
     g.n_nodes = z.n_nodes[i]; g.n_edges = z.n_total[i]; g.n_real_edges = n_real[i];
     g.rowptr = L.rowptr[i]; g.col = L.col[i]; g.row = L.row[i]; g.eid = L.eid[i]; g.slot_of_eid = L.slot_of_eid[i];
     g.rrowptr = L.rrowptr[i]; g.rslot = L.rslot[i]; g.rdst = L.rdst[i]; g.edge_attr = nullptr;
-    g.tile_range = staging ? L.tile_range[i] : nullptr; g.rtile_range = staging ? L.rtile_range[i] : nullptr;
-    g.comp_ptr = comps ? comp_ptr[i] : nullptr; g.n_comps = comps ? in->n_graphs : 0;
-    g.comp_bucket = comps ? L.comp_bucket[i] : nullptr;
-    g.comp_open = comps ? L.status + 8 + i : nullptr;
   }
   out->bond.edge_attr = L.attr_bond;
   out->fbond.edge_attr = L.attr_fbond;
@@ -489,8 +398,7 @@ int fnb_batch_plan_view(const fnb_batch_inputs *in, void *arena, size_t arena_by
   if (reinterpret_cast<uintptr_t>(arena) & 255u) return FNB_ERR_ALIGN;
   const PlanLayout L = plan_layout(in, (char *)arena);
   if (L.total > arena_bytes) return FNB_ERR_WORKSPACE;
-  const bool comps = in->batch != nullptr && in->n_graphs > 0 && fnb_fused_bwd_enabled();
-  fill_plan(in, L, sizes(in), fnb_use_staging(), comps, out);
+  fill_plan(in, L, sizes(in), out);
   return 0;
 }
 
@@ -500,7 +408,7 @@ extern "C" int fnb_batch_plan_build(const fnb_batch_inputs *in, void *arena, siz
 }
 
 // forward_ready (optional): recorded once everything the FORWARD attention kernels read is complete -- destination-
-// sorted CSRs, slot-ordered edge attributes, the pooling CSR.  The reverse CSRs, the tile ranges and the int32 /
+// sorted CSRs, slot-ordered edge attributes, the pooling CSR.  The reverse CSRs and the int32 /
 // per-molecule arrays (backward, readout) follow; a step's first attention kernel starts ~20 us earlier by waiting
 // for this event instead of for the whole plan.
 int fnb_batch_plan_build_impl(const fnb_batch_inputs *in, void *arena, size_t arena_bytes, fnb_batch_plan *out,
@@ -549,7 +457,7 @@ int fnb_batch_plan_build_impl(const fnb_batch_inputs *in, void *arena, size_t ar
   a.cnt_dst = L.cnt_dst; a.cnt_src = L.cnt_src; a.x_dst = L.x_dst; a.x_src = L.x_src;
   a.tmp_eid = L.tmp_eid; a.tmp_reid = L.tmp_reid; a.status = L.status;
 
-  cudaError_t err = cudaMemsetAsync(L.status, 0, 256, stream);
+  cudaError_t err = cudaMemsetAsync(L.status, 0, sizeof(int), stream);
   if (err != cudaSuccess) return (int)err;
   if (z.n_total_nodes > 0) {
     err = cudaMemsetAsync(L.cnt_dst, 0, L.cnt_bytes, stream);
@@ -589,54 +497,14 @@ int fnb_batch_plan_build_impl(const fnb_batch_inputs *in, void *arena, size_t ar
     if (cudaError_t le = fnb_launch(k_plan_rank_reverse, dim3(grid_for(z.e_total)), dim3(256), 0, stream, a)) return (int)le;
     FNB_CHECK_LAUNCH();
   }
-  const bool staging = fnb_use_staging();
-  if (staging) {  // source ranges of every 64-node tile (forward and reverse CSR of the four graphs): one launch
-    RangeJobs rj{};
-    int tiles = 0;
-    for (int i = 0; i < 4; ++i) {
-      if (z.n_nodes[i] == 0) continue;
-      const int nt = (z.n_nodes[i] + kRangeTile - 1) / kRangeTile;
-      const int *rp[2] = {L.rowptr[i], L.rrowptr[i]};
-      const int *cl[2] = {L.col[i], L.rdst[i]};
-      int *outp[2] = {L.tile_range[i], L.rtile_range[i]};
-      for (int d = 0; d < 2; ++d) {
-        const int k = rj.n_jobs++;
-        rj.rowptr[k] = rp[d]; rj.col[k] = cl[d]; rj.n_nodes[k] = z.n_nodes[i]; rj.out[k] = outp[d];
-        rj.tile_base[k] = tiles;
-        tiles += nt;
-      }
-    }
-    rj.total_tiles = tiles;
-    for (int k = rj.n_jobs; k < 8; ++k) rj.tile_base[k] = tiles;
-    const int rc = fnb_launch_tile_ranges(rj, stream);
-    if (rc) return rc;
-  }
   AuxArgs x;
   x.a2f = in->atom_to_frag_ids; x.batch = in->batch; x.frag_batch = in->frag_batch; x.a2f32 = L.a2f32;
   x.batch32 = L.batch32; x.frag_batch32 = L.frag_batch32; x.atom_ptr = L.atom_ptr; x.frag_ptr = L.frag_ptr;
   x.n_atoms = (int)in->n_atoms; x.n_frags = (int)in->n_frags; x.n_graphs = (int)in->n_graphs;
-  // component tables for the one-kernel attention backward (opt-in): molecule boundaries in the node order of each graph
-  const bool comps = in->batch != nullptr && in->n_graphs > 0 && fnb_fused_bwd_enabled();
-  x.bond_src = in->edge_index; x.fbond_src = in->frag_index; x.n_bonds = (int)in->n_bonds;
-  x.n_fbond_nodes = (int)in->n_fbond_nodes; x.bond_ptr = comps ? L.bond_ptr : nullptr; x.fbond_ptr = L.fbond_ptr;
   if (cudaError_t le = fnb_launch(k_plan_aux, dim3(grid_for(in->n_atoms > in->n_graphs ? in->n_atoms : in->n_graphs + 1)), dim3(256), 0, stream, x))
     return (int)le;
   FNB_CHECK_LAUNCH();
-  int *comp_ptr[4] = {L.bond_ptr, L.atom_ptr, L.fbond_ptr, L.frag_ptr};
-  if (comps) {
-    CompJobs cj{};
-    cj.n_comps = (int)in->n_graphs;
-    for (int i = 0; i < 4; ++i) {
-      const int k = cj.n_jobs++;
-      cj.rowptr[k] = L.rowptr[i]; cj.col[k] = L.col[i]; cj.rrowptr[k] = L.rrowptr[i]; cj.rdst[k] = L.rdst[i];
-      cj.comp_ptr[k] = comp_ptr[i]; cj.n_nodes[k] = z.n_nodes[i]; cj.open[k] = L.status + 8 + i;
-      cj.bucket[k] = L.comp_bucket[i];
-    }
-    const int64_t warps = (int64_t)cj.n_jobs * (cj.n_comps + 1);
-    if (cudaError_t le = fnb_launch(k_plan_comp_check, dim3(grid_for(warps * 32)), dim3(256), 0, stream, cj)) return (int)le;
-    FNB_CHECK_LAUNCH();
-  }
 
-  fill_plan(in, L, z, staging, comps, out);
+  fill_plan(in, L, z, out);
   return 0;
 }

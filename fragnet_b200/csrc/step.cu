@@ -7,8 +7,6 @@
 // ~3 us each.  Everything lives in one caller-provided workspace whose layout is a pure function of the batch sizes.
 // The optimizer update (fnb_adam_step over the flat parameter buffer) and, with several GPUs, the gradient
 // all-reduce stay separate calls so that NCCL can sit between them.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace {
@@ -140,10 +138,7 @@ extern "C" int fnb_pretrain_step(const fnb_pretrain_step_args *a, void *workspac
     RC((int)cudaStreamWaitEvent(aux.wstream, aux.ready[1], 0));
     RC(fnb_batch_plan_build_impl(in, B.plan_arena, B.plan_bytes, &plan, (void *)aux.wstream, aux.plan_fwd));
     RC((int)cudaEventRecord(aux.wjoin, aux.wstream));
-    // forward CSRs: what the first attention kernels wait for (the experimental staged forward, FNB_STAGE=1, also reads
-    // the tile ranges: it waits for the whole plan)
-    static const bool staged = getenv("FNB_STAGE") && getenv("FNB_STAGE")[0] == '1';
-    plan_ready = staged ? aux.wjoin : aux.plan_fwd;
+    plan_ready = aux.plan_fwd;       // forward CSRs: what the first attention kernels wait for
     plan_complete = aux.wjoin;       // + reverse CSRs, per-molecule arrays: waited for behind those kernels
   } else {
     RC(fnb_batch_plan_build(in, B.plan_arena, B.plan_bytes, &plan, stream));
@@ -199,9 +194,7 @@ extern "C" int fnb_pretrain_plan_prefetch(const fnb_batch_inputs *next, void *ar
   FnbAux aux{};
   if (fnb_aux_streams(&aux) != 0) return FNB_ERR_MODE;
   // Starts once the encoder forward of the step launched last is complete (aux.step_begin is recorded there): by then
-  // the arena's previous tenant -- the step before that one, two arenas alternate -- is long finished.  The staged
-  // forward (FNB_STAGE=1) waits for the whole plan, which this path does not distinguish: not supported together.
-  if (fnb_use_staging()) return FNB_ERR_MODE;
+  // the arena's previous tenant -- the step before that one, two arenas alternate -- is long finished.
   RC((int)cudaStreamWaitEvent(aux.pstream, aux.step_begin, 0));
   if (batch_ready) RC((int)cudaStreamWaitEvent(aux.pstream, (cudaEvent_t)batch_ready, 0));
   fnb_batch_plan plan{};

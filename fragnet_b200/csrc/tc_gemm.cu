@@ -31,8 +31,6 @@
 //  (K > 128 with <= 8192 rows) where a 128-row tile would leave most SMs idle.
 #include <cuda.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace {
@@ -210,7 +208,6 @@ struct TcArgs {
   int64_t M;
   int n_kb;             // K-blocks of 32
   int n_stages;         // depth of the A ring (<= TC_STAGES; fewer for K = 256 so that W + ring + staging fit)
-  int dbg;              // FNB_X3_DBG experiments (k_tc_proj3): 1 = converters only signal, 2 = hi*hi only, 4 = no stores
 };
 
 __global__ void __launch_bounds__(TC_THREADS, 1)
@@ -346,7 +343,7 @@ k_tc_proj(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
 #pragma unroll
         for (int i = 0; i < 8; ++i) {                       // 4 rows x 128 bytes per store instruction
           const int rr = 4 * i + (lane >> 3), cc = (lane & 7) * 4;
-          if (row0 + rr < g.M && !(g.dbg & 4)) st4(g.C + (row0 + rr) * TC_BN + hh * 32 + cc, ld4(stg + rr * TC_EPI_LD + cc));
+          if (row0 + rr < g.M) st4(g.C + (row0 + rr) * TC_BN + hh * 32 + cc, ld4(stg + rr * TC_EPI_LD + cc));
         }
       }
       tc_fence_before();
@@ -493,7 +490,7 @@ k_tc_proj3(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUt
     for (int64_t tile = pair; tile < n_tiles; tile += n_pairs) {
       for (int kb = 0; kb < g.n_kb; ++kb) {
         mbar_wait(bar_full + 8 * stage, phase);
-        if (!(g.dbg & 1)) split_block(ring + stage * kStage, TC_STAGE_BYTES, TC_STAGE_BYTES, ct, X3_CONV_THREADS);
+        split_block(ring + stage * kStage, TC_STAGE_BYTES, TC_STAGE_BYTES, ct, X3_CONV_THREADS);
         fence_proxy_async_smem();
         mbar_arrive(bar_conv + 8 * stage);
         if (++stage == (uint32_t)g.n_stages) { stage = 0; phase ^= 1; }
@@ -536,7 +533,7 @@ k_tc_proj3(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUt
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const int rr = 4 * i + (lane >> 3), cc = (lane & 7) * 4;
-          if (row0 + rr < g.M && !(g.dbg & 4))
+          if (row0 + rr < g.M)
             st4(g.C + (row0 + rr) * TC_BN + half * X3_BN + hh * 32 + cc, ld4(stg + rr * TC_EPI_LD + cc));
         }
       }
@@ -560,7 +557,7 @@ k_tc_proj3(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUt
 
 // ------------------------------------------------------------------------------------------------
 // 3xTF32, K <= 128: full-width version (one CTA per row tile, no pairs).  Measured on the pair kernel above
-// (gpurun_out/r4c: FNB_X3_DBG experiments at 215 k rows): the three N = 64 MMAs per K-step cost as much tensor time as
+// (ablations at 215 k rows): the three N = 64 MMAs per K-step cost as much tensor time as
 // three N = 128 ones (~65 clocks each), converting every A block in both CTAs of a pair doubles that work, and only
 // 32 KB of distinct A bytes per SM are in flight.  Here
 //   * W lives in shared memory as [W_hi (128 rows) ; W_lo (128 rows)] per K-block, so ONE MMA with N = 256 yields
@@ -660,12 +657,9 @@ k_tc_proj3r(const float *__restrict__ A, int lda, const __grid_constant__ CUtens
           for (int k = 0; k < TC_BK / UMMA_K; ++k) {
             const uint32_t ko = k * UMMA_K * 4;
             const uint64_t db = make_desc_sw128_kmajor(b + ko);
-            if (g.dbg & 2) continue;
             tc_mma_tf32(tmem_d, make_desc_sw128_kmajor(a_hi + ko), db, kIdescTf32N256, (kb | k) != 0);
-            if (g.dbg & 16)      // experiment: lo*hi and lo*lo on top of the same columns
-              tc_mma_tf32(tmem_d, make_desc_sw128_kmajor(a_lo + ko), db, kIdescTf32N256, 1);
-            else                 // lo*hi joins hi*lo in the small accumulator: the large one only ever adds hi*hi
-              tc_mma_tf32(tmem_d + 128, make_desc_sw128_kmajor(a_lo + ko), db, kIdescTf32, 1);
+            // lo*hi joins hi*lo in the small accumulator: the large one only ever adds hi*hi
+            tc_mma_tf32(tmem_d + 128, make_desc_sw128_kmajor(a_lo + ko), db, kIdescTf32, 1);
           }
           tc_commit(bar_empty + 8 * slot);
           if (++slot == X3R_SLOTS) { slot = 0; phase ^= 1; }
@@ -721,7 +715,6 @@ k_tc_proj3r(const float *__restrict__ A, int lda, const __grid_constant__ CUtens
           mbar_wait(bar_empty + 8 * grp, (uint32_t)(j & 1) ^ 1);
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
-            if (g.dbg & 1) break;
             const int row = prow + i * 16;
             const uint32_t off = (uint32_t)(row >> 3) * 1024u + (uint32_t)(row & 7) * 128u + (uint32_t)((pc ^ (row & 7)) << 4);
             float4 hi, lo;
@@ -737,7 +730,7 @@ k_tc_proj3r(const float *__restrict__ A, int lda, const __grid_constant__ CUtens
     }
   } else {
     // ===== epilogue warps 0..3: (hi*hi + lo*hi) + hi*lo, bias, logit scalars; rows leave through TMA stores =====
-    // Measured (FNB_X3_DBG ablations, 215 k rows): the epilogue was 16 of 60 us, half of it the st.global path
+    // Measured (ablations, 215 k rows): the epilogue was 16 of 60 us, half of it the st.global path
     // (a thread owns a ROW of the accumulator, so even staged through shared memory a warp needs 8 store
     // instructions per 32 columns); spreading it over 8 warps with 16-column pieces made it slower (64-byte pieces).
     // Here a warp writes its 32 x 32 piece into a 128-byte-swizzled staging box (conflict-free: chunk q of row r
@@ -754,7 +747,6 @@ k_tc_proj3r(const float *__restrict__ A, int lda, const __grid_constant__ CUtens
       float st[4], ss[4];
 #pragma unroll
       for (int hh = 0; hh < 4; ++hh) {
-        if (g.dbg & 8) { st[hh] = ss[hh] = 0.f; continue; }
         uint32_t r[32], r2[32];
         const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + acc * 256 + hh * 32;
         tc_ld_32x32_nowait(taddr, r);
@@ -782,7 +774,7 @@ k_tc_proj3r(const float *__restrict__ A, int lda, const __grid_constant__ CUtens
         }
         fence_proxy_async_smem();
         __syncwarp();
-        if (lane == 0 && !(g.dbg & 4)) {
+        if (lane == 0) {
           asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
                        ::"l"(reinterpret_cast<uint64_t>(&tm_c)), "r"(stg), "r"(hh * 32), "r"((int)row0)
                        : "memory");
@@ -1117,24 +1109,14 @@ int make_map(CUtensorMap *map, const float *ptr, int64_t rows, int cols, int box
   return r == CUDA_SUCCESS ? 0 : FNB_ERR_MODE;
 }
 
-// CTA cap for the projection launches of the calling thread (0 = none): the encoder programs set it around the GEMMs of
-// their side chains (atom / fragment-connection graphs), see fnb_tc_set_cta_cap.
-thread_local int t_cta_cap = 0;
-
 // Persistent grid with the same number of tiles on every CTA: 203 tiles on 148 SMs are two rounds either way, and 102
 // CTAs with two tiles each leave 46 SMs to the kernels of the other streams (a GEMM CTA owns its SM's shared memory).
 int balanced_grid(int64_t n_tiles, int max_ctas) {
-  if (t_cta_cap > 0 && t_cta_cap < max_ctas) max_ctas = t_cta_cap;
   const int64_t per = (n_tiles + max_ctas - 1) / max_ctas;
   return (int)((n_tiles + per - 1) / per);
 }
 
 }  // namespace
-
-// A tcgen05 GEMM CTA owns its SM's shared memory: while a 148-CTA projection runs, the gather kernels of the other
-// streams cannot start anywhere.  GEMMs that nothing on the critical path waits for (side chains) are therefore capped
-// to a fraction of the SMs: they take longer, the bond chain keeps the rest of the GPU.
-void fnb_tc_set_cta_cap(int cap) { t_cta_cap = cap; }
 
 // C[M,128] = A[M,K] @ B[128,K]^T (+bias) with optional fused S; returns FNB_ERR_MODE if the shape cannot take the
 // TMA path (K*4 not a multiple of 16 bytes, K > 256, unaligned pointers) so the caller can fall back to proj.cu.
@@ -1152,10 +1134,7 @@ int fnb_tc_proj_launch(const float *A, const float *B, const float *bias, int64_
   TcArgs g;
   g.C = C; g.bias = bias; g.alpha = alpha; g.alpha_stride = alpha_stride; g.off_t = off_t; g.off_s = off_s;
   g.S = alpha ? S : nullptr; g.M = M; g.n_kb = (K + TC_BK - 1) / TC_BK;
-  g.dbg = 0;
   if (x3) {
-    static const int dbg_env = getenv("FNB_X3_DBG") ? atoi(getenv("FNB_X3_DBG")) : 0;
-    g.dbg = dbg_env;
     // [W_hi | W_lo] of this CTA's 64 columns + ring of [A_hi | A_lo] stages + alignment slack, next to ~20 KB static
     constexpr size_t kDynMax3 = (size_t)206 * 1024;
     const size_t w2 = (size_t)2 * g.n_kb * X3_W_BYTES;
@@ -1173,8 +1152,7 @@ int fnb_tc_proj_launch(const float *A, const float *B, const float *bias, int64_
       done3[dev] = true;
     }
     const int64_t n_tiles3 = (M + TC_BM - 1) / TC_BM;
-    static const bool use_r = !(getenv("FNB_X3_PAIR") && atoi(getenv("FNB_X3_PAIR")));
-    if (use_r && g.n_kb <= 4 && (K & 31) == 0) {   // full-width register-staged kernel
+    if (g.n_kb <= 4 && (K & 31) == 0) {   // full-width register-staged kernel
       constexpr size_t kDynR = (size_t)4 * 2 * TC_STAGE_BYTES + (size_t)X3R_SLOTS * 2 * TC_STAGE_BYTES + 1024;
       void (*kern)(const float *, int, const CUtensorMap, const CUtensorMap, TcArgs) = k_tc_proj3r;
       static bool doneR[64] = {};
@@ -1254,20 +1232,12 @@ int fnb_tc_dw_launch(const float *dh, const float *x, int64_t n_rows, int x_cols
   // stream at least kDwMinBlocks row blocks (512 rows = 512 KiB of operands) so that the partials stay a small
   // fraction of the traffic; the GEMM shares the GPU with the gather kernels of the other streams anyway.
   constexpr int64_t kDwMinBlocks = 16;
-  static const int dw_cap = getenv("FNB_DW_MAX_CTAS") ? atoi(getenv("FNB_DW_MAX_CTAS")) : kNumSMs;
-  const int cap = dw_cap > 0 && dw_cap < kNumSMs ? dw_cap : kNumSMs;
-  int64_t per = (n_rb + cap - 1) / cap;
+  int64_t per = (n_rb + kNumSMs - 1) / kNumSMs;
   if (per < kDwMinBlocks) per = kDwMinBlocks;
   const int grid = (int)((n_rb + per - 1) / per);
   const size_t stage_bytes = ((size_t)TC_STAGE_BYTES + (size_t)n_chunks * 4096) * (x3 ? 2 : 1);
   int n_stages = (int)((200 * 1024) / stage_bytes);
   if (n_stages > DW_MAX_STAGES) n_stages = DW_MAX_STAGES;
-  {
-    // FNB_DW_STAGES (measurement switch): fewer stages = less shared memory, so that gather CTAs of the other streams
-    // can share the SM with a weight-gradient CTA
-    static const int cap = [] { const char *e = getenv("FNB_DW_STAGES"); return e ? atoi(e) : 0; }();
-    if (cap > 0 && n_stages > cap) n_stages = cap;
-  }
   if (n_stages < 1) return FNB_ERR_MODE;
   const size_t smem = (size_t)n_stages * stage_bytes + 1024;
   uint32_t tmem_cols = 32;

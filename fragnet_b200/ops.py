@@ -83,8 +83,6 @@ class GraphCSR:
     rdst: Optional[torch.Tensor] = None
     status: Optional[torch.Tensor] = None   # int32[1], non-zero if an index was out of range
     attr: Optional[torch.Tensor] = None     # per-edge attributes permuted into slot order
-    tile_range: Optional[torch.Tensor] = None    # [ceil(N/64), 2] source range of every 64-destination tile
-    rtile_range: Optional[torch.Tensor] = None   # same for the reverse CSR
     _c: Optional[_abi.CGraph] = field(default=None, repr=False)
 
     def cstruct(self) -> _abi.CGraph:
@@ -93,7 +91,7 @@ class GraphCSR:
             a = lambda t: None if t is None else t.data_ptr()
             self._c = _abi.CGraph(self.n_nodes, self.n_edges, self.n_real, a(self.rowptr), a(self.col), a(self.row),
                                   a(self.eid), a(self.slot_of_eid), a(self.rrowptr), a(self.rslot), a(self.rdst),
-                                  a(self.tile_range), a(self.rtile_range), a(self.attr))
+                                  a(self.attr))
         return self._c
 
 
@@ -124,15 +122,7 @@ def csr_build(dst: torch.Tensor, src: Optional[torch.Tensor], n_nodes: int, self
     rc = lib.fnb_csr_build(_p(dst), _p(src), E, n_nodes, int(self_loops), _p(rowptr), _p(col), _p(row), _p(eid),
                            _p(slot_of_eid), _p(rrowptr), _p(rslot), _p(rdst), _p(ws), ws_bytes, _p(status), _stream())
     _abi.check(rc, "csr_build")
-    g = GraphCSR(n_nodes, total, E, rowptr, col, row, eid, slot_of_eid, rrowptr, rslot, rdst, status)
-    if n_nodes > 0 and src is not None:
-        nt = (n_nodes + 63) // 64
-        g.tile_range = torch.empty((nt, 2), **i32)
-        _abi.check(lib.fnb_tile_ranges(_p(rowptr), _p(col), n_nodes, _p(g.tile_range), _stream()), "tile_ranges")
-        if reverse:
-            g.rtile_range = torch.empty((nt, 2), **i32)
-            _abi.check(lib.fnb_tile_ranges(_p(rrowptr), _p(rdst), n_nodes, _p(g.rtile_range), _stream()), "tile_ranges")
-    return g
+    return GraphCSR(n_nodes, total, E, rowptr, col, row, eid, slot_of_eid, rrowptr, rslot, rdst, status)
 
 
 def gather_rows(src: torch.Tensor, index: torch.Tensor, n_rows: int) -> torch.Tensor:
@@ -229,9 +219,6 @@ class LayerPlan:
                              self._view(cg.row, e), self._view(cg.eid, e), self._view(cg.slot_of_eid, e),
                              self._view(cg.rrowptr, n + 1), self._view(cg.rslot, e), self._view(cg.rdst, e),
                              self._view(self.c.status, 1), attr.view(e, aw) if aw > 1 else attr)
-                nt = (n + 63) // 64
-                g.tile_range = self._view(cg.tile_range, 2 * nt)
-                g.rtile_range = self._view(cg.rtile_range, 2 * nt)
                 g._c = cg
             self._views[name] = g
         return self._views[name]
@@ -249,14 +236,6 @@ class LayerPlan:
     @property
     def status(self):
         return self._view(self.c.status, 1)
-
-    @property
-    def comp_open(self):
-        """int32[4] (bond, atom, fbond, frag): 0 = the graph's molecules are closed, tile-sized components, so its
-        attention backward runs as one kernel (gat_tiled.cu: k_gat_bwd_fused); None without batch vectors."""
-        if not self.c.bond.comp_open:
-            return None
-        return self._view(self.c.bond.comp_open, 4)
 
     @property
     def readout(self) -> Optional[ReadoutPlan]:

@@ -17,10 +17,7 @@
  *     fnb_pretrain_step) fork onto three lazily created, library-owned auxiliary streams (+ events) per device and join
  *     back before they return, so one host thread per device should drive them (the reference's loops are single
  *     threaded).  FNB_STREAMS=1 in the environment keeps every launch on the caller's stream, FNB_PDL=0 turns
- *     programmatic dependent launch off, FNB_DEEP=<mean in-degree> sets the threshold from which the attention
- *     kernels use their deep-gather instantiations (default 24, 0 = never); experiment switches that measured slower
- *     and are off: FNB_PRIO=1 (highest priority for the atom-chain stream), FNB_PREFETCH=1 (L2 prefetch of the source
- *     rows), FNB_STAGE=1 (bulk-copy staging of the source-row range).
+ *     programmatic dependent launch off.
  *     Process-wide state otherwise: a diagnostic launch counter;
  *   - all feature matrices are row-major fp32 with D = 128
  *     columns, H = 4 heads of d = 32 (the only geometry FragNet's gat2 uses with emb_dim 128);
@@ -39,7 +36,7 @@ extern "C" {
 
 #define FNB_D 128 /* embedding width  */
 #define FNB_H 4   /* attention heads  */
-#define FNB_ABI_VERSION 8
+#define FNB_ABI_VERSION 9
 
 /* edge-term modes of the fused attention kernels (SURVEY.md App. A.5) */
 /* arithmetic of the dense projections */
@@ -78,10 +75,6 @@ int fnb_csr_build(const int64_t *dst, const int64_t *src, int64_t n_edges, int64
                   int append_self_loops, int32_t *rowptr, int32_t *col, int32_t *row, int32_t *eid,
                   int32_t *slot_of_eid, int32_t *rrowptr, int32_t *rslot, int32_t *rdst,
                   void *workspace, size_t workspace_bytes, int32_t *status, void *stream);
-
-/* Per tile of 64 consecutive rows of a CSR (rowptr/col), the half-open range [lo, hi) of the column indices met:
- * ranges[2*t] = lo, ranges[2*t+1] = hi (lo = hi = 0 for a tile without edges).  n_tiles = ceil(n_nodes / 64). */
-int fnb_tile_ranges(const int32_t *rowptr, const int32_t *col, int64_t n_nodes, int32_t *ranges, void *stream);
 
 /* out[r, 0:width] = in[index[r], 0:width]  -- puts per-edge attributes into CSR slot order. */
 int fnb_gather_rows(const float *in, const int32_t *index, int64_t n_rows, int width, float *out,
@@ -181,23 +174,8 @@ typedef struct fnb_graph {
   int64_t n_nodes, n_edges, n_real_edges; /* n_edges includes appended self loops */
   const int32_t *rowptr, *col, *row, *eid, *slot_of_eid; /* destination-sorted CSR (fnb_csr_build) */
   const int32_t *rrowptr, *rslot, *rdst;                 /* reverse (source-sorted) CSR             */
-  /* Optional locality hints for the bulk-copy (TMA) staging of gathered rows: for every tile of 64 consecutive
-   * destination nodes, [lo, hi) bounds the SOURCE nodes of its edges (tile_range[2*t], tile_range[2*t+1]); rtile_range
-   * likewise bounds the DESTINATIONS met by 64 consecutive sources in the reverse CSR.  NULL = always gather. */
-  const int32_t *tile_range, *rtile_range;
   const float *edge_attr; /* slot-ordered attributes: [E] (bond graph), [E,6] (fragment-connection graph), else NULL */
-  /* Optional component table (fnb_batch_plan_build with batch vectors while fnb_debug_set_fused_bwd(1)): nodes [comp_ptr[c], comp_ptr[c+1]) are the
-   * nodes of molecule c.  comp_open is a device word the plan writes: 0 = every component is CLOSED (no edge of the
-   * graph leaves it, in either direction) and fits one tile of the fused attention backward (FNB_FUSED_NODES nodes,
-   * FNB_FUSED_SLOTS edge slots), so destination and source pass run as ONE kernel with the tile's gradient rows in
-   * shared memory; non-zero = the two-pass kernels run instead.  comp_ptr == NULL: unknown, two passes. */
-  const int32_t *comp_ptr;    /* [n_comps + 1]; n_comps may exceed the molecule count (trailing empty components) */
-  int64_t n_comps;
-  const int32_t *comp_bucket; /* [ceil(n_nodes / 8) + 1]: first component whose first node is >= 8 k */
-  const int32_t *comp_open;
 } fnb_graph;
-#define FNB_FUSED_NODES 128
-#define FNB_FUSED_SLOTS 896
 
 typedef struct fnb_post_act { /* y = ReLU(Dropout_p(out)); RNG counter of element i is offset + i/4 */
   float p;
@@ -242,10 +220,6 @@ int fnb_gat_bwd_tiled(const fnb_graph *g, const fnb_gat_bwd_args *args, void *st
 /* Same two launches with `between_passes` (a cudaEvent_t of the caller, may be NULL) recorded on `stream` after the
  * destination pass: lets a caller time the two passes separately (bench.py's roofline.kernels). */
 int fnb_gat_bwd_tiled_marked(const fnb_graph *g, const fnb_gat_bwd_args *args, void *between_passes, void *stream);
-/* Opt-in (also FNB_FUSED_BWD=1 in the environment; default 0): plans built while it is 1 carry component tables and
- * their attention backward runs as one kernel.  Measured no faster than the two passes on B200 (DESIGN.md section 3);
- * kept for graphs / parts where it may pay, and exercised by the tests. */
-void fnb_debug_set_fused_bwd(int on);
 /* g_feat[e,:] = g_base[e,:] (if given) + dy[e,:]*(y[e,:]>0)*post_scale (if given) + sum_h dz[slot_of_eid[e],h]*alpha_e[h,:];
  * d_alpha[h, off_e:off_e+128] = sum_e dz[slot_of_eid[e],h] * feat[e,:] */
 int fnb_edge_table_bwd_fused(const fnb_graph *g, const float *dz, const float *feat, const float *alpha,

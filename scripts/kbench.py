@@ -32,7 +32,6 @@ def main():
     Nf, Nfb = b["x_frags"].shape[0], b["node_features_fbonds"].shape[0]
     plan = ops.build_layer_plan(b["edge_index"], b["frag_index"], b["atom_to_frag_ids"], b["edge_index_bonds_graph"],
                                 b["edge_attr_bonds"], b["edge_index_fbonds"], b["edge_attr_fbonds"], Na, Nf, Nb, Nfb, dev)
-    print("FNB_STAGE =", os.environ.get("FNB_STAGE"), " FNB_NPC =", os.environ.get("FNB_NPC"), flush=True)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)
     results = []
 

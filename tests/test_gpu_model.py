@@ -256,61 +256,10 @@ def test_device_prefetcher_yields_identical_batches():
         assert torch.equal(m(lean), m({k: v.cuda() for k, v in host[0].items()}))
 
 
-def _plan_of(b):
-    from fragnet_b200 import ops
-    return ops.build_layer_plan(b["edge_index"], b["frag_index"], b["atom_to_frag_ids"], b["edge_index_bonds_graph"],
-                                b["edge_attr_bonds"], b["edge_index_fbonds"], b["edge_attr_fbonds"],
-                                b["x_atoms"].shape[0], b["x_frags"].shape[0], b["edge_index"].shape[1],
-                                b["frag_index"].shape[1], b["x_atoms"].device, b["batch"], b["frag_batch"])
-
-
-@pytest.mark.parametrize("shape,n,open_expected", [("esol", 16, [0, 0, 0, 0]), ("unimol", 64, [0, 0, 0, 0]),
-                                                    ("stress", 3, None)])
-def test_one_kernel_attention_backward_equals_two_pass(shape, n, open_expected):
-    """Graphs whose molecules are closed, tile-sized components take the one-kernel attention backward
-    (gat_tiled.cu: k_gat_bwd_fused); the two-pass kernels stay as the path for everything else.  Same arithmetic per
-    row, so input gradients agree bitwise and parameter gradients to reduction-order rounding."""
+def test_unsorted_fragment_connections_match_oracle():
+    """A batch whose fragment-connection list is not sorted by molecule (the nodes of the fragment-connection graph
+    are then not grouped by molecule) gives the oracle's forward and gradients."""
     from fragnet.model.gat.gat2 import FragNetFineTune
-    from fragnet_b200 import _abi, ops
-    lib = _abi.load()
-    b = _to(_batch(shape, n, 33, pretrain=False), "cuda")
-    torch.manual_seed(5)
-    m = FragNetFineTune(n_classes=1, num_layer=3, drop_ratio=0.1, h1=64, h2=64, h3=64, h4=64, act="relu").cuda().eval()
-    assert _plan_of(b).comp_open is None               # opt-in: plans carry no component tables by default
-    lib.fnb_debug_set_fused_bwd(1)
-    try:
-        flags = _plan_of(b).comp_open.cpu().tolist()      # bond, atom, fbond, frag
-    finally:
-        lib.fnb_debug_set_fused_bwd(0)
-    if open_expected is not None:
-        assert flags == open_expected
-    else:                               # stress shape: the fragment-connection molecules exceed a tile
-        assert flags[2] == 1 and flags[1] == 0
-    x = {k: (v.clone().requires_grad_(True) if k == "x_atoms" else v) for k, v in b.items()}
-    grads = []
-    try:
-        for on in (1, 0):
-            lib.fnb_debug_set_fused_bwd(on)
-            ops.clear_plan_cache()
-            m.zero_grad()
-            x["x_atoms"].grad = None
-            m(x).sum().backward()
-            g = {k: p.grad.clone() for k, p in m.named_parameters() if p.grad is not None}
-            g["x_atoms"] = x["x_atoms"].grad.clone()
-            grads.append(g)
-    finally:
-        lib.fnb_debug_set_fused_bwd(0)
-    assert grads[0].keys() == grads[1].keys()
-    for k in grads[0]:
-        scale = grads[1][k].abs().max().clamp_min(1e-30)
-        assert (grads[0][k] - grads[1][k]).abs().max() <= 2e-6 * scale, k
-
-
-def test_one_kernel_backward_falls_back_on_unsorted_edges():
-    """A batch whose bond list is not molecule-sorted has no closed components: the device-side check marks the graphs
-    open and the two-pass kernels produce the same gradients as for the sorted batch (permuted back)."""
-    from fragnet.model.gat.gat2 import FragNetFineTune
-    from fragnet_b200 import ops
     from oracle import gat2_oracle as O
     b = _batch("esol", 64, 4, pretrain=False)
     torch.manual_seed(6)
@@ -330,19 +279,10 @@ def test_one_kernel_backward_falls_back_on_unsorted_edges():
     b2["edge_index_fbonds"] = inv[b["edge_index_fbonds"]]
     ref = O.finetune_forward(P, b2)
     ref.sum().backward()
-    from fragnet_b200 import _abi
-    lib = _abi.load()
     m = m.cuda()
-    ops.clear_plan_cache()
-    lib.fnb_debug_set_fused_bwd(1)
-    try:
-        assert _plan_of(_to(b2, "cuda")).comp_open.cpu().tolist()[2] == 1
-        pred = m(_to(b2, "cuda"))
-        assert rel_err(pred, ref) <= FP32_REL_TOL
-        pred.sum().backward()
-    finally:
-        lib.fnb_debug_set_fused_bwd(0)
-        ops.clear_plan_cache()
+    pred = m(_to(b2, "cuda"))
+    assert rel_err(pred, ref) <= FP32_REL_TOL
+    pred.sum().backward()
     _assert_grads([(k, p.grad, P[k].grad) for k, p in m.named_parameters() if p.grad is not None])
 
 

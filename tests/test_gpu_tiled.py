@@ -12,7 +12,7 @@ pytestmark = pytest.mark.gpu
 def _graph(n_nodes, n_edges, seed, hub_edges=0, band=0):
     g = torch.Generator().manual_seed(seed)
     dst = torch.randint(0, n_nodes, (n_edges,), generator=g)
-    if band:     # block-diagonal-like locality (sources within +-band of the destination): the bulk-copy staged path
+    if band:     # block-diagonal-like locality (sources within +-band of the destination), as in batched molecules
         src = (dst + torch.randint(-band, band + 1, (n_edges,), generator=g)).clamp_(0, n_nodes - 1)
     else:
         src = torch.randint(0, n_nodes, (n_edges,), generator=g)
@@ -24,8 +24,8 @@ def _graph(n_nodes, n_edges, seed, hub_edges=0, band=0):
 
 
 CASES = [
-    (20000, 130000, -30),  # 64-node tiles with local sources: rows staged by cp.async.bulk (negative = band width)
-    (20000, 130000, -100), # ranges above the staging capacity: gather fallback inside the staged kernel
+    (20000, 130000, -30),  # 64-node tiles with local sources (negative = band width)
+    (20000, 130000, -100), # wider band: each tile's sources span a longer id range
     (40, 200, 0),          # one partial tile
     (64, 3000, 0),         # one tile, several sub-tiles (3000 slots > capacity)
     (50, 6000, 2500),      # hub paths: in-degree and out-degree above the capacity of a sub-tile
