@@ -107,9 +107,12 @@ class EncoderFn(torch.autograd.Function):
         lib = ops._lib()
         layers = _layer_structs(cfg, params, dev)
         dropping = cfg.post_act and cfg.training and cfg.drop_p > 0
+        # the forward gets the backward's need_dx_* as well: with a wanted d x_atoms, input dropout then runs as its own
+        # kernel instead of inside the padding kernel (the backward's results do not depend on which one ran)
+        need_dx = [int(need_grad and n) for n in ctx.needs_input_grad[2:5]]
         opts = _abi.CEncoderOpts(n_layers, int(cfg.post_act), float(cfg.drop_p), int(cfg.training),
                                  torch.initial_seed() & 0xFFFFFFFFFFFFFFFF, 0, cfg.precision, int(need_grad),
-                                 0, 0, 0)
+                                 *need_dx)
         cplan = plan.cstruct()
         if dropping:
             opts.offset = ops.reserve_rng(lib.fnb_encoder_rng_span(C.byref(cplan), C.byref(opts), layers))

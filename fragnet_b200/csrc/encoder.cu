@@ -737,12 +737,14 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
         if (two) RC((int)cudaStreamWaitEvent(stream, aux.a_dz, 0));
         RC(w_begin(0, sA));
         float *dx = need_dx ? W.dx_atom : (o->need_dx_atoms ? io->dx_atoms : nullptr);
-        if (l == 0 && b.k_pad[1] && !dx) {
+        // layer 0 with padded operands: d Wa always from the padded copy, which holds exactly what the forward
+        // multiplied (dropped or not).  The unpadded dropped copy xa0 exists only if the forward call already had
+        // need_dx_atoms set; with input dropout applied inside the padding kernel it was never written.
+        if (dx) RC(fnb_proj_bwd_dx(P.Wa, wt_of(l, 1), dh_a, z.Na, P.K_atom, dx, o->precision, scratchA, sA_));
+        if (l == 0 && b.k_pad[1])
           RC(fnb_tc_dw_launch(dh_a, b.x_pad[1], z.Na, b.k_pad[1], P.K_atom, D.Wa, scratch_body(scratchWs[0]), sWs[0], x3));
-        } else {
-          RC(fnb_proj_bwd_dx(P.Wa, wt_of(l, 1), dh_a, z.Na, P.K_atom, dx, o->precision, scratchA, sA_));
+        else
           RC(fnb_proj_bwd_dw(xa, dh_a, z.Na, P.K_atom, D.Wa, nullptr, o->precision, scratchWs[0], (void *)sWs[0]));
-        }
         RC(w_end(0, par));
         // bond features were this graph's edge vectors (gat2.py:203-208): the head-vector gradient of that term is
         // nobody's input.  On the atom chain it delayed the next layer's dz (which the bond chain, the critical path,

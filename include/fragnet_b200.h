@@ -306,7 +306,10 @@ typedef struct fnb_encoder_opts {
   uint64_t seed, offset; /* RNG key / first counter; the call consumes fnb_encoder_rng_span() counters */
   int precision;         /* FNB_PRECISION_* for the dense projections */
   int save_for_backward; /* keep what fnb_encoder_backward needs */
-  int need_dx_atoms, need_dx_bond, need_dx_fbond; /* backward: gradients of the layer-0 inputs */
+  int need_dx_atoms, need_dx_bond, need_dx_fbond; /* backward: gradients of the layer-0 inputs.  In the forward,
+                                                     need_dx_atoms only selects where input dropout runs (its own
+                                                     kernel instead of the padding kernel); the backward is right
+                                                     whichever values the forward call had */
 } fnb_encoder_opts;
 
 typedef struct fnb_encoder_io {

@@ -15,7 +15,7 @@ written by ``tests/golden/make_golden.py``.
 """
 from __future__ import annotations
 
-from typing import Dict, Mapping, Optional, Sequence
+from typing import Callable, Dict, Mapping, Optional, Sequence
 
 import torch
 import torch.nn.functional as F
@@ -24,6 +24,16 @@ from .shims import add_self_loops, scatter_add, scatter_softmax
 
 Params = Mapping[str, torch.Tensor]
 NEG_SLOPE = 0.2          # nn.LeakyReLU(0.2), gat2.py:83
+# ``drop_fn(site, t)``: replaces ``F.dropout(t, drop_ratio, training)`` at one dropout site of an encoder.  ``site`` is
+# ("input", "atoms" | "frags") for the dropout on the raw features, (layer, "atoms" | "frags" | "bond" | "fbond") for
+# the ReLU(Dropout(.)) after a layer.  Tests pass one that applies a known keep-mask, to replay the masks of a run.
+DropFn = Callable[[tuple, torch.Tensor], torch.Tensor]
+
+
+def _dropper(drop_fn: Optional[DropFn], drop_ratio: float, training: bool):
+    if drop_fn is None:
+        return lambda site, t: F.dropout(t, drop_ratio, training)
+    return drop_fn
 
 
 def _linear(P: Params, name: str, x: torch.Tensor) -> torch.Tensor:
@@ -109,19 +119,20 @@ def layer_forward(P: Params, prefix: str, num_heads: int,
 
 def fragnet_forward(P: Params, batch: Dict[str, torch.Tensor], num_layer: int, num_heads: int = 4,
                     drop_ratio: float = 0.0, training: bool = False, prefix: str = "pretrain.",
-                    masks: Optional[dict] = None, return_attentions: bool = False):
+                    masks: Optional[dict] = None, return_attentions: bool = False,
+                    drop_fn: Optional[DropFn] = None):
     """``FragNet.forward`` (gat2.py:381-442): input dropout, layer 0 on raw features, then
     ``ReLU(Dropout(.))`` on the four outputs of every layer; layers >= 1 receive the bond
     features as both ``edge_attr`` and bond-graph node features (:421-434).
 
     With ``return_attentions`` the attention tensors of the LAST layer are appended, which is
-    the arrangement of ``vizualize/model.py:72-142``.
+    the arrangement of ``vizualize/model.py:72-142``.  ``drop_fn`` replaces ``F.dropout`` at every site (``DropFn``).
     """
     masks = masks or {}
-    drop = lambda t: F.dropout(t, drop_ratio, training)
-    post = lambda t: F.relu(drop(t))
-    x_atoms = drop(batch["x_atoms"])
-    x_frags = drop(batch["x_frags"])
+    drop = _dropper(drop_fn, drop_ratio, training)
+    post = lambda site, t: F.relu(drop(site, t))
+    x_atoms = drop(("input", "atoms"), batch["x_atoms"])
+    x_frags = drop(("input", "frags"), batch["x_frags"])
     edge_feat = batch["edge_attr"]
     bond_nodes = batch["node_features_bonds"]
     fbond_nodes = batch["node_features_fbonds"]
@@ -133,9 +144,9 @@ def fragnet_forward(P: Params, batch: Dict[str, torch.Tensor], num_layer: int, n
             batch["atom_to_frag_ids"], bond_nodes, batch["edge_index_bonds_graph"],
             batch["edge_attr_bonds"], fbond_nodes, batch["edge_index_fbonds"],
             batch["edge_attr_fbonds"], **masks)
-        x_atoms, x_frags = post(out[0]), post(out[1])
-        edge_feat = post(out[2])
-        fedge_feat = post(out[3])
+        x_atoms, x_frags = post((li, "atoms"), out[0]), post((li, "frags"), out[1])
+        edge_feat = post((li, "bond"), out[2])
+        fedge_feat = post((li, "fbond"), out[3])
         bond_nodes, fbond_nodes = edge_feat, fedge_feat
         attn = out[4:]
     if return_attentions:
@@ -205,18 +216,19 @@ def lite_layer_forward(P: Params, prefix: str, num_heads: int, x_atoms, edge_ind
 
 
 def lite_fragnet_forward(P: Params, batch, num_layer: int, num_heads: int = 4, drop_ratio: float = 0.0,
-                         training: bool = False, prefix: str = "pretrain."):
+                         training: bool = False, prefix: str = "pretrain.", drop_fn: Optional[DropFn] = None):
     """``gat2_lite.FragNet.forward`` (gat2_lite.py:174-216): ``ReLU(Dropout(.))`` on atoms, pooled fragments and bond
-    features after every layer; layers >= 1 take the bond features as edge attributes and bond-graph nodes."""
-    drop = lambda t: F.dropout(t, drop_ratio, training)
-    post = lambda t: F.relu(drop(t))
-    x_atoms, x_frags = drop(batch["x_atoms"]), drop(batch["x_frags"])
+    features after every layer; layers >= 1 take the bond features as edge attributes and bond-graph nodes.
+    ``drop_fn``: as in ``fragnet_forward`` (no "fbond" site)."""
+    drop = _dropper(drop_fn, drop_ratio, training)
+    post = lambda site, t: F.relu(drop(site, t))
+    x_atoms, x_frags = drop(("input", "atoms"), batch["x_atoms"]), drop(("input", "frags"), batch["x_frags"])
     edge_feat, bond_nodes = batch["edge_attr"], batch["node_features_bonds"]
     for li in range(num_layer):
         out = lite_layer_forward(P, f"{prefix}layers.{li}.", num_heads, x_atoms, batch["edge_index"], edge_feat, x_frags,
                                  batch["atom_to_frag_ids"], bond_nodes, batch["edge_index_bonds_graph"],
                                  batch["edge_attr_bonds"])
-        x_atoms, x_frags, edge_feat = post(out[0]), post(out[1]), post(out[2])
+        x_atoms, x_frags, edge_feat = post((li, "atoms"), out[0]), post((li, "frags"), out[1]), post((li, "bond"), out[2])
         bond_nodes = edge_feat
     return x_atoms, x_frags, edge_feat, None
 
@@ -253,17 +265,18 @@ def edge_layer_forward(P: Params, prefix: str, num_heads: int, x_atoms, edge_ind
 
 
 def edge_fragnet_forward(P: Params, batch, num_layer: int, num_heads: int = 4, drop_ratio: float = 0.0,
-                         training: bool = False, prefix: str = "pretrain."):
-    """``gat2_edge.FragNet.forward`` (gat2_edge.py:198-239)."""
-    drop = lambda t: F.dropout(t, drop_ratio, training)
-    post = lambda t: F.relu(drop(t))
-    x_atoms, x_frags = drop(batch["x_atoms"]), drop(batch["x_frags"])
+                         training: bool = False, prefix: str = "pretrain.", drop_fn: Optional[DropFn] = None):
+    """``gat2_edge.FragNet.forward`` (gat2_edge.py:198-239).  ``drop_fn``: as in ``fragnet_forward`` (no "fbond"
+    site)."""
+    drop = _dropper(drop_fn, drop_ratio, training)
+    post = lambda site, t: F.relu(drop(site, t))
+    x_atoms, x_frags = drop(("input", "atoms"), batch["x_atoms"]), drop(("input", "frags"), batch["x_frags"])
     edge_feat, bond_nodes = batch["edge_attr"], batch["node_features_bonds"]
     for li in range(num_layer):
         out = edge_layer_forward(P, f"{prefix}layers.{li}.", num_heads, x_atoms, batch["edge_index"], edge_feat,
                                  batch["frag_index"], x_frags, batch["atom_to_frag_ids"], bond_nodes,
                                  batch["edge_index_bonds_graph"], batch["edge_attr_bonds"], batch["cnx_attr"])
-        x_atoms, x_frags, edge_feat = post(out[0]), post(out[1]), post(out[2])
+        x_atoms, x_frags, edge_feat = post((li, "atoms"), out[0]), post((li, "frags"), out[1]), post((li, "bond"), out[2])
         bond_nodes = edge_feat
     return x_atoms, x_frags, edge_feat
 
@@ -298,9 +311,10 @@ def pretrain_heads_forward(P: Params, x_atoms, x_frags, edge_feat, batch, L: int
 
 
 def pretrain_forward(P: Params, batch, num_layer: int = 4, num_heads: int = 4, drop_ratio: float = 0.0,
-                     training: bool = False):
-    """``FragNetPreTrain.forward`` (pretrain_heads.py:134-141)."""
-    x_atoms, x_frags, e_edge, _ = fragnet_forward(P, batch, num_layer, num_heads, drop_ratio, training)
+                     training: bool = False, drop_fn: Optional[DropFn] = None):
+    """``FragNetPreTrain.forward`` (pretrain_heads.py:134-141).  ``drop_fn``: see ``fragnet_forward``."""
+    x_atoms, x_frags, e_edge, _ = fragnet_forward(P, batch, num_layer, num_heads, drop_ratio, training,
+                                                  drop_fn=drop_fn)
     return pretrain_heads_forward(P, x_atoms, x_frags, e_edge, batch)
 
 
