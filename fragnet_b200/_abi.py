@@ -63,6 +63,9 @@ SIGNATURES = {
     "fnb_pretrain_step_rng_span": (_u64, [_vp]),
     "fnb_pretrain_step": (C.c_int, [_vp, _vp, _sz, _vp, _vp]),
     "fnb_pretrain_plan_prefetch": (C.c_int, [_vp, _vp, _sz, _vp]),
+    "fnb_finetune_step_workspace_bytes": (_sz, [_vp]),
+    "fnb_finetune_step_rng_span": (_u64, [_vp]),
+    "fnb_finetune_step": (C.c_int, [_vp, _vp, _sz, _vp, _vp]),
     "fnb_arena_workspace_bytes": (_sz, [_i64, _i32]),
     "fnb_arena_assemble": (C.c_int, [_vp, _i64, _i64, _vp, _i32, _vp, _i32, _vp, _sz, _vp, _vp]),
 }
@@ -112,7 +115,7 @@ class CWidenJob(C.Structure):
 WIDEN_U8_F32, WIDEN_I32_I64, WIDEN_MAX_JOBS = 0, 1, 16
 ARENA_COPY32, ARENA_INDEX, ARENA_FILL = 0, 1, 2
 ARENA_MAX_KINDS, ARENA_MAX_JOBS = 24, 32
-ABI_VERSION = 9
+ABI_VERSION = 10
 EDGE_NONE, EDGE_AFFINE1, EDGE_AFFINE6, EDGE_TABLE = 0, 1, 2, 3
 PRECISION_FP32, PRECISION_TF32, PRECISION_TF32X3 = 0, 1, 2
 
@@ -224,3 +227,22 @@ class CPretrainStepArgs(C.Structure):
                 ("drop_p", _f32), ("training", _i32), ("seed", _u64), ("offset", _u64), ("precision", _i32),
                 ("backward", _i32)] + \
                [(n, _vp) for n in ("loss", "bond_length", "bond_angle", "dihedral", "energy", "plan_arena")]
+
+
+ACT_NONE, ACT_RELU, ACT_CELU, ACT_SILU, ACT_GELU, ACT_SELU, ACT_RELU6, ACT_LEAKYRELU = range(8)
+MLP_MAX_LAYERS = 8
+LOSS_MSE, LOSS_BCE_MASKED = 0, 1
+
+
+class CMlpLayer(C.Structure):
+    _fields_ = [(n, _vp) for n in ("W", "b", "dW", "db")] + [("in_dim", _i32), ("out_dim", _i32), ("p_in", _f32),
+                                                               ("p_out", _f32), ("act", _i32)]
+
+
+class CFinetuneStepArgs(C.Structure):
+    _fields_ = [("batch", CBatchInputs)] + \
+               [(n, _vp) for n in ("x_atoms", "x_bond", "x_fbond", "target")] + \
+               [("n_layers", _i32), ("layers", _vp), ("layer_grads", _vp), ("n_head_layers", _i32), ("head", _vp),
+                ("loss_kind", _i32), ("drop_p", _f32), ("training", _i32), ("seed", _u64), ("offset", _u64),
+                ("precision", _i32), ("backward", _i32)] + \
+               [(n, _vp) for n in ("loss", "predictions", "plan_arena")]

@@ -267,6 +267,31 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
                                     void *workspace, size_t workspace_bytes, void *scratch, void *stream,
                                     int skip_tails);
 
+// Finetuning head (finetune.cu).  One run of an fnb_mlp_layer list over G rows; every buffer is caller-provided.
+struct FnbMlpRun {
+  const fnb_mlp_layer *L;
+  int n;
+  int64_t G;
+  int training;
+  uint64_t seed;
+  uint64_t in_base[FNB_MLP_MAX_LAYERS], out_base[FNB_MLP_MAX_LAYERS];   // fnb_mlp_rng
+  float *x0;                        // [G, L[0].in_dim] head input
+  float *xd[FNB_MLP_MAX_LAYERS];    // [G, L[l].in_dim] what layer l multiplies; xd[0] == x0 when nothing drops there
+  float *u[FNB_MLP_MAX_LAYERS];     // [G, L[l].out_dim] pre-activation of the hidden layers (NULL: not kept)
+  float *out;                       // [G, L[n-1].out_dim] predictions
+  float *dz[FNB_MLP_MAX_LAYERS];    // backward: [G, L[l].out_dim] gradient of layer l's pre-dropout output; dz[n-1] is input
+  float *dx0;                       // backward: [G, L[0].in_dim] gradient of x0
+  float *rec;                       // backward: fnb_mlp_dw_record_floats() floats
+};
+int fnb_mlp_check(const fnb_mlp_layer *L, int n, int64_t G, int in0, int backward);
+uint64_t fnb_mlp_rng(const fnb_mlp_layer *L, int n, int64_t G, uint64_t offset, uint64_t *in_base, uint64_t *out_base);
+size_t fnb_mlp_dw_record_floats(const fnb_mlp_layer *L, int n, int64_t G);
+int fnb_mlp_forward(const FnbMlpRun *r, cudaStream_t stream);
+int fnb_mlp_backward(const FnbMlpRun *r, cudaStream_t stream);
+// loss[0] = mean of BCE-with-logits over the labels > -0.5 (NaN if none); grad (may be NULL) = its logit gradient.
+int fnb_bce_masked_loss(const float *logits, const float *labels, int64_t n, float *loss, float *grad,
+                        cudaStream_t stream);
+
 // Tensor-core (tcgen05, TF32) projection path, tc_gemm.cu.  Returns FNB_ERR_MODE when the shape cannot use TMA.
 // x3 != 0: 3xTF32 (error-compensated, FP32-grade) instead of one TF32 product.
 int fnb_tc_proj_launch(const float *A, const float *B, const float *bias, int64_t M, int K, const float *alpha,

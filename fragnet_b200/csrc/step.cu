@@ -35,7 +35,9 @@ fnb_batch_plan sizes_plan(const fnb_batch_inputs *in) {
   return p;
 }
 
-fnb_encoder_opts opts_of(const fnb_pretrain_step_args *a) {
+// the encoder options of a step (fnb_pretrain_step_args and fnb_finetune_step_args name these fields alike)
+template <class StepArgs>
+fnb_encoder_opts opts_of(const StepArgs *a) {
   fnb_encoder_opts o{};
   o.n_layers = a->n_layers; o.post_act = 1; o.drop_p = a->drop_p; o.training = a->training; o.seed = a->seed;
   o.offset = a->offset; o.precision = a->precision; o.save_for_backward = a->backward ? 1 : 0;
@@ -93,6 +95,39 @@ size_t step_layout(const fnb_pretrain_step_args *a, char *base, StepBufs *out) {
     if (rc__) return rc__;   \
   } while (0)
 
+// The first half of both step programs: the on-device collate of the batch (north-star kernel a) and the encoder
+// forward (FragNet.forward, gat2.py:381-442).  The collate runs on an auxiliary stream, underneath the plan-independent
+// head of the forward pass (input dropout, operand padding, layer-0 projections), or was done ahead of the step by
+// fnb_pretrain_plan_prefetch (`prefetched`: its arena, on its own stream, underneath the previous step).
+int collate_and_encode(const fnb_batch_inputs *in, const void *prefetched, char *plan_arena, size_t plan_bytes,
+                       const fnb_encoder_opts *o, const fnb_layer_params *layers, const fnb_encoder_io *eio,
+                       char *enc_ws, size_t enc_bytes, void *scratch, void *stream, const FnbAux &aux, bool two,
+                       fnb_batch_plan *plan_out) {
+  fnb_batch_plan plan{};
+  cudaEvent_t plan_ready = nullptr, plan_complete = nullptr;
+  if (two && prefetched) {
+    RC(fnb_batch_plan_view(in, const_cast<void *>(prefetched), fnb_batch_plan_bytes(in), &plan));
+    plan_ready = aux.p_fwd;
+    plan_complete = aux.p_done;
+  } else if (two) {
+    cudaStream_t s = (cudaStream_t)stream;
+    RC((int)cudaEventRecord(aux.ready[1], s));               // the batch tensors are complete on the caller's stream
+    RC((int)cudaStreamWaitEvent(aux.wstream, aux.ready[1], 0));
+    RC(fnb_batch_plan_build_impl(in, plan_arena, plan_bytes, &plan, (void *)aux.wstream, aux.plan_fwd));
+    RC((int)cudaEventRecord(aux.wjoin, aux.wstream));
+    plan_ready = aux.plan_fwd;       // forward CSRs: what the first attention kernels wait for
+    plan_complete = aux.wjoin;       // + reverse CSRs, per-molecule arrays: waited for behind those kernels
+  } else {
+    RC(fnb_batch_plan_build(in, plan_arena, plan_bytes, &plan, stream));
+  }
+  RC(fnb_encoder_forward_impl(&plan, o, layers, eio, enc_ws, enc_bytes, scratch, stream, plan_ready, plan_complete));
+  // the collate of the next batch (fnb_pretrain_plan_prefetch) starts here: underneath the heads, where one or two
+  // kernels are in flight, rather than underneath the forward, whose chains it slowed (gpurun_out/r5q)
+  if (two) RC((int)cudaEventRecord(aux.step_begin, (cudaStream_t)stream));
+  *plan_out = plan;
+  return 0;
+}
+
 }  // namespace
 
 extern "C" size_t fnb_pretrain_step_workspace_bytes(const fnb_pretrain_step_args *a) {
@@ -121,37 +156,15 @@ extern "C" int fnb_pretrain_step(const fnb_pretrain_step_args *a, void *workspac
   StepBufs B;
   if (step_layout(a, (char *)workspace, &B) > workspace_bytes) return FNB_ERR_WORKSPACE;
 
-  // ---- on-device collate (north-star kernel a): on an auxiliary stream, underneath the plan-independent head of the
-  // forward pass (input dropout, operand padding, layer-0 projections)
-  fnb_batch_plan plan{};
   FnbAux aux{};
   const bool two = fnb_aux_streams(&aux) == 0;
-  cudaEvent_t plan_ready = nullptr, plan_complete = nullptr;
-  if (two && a->plan_arena) {
-    // collated ahead of this step by fnb_pretrain_plan_prefetch (on its own stream, underneath the previous step)
-    RC(fnb_batch_plan_view(in, const_cast<void *>(a->plan_arena), fnb_batch_plan_bytes(in), &plan));
-    plan_ready = aux.p_fwd;
-    plan_complete = aux.p_done;
-  } else if (two) {
-    cudaStream_t s = (cudaStream_t)stream;
-    RC((int)cudaEventRecord(aux.ready[1], s));               // the batch tensors are complete on the caller's stream
-    RC((int)cudaStreamWaitEvent(aux.wstream, aux.ready[1], 0));
-    RC(fnb_batch_plan_build_impl(in, B.plan_arena, B.plan_bytes, &plan, (void *)aux.wstream, aux.plan_fwd));
-    RC((int)cudaEventRecord(aux.wjoin, aux.wstream));
-    plan_ready = aux.plan_fwd;       // forward CSRs: what the first attention kernels wait for
-    plan_complete = aux.wjoin;       // + reverse CSRs, per-molecule arrays: waited for behind those kernels
-  } else {
-    RC(fnb_batch_plan_build(in, B.plan_arena, B.plan_bytes, &plan, stream));
-  }
-  // ---- encoder forward (FragNet.forward, gat2.py:381-442)
+  fnb_batch_plan plan{};
   fnb_encoder_opts o = opts_of(a);
   fnb_encoder_io eio{};
   eio.x_atoms = a->x_atoms; eio.x_bond = a->x_bond; eio.x_fbond = a->x_fbond;
   eio.out_atoms = B.out_atoms; eio.out_frags = B.out_frags; eio.out_bond = B.out_bond; eio.out_fbond = B.out_fbond;
-  RC(fnb_encoder_forward_impl(&plan, &o, a->layers, &eio, B.enc_ws, B.enc_bytes, scratch, stream, plan_ready, plan_complete));
-  // the collate of the next batch (fnb_pretrain_plan_prefetch) starts here: underneath the heads, where one or two
-  // kernels are in flight, rather than underneath the forward, whose chains it slowed (gpurun_out/r5q)
-  if (two) RC((int)cudaEventRecord(aux.step_begin, (cudaStream_t)stream));
+  RC(collate_and_encode(in, a->plan_arena, B.plan_arena, B.plan_bytes, &o, a->layers, &eio, B.enc_ws, B.enc_bytes,
+                        scratch, stream, aux, two, &plan));
   // ---- heads (PretrainTask.forward, pretrain_heads.py:64-102)
   fnb_pretrain_head_io hio{};
   hio.x_atoms = B.out_atoms; hio.x_frags = B.out_frags; hio.edge_feat = B.out_bond; hio.edge_index = in->edge_index;
@@ -203,3 +216,139 @@ extern "C" int fnb_pretrain_plan_prefetch(const fnb_batch_inputs *next, void *ar
   return 0;
 }
 
+
+// ---------------------------------------------------------------------------------------------------------------------
+// One finetuning step (TrainerFineTune.train_regr / train_clsf_bce, fragnet/train/utils.py:330-470, on FragNetFineTune):
+// collate, encoder forward, readout cat(sum atoms, sum fragments) (gat2.py:820-823), FTHead forward, loss, FTHead
+// backward, readout backward, encoder backward -- in stream order on the caller's stream, the encoder's own forks aside.
+namespace {
+
+bool ft_args_ok(const fnb_finetune_step_args *a) {
+  return a && a->n_layers >= 1 && a->n_layers <= 16 && a->layers && a->batch.n_atoms >= 0 && a->batch.n_frags >= 0 &&
+         a->batch.n_bonds >= 0 && a->batch.n_graphs >= 1 &&
+         fnb_mlp_check(a->head, a->n_head_layers, a->batch.n_graphs, 2 * kD, 0) == 0;
+}
+
+struct FtBufs {
+  char *plan_arena; size_t plan_bytes;
+  char *enc_ws; size_t enc_bytes;
+  char *enc_bws; size_t enc_bws_bytes;
+  float *out_atoms, *out_frags, *out_bond, *out_fbond;
+  float *readout, *xd0, *pred;
+  float *xd[FNB_MLP_MAX_LAYERS], *u[FNB_MLP_MAX_LAYERS], *dz[FNB_MLP_MAX_LAYERS];
+  float *d_readout, *g_atoms, *g_frags, *rec;
+};
+
+size_t ft_layout(const fnb_finetune_step_args *a, char *base, FtBufs *out) {
+  const fnb_batch_inputs *in = &a->batch;
+  const fnb_batch_plan sp = sizes_plan(in);
+  const fnb_encoder_opts o = opts_of(a);
+  const int64_t Na = in->n_atoms, Nf = in->n_frags, Nb = in->n_bonds, Nfb = in->n_fbond_nodes, G = in->n_graphs;
+  const fnb_mlp_layer *L = a->head;
+  const int n = a->n_head_layers;
+  Arena ar{base, 0};
+  FtBufs b{};
+  b.plan_bytes = fnb_batch_plan_bytes(in);
+  b.plan_arena = ar.bytes(b.plan_bytes);
+  b.enc_bytes = fnb_encoder_workspace_bytes(&sp, &o, a->layers);
+  b.enc_ws = ar.bytes(b.enc_bytes);
+  b.out_atoms = ar.take<float>(Na * kD); b.out_frags = ar.take<float>(Nf * kD);
+  b.out_bond = ar.take<float>(Nb * kD);  b.out_fbond = ar.take<float>(Nfb * kD);
+  b.readout = ar.take<float>(G * 2 * kD);
+  if (L[0].p_in > 0.f) b.xd0 = ar.take<float>(G * 2 * kD);
+  b.pred = ar.take<float>(G * L[n - 1].out_dim);
+  for (int l = 0; l + 1 < n; ++l) {
+    b.xd[l + 1] = ar.take<float>(G * L[l].out_dim);
+    if (a->backward) b.u[l] = ar.take<float>(G * L[l].out_dim);
+  }
+  if (a->backward) {
+    for (int l = 0; l < n; ++l) b.dz[l] = ar.take<float>(G * L[l].out_dim);
+    b.d_readout = ar.take<float>(G * 2 * kD);
+    b.rec = ar.take<float>(fnb_mlp_dw_record_floats(L, n, G));
+    b.g_atoms = ar.take<float>(Na * kD); b.g_frags = ar.take<float>(Nf * kD);
+    b.enc_bws_bytes = fnb_encoder_bwd_workspace_bytes(&sp, &o, a->layers);
+    b.enc_bws = ar.bytes(b.enc_bws_bytes);
+  }
+  if (out) *out = b;
+  return (ar.off + 255) & ~(size_t)255;
+}
+
+}  // namespace
+
+extern "C" size_t fnb_finetune_step_workspace_bytes(const fnb_finetune_step_args *a) {
+  if (!ft_args_ok(a)) return 0;
+  return ft_layout(a, nullptr, nullptr);
+}
+
+extern "C" uint64_t fnb_finetune_step_rng_span(const fnb_finetune_step_args *a) {
+  if (!ft_args_ok(a)) return 0;
+  const fnb_batch_plan sp = sizes_plan(&a->batch);
+  const fnb_encoder_opts o = opts_of(a);
+  return fnb_encoder_rng_span(&sp, &o, a->layers) +
+         fnb_mlp_rng(a->head, a->n_head_layers, a->batch.n_graphs, 0, nullptr, nullptr);
+}
+
+extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspace, size_t workspace_bytes, void *scratch,
+                                 void *stream) {
+  if (!a || !workspace || !scratch) return FNB_ERR_NULL;
+  if (!a->head || !a->layers) return FNB_ERR_NULL;
+  if (a->n_layers < 1 || a->n_layers > 16) return FNB_ERR_SIZE;
+  const fnb_batch_inputs *in = &a->batch;
+  if (in->n_atoms < 1 || in->n_bonds < 0 || in->n_frags < 0 || in->n_graphs < 1 || !in->batch || !in->frag_batch)
+    return FNB_ERR_SIZE;
+  RC(fnb_mlp_check(a->head, a->n_head_layers, in->n_graphs, 2 * kD, a->backward));
+  if (a->loss_kind != FNB_LOSS_MSE && a->loss_kind != FNB_LOSS_BCE_MASKED) return FNB_ERR_MODE;
+  if (!a->loss || !a->target || !a->x_atoms || !a->x_bond || !a->x_fbond) return FNB_ERR_NULL;
+  if (a->backward && !a->layer_grads) return FNB_ERR_NULL;
+  if (reinterpret_cast<uintptr_t>(workspace) & 255u) return FNB_ERR_ALIGN;
+  FtBufs B;
+  if (ft_layout(a, (char *)workspace, &B) > workspace_bytes) return FNB_ERR_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream;
+  const fnb_mlp_layer *L = a->head;
+  const int n = a->n_head_layers;
+  const int64_t G = in->n_graphs, n_out = G * L[n - 1].out_dim;
+
+  // ---- collate + encoder forward
+  FnbAux aux{};
+  const bool two = fnb_aux_streams(&aux) == 0;
+  fnb_batch_plan plan{};
+  fnb_encoder_opts o = opts_of(a);
+  fnb_encoder_io eio{};
+  eio.x_atoms = a->x_atoms; eio.x_bond = a->x_bond; eio.x_fbond = a->x_fbond;
+  eio.out_atoms = B.out_atoms; eio.out_frags = B.out_frags; eio.out_bond = B.out_bond; eio.out_fbond = B.out_fbond;
+  RC(collate_and_encode(in, a->plan_arena, B.plan_arena, B.plan_bytes, &o, a->layers, &eio, B.enc_ws, B.enc_bytes,
+                        scratch, stream, aux, two, &plan));
+  // ---- readout: [G,256] = cat(sum over each molecule's atoms, sum over its fragments)
+  RC(fnb_segment_sum(plan.mol_atom_ptr, nullptr, G, B.out_atoms, B.readout, 2 * kD, nullptr, 0, 0, 0, nullptr, stream));
+  RC(fnb_segment_sum(plan.mol_frag_ptr, nullptr, G, B.out_frags, B.readout + kD, 2 * kD, nullptr, 0, 0, 0, nullptr,
+                     stream));
+  // ---- head forward; its dropout sites follow the encoder's
+  FnbMlpRun r{};
+  r.L = L; r.n = n; r.G = G; r.training = a->training; r.seed = a->seed;
+  fnb_mlp_rng(L, n, G, a->offset + fnb_encoder_rng_span(&plan, &o, a->layers), r.in_base, r.out_base);
+  r.x0 = B.readout;
+  r.xd[0] = (a->training && L[0].p_in > 0.f) ? B.xd0 : B.readout;
+  for (int l = 0; l + 1 < n; ++l) { r.xd[l + 1] = B.xd[l + 1]; r.u[l] = B.u[l]; }
+  r.out = a->predictions ? a->predictions : B.pred;
+  RC(fnb_mlp_forward(&r, s));
+  // ---- loss (and, training, the gradient of the predictions)
+  float *d_pred = a->backward ? B.dz[n - 1] : nullptr;
+  if (a->loss_kind == FNB_LOSS_MSE) {
+    fnb_mse_term t{};
+    t.pred = r.out; t.target = a->target; t.n = n_out; t.weight = 1.f; t.grad = d_pred;
+    RC(fnb_mse_sum_loss(&t, 1, a->loss, scratch, stream));
+  } else {
+    RC(fnb_bce_masked_loss(r.out, a->target, n_out, a->loss, d_pred, s));
+  }
+  if (!a->backward) return 0;
+  // ---- head backward, readout backward, encoder backward
+  for (int l = 0; l < n; ++l) r.dz[l] = B.dz[l];
+  r.dx0 = B.d_readout; r.rec = B.rec;
+  RC(fnb_mlp_backward(&r, s));
+  RC(fnb_segment_gather(B.d_readout, 2 * kD, plan.batch32, in->n_atoms, nullptr, B.g_atoms, stream));
+  RC(fnb_segment_gather(B.d_readout + kD, 2 * kD, plan.frag_batch32, in->n_frags, nullptr, B.g_frags, stream));
+  eio.g_atoms = B.g_atoms; eio.g_frags = B.g_frags; eio.g_bond = nullptr; eio.g_fbond = nullptr;
+  RC(fnb_encoder_backward(&plan, &o, a->layers, a->layer_grads, &eio, B.enc_ws, B.enc_bytes, B.enc_bws, B.enc_bws_bytes,
+                          scratch, stream));
+  return 0;
+}

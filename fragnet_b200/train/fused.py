@@ -1,4 +1,4 @@
-"""One pretraining step per library call: ``FusedPretrainStep``.
+"""One training step per library call: ``FusedPretrainStep`` (pretraining) and ``FusedFineTuneStep`` (finetuning).
 
 The reference's loop body (fragnet/train/pretrain/pretrain_utils.py:12-30) is::
 
@@ -11,6 +11,9 @@ model as ``fnb_pretrain_step`` (collate, forward, loss, backward: one call) + op
 ``fnb_adam_step`` (one launch over a flat parameter buffer).  The model's parameters stay ordinary ``nn.Parameter``
 objects with their names and shapes (``state_dict`` round-trips); those that receive gradients are re-homed as views
 into one flat buffer and their ``.grad`` are views into a second one.
+
+``FusedFineTuneStep`` does the same for a ``FragNetFineTune`` model and the finetuning loop's body
+(fragnet/train/utils.py:330-470: ``model(batch)`` -> MSE or masked BCE -> backward -> Adam) with ``fnb_finetune_step``.
 """
 from __future__ import annotations
 
@@ -26,7 +29,225 @@ from ..autograd import N_PARAMS, _F_INDEX
 from .optim import flat_views as _flat_views
 
 
-class FusedPretrainStep:
+def _on(batch, k, dev, dtype):
+    t = batch[k]
+    if t.device != dev or t.dtype != dtype or not t.is_contiguous():
+        t = t.to(device=dev, dtype=dtype).contiguous()
+    return t
+
+
+def _encoder_structs(layer_params, grad_of):
+    """``fnb_layer_params`` / ``fnb_layer_grads`` arrays of an encoder's layers (fragment block in the last one only)."""
+    n_layers = len(layer_params)
+    layers, grads = (_abi.CLayerParams * n_layers)(), (_abi.CLayerGrads * n_layers)()
+    for li, ps in enumerate(layer_params):
+        L, G = layers[li], grads[li]
+        for name, p in zip(_abi.PARAM_FIELDS, ps):
+            setattr(L, name, p.data_ptr())
+            g = grad_of.get(id(p))
+            setattr(G, name, None if g is None else g.data_ptr())
+        L.K_bond, L.K_fbond, L.K_atom = ps[0].shape[1], ps[2].shape[1], ps[8].shape[1]
+        L.run_frag_block, L.want_attention = int(li == n_layers - 1), 0
+        L.bond_mask = L.frag_bond_mask = L.atom_mask = -1
+        L.atom_mask_list, L.n_atom_mask = None, 0
+    assert len(layer_params[0]) == N_PARAMS
+    return layers, grads
+
+
+class _FlatStep:
+    """What the one-call steps share: the live parameters re-homed as views of one flat buffer (their ``.grad`` views
+    of a second one), the flat Adam update, a caller's ``torch.optim.Adam`` kept truthful, and the collate of the next
+    batch underneath the running step."""
+
+    def _bind_flat(self, live, dev, g_store=None):
+        """Re-homes ``live`` into the flat buffers; returns the gradient views."""
+        self.live = live
+        self.flat_p, p_views = _flat_views(live, dev)
+        self.flat_g, g_views = _flat_views(live, dev, storage=g_store)
+        with torch.no_grad():
+            torch._foreach_copy_(p_views, [p.data for p in live])
+            for p, v, g in zip(live, p_views, g_views):
+                p.data = v
+                p.grad = g
+        self.exp_avg = torch.zeros_like(self.flat_p)
+        self.exp_avg_sq = torch.zeros_like(self.flat_p)
+        self.t = 0
+        self._p_views = p_views
+        self._ws: Optional[torch.Tensor] = None
+        self._loss = torch.zeros(8, dtype=torch.float32, device=dev)      # ring of loss scalars
+        self._loss_i = 0
+        # collate of the next batch underneath the running step (prefetch_plan): two alternating plan arenas
+        self._plan_arenas: List[Optional[torch.Tensor]] = [None, None]
+        self._step_parity: Optional[int] = None     # arena the step launched last reads, if it found its plan prefetched
+        self._prefetched = None          # (key of the batch inputs, arena, tensors kept alive)
+        self.plan_hits = 0               # steps that found their plan prefetched
+        return g_views
+
+    def bound_to_model(self) -> bool:
+        """True while every live parameter still is its view of the flat buffer (``model.to()``, ``.cpu()`` or a
+        re-assigned ``p.data`` break the binding; the caller then has to fall back to the generic loop)."""
+        return all(p.data_ptr() == v.data_ptr() and p.device == v.device for p, v in zip(self.live, self._p_views))
+
+    def attach_optimizer(self, optimizer) -> None:
+        """Keep a caller-owned ``torch.optim.Adam`` truthful: its ``state`` entries of the live parameters become VIEWS
+        of this object's moment buffers plus a shared step counter, so ``optimizer.state_dict()`` checkpoints the real
+        state; moments already present in ``optimizer.state`` (a resumed run) are adopted first."""
+        from .optim import flat_views
+        _, m_views = flat_views(self.live, self.dev, storage=self.exp_avg)
+        _, v_views = flat_views(self.live, self.dev, storage=self.exp_avg_sq)
+        steps = [int(optimizer.state[p]["step"]) for p in self.live if p in optimizer.state and "step" in optimizer.state[p]]
+        with torch.no_grad():
+            for p, m, v in zip(self.live, m_views, v_views):
+                st = optimizer.state.get(p)
+                if st and "exp_avg" in st:
+                    m.copy_(st["exp_avg"])
+                    v.copy_(st["exp_avg_sq"])
+        if steps:
+            self.t = max(steps)
+        self._opt_step = torch.tensor(float(self.t))
+        for p, m, v in zip(self.live, m_views, v_views):
+            optimizer.state[p] = {"step": self._opt_step, "exp_avg": m, "exp_avg_sq": v}
+
+    def _adam(self) -> None:
+        """``fnb_adam_step`` over the flat buffers at step ``self.t``."""
+        _abi.check(ops._lib().fnb_adam_step(ops._p(self.flat_p), ops._p(self.flat_g), ops._p(self.exp_avg),
+                                            ops._p(self.exp_avg_sq), self.flat_p.numel(), self.lr, self.betas[0],
+                                            self.betas[1], self.eps, self.weight_decay, self.t, ops._stream()), "adam_step")
+        if getattr(self, "_opt_step", None) is not None:
+            self._opt_step.fill_(float(self.t))
+
+    def _next_loss(self) -> torch.Tensor:
+        self._loss_i = (self._loss_i + 1) % self._loss.numel()
+        return self._loss[self._loss_i]
+
+    def _batch_inputs(self, batch, g: int):
+        """``fnb_batch_inputs`` of a batch dict with ``g`` molecules, the tensors it points into, and the raw features."""
+        dev = self.dev
+        idx = lambda k: _on(batch, k, dev, torch.int64)
+        f32 = lambda k: _on(batch, k, dev, torch.float32)
+        ei, fi, a2f = idx("edge_index"), idx("frag_index"), idx("atom_to_frag_ids")
+        eb, efb = idx("edge_index_bonds_graph"), idx("edge_index_fbonds")
+        bv, fbv = idx("batch"), idx("frag_batch")
+        cos, a6 = f32("edge_attr_bonds"), f32("edge_attr_fbonds")
+        xa, xb, xfb = f32("x_atoms"), f32("node_features_bonds"), f32("node_features_fbonds")
+        na, nf, nb, nfb = xa.shape[0], batch["x_frags"].shape[0], xb.shape[0], xfb.shape[0]
+        if ei.shape[1] != nb or fi.shape[1] != nfb:
+            raise ValueError("fragnet_b200: the bond graph needs one node per column of edge_index and the "
+                             "fragment-connection graph one node per column of frag_index")
+        pt = ops._ptr
+        inp = _abi.CBatchInputs(pt(ei), pt(fi), pt(a2f), pt(eb), pt(efb), pt(bv), pt(fbv), pt(cos), pt(a6),
+                                na, nf, nb, eb.shape[1], nfb, efb.shape[1], g)
+        return inp, (ei, fi, a2f, eb, efb, bv, fbv, cos, a6, xa, xb, xfb), (xa, xb, xfb)
+
+    def _take_prefetched(self, inp) -> Optional[int]:
+        """Arena address of the plan ``prefetch_plan`` built for exactly these batch inputs, or None."""
+        pre, self._prefetched = self._prefetched, None       # one prefetch serves one step
+        self._step_parity = None
+        if pre is not None and pre[0] == self._plan_key(inp):
+            self._step_parity = pre[3]             # this arena is now in use until the step has run
+            self.plan_hits += 1
+            return pre[1].data_ptr()
+        return None
+
+    # ---- collate of the next batch underneath the running step -------------------------------------------------------
+    _PLAN_TENSORS = ("edge_index", "frag_index", "atom_to_frag_ids", "edge_index_bonds_graph", "edge_index_fbonds",
+                     "batch", "frag_batch")
+
+    @staticmethod
+    def _plan_key(inp: "_abi.CBatchInputs"):
+        return tuple(getattr(inp, n) for n, _ in _abi.CBatchInputs._fields_)
+
+    def prefetch_plan(self, next_batch, ready_event: Optional["torch.cuda.Event"] = None) -> bool:
+        """Queue the on-device collate (``fnb_batch_plan_build``) of the batch the NEXT ``step`` call will get, on a
+        library stream underneath the step that is running -- the plan depends on nothing but the batch's index tensors,
+        and without it the first attention kernel of a step waits ~50 us for nine small launches that compete with the
+        layer-0 GEMMs for SMs.  ``ready_event``: recorded once the tensors of ``next_batch`` are complete (a
+        ``DevicePrefetcher`` slot still being copied); None if they already are.  Only batches that need no dtype /
+        device conversion qualify (returns False otherwise: the step then collates by itself, as always).  The tensors
+        must not be modified until that step has been launched."""
+        self._prefetched = None
+        dev = self.dev
+        for k in self._PLAN_TENSORS:
+            t = next_batch.get(k)
+            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.int64 or not t.is_contiguous():
+                return False
+        for k in ("edge_attr_bonds", "edge_attr_fbonds"):
+            t = next_batch.get(k)
+            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.float32 or not t.is_contiguous():
+                return False
+        b = next_batch
+        na, nf = b["x_atoms"].shape[0], b["x_frags"].shape[0]
+        nb, nfb, g = b["edge_index"].shape[1], b["frag_index"].shape[1], b["y"].numel() // self._y_width
+        pt = ops._ptr
+        inp = _abi.CBatchInputs(pt(b["edge_index"]), pt(b["frag_index"]), pt(b["atom_to_frag_ids"]),
+                                pt(b["edge_index_bonds_graph"]), pt(b["edge_index_fbonds"]), pt(b["batch"]),
+                                pt(b["frag_batch"]), pt(b["edge_attr_bonds"]), pt(b["edge_attr_fbonds"]),
+                                na, nf, nb, b["edge_index_bonds_graph"].shape[1], nfb, b["edge_index_fbonds"].shape[1], g)
+        lib = ops._lib()
+        need = lib.fnb_batch_plan_bytes(C.byref(inp))
+        if need == 0:
+            return False
+        # never the arena the step launched last reads (its backward still needs the plan); a second prefetch before the
+        # next step simply replaces the first
+        parity = 0 if self._step_parity is None else 1 - self._step_parity
+        arena = self._plan_arenas[parity]
+        if arena is None or arena.numel() < need:
+            # (re)allocation: the block may have been freed by work still running on the compute stream, and the collate
+            # writes it from another stream -- rare (first steps, a larger batch), so simply wait
+            torch.cuda.current_stream(dev).synchronize()
+            arena = torch.empty(int(need * 1.25) + 256, dtype=torch.uint8, device=dev)
+            self._plan_arenas[parity] = arena
+        ev = C.c_void_p(ready_event.cuda_event) if ready_event is not None else None
+        rc = lib.fnb_pretrain_plan_prefetch(C.byref(inp), ops._ptr(arena), arena.numel(), ev)
+        if rc != 0:
+            return False                 # single-stream mode: the step collates by itself
+        keep = tuple(b[k] for k in self._PLAN_TENSORS) + (b["edge_attr_bonds"], b["edge_attr_fbonds"])
+        self._prefetched = (self._plan_key(inp), arena, keep, parity)
+        return True
+
+    # ---- the step: what the subclass's _args / _NATIVE describe --------------------------------------------------------
+    _y_width = 1          # entries of batch["y"] per molecule
+
+    def _run(self, batch, backward: bool, want_preds: bool = False):
+        lib = ops._lib()
+        a, loss, preds, keep = self._args(batch, backward, want_preds)
+        if self._draws(a):
+            a.offset = ops.reserve_rng(getattr(lib, f"fnb_{self._NATIVE}_rng_span")(C.byref(a)))
+        need = getattr(lib, f"fnb_{self._NATIVE}_workspace_bytes")(C.byref(a))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(int(need * 1.25) + 256, dtype=torch.uint8, device=self.dev)
+        _abi.check(getattr(lib, f"fnb_{self._NATIVE}")(C.byref(a), ops._ptr(self._ws), self._ws.numel(),
+                                                       ops._ptr(ops.scratch(self.dev)), ops._stream()), self._NATIVE)
+        del keep        # stream-ordered allocator: safe to release once the launches are queued on this stream
+        return loss, preds
+
+    def step(self, batch, next_batch=None, next_ready=None) -> torch.Tensor:
+        """collate + forward + loss + backward (+ all-reduce) + Adam on one batch dict; returns the loss.
+        ``next_batch`` (optional): the batch of the following call, whose collate is then queued underneath this step
+        (``prefetch_plan``); ``next_ready``: the CUDA event after which its tensors are complete, if they are not yet."""
+        loss = self._step(batch)
+        if next_batch is not None:
+            self.prefetch_plan(next_batch, next_ready)
+        return loss
+
+    def _step(self, batch) -> torch.Tensor:
+        loss, _ = self._run(batch, backward=True)
+        self.t += 1
+        self._adam()
+        return loss
+
+    def forward_backward(self, batch) -> torch.Tensor:
+        """Gradients only (``p.grad`` of the live parameters are views of ``flat_g``), no parameter update."""
+        return self._run(batch, backward=True)[0]
+
+    @torch.no_grad()
+    def evaluate(self, batch, return_predictions: bool = False):
+        """Forward + loss without gradients (validation)."""
+        loss, preds = self._run(batch, backward=False, want_preds=return_predictions)
+        return (loss, preds) if return_predictions else loss
+
+
+class FusedPretrainStep(_FlatStep):
     """``step(batch) -> loss`` (0-dim CUDA tensor) for a ``FragNetPreTrain`` model; Adam hyper-parameters as
     ``torch.optim.Adam``.  ``group``: a ``torch.distributed`` process group for data-parallel training (mean of the
     per-rank gradients, the DDP semantics of finetune_gat2_pl.py:230); ``None`` uses the default group if one is
@@ -52,39 +273,16 @@ class FusedPretrainStep:
         live += head_params[8:]                       # ba, da, FC stacks (the bond-length head is never trained)
         if any(p.dtype != torch.float32 or p.device != dev for p in live):
             raise ValueError("FusedPretrainStep needs fp32 parameters on one CUDA device")
-        self.live = live
-        self.flat_p, p_views = _flat_views(live, dev)
         self._peers = None
-        g_store = self._symmetric_gradient_buffer(live, dev, group)
-        self.flat_g, g_views = _flat_views(live, dev, storage=g_store)
-        with torch.no_grad():
-            torch._foreach_copy_(p_views, [p.data for p in live])
-            for p, v, g in zip(live, p_views, g_views):
-                p.data = v
-                p.grad = g
-        self.exp_avg = torch.zeros_like(self.flat_p)
-        self.exp_avg_sq = torch.zeros_like(self.flat_p)
-        self.t = 0
-        self._p_views = p_views
+        g_views = self._bind_flat(live, dev, self._symmetric_gradient_buffer(live, dev, group))
+        p_views = self._p_views
         if self.world_size > 1:
             # DDP / Fabric broadcast rank 0's parameters at wrap time (finetune_gat2_pl.py:230): differently seeded
             # ranks, or a checkpoint loaded on one rank only, must not diverge silently
             dist.broadcast(self.flat_p, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
         grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
         # ---- C structs (built once: parameter storage never moves afterwards)
-        self._layers = (_abi.CLayerParams * n_layers)()
-        self._layer_grads = (_abi.CLayerGrads * n_layers)()
-        for li, ps in enumerate(layer_params):
-            L, G = self._layers[li], self._layer_grads[li]
-            for name, p in zip(_abi.PARAM_FIELDS, ps):
-                setattr(L, name, p.data_ptr())
-                g = grad_of.get(id(p))
-                setattr(G, name, None if g is None else g.data_ptr())
-            L.K_bond, L.K_fbond, L.K_atom = ps[0].shape[1], ps[2].shape[1], ps[8].shape[1]
-            L.run_frag_block, L.want_attention = int(li == n_layers - 1), 0
-            L.bond_mask = L.frag_bond_mask = L.atom_mask = -1
-            L.atom_mask_list, L.n_atom_mask = None, 0
-        assert len(layer_params[0]) == N_PARAMS
+        self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of)
         self._heads, self._head_grads = _abi.CPretrainHeadParams(), _abi.CPretrainHeadParams()
         self._heads.Wr, self._heads.br = head_params[0].data_ptr(), head_params[1].data_ptr()
         for gi, group_name in enumerate(("bl", "ba", "da", "fc")):
@@ -94,15 +292,7 @@ class FusedPretrainStep:
                 g = grad_of.get(id(p))
                 setattr(getattr(self._head_grads, group_name), fname, None if g is None else g.data_ptr())
         self._keep = (layer_params, head_params, p_views, g_views)
-        self._ws: Optional[torch.Tensor] = None
-        self._loss = torch.zeros(8, dtype=torch.float32, device=dev)      # ring of loss scalars
-        self._loss_i = 0
         self.n_layers = n_layers
-        # collate of the next batch underneath the running step (prefetch_plan): two alternating plan arenas
-        self._plan_arenas: List[Optional[torch.Tensor]] = [None, None]
-        self._step_parity: Optional[int] = None     # arena the step launched last reads, if it found its plan prefetched
-        self._prefetched = None          # (key of the batch inputs, arena, tensors kept alive)
-        self.plan_hits = 0               # steps that found their plan prefetched
 
     # ------------------------------------------------------------------------------------------
     def _symmetric_gradient_buffer(self, live, dev, group):
@@ -144,66 +334,22 @@ class FusedPretrainStep:
         self._symm_keep = (hg, hf)
         return g
 
-    def bound_to_model(self) -> bool:
-        """True while every live parameter still is its view of the flat buffer (``model.to()``, ``.cpu()`` or a
-        re-assigned ``p.data`` break the binding; the caller then has to fall back to the generic loop)."""
-        return all(p.data_ptr() == v.data_ptr() and p.device == v.device for p, v in zip(self.live, self._p_views))
-
-    def attach_optimizer(self, optimizer) -> None:
-        """Keep a caller-owned ``torch.optim.Adam`` truthful: its ``state`` entries of the live parameters become VIEWS
-        of this object's moment buffers plus a shared step counter, so ``optimizer.state_dict()`` checkpoints the real
-        state; moments already present in ``optimizer.state`` (a resumed run) are adopted first."""
-        from .optim import flat_views
-        _, m_views = flat_views(self.live, self.dev, storage=self.exp_avg)
-        _, v_views = flat_views(self.live, self.dev, storage=self.exp_avg_sq)
-        steps = [int(optimizer.state[p]["step"]) for p in self.live if p in optimizer.state and "step" in optimizer.state[p]]
-        with torch.no_grad():
-            for p, m, v in zip(self.live, m_views, v_views):
-                st = optimizer.state.get(p)
-                if st and "exp_avg" in st:
-                    m.copy_(st["exp_avg"])
-                    v.copy_(st["exp_avg_sq"])
-        if steps:
-            self.t = max(steps)
-        self._opt_step = torch.tensor(float(self.t))
-        for p, m, v in zip(self.live, m_views, v_views):
-            optimizer.state[p] = {"step": self._opt_step, "exp_avg": m, "exp_avg_sq": v}
-
     @property
     def world_size(self) -> int:
         return dist.get_world_size(self.group) if dist.is_available() and dist.is_initialized() else 1
 
     def _args(self, batch, backward: bool, want_preds: bool):
         dev = self.dev
-
-        def idx(k):
-            t = batch[k]
-            if t.device != dev or t.dtype != torch.int64 or not t.is_contiguous():
-                t = t.to(device=dev, dtype=torch.int64).contiguous()
-            return t
-
-        def f32(k):
-            t = batch[k]
-            if t.device != dev or t.dtype != torch.float32 or not t.is_contiguous():
-                t = t.to(device=dev, dtype=torch.float32).contiguous()
-            return t
-
-        ei, fi, a2f = idx("edge_index"), idx("frag_index"), idx("atom_to_frag_ids")
-        eb, efb = idx("edge_index_bonds_graph"), idx("edge_index_fbonds")
-        bv, fbv = idx("batch"), idx("frag_batch")
-        cos, a6 = f32("edge_attr_bonds"), f32("edge_attr_fbonds")
-        xa, xb, xfb = f32("x_atoms"), f32("node_features_bonds"), f32("node_features_fbonds")
+        f32 = lambda k: _on(batch, k, dev, torch.float32)
         t_ba, t_dh, y = f32("bnd_angl"), f32("dh_angl"), f32("y")
-        na, nf, nb, nfb, g = xa.shape[0], batch["x_frags"].shape[0], xb.shape[0], xfb.shape[0], y.numel()
-        if ei.shape[1] != nb or fi.shape[1] != nfb:
-            raise ValueError("fragnet_b200: the bond graph needs one node per column of edge_index and the "
-                             "fragment-connection graph one node per column of frag_index")
+        g = y.numel()
+        inp, tensors, (xa, xb, xfb) = self._batch_inputs(batch, g)
+        na, nb = inp.n_atoms, inp.n_bonds
         if t_ba.numel() != na or t_dh.numel() != nb:
             raise ValueError("fragnet_b200: bnd_angl / dh_angl must have one entry per atom / directed bond")
         pt = ops._ptr
         a = _abi.CPretrainStepArgs()
-        a.batch = _abi.CBatchInputs(pt(ei), pt(fi), pt(a2f), pt(eb), pt(efb), pt(bv), pt(fbv), pt(cos), pt(a6),
-                                    na, nf, nb, eb.shape[1], nfb, efb.shape[1], g)
+        a.batch = inp
         a.x_atoms, a.x_bond, a.x_fbond = pt(xa), pt(xb), pt(xfb)
         a.t_bond_angle, a.t_dihedral, a.t_energy = pt(t_ba), pt(t_dh), pt(y)
         a.n_layers = self.n_layers
@@ -216,100 +362,22 @@ class FusedPretrainStep:
         a.drop_p, a.training = float(enc.dropout.p), int(training)
         a.seed, a.offset = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF, 0
         a.precision, a.backward = config.precision_id(), int(backward)
-        self._loss_i = (self._loss_i + 1) % self._loss.numel()
-        loss = self._loss[self._loss_i]
+        loss = self._next_loss()
         a.loss = loss.data_ptr()
         preds = None
         if want_preds:
             new = lambda n: torch.empty((n, 1), dtype=torch.float32, device=dev)
             preds = (new(nb), new(na), new(nb), new(g))
             a.bond_length, a.bond_angle, a.dihedral, a.energy = (pt(t) for t in preds)
-        keep = (ei, fi, a2f, eb, efb, bv, fbv, cos, a6, xa, xb, xfb, t_ba, t_dh, y)
-        pre, self._prefetched = self._prefetched, None       # one prefetch serves one step
-        self._step_parity = None
-        if pre is not None and pre[0] == self._plan_key(a.batch):
-            a.plan_arena = pre[1].data_ptr()       # collated ahead of this step (see prefetch_plan)
-            self._step_parity = pre[3]             # ... and this arena is now in use until the step has run
-            self.plan_hits += 1
+        keep = tensors + (t_ba, t_dh, y)
+        a.plan_arena = self._take_prefetched(a.batch)       # collated ahead of this step (see prefetch_plan)
         return a, loss, preds, keep
 
-    # ---- collate of the next batch underneath the running step -------------------------------------------------------
-    _PLAN_TENSORS = ("edge_index", "frag_index", "atom_to_frag_ids", "edge_index_bonds_graph", "edge_index_fbonds",
-                     "batch", "frag_batch")
+    _NATIVE = "pretrain_step"
 
     @staticmethod
-    def _plan_key(inp: "_abi.CBatchInputs"):
-        return tuple(getattr(inp, n) for n, _ in _abi.CBatchInputs._fields_)
-
-    def prefetch_plan(self, next_batch, ready_event: Optional["torch.cuda.Event"] = None) -> bool:
-        """Queue the on-device collate (``fnb_batch_plan_build``) of the batch the NEXT ``step`` call will get, on a
-        library stream underneath the step that is running -- the plan depends on nothing but the batch's index tensors,
-        and without it the first attention kernel of a step waits ~50 us for nine small launches that compete with the
-        layer-0 GEMMs for SMs.  ``ready_event``: recorded once the tensors of ``next_batch`` are complete (a
-        ``DevicePrefetcher`` slot still being copied); None if they already are.  Only batches that need no dtype /
-        device conversion qualify (returns False otherwise: the step then collates by itself, as always).  The tensors
-        must not be modified until that step has been launched."""
-        self._prefetched = None
-        dev = self.dev
-        for k in self._PLAN_TENSORS:
-            t = next_batch.get(k)
-            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.int64 or not t.is_contiguous():
-                return False
-        for k in ("edge_attr_bonds", "edge_attr_fbonds"):
-            t = next_batch.get(k)
-            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.float32 or not t.is_contiguous():
-                return False
-        b = next_batch
-        na, nf = b["x_atoms"].shape[0], b["x_frags"].shape[0]
-        nb, nfb, g = b["edge_index"].shape[1], b["frag_index"].shape[1], b["y"].numel()
-        pt = ops._ptr
-        inp = _abi.CBatchInputs(pt(b["edge_index"]), pt(b["frag_index"]), pt(b["atom_to_frag_ids"]),
-                                pt(b["edge_index_bonds_graph"]), pt(b["edge_index_fbonds"]), pt(b["batch"]),
-                                pt(b["frag_batch"]), pt(b["edge_attr_bonds"]), pt(b["edge_attr_fbonds"]),
-                                na, nf, nb, b["edge_index_bonds_graph"].shape[1], nfb, b["edge_index_fbonds"].shape[1], g)
-        lib = ops._lib()
-        need = lib.fnb_batch_plan_bytes(C.byref(inp))
-        if need == 0:
-            return False
-        # never the arena the step launched last reads (its backward still needs the plan); a second prefetch before the
-        # next step simply replaces the first
-        parity = 0 if self._step_parity is None else 1 - self._step_parity
-        arena = self._plan_arenas[parity]
-        if arena is None or arena.numel() < need:
-            # (re)allocation: the block may have been freed by work still running on the compute stream, and the collate
-            # writes it from another stream -- rare (first steps, a larger batch), so simply wait
-            torch.cuda.current_stream(dev).synchronize()
-            arena = torch.empty(int(need * 1.25) + 256, dtype=torch.uint8, device=dev)
-            self._plan_arenas[parity] = arena
-        ev = C.c_void_p(ready_event.cuda_event) if ready_event is not None else None
-        rc = lib.fnb_pretrain_plan_prefetch(C.byref(inp), ops._ptr(arena), arena.numel(), ev)
-        if rc != 0:
-            return False                 # single-stream mode: the step collates by itself
-        keep = tuple(b[k] for k in self._PLAN_TENSORS) + (b["edge_attr_bonds"], b["edge_attr_fbonds"])
-        self._prefetched = (self._plan_key(inp), arena, keep, parity)
-        return True
-
-    def _run(self, batch, backward: bool, want_preds: bool = False):
-        lib = ops._lib()
-        a, loss, preds, keep = self._args(batch, backward, want_preds)
-        if a.training and a.drop_p > 0:
-            a.offset = ops.reserve_rng(lib.fnb_pretrain_step_rng_span(C.byref(a)))
-        need = lib.fnb_pretrain_step_workspace_bytes(C.byref(a))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty(int(need * 1.25) + 256, dtype=torch.uint8, device=self.dev)
-        _abi.check(lib.fnb_pretrain_step(C.byref(a), ops._ptr(self._ws), self._ws.numel(), ops._ptr(ops.scratch(self.dev)),
-                                         ops._stream()), "pretrain_step")
-        del keep        # stream-ordered allocator: safe to release once the launches are queued on this stream
-        return loss, preds
-
-    def step(self, batch, next_batch=None, next_ready=None) -> torch.Tensor:
-        """collate + forward + loss + backward (+ all-reduce) + Adam on one batch dict; returns the loss.
-        ``next_batch`` (optional): the batch of the following call, whose collate is then queued underneath this step
-        (``prefetch_plan``); ``next_ready``: the CUDA event after which its tensors are complete, if they are not yet."""
-        loss = self._step(batch)
-        if next_batch is not None:
-            self.prefetch_plan(next_batch, next_ready)
-        return loss
+    def _draws(a) -> bool:
+        return bool(a.training and a.drop_p > 0)
 
     def _step(self, batch) -> torch.Tensor:
         loss, _ = self._run(batch, backward=True)
@@ -328,22 +396,130 @@ class FusedPretrainStep:
         if w > 1:
             dist.all_reduce(self.flat_g, op=dist.ReduceOp.SUM, group=self.group)
             self.flat_g.mul_(1.0 / w)
-        _abi.check(ops._lib().fnb_adam_step(ops._p(self.flat_p), ops._p(self.flat_g), ops._p(self.exp_avg),
-                                            ops._p(self.exp_avg_sq), self.flat_p.numel(), self.lr, self.betas[0],
-                                            self.betas[1], self.eps, self.weight_decay, self.t, ops._stream()), "adam_step")
-        if getattr(self, "_opt_step", None) is not None:
-            self._opt_step.fill_(float(self.t))
+        self._adam()
         return loss
 
-    def forward_backward(self, batch) -> torch.Tensor:
-        """Gradients only (``p.grad`` of the live parameters are views of ``flat_g``), no parameter update."""
-        return self._run(batch, backward=True)[0]
 
-    @torch.no_grad()
-    def evaluate(self, batch, return_predictions: bool = False):
-        """Forward + loss without gradients (Trainer.validate, pretrain_utils.py:33-57)."""
-        loss, preds = self._run(batch, backward=False, want_preds=return_predictions)
-        return (loss, preds) if return_predictions else loss
+def _act_id(module) -> Optional[int]:
+    """The library's activation code of an FTHead activation module, or None if it has none."""
+    import torch.nn as nn
+    exact = {nn.ReLU: _abi.ACT_RELU, nn.SiLU: _abi.ACT_SILU, nn.SELU: _abi.ACT_SELU, nn.ReLU6: _abi.ACT_RELU6}
+    if type(module) in exact:
+        return exact[type(module)]
+    if type(module) is nn.CELU and module.alpha == 1.0:
+        return _abi.ACT_CELU
+    if type(module) is nn.GELU and module.approximate == "none":
+        return _abi.ACT_GELU
+    if type(module) is nn.LeakyReLU and module.negative_slope == 0.01:
+        return _abi.ACT_LEAKYRELU
+    return None
+
+
+def _head_layers(head):
+    """(linears, p_in, p_out, act) per layer of an FTHead1-4, the arrangement of gat2.py:569-751."""
+    from ..model.gat import gat2
+    kind = type(head)
+    if kind in (gat2.FTHead3, gat2.FTHead2):
+        # act(dropout(linear(x))) per hidden layer, bare last linear; FTHead2: ReLU, its own p = 0.1 (gat2.py:745-751)
+        act = _abi.ACT_RELU if kind is gat2.FTHead2 else _act_id(getattr(head, "activation", None))
+        lins = list(head.predictor)
+        p = float(head.dropout.p)
+        return [(lin, 0.0, p if i + 1 < len(lins) else 0.0, act if i + 1 < len(lins) else _abi.ACT_NONE)
+                for i, lin in enumerate(lins)]
+    if kind in (gat2.FTHead1, gat2.FTHead4):
+        # out(dropout(act(linear(dropout(x))))) (gat2.py:580-588, :669-675)
+        first, last = (head.lin1, head.out) if kind is gat2.FTHead1 else (head.dense, head.out_proj)
+        act = _abi.ACT_RELU if kind is gat2.FTHead1 else _act_id(getattr(head, "activation", None))
+        p = float(head.dropout.p)
+        return [(first, p, 0.0, act), (last, p, 0.0, _abi.ACT_NONE)]
+    return None
+
+
+class FusedFineTuneStep(_FlatStep):
+    """``step(batch) -> loss`` (0-dim CUDA tensor) for this package's gat2 ``FragNetFineTune`` with an FTHead1-4 head:
+    collate, encoder, readout, head, loss and every gradient in one ``fnb_finetune_step`` call, then Adam over the flat
+    buffers (hyper-parameters as ``torch.optim.Adam``).  ``loss``: ``"mse"`` (``nn.MSELoss`` over the flattened
+    predictions, ``TrainerFineTune.train_regr``) or ``"bce"`` (BCE-with-logits over the labels > -0.5,
+    ``TrainerFineTune.train_clsf_bce``).  Models the library does not cover raise ``NotImplementedError``: other heads
+    or activations (PReLU and RReLU among them), the lite / edge variants, other encoder geometries, several ranks."""
+
+    _NATIVE = "finetune_step"
+
+    def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.0,
+                 loss: str = "mse"):
+        from ..model.gat import gat2
+        if type(model) is not gat2.FragNetFineTune:
+            raise NotImplementedError("FusedFineTuneStep needs fragnet_b200's gat2 FragNetFineTune "
+                                      f"(got {type(model).__module__}.{type(model).__name__})")
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise NotImplementedError("FusedFineTuneStep runs on one GPU")
+        if loss not in ("mse", "bce"):
+            raise ValueError(f"FusedFineTuneStep: loss must be 'mse' or 'bce', got {loss!r}")
+        enc = model.pretrain
+        spec = _head_layers(getattr(model, "fthead", None))
+        if spec is None or any(act is None for _, _, _, act in spec):
+            raise NotImplementedError("FusedFineTuneStep needs an FTHead1-4 head with a relu, celu, silu, gelu, selu, "
+                                      "relu6 or leakyrelu activation")
+        if len(spec) > _abi.MLP_MAX_LAYERS or spec[0][0].in_features != 2 * ops.D:
+            raise NotImplementedError("FusedFineTuneStep: unsupported head shape")
+        for layer in enc.layers:
+            layer._check_geometry()
+        self.model, self.loss_kind = model, loss
+        self.lr, self.betas, self.eps, self.weight_decay = float(lr), betas, float(eps), float(weight_decay)
+        self.dev = dev = ops.require_cuda(enc.layers[0].a.device)
+        n_layers = len(enc.layers)
+        layer_params = [list(layer._live_parameters()) for layer in enc.layers]
+        live: List[torch.nn.Parameter] = []
+        for li, ps in enumerate(layer_params):
+            live += [p for j, p in enumerate(ps) if j != _F_INDEX or li == n_layers - 1]
+        for lin, _, _, _ in spec:
+            live += [lin.weight, lin.bias]
+        if any(p.dtype != torch.float32 or p.device != dev for p in live):
+            raise ValueError("FusedFineTuneStep needs fp32 parameters on one CUDA device")
+        g_views = self._bind_flat(live, dev)
+        grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
+        self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of)
+        self._head = (_abi.CMlpLayer * len(spec))()
+        for h, (lin, p_in, p_out, act) in zip(self._head, spec):
+            h.W, h.b = lin.weight.data_ptr(), lin.bias.data_ptr()
+            h.dW, h.db = grad_of[id(lin.weight)].data_ptr(), grad_of[id(lin.bias)].data_ptr()
+            h.in_dim, h.out_dim, h.p_in, h.p_out, h.act = lin.in_features, lin.out_features, p_in, p_out, act
+        self.n_classes = self._y_width = spec[-1][0].out_features
+        self._head_drops = any(p_in > 0 or p_out > 0 for _, p_in, p_out, _ in spec)
+        self._keep = (layer_params, self._p_views, g_views)
+        self.n_layers = n_layers
+
+    def _draws(self, a) -> bool:
+        return bool(a.training and (a.drop_p > 0 or self._head_drops))
+
+    def _args(self, batch, backward: bool, want_preds: bool):
+        dev = self.dev
+        y = _on(batch, "y", dev, torch.float32)
+        if y.numel() % self.n_classes:
+            raise ValueError(f"fragnet_b200: batch['y'] has {y.numel()} entries, not a multiple of the head's "
+                             f"{self.n_classes} outputs")
+        g = y.numel() // self.n_classes
+        inp, tensors, (xa, xb, xfb) = self._batch_inputs(batch, g)
+        pt = ops._ptr
+        a = _abi.CFinetuneStepArgs()
+        a.batch = inp
+        a.x_atoms, a.x_bond, a.x_fbond, a.target = pt(xa), pt(xb), pt(xfb), pt(y)
+        a.n_layers = self.n_layers
+        a.layers = C.cast(self._layers, C.c_void_p)
+        a.layer_grads = C.cast(self._layer_grads, C.c_void_p)
+        a.n_head_layers, a.head = len(self._head), C.cast(self._head, C.c_void_p)
+        a.loss_kind = _abi.LOSS_MSE if self.loss_kind == "mse" else _abi.LOSS_BCE_MASKED
+        a.drop_p, a.training = float(self.model.pretrain.dropout.p), int(bool(self.model.training))
+        a.seed, a.offset = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF, 0
+        a.precision, a.backward = config.precision_id(), int(backward)
+        loss = self._next_loss()
+        a.loss = loss.data_ptr()
+        preds = None
+        if want_preds:
+            preds = torch.empty((g, self.n_classes), dtype=torch.float32, device=dev)
+            a.predictions = pt(preds)
+        a.plan_arena = self._take_prefetched(a.batch)
+        return a, loss, preds, tensors + (y,)
 
 
 class LaggedScalars:

@@ -7,6 +7,11 @@ Same signatures, same returned quantities (epoch loss = sum of the per-batch los
 staged by ``DevicePrefetcher`` (pinned, double-buffered copies on a side stream, only the tensors the model reads)
 instead of 16 blocking ``batch[k].to(device)`` calls per step (utils.py:335-336), and the per-batch losses are summed
 on the device and read back once per epoch instead of one ``loss.item()`` synchronisation per step (utils.py:344).
+
+``TrainerFineTune(..., fused=True)`` runs each training batch of this package's ``FragNetFineTune`` as one library call
+(``FusedFineTuneStep``: collate, encoder, readout, head, loss, backward, then Adam over flat buffers) when the
+optimizer is a plain ``torch.optim.Adam`` and the model is one the library covers; anything else silently takes the
+generic loop below.  Validation and test always call ``model(batch)``.
 """
 from __future__ import annotations
 
@@ -81,9 +86,11 @@ test_fn.__test__ = False      # not a pytest test
 class TrainerFineTune:
     """utils.py:307-520 for ``target_type`` ``regr`` (MSE) and ``clsf`` (masked BCE, ROC-AUC validation)."""
 
-    def __init__(self, target_pos=None, target_type="regr", n_multi_task_heads=0):
+    def __init__(self, target_pos=None, target_type="regr", n_multi_task_heads=0, fused: bool = False):
         self.target_pos = target_pos
         self.n_multi_task_heads = n_multi_task_heads
+        self.fused = fused
+        self._fused_steps = []       # [(weakref(model), weakref(optimizer), FusedFineTuneStep | None)]
         if target_type == "regr":
             self.train, self.validate, self.test = self.train_regr, self.validate_regr, self.test_regr
             self.loss_fn = nn.MSELoss()
@@ -106,10 +113,62 @@ class TrainerFineTune:
             total += loss.detach().double()
         return float(total) / len(loader.dataset)
 
+    # ---- fused path (fused=True): one library call per training batch
+    def _fused_for(self, model, optimizer, device, loss):
+        """The ``FusedFineTuneStep`` bound to (model, optimizer), or None when the fused path does not apply."""
+        if not self.fused or torch.device(device).type != "cuda" or optimizer is None:
+            return None
+        from .pretrain_utils import _plain_adam
+        if loss == "mse":
+            ok = type(self.loss_fn) is nn.MSELoss and self.loss_fn.reduction == "mean"
+        else:
+            ok = type(self.loss_fn) is nn.BCEWithLogitsLoss and self.loss_fn.reduction == "none" and \
+                self.loss_fn.weight is None and self.loss_fn.pos_weight is None
+        p0 = next(model.parameters(), None)
+        if not (ok and _plain_adam(optimizer) and torch.is_tensor(p0) and p0.is_cuda):
+            return None
+        import weakref
+        self._fused_steps = [e for e in self._fused_steps if e[0]() is not None and e[1]() is not None]
+        for wm, wo, fs in self._fused_steps:
+            if wm() is model and wo() is optimizer:
+                return fs if fs is not None and fs.bound_to_model() else None
+        from .fused import FusedFineTuneStep
+        g = optimizer.param_groups[0]
+        try:
+            fs = FusedFineTuneStep(model, lr=g["lr"], betas=g["betas"], eps=g["eps"], weight_decay=g["weight_decay"],
+                                   loss=loss)
+            fs.attach_optimizer(optimizer)          # optimizer.state_dict() keeps checkpointing the real moments
+        except NotImplementedError:
+            fs = None
+        self._fused_steps.append((weakref.ref(model), weakref.ref(optimizer), fs))
+        return fs
+
+    @staticmethod
+    def _fused_epoch(fs, loader, device, optimizer):
+        """One training epoch through ``fs``; the next batch's collate is queued underneath every step."""
+        from ..dataset.prefetch import DevicePrefetcher
+        staged = DevicePrefetcher(loader, device, depth=2, hot_path_only=True)
+        feed = iter(staged)
+        total = torch.zeros((), dtype=torch.float64, device=device)
+        batch = next(feed, None)
+        while batch is not None:
+            g = optimizer.param_groups[0]            # LR schedulers / edited hyper-parameters are honoured per step
+            fs.lr, fs.betas, fs.eps, fs.weight_decay = float(g["lr"]), g["betas"], float(g["eps"]), float(g["weight_decay"])
+            loss = fs.step(batch)
+            batch = next(feed, None)
+            if batch is not None:
+                fs.prefetch_plan(batch, staged.last_event)
+            total += loss.double()
+        return float(total) / len(loader.dataset)
+
     # ---- regression (utils.py:330-385)
     def train_regr(self, model, loader, optimizer, scheduler, device, val_loader):
         model.train()
-        mean = self._epoch(model, loader, device, lambda b: self.loss_fn(model(b).view(-1), b["y"]), optimizer)
+        fs = self._fused_for(model, optimizer, device, "mse")
+        if fs is not None:
+            mean = self._fused_epoch(fs, loader, device, optimizer)
+        else:
+            mean = self._epoch(model, loader, device, lambda b: self.loss_fn(model(b).view(-1), b["y"]), optimizer)
         if scheduler:
             self.validate(model, val_loader, device)
             scheduler.step()
@@ -132,7 +191,11 @@ class TrainerFineTune:
 
     def train_clsf_bce(self, model, loader, optimizer, scheduler, device, val_loader):
         model.train()
-        mean = self._epoch(model, loader, device, lambda b: self._bce(model(b), b["y"]), optimizer)
+        fs = self._fused_for(model, optimizer, device, "bce")
+        if fs is not None:
+            mean = self._fused_epoch(fs, loader, device, optimizer)
+        else:
+            mean = self._epoch(model, loader, device, lambda b: self._bce(model(b), b["y"]), optimizer)
         if scheduler:
             scheduler.step(self.validate(model, val_loader, device))
         return mean

@@ -36,7 +36,7 @@ extern "C" {
 
 #define FNB_D 128 /* embedding width  */
 #define FNB_H 4   /* attention heads  */
-#define FNB_ABI_VERSION 9
+#define FNB_ABI_VERSION 10
 
 /* edge-term modes of the fused attention kernels (SURVEY.md App. A.5) */
 /* arithmetic of the dense projections */
@@ -496,6 +496,64 @@ int fnb_pretrain_step(const fnb_pretrain_step_args *args, void *workspace, size_
  * result through args->plan_arena.  Returns FNB_ERR_MODE
  * when the library runs single-stream (FNB_STREAMS=1): nothing was queued, build inside the step as usual. */
 int fnb_pretrain_plan_prefetch(const fnb_batch_inputs *next, void *arena, size_t arena_bytes, void *batch_ready);
+
+/* ---- one finetuning step (finetune.cu, step.cu) -------------------------------------------------------------------
+ * The body of TrainerFineTune.train_regr / train_clsf_bce (fragnet/train/utils.py:330-385, :406-470) for a
+ * FragNetFineTune model (gat2.py:758-826) as ONE call: on-device collate, FragNet.forward, the graph readout
+ * cat(sum atoms, sum fragments), the FTHead, the loss and, with backward != 0, every parameter gradient (written, not
+ * accumulated).  The optimizer update is fnb_adam_step on the caller's flat buffers.
+ *
+ * The head is a list of linear layers, each  y = act(drop_out(drop_in(x) W^T + b)), in exact FP32 in every precision
+ * mode.  drop_in covers FTHead1 / FTHead4 (dropout in front of a linear, gat2.py:580-588, :669-675), drop_out FTHead2 /
+ * FTHead3 (dropout between a linear and its activation, :719-725, :745-751).  The last layer is a bare linear
+ * (act = FNB_ACT_NONE, p_out = 0); its out_dim is the number of classes. */
+#define FNB_ACT_NONE 0
+#define FNB_ACT_RELU 1
+#define FNB_ACT_CELU 2      /* alpha = 1 */
+#define FNB_ACT_SILU 3
+#define FNB_ACT_GELU 4      /* exact (erf) form */
+#define FNB_ACT_SELU 5
+#define FNB_ACT_RELU6 6
+#define FNB_ACT_LEAKYRELU 7 /* negative slope 0.01 */
+#define FNB_MLP_MAX_LAYERS 8
+typedef struct fnb_mlp_layer {
+  const float *W, *b;  /* nn.Linear weight [out,in] and bias [out] */
+  float *dW, *db;      /* their gradients (backward only; written) */
+  int in_dim, out_dim; /* any positive widths; in_dim of layer 0 = 2 * FNB_D (the readout), of layer l = out_dim of l-1 */
+  float p_in, p_out;   /* dropout probability on the layer's input / on its pre-activation output; 0 = none */
+  int act;             /* FNB_ACT_* */
+} fnb_mlp_layer;
+
+#define FNB_LOSS_MSE 0        /* nn.MSELoss over the flattened predictions (train_regr)                        */
+#define FNB_LOSS_BCE_MASKED 1 /* BCE-with-logits over the labels > -0.5, divided by their count (train_clsf_bce) */
+
+/* Dropout counters: the encoder's sites as fnb_encoder_rng_span lays them out from `offset`, then the head's, in layer
+ * order (a layer's input site, then its output site; a site exists where its p is non-zero), each a contiguous block
+ * of ceil(G * width / 4) counters over the row-major [G, width] tensor. */
+typedef struct fnb_finetune_step_args {
+  fnb_batch_inputs batch;                   /* as fnb_pretrain_step_args.batch; n_graphs = G molecules */
+  const float *x_atoms, *x_bond, *x_fbond;  /* [Na,K_atom] [Nb,K_bond] [Nfb,K_fbond] raw features */
+  const float *target;                      /* y: [G * n_classes] (labels < -0.5 are missing with FNB_LOSS_BCE_MASKED) */
+  int n_layers;
+  const fnb_layer_params *layers;           /* run_frag_block: 1 for the last layer only */
+  const fnb_layer_grads *layer_grads;
+  int n_head_layers;                        /* 1 .. FNB_MLP_MAX_LAYERS */
+  const fnb_mlp_layer *head;
+  int loss_kind;                            /* FNB_LOSS_* */
+  float drop_p;                             /* the encoder's dropout (the head layers carry their own) */
+  int training;
+  uint64_t seed, offset;                    /* dropout RNG key / first counter (fnb_finetune_step_rng_span) */
+  int precision;                            /* FNB_PRECISION_* of the encoder; the head is FP32 in every mode */
+  int backward;                             /* 0: forward + loss only */
+  float *loss;                              /* device scalar */
+  float *predictions;                       /* optional [G, n_classes] output */
+  const void *plan_arena;                   /* NULL, or an arena fnb_pretrain_plan_prefetch() filled for `batch` */
+} fnb_finetune_step_args;
+size_t fnb_finetune_step_workspace_bytes(const fnb_finetune_step_args *args);
+uint64_t fnb_finetune_step_rng_span(const fnb_finetune_step_args *args);
+/* workspace: 256-byte aligned, fnb_finetune_step_workspace_bytes() bytes; scratch: fnb_scratch_bytes(). */
+int fnb_finetune_step(const fnb_finetune_step_args *args, void *workspace, size_t workspace_bytes, void *scratch,
+                      void *stream);
 
 /* ---- device-side batch assembly from a packed dataset arena (arena.cu) ---------------------------
  * Replaces, for a dataset resident in device memory, collate_fn / collate_fn_pt (fragnet/dataset/data.py:877-948,
