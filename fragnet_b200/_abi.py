@@ -26,15 +26,7 @@ SIGNATURES = {
     "fnb_proj_fwd": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp]),
     "fnb_proj_bwd": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _i32, _vp, _vp]),
     "fnb_node_scalars": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _i32, _vp, _vp]),
-    "fnb_edge_coef_fwd": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _i32, _vp, _vp]),
-    "fnb_edge_coef_bwd": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
-    "fnb_gat_fwd": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _i64, _i64,
-                              _vp, _i32, _vp, _vp]),
     "fnb_attn_by_source": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp]),
-    "fnb_gat_bwd_dst": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "fnb_gat_bwd_src": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp,
-                                  _vp, _vp, _vp]),
-    "fnb_edge_table_bwd": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "fnb_segment_sum": (C.c_int, [_vp, _vp, _i64, _vp, _vp, _i64, _vp, _i32, _i32, _i32, _vp, _vp]),
     "fnb_segment_gather": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _vp]),
     "fnb_dropout_relu_fwd": (C.c_int, [_vp, _vp, _i64, _f32, _i32, _i32, _u64, _u64, _vp]),
@@ -115,7 +107,7 @@ class CWidenJob(C.Structure):
 WIDEN_U8_F32, WIDEN_I32_I64, WIDEN_MAX_JOBS = 0, 1, 16
 ARENA_COPY32, ARENA_INDEX, ARENA_FILL = 0, 1, 2
 ARENA_MAX_KINDS, ARENA_MAX_JOBS = 24, 32
-ABI_VERSION = 10
+ABI_VERSION = 11
 EDGE_NONE, EDGE_AFFINE1, EDGE_AFFINE6, EDGE_TABLE = 0, 1, 2, 3
 PRECISION_FP32, PRECISION_TF32, PRECISION_TF32X3 = 0, 1, 2
 

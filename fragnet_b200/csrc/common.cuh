@@ -18,8 +18,6 @@ constexpr float kNegSlope = 0.2f;  // nn.LeakyReLU(0.2), reference gat2.py:83
 constexpr int kNumSMs = 148;       // B200
 constexpr unsigned kFull = 0xffffffffu;
 
-// Upper bound on the number of CTAs of any kernel that emits per-CTA partial sums.
-constexpr int kMaxPartialBlocks = 148 * 8;
 // Scratch floats a caller must provide to the backward entry points (fnb_scratch_bytes): the widest
 // user is the projection weight gradient, kNumSMs CTAs x (128 x (K<=256) + 128) floats.
 constexpr int kProjBwdMaxK = 256;
@@ -28,7 +26,6 @@ constexpr int kProjBwdMaxK = 256;
 constexpr int kScratchCounters = 64;
 constexpr size_t kScratchFloats = kScratchCounters + (size_t)kNumSMs * (128 * kProjBwdMaxK + 128);
 static inline float *scratch_body(void *scratch) { return reinterpret_cast<float *>(scratch) + kScratchCounters; }
-static_assert(kScratchFloats >= 64 + (size_t)64 * 512 + (size_t)kMaxPartialBlocks * 512, "scratch must hold the edge-table partials");
 
 // Diagnostic only (bench.py's "gpu_launches"): kernels launched by this library in this process.
 extern unsigned long long g_fnb_launches;
@@ -195,7 +192,7 @@ __device__ __forceinline__ bool cta_finish(const float *s_rec, float *s_final, f
 }
 constexpr size_t finish_scratch_floats(int W, int n_ctas) { return 64 + (size_t)64 * W + (size_t)n_ctas * W; }
 
-// Up to 4 output segments of one partial record, reduced by a single launch (gat_bwd.cu).
+// Up to 4 output segments of one partial record, reduced by a single launch (reduce.cu).
 struct ReduceSegments {
   int n;
   int rec_off[4];       // float offset of the segment inside a record
@@ -208,11 +205,6 @@ struct ReduceSegments {
 };
 int fnb_launch_reduce_segments(const float *partials, int n_blocks, int pstride, ReduceSegments segs,
                                cudaStream_t stream);
-
-// Deterministic second stage for per-CTA partial sums (gat_bwd.cu):
-//   out[(j / row_len) * out_stride + j % row_len] (+)= sum_b partials[b * pstride + j],  j < width.
-int fnb_launch_reduce_partials(const float *partials, int n_blocks, int pstride, int width, float *out, int row_len,
-                               int out_stride, int accumulate, cudaStream_t stream);
 
 // Auxiliary stream of the calling thread's current device (abi.cu); returns non-zero when only the caller's stream
 // should be used.

@@ -1,4 +1,5 @@
-// Node-tiled fused GAT2 attention kernels (forward, destination-side backward, source-side backward).
+// Node-tiled fused GAT2 attention kernels (forward, destination-side backward, source-side backward) and the
+// by-source attention sums.
 //
 // Reference math (fragnet/model/gat/gat2.py:146-169 bond graph, :196-224 atom graph, :250-272 fragment-connection
 // graph, :286-316 fragment graph; SURVEY.md App. A):
@@ -854,6 +855,13 @@ inline int tile_grid(int64_t n_nodes, int npc, int ctas_per_sm) {
   return (int)tiles;
 }
 
+// The cross-CTA reductions (cta_finish) keep one record per CTA in the caller's scratch.  Largest grids: the
+// destination pass (32-float record) and the source pass (384) tile_grid(., ., <= 6), the edge-table backward (512)
+// kNumSMs * 4.
+static_assert(kScratchFloats >= finish_scratch_floats(32, kNumSMs * 6), "scratch must hold the destination-pass records");
+static_assert(kScratchFloats >= finish_scratch_floats(384, kNumSMs * 6), "scratch must hold the source-pass records");
+static_assert(kScratchFloats >= finish_scratch_floats(512, kNumSMs * 4), "scratch must hold the edge-table records");
+
 template <int MODE>
 int launch_fwd(const FwdT &a, cudaStream_t stream) {
   if (a.deep) {
@@ -876,6 +884,23 @@ inline bool deep_graph(const fnb_graph *g) {
 
 inline bool graph_ok(const fnb_graph *g) {
   return g && g->n_nodes >= 0 && g->n_edges >= 0 && g->n_nodes < INT32_MAX && g->n_edges < INT32_MAX;
+}
+
+// w[n,:] = sum of |p| over the reverse-CSR slots of source n.
+__global__ void k_attn_by_source(const int *__restrict__ rrowptr, const int *__restrict__ rslot,
+                                 const float *__restrict__ p_saved, int64_t n_nodes, float *__restrict__ w) {
+  for (int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; n < n_nodes; n += (int64_t)gridDim.x * blockDim.x) {
+    const int beg = rrowptr[n], end = rrowptr[n + 1];
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int r = beg; r < end; ++r) {
+      const float4 p = ldg4(p_saved + (int64_t)rslot[r] * 4);
+      acc.x += fabsf(p.x);
+      acc.y += fabsf(p.y);
+      acc.z += fabsf(p.z);
+      acc.w += fabsf(p.w);
+    }
+    st4(w + n * 4, acc);
+  }
 }
 
 }  // namespace
@@ -1036,6 +1061,18 @@ extern "C" int fnb_edge_table_bwd_fused(const fnb_graph *g, const float *dz, con
   if (blocks > kNumSMs * 4) blocks = kNumSMs * 4;
   if (blocks < 1) blocks = 1;
   if (cudaError_t le = fnb_launch(k_edge_table_bwd_tiled, dim3((int)blocks), dim3(T_THREADS), 0, (cudaStream_t)stream_, a)) return (int)le;
+  FNB_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fnb_attn_by_source(const int32_t *rrowptr, const int32_t *rslot, const float *p_saved, int64_t n_nodes,
+                                  float *w, void *stream) {
+  if (n_nodes < 0) return FNB_ERR_SIZE;
+  if (n_nodes == 0) return 0;
+  if (!rrowptr || !rslot || !p_saved || !w) return FNB_ERR_NULL;
+  int64_t blocks = (n_nodes + 255) / 256;
+  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
+  k_attn_by_source<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(rrowptr, rslot, p_saved, n_nodes, w);
   FNB_CHECK_LAUNCH();
   return 0;
 }

@@ -280,48 +280,6 @@ __global__ void __launch_bounds__(256) k_node_scalars(const float *__restrict__ 
   }
 }
 
-// coef[h*in + k] = sum_j We[j,k] alpha_e[h,j];  coef[4*in + h] = sum_j be[j] alpha_e[h,j]
-__global__ void k_edge_coef_fwd(const float *__restrict__ We, const float *__restrict__ be, int in_dim,
-                                const float *__restrict__ alpha, int alpha_stride, int off_e,
-                                float *__restrict__ coef) {
-  const int o = threadIdx.x;
-  if (o >= 4 * in_dim + 4) return;
-  float s = 0.f;
-  if (o < 4 * in_dim) {
-    const int hh = o / in_dim, k = o % in_dim;
-    for (int j = 0; j < kHd; ++j) s = fmaf(We[j * in_dim + k], alpha[hh * alpha_stride + off_e + j], s);
-  } else {
-    const int hh = o - 4 * in_dim;
-    for (int j = 0; j < kHd; ++j) s = fmaf(be[j], alpha[hh * alpha_stride + off_e + j], s);
-  }
-  coef[o] = s;
-}
-
-__global__ void k_edge_coef_bwd(const float *__restrict__ We, const float *__restrict__ be, int in_dim,
-                                const float *__restrict__ alpha, int alpha_stride, int off_e,
-                                const float *__restrict__ d_coef, float *__restrict__ dWe, float *__restrict__ dbe,
-                                float *__restrict__ d_alpha) {
-  const int tid = threadIdx.x;
-  const int n_w = kHd * in_dim;
-  if (tid < n_w) {  // dWe[j,k] = sum_h d_coef[h*in+k] alpha_e[h,j]
-    const int j = tid / in_dim, k = tid % in_dim;
-    float s = 0.f;
-    for (int hh = 0; hh < kH; ++hh) s = fmaf(d_coef[hh * in_dim + k], alpha[hh * alpha_stride + off_e + j], s);
-    dWe[tid] = s;
-  } else if (tid < n_w + kHd) {  // dbe[j] = sum_h d_coef[4in+h] alpha_e[h,j]
-    const int j = tid - n_w;
-    float s = 0.f;
-    for (int hh = 0; hh < kH; ++hh) s = fmaf(d_coef[4 * in_dim + hh], alpha[hh * alpha_stride + off_e + j], s);
-    dbe[j] = s;
-  } else if (tid < n_w + kHd + kH * kHd) {  // d alpha_e[h,j] = sum_k d_coef[h*in+k] We[j,k] + d_coef[4in+h] be[j]
-    const int r = tid - n_w - kHd;
-    const int hh = r / kHd, j = r % kHd;
-    float s = d_coef[4 * in_dim + hh] * be[j];
-    for (int k = 0; k < in_dim; ++k) s = fmaf(d_coef[hh * in_dim + k], We[j * in_dim + k], s);
-    d_alpha[hh * alpha_stride + off_e + j] = s;
-  }
-}
-
 // Small-M linear layer: C[M, Nc] = A[M, Kd] @ op(B) (+ bias) for a few thousand rows at most (the energy head:
 // one row per molecule, [G, 256] x [256 -> 128] forward and [G, 128] x [128 -> 256] input gradient).  k_gemm tiles 64
 // rows per CTA: 16 CTAs at G = 1024 and 45 us of pure latency on the critical path between the encoder's forward and
@@ -558,26 +516,6 @@ extern "C" int fnb_node_scalars(const float *h, int64_t n_rows, const float *alp
   int64_t blocks = (n_rows + 7) / 8;
   if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
   k_node_scalars<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(h, n_rows, alpha, alpha_stride, off_t, off_s, S);
-  FNB_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" int fnb_edge_coef_fwd(const float *We, const float *be, int in_dim, const float *alpha, int alpha_stride,
-                                 int off_e, float *coef, void *stream) {
-  if (in_dim != 1 && in_dim != 6) return FNB_ERR_MODE;
-  if (!We || !be || !alpha || !coef) return FNB_ERR_NULL;
-  k_edge_coef_fwd<<<1, 32, 0, (cudaStream_t)stream>>>(We, be, in_dim, alpha, alpha_stride, off_e, coef);
-  FNB_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" int fnb_edge_coef_bwd(const float *We, const float *be, int in_dim, const float *alpha, int alpha_stride,
-                                 int off_e, const float *d_coef, float *dWe, float *dbe, float *d_alpha,
-                                 void *stream) {
-  if (in_dim != 1 && in_dim != 6) return FNB_ERR_MODE;
-  if (!We || !be || !alpha || !d_coef || !dWe || !dbe || !d_alpha) return FNB_ERR_NULL;
-  k_edge_coef_bwd<<<1, 512, 0, (cudaStream_t)stream>>>(We, be, in_dim, alpha, alpha_stride, off_e, d_coef, dWe, dbe,
-                                                       d_alpha);
   FNB_CHECK_LAUNCH();
   return 0;
 }

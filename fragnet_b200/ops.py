@@ -366,67 +366,11 @@ def node_scalars(h, alpha, alpha_stride, off_t, off_s):
     return S
 
 
-def edge_coef_fwd(We, be, in_dim, alpha, alpha_stride, off_e):
-    coef = torch.empty(4 * in_dim + 4, dtype=torch.float32, device=We.device)
-    _abi.check(_lib().fnb_edge_coef_fwd(_p(We), _p(be), in_dim, _p(alpha), alpha_stride, off_e, _p(coef), _stream()),
-               "edge_coef_fwd")
-    return coef
-
-
-def edge_coef_bwd(We, be, in_dim, alpha, alpha_stride, off_e, d_coef, d_alpha):
-    dWe, dbe = torch.empty_like(We), torch.empty_like(be)
-    _abi.check(_lib().fnb_edge_coef_bwd(_p(We), _p(be), in_dim, _p(alpha), alpha_stride, off_e, _p(d_coef), _p(dWe),
-                                        _p(dbe), _p(d_alpha), _stream()), "edge_coef_bwd")
-    return dWe, dbe
-
-
-def gat_fwd(g: GraphCSR, h, S, mode, edge_attr=None, coef=None, save_p=True, mask=(-1, -1),
-            next_alpha=None, next_alpha_stride=0):
-    """Returns (out [N,128], p_saved [E,4] or None, next_Se [N,4] or None)."""
-    out = torch.empty((g.n_nodes, D), dtype=torch.float32, device=h.device)
-    p = torch.empty((g.n_edges, H), dtype=torch.float32, device=h.device) if save_p else None
-    nse = torch.empty((g.n_nodes, H), dtype=torch.float32, device=h.device) if next_alpha is not None else None
-    _abi.check(_lib().fnb_gat_fwd(_p(g.rowptr), _p(g.col), g.n_nodes, g.n_edges, _p(h), _p(S), mode, _p(edge_attr),
-                                  _p(coef), _p(g.eid), g.n_real, _p(out), _p(p), mask[0], mask[1], _p(next_alpha),
-                                  next_alpha_stride, _p(nse), _stream()), "gat_fwd")
-    return out, p, nse
-
-
 def attn_by_source(g: GraphCSR, p):
     w = torch.empty((g.n_nodes, H), dtype=torch.float32, device=p.device)
     _abi.check(_lib().fnb_attn_by_source(_p(g.rrowptr), _p(g.rslot), _p(p), g.n_nodes, _p(w), _stream()),
                "attn_by_source")
     return w
-
-
-def gat_bwd_dst(g: GraphCSR, h, dout, p, mode=EDGE_NONE, edge_attr=None, want_coef=False):
-    dz = torch.empty((g.n_edges, H), dtype=torch.float32, device=h.device)
-    dSt = torch.empty((g.n_nodes, H), dtype=torch.float32, device=h.device)
-    d_coef = None
-    if want_coef:
-        d_coef = torch.empty(8 if mode == EDGE_AFFINE1 else 28, dtype=torch.float32, device=h.device)
-    _abi.check(_lib().fnb_gat_bwd_dst(_p(g.rowptr), _p(g.col), g.n_nodes, g.n_edges, _p(h), _p(dout), _p(p), mode,
-                                      _p(edge_attr), _p(dz), _p(dSt), _p(d_coef), _p(scratch(h.device)), _stream()),
-               "gat_bwd_dst")
-    return dz, dSt, d_coef
-
-
-def gat_bwd_src(g: GraphCSR, h, dout, p, dz, dSt, alpha, alpha_stride, off_t, off_s, d_alpha, want_bias_grad=False):
-    """Returns dh, or (dh, d_bias) with ``want_bias_grad`` (d_bias = column sums of dh)."""
-    dh = torch.empty((g.n_nodes, D), dtype=torch.float32, device=h.device)
-    db = torch.empty(D, dtype=torch.float32, device=h.device) if want_bias_grad else None
-    _abi.check(_lib().fnb_gat_bwd_src(_p(g.rrowptr), _p(g.rslot), _p(g.rdst), g.n_nodes, _p(h), _p(dout), _p(p),
-                                      _p(dz), _p(dSt), _p(alpha), alpha_stride, off_t, off_s, _p(dh), _p(d_alpha),
-                                      _p(db), _p(scratch(h.device)), _stream()), "gat_bwd_src")
-    return (dh, db) if want_bias_grad else dh
-
-
-def edge_table_bwd(g: GraphCSR, dz, feat, alpha, alpha_stride, off_e, g_base, d_alpha):
-    g_feat = torch.empty((g.n_real, D), dtype=torch.float32, device=feat.device)
-    _abi.check(_lib().fnb_edge_table_bwd(_p(dz), _p(g.slot_of_eid), g.n_real, _p(feat), _p(alpha), alpha_stride,
-                                         off_e, _p(g_base), _p(g_feat), _p(d_alpha), _p(scratch(feat.device)),
-                                         _stream()), "edge_table_bwd")
-    return g_feat
 
 
 # ---- node-tiled attention kernels (gat_tiled.cu) ------------------------------------------------

@@ -36,15 +36,15 @@ extern "C" {
 
 #define FNB_D 128 /* embedding width  */
 #define FNB_H 4   /* attention heads  */
-#define FNB_ABI_VERSION 10
+#define FNB_ABI_VERSION 11
 
-/* edge-term modes of the fused attention kernels (SURVEY.md App. A.5) */
 /* arithmetic of the dense projections */
 #define FNB_PRECISION_FP32 0 /* FP32 FFMA: bit-for-bit comparable with the reference within 1e-5            */
 #define FNB_PRECISION_TF32 1 /* tcgen05 tensor cores, TF32 operands, FP32 accumulate (stated tolerance 2e-3) */
 #define FNB_PRECISION_TF32X3 2 /* tcgen05 tensor cores, 3xTF32 error-compensated split (hi*hi + hi*lo + lo*hi),
                                   FP32 accumulate: FP32-grade results, within 1e-5 of the reference             */
 
+/* edge-term modes of the fused attention kernels (SURVEY.md App. A.5) */
 #define FNB_EDGE_NONE 0   /* no edge term                                              */
 #define FNB_EDGE_AFFINE1 1 /* bond graph: S_e[h] = attr[slot]*coef[h] + coef[4+h]       */
 #define FNB_EDGE_AFFINE6 2 /* fragment-connection graph: attr[slot,0:6] . coef[h,0:6] + coef[24+h] */
@@ -97,77 +97,46 @@ int fnb_narrow_index(const int64_t *in, int64_t n, int32_t *out, void *stream);
 int fnb_proj_fwd(const float *x, const float *W, const float *b, int64_t n_rows, int K,
                  const float *alpha, int alpha_stride, int off_t, int off_s, float *h, float *S,
                  int precision, void *stream);
-/* dx = dh @ W (dx may be NULL); dW = dh^T @ x; db = column sums of dh (may be NULL: fnb_gat_bwd_src can emit
- * it for free).  scratch: fnb_scratch_bytes(). */
+/* dx = dh @ W (dx may be NULL); dW = dh^T @ x; db = column sums of dh (may be NULL: fnb_gat_bwd_tiled can emit
+ * it for free as d_bias).  scratch: fnb_scratch_bytes(). */
 int fnb_proj_bwd(const float *x, const float *W, const float *dh, int64_t n_rows, int K, float *dx,
                  float *dW, float *db, int precision, void *scratch, void *stream);
 /* S for features that are not projected (fragment graph: hf = pooled atoms, gat2.py:285). */
 int fnb_node_scalars(const float *h, int64_t n_rows, const float *alpha, int alpha_stride,
                      int off_t, int off_s, float *S, void *stream);
 
-/* Constants of the affine edge term from the tiny edge-attribute embedding (App. A.5):
- * coef[h, 0:in] = We^T alpha_e[h], coef[4*in + h] = <be, alpha_e[h]>,
- * We [32,in] = edge_attr_{bond,fbond}_embed.weight, alpha_e = alpha[h, off_e : off_e+32]. */
-int fnb_edge_coef_fwd(const float *We, const float *be, int in_dim, const float *alpha,
-                      int alpha_stride, int off_e, float *coef, void *stream);
-/* d_coef [4*in+4] -> dWe [32,in], dbe [32], d_alpha[h, off_e:off_e+32] (written, not accumulated). */
-int fnb_edge_coef_bwd(const float *We, const float *be, int in_dim, const float *alpha,
-                      int alpha_stride, int off_e, const float *d_coef, float *dWe, float *dbe,
-                      float *d_alpha, void *stream);
-
-/* ---- (b) fused gather -> edge logit -> LeakyReLU(0.2) -> segment softmax -> aggregate -------
- * One warp per destination node (gat2.py:146-169, 196-224, 250-272, 286-316 in one pass):
- *   z[e,h] = S[t,h] + S_e[e,h] + S[s,4+h];  p = softmax over the slots of t;  out[t] = sum p*h[s]
- * p_saved [n_edges,4] (slot order; sign bit carries z>0 for the LeakyReLU derivative) may be
- * NULL for inference.  Rows [mask_lo, mask_hi) of out are zeroed (bond / frag-bond / atom masks,
- * gat2.py:173-176,227-231,275-278); pass mask_lo = mask_hi = -1 for none.
- * If next_alpha_e != NULL, also emits next_Se[t,h] = <out[t,:], next_alpha_e[h, 0:128]>, the edge
- * term of the graph whose edges are this graph's nodes (bond -> atom, fbond -> fragment).
- */
-int fnb_gat_fwd(const int32_t *rowptr, const int32_t *col, int64_t n_nodes, int64_t n_edges,
-                const float *h, const float *S, int edge_mode, const float *edge_attr,
-                const float *edge_coef, const int32_t *eid, int64_t n_real_edges, float *out,
-                float *p_saved, int64_t mask_lo, int64_t mask_hi, const float *next_alpha_e,
-                int next_alpha_stride, float *next_Se, void *stream);
-
 /* w[n,h] = sum of p over the edges whose SOURCE is n (gat2.py:165,219,268,312), atomics-free over
  * the reverse CSR. */
 int fnb_attn_by_source(const int32_t *rrowptr, const int32_t *rslot, const float *p_saved,
                        int64_t n_nodes, float *w, void *stream);
 
-/* ---- (c) atomics-free backward --------------------------------------------------------------
- * Pass 1, destination segments: dz[slot,h] (gradient of the pre-LeakyReLU logit), dSt[t,h], and
- * the gradient of the affine edge-term constants d_coef (same layout as coef; NULL unless the
- * mode is AFFINE1/AFFINE6).  With extra_g/extra_index, dout[t] += extra_g[extra_index[t]] is
- * applied on the fly and the combined rows are written to dout_combined (atom->fragment pooling
- * backward, gat2.py:234).  scratch: fnb_scratch_bytes().
- */
-int fnb_gat_bwd_dst(const int32_t *rowptr, const int32_t *col, int64_t n_nodes, int64_t n_edges,
-                    const float *h, const float *dout, const float *p_saved, int edge_mode,
-                    const float *edge_attr, float *dz, float *dSt, float *d_coef, void *scratch,
-                    void *stream);
-/* Pass 2, source segments over the reverse CSR: dh[s] = sum p*dout[t] + dSt[s]*alpha_t + dSs[s]*alpha_s,
- * d_alpha[h, off_t:+32], d_alpha[h, off_s:+32] (written), and optionally d_bias[128] = column sums of dh
- * (the bias gradient of the projection that produced h; NULL to skip). */
-int fnb_gat_bwd_src(const int32_t *rrowptr, const int32_t *rslot, const int32_t *rdst,
-                    int64_t n_nodes, const float *h, const float *dout, const float *p_saved,
-                    const float *dz, const float *dSt, const float *alpha, int alpha_stride,
-                    int off_t, int off_s, float *dh, float *d_alpha, float *d_bias, void *scratch,
-                    void *stream);
-/* Edge-term backward for TABLE mode: for every real edge e with feature row feat[e,:]:
- *   g_feat[e,:] = g_base[e,:] + sum_h dz[slot_of_eid[e],h] * alpha_e[h,:]   (g_base NULL = 0; may alias g_feat)
- *   d_alpha[h, off_e:off_e+128] = sum_e dz[slot_of_eid[e],h] * feat[e,:] */
-int fnb_edge_table_bwd(const float *dz, const int32_t *slot_of_eid, int64_t n_real_edges,
-                       const float *feat, const float *alpha, int alpha_stride, int off_e,
-                       const float *g_base, float *g_feat, float *d_alpha, void *scratch, void *stream);
-
-/* ---- node-tiled attention kernels (gat_tiled.cu): the production path ------------------------
- * Same math as fnb_gat_fwd / fnb_gat_bwd_dst / fnb_gat_bwd_src / fnb_edge_table_bwd above, restructured after
- * profiling (DESIGN.md section 3): a CTA owns 64 consecutive destination nodes, logits are computed one thread per
+/* ---- fused attention block (gat_tiled.cu) --------------------------------------------------------------
+ * Forward, gather -> edge logit -> LeakyReLU(0.2) -> segment softmax -> aggregate in one launch
+ * (gat2.py:146-169, 196-224, 250-272, 286-316):
+ *   z[e,h] = S[t,h] + S_e[e,h] + S[s,4+h];  p = softmax over the slots of t;  out[t] = sum p*h[s]
+ * with t, s the destination and source of slot e and S_e the edge term of edge_mode (FNB_EDGE_*).  The affine modes
+ * compute their constants from the tiny edge-attribute embedding (App. A.5) in the kernel's prologue:
+ *   coef[h*in + k] = sum_j We[j,k] alpha_e[h,j],  coef[4*in + h] = <be, alpha_e[h,:]>   (in = 1 or 6).
+ * p_saved [n_edges,4] (slot order; the sign bit carries z>0 for the LeakyReLU derivative) may be NULL for inference.
+ * Rows [mask_lo, mask_hi) of out and y are zeroed (bond / frag-bond / atom masks, gat2.py:173-176,227-231,275-278);
+ * pass mask_lo = mask_hi = -1 for none.  If next_alpha_e != NULL, also emits
+ * next_Se[t,h] = <out[t,:], next_alpha_e[h, 0:128]>, the edge term of the graph whose edges are this graph's nodes
+ * (bond -> atom, fbond -> fragment).
+ *
+ * Backward, destination pass then source pass, both atomics-free.  The destination pass (CSR) writes dz[slot,h], the
+ * gradient of the pre-LeakyReLU logit z, and dSt[t,h] = sum of dz over the slots of t (the gradient of S[t,h]).  The
+ * source pass (reverse CSR) writes
+ *   dh[s] = sum p*dout[t] + dSt[s]*alpha_t + dSs[s]*alpha_s,   dSs[s,h] = sum of dz over the edges leaving s,
+ * with alpha_t = alpha[h, off_t:+32], alpha_s = alpha[h, off_s:+32], and the head-vector gradients
+ * d_alpha[h, off_t:+32] and d_alpha[h, off_s:+32] (written, not accumulated); the affine modes also write
+ * d_alpha[h, off_e:+32], dWe and dbe.  d_bias[128] = column sums of dh (the bias gradient of the projection that
+ * produced h), or NULL to skip.  The 128-wide edge slice of TABLE mode is fnb_edge_table_bwd_fused's.
+ *
+ * Layout (DESIGN.md section 3): a CTA owns up to 64 consecutive destination nodes, logits are computed one thread per
  * edge slot, the softmax one thread per (node, head) in shared memory, the row aggregation one warp per node.
- * Folded in: the edge-embedding constants (fnb_edge_coef_fwd/bwd), the inter-layer ReLU(Dropout(.)) of
- * gat2.py:414-418 (forward epilogue / edge-table backward), and the cross-CTA reduction of every parameter
- * gradient (last CTA to finish; deterministic, no atomics on floats, no second launch).
+ * Also folded in: the inter-layer ReLU(Dropout(.)) of gat2.py:414-418 (forward epilogue / edge-table backward) and
+ * the cross-CTA reduction of every parameter gradient (last CTA to finish; deterministic, no atomics on floats, no
+ * second launch).
  * scratch: fnb_scratch_bytes() bytes whose first 256 bytes are ZERO before the first call and are left zero by
  * every call (arrival counters). */
 typedef struct fnb_graph {

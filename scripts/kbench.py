@@ -65,23 +65,16 @@ def main():
         S = ops.node_scalars(h, alpha, stride, 0, off_s)
         X = {ops.EDGE_AFFINE1: E * 4, ops.EDGE_AFFINE6: E * 24, ops.EDGE_TABLE: E * 16 + E * 4}[mode]
         fwd_bytes = 2 * N * 512 + X + 2 * E * 4 + (N + 1) * 4 + E * 16 + 2 * N * 32
-        kw_old, kw_new, kw_b = {}, {}, {}
+        kw_b = {}
         if mode == ops.EDGE_AFFINE1:
-            coef = ops.edge_coef_fwd(We1, be1, 1, alpha, stride, 32)
-            kw_old = dict(edge_attr=g.attr, coef=coef)
             kw_new = dict(We=We1, be=be1, alpha_e=alpha[:, 32:], alpha_stride=stride)
             kw_b = dict(We=We1, be=be1)
         elif mode == ops.EDGE_AFFINE6:
-            coef = ops.edge_coef_fwd(We6, be6, 6, alpha, stride, 32)
-            kw_old = dict(edge_attr=g.attr, coef=coef)
             kw_new = dict(We=We6, be=be6, alpha_e=alpha[:, 32:], alpha_stride=stride)
             kw_b = dict(We=We6, be=be6)
         else:
-            table = rnd(g.n_real, 4)
-            kw_old = dict(edge_attr=table)
-            kw_new = dict(table=table)
-        timeit(f"{name}: gat_fwd warp-per-node (N={N},E={E})", lambda: ops.gat_fwd(g, h, S, mode, **kw_old), fwd_bytes)
-        timeit(f"{name}: gat_fwd tiled", lambda: ops.gat_fwd_tiled(g, h, S, mode, **kw_new), fwd_bytes)
+            kw_new = dict(table=rnd(g.n_real, 4))
+        timeit(f"{name}: gat_fwd tiled (N={N},E={E})", lambda: ops.gat_fwd_tiled(g, h, S, mode, **kw_new), fwd_bytes)
         timeit(f"{name}: gat_fwd tiled +y(drop .2)+nextSe",
                lambda: ops.gat_fwd_tiled(g, h, S, mode, post=(0.2, 1, 1, 1, 0), next_alpha=a192[:, 32:],
                                          next_alpha_stride=192, **kw_new), fwd_bytes + N * 512 + N * 16)
@@ -91,12 +84,6 @@ def main():
         _, _, p, _ = ops.gat_fwd_tiled(g, h, S, mode, **kw_new)
         d_alpha = torch.zeros(4, stride, device=dev)
         bwd_bytes = 5 * N * 512 + 4 * E * 16 + 3 * E * 4 + 2 * N * 16 + 2 * (N + 1) * 4
-        old_mode = mode if mode in (ops.EDGE_AFFINE1, ops.EDGE_AFFINE6) else ops.EDGE_NONE
-
-        def old_bwd():
-            dz, dSt, _ = ops.gat_bwd_dst(g, h, go, p, old_mode, g.attr if old_mode else None, bool(old_mode))
-            ops.gat_bwd_src(g, h, go, p, dz, dSt, alpha, stride, 0, off_s, d_alpha, want_bias_grad=True)
-        timeit(f"{name}: gat_bwd dst+src warp-per-node", old_bwd, bwd_bytes)
         timeit(f"{name}: gat_bwd dst+src tiled",
                lambda: ops.gat_bwd_tiled(g, h, go, p, mode, alpha, stride, 0, 32, off_s, d_alpha, want_bias_grad=True,
                                          **kw_b), bwd_bytes)
@@ -104,8 +91,6 @@ def main():
             dz = rnd(E, 4)
             feat, dy = rnd(g.n_real, 128), rnd(g.n_real, 128)
             y = torch.relu(feat)
-            timeit(f"{name}: edge_table_bwd (old, g_base)",
-                   lambda: ops.edge_table_bwd(g, dz, feat, alpha, stride, 32, dy, d_alpha), 3 * g.n_real * 512)
             timeit(f"{name}: edge_table_bwd fused dropout-relu bwd",
                    lambda: ops.edge_table_bwd_fused(g, dz, feat, alpha, stride, 32, d_alpha, dy=dy, y=y, post_scale=1.25),
                    4 * g.n_real * 512)

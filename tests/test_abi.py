@@ -36,7 +36,6 @@ def test_argument_validation_needs_no_gpu():
     assert lib.fnb_csr_build(None, None, -1, 4, 0, None, None, None, None, None, None, None, None, None, 0, None, None) == -2
     assert lib.fnb_csr_build(None, None, 0, 4, 0, None, None, None, None, None, None, None, None, None, 0, None, None) == -1
     assert lib.fnb_proj_fwd(None, None, None, 8, 128, None, 0, 0, 0, None, None, 0, None) == -1
-    assert lib.fnb_edge_coef_fwd(None, None, 3, None, 96, 32, None, None) == -3
     assert lib.fnb_dropout_relu_fwd(None, None, 4, 1.5, 1, 1, 0, 0, None) == -2
     assert lib.fnb_gat_fwd_tiled(None, None, None) == -1
     assert lib.fnb_gat_bwd_tiled(None, None, None) == -1

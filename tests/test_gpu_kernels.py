@@ -30,106 +30,6 @@ def test_projection_forward_backward(n, K):
     assert rel_err(ops.node_scalars(h, alpha.cuda(), 96, 0, 64), Sref) <= FP32_REL_TOL
 
 
-def _random_graph(n_nodes, n_edges, seed, hub=False):
-    g = torch.Generator().manual_seed(seed)
-    dst = torch.randint(0, n_nodes, (n_edges,), generator=g)
-    src = torch.randint(0, n_nodes, (n_edges,), generator=g)
-    dst[:n_nodes] = torch.arange(n_nodes)           # every node is a target (reference requirement, App. B)
-    if hub:
-        dst[n_nodes:n_nodes + 300] = 0              # one segment spanning 10 chunks of 32 edges
-    return dst, src
-
-
-@pytest.mark.parametrize("mode", ["none", "affine1", "affine6", "table"])
-@pytest.mark.parametrize("n_nodes,n_edges,hub", [(40, 200, False), (64, 1500, True), (3000, 20000, False)])
-def test_attention_block_forward_backward(mode, n_nodes, n_edges, hub):
-    """gat_fwd / gat_bwd_dst / gat_bwd_src / edge_table_bwd / edge_coef_* against autograd of the oracle block."""
-    from fragnet_b200 import ops
-    from oracle import gat2_oracle as O
-    dst, src = _random_graph(n_nodes, n_edges, 7 + n_nodes, hub)
-    gen = torch.Generator().manual_seed(n_edges)
-    h = torch.randn(n_nodes, 128, generator=gen).requires_grad_()
-    gout = torch.randn(n_nodes, 128, generator=gen)
-    graph = ops.csr_build(dst.cuda(), src.cuda(), n_nodes)
-    sc = ops.scratch(torch.device("cuda", 0))  # noqa: F841
-    if mode in ("none", "affine1", "affine6"):
-        stride, off_t, off_e, off_s = 96, 0, 32, 64
-    else:
-        stride, off_t, off_e, off_s = 192, 0, 32, 160
-    alpha = (torch.randn(4, stride, generator=gen) * 0.3).requires_grad_()
-    edge_vec = None
-    kw = {}
-    if mode == "none":
-        a_used = torch.cat([alpha[:, 0:32], alpha[:, 64:96]], dim=1)
-        edge_vec = torch.zeros(n_edges, 0)
-    elif mode in ("affine1", "affine6"):
-        k = 1 if mode == "affine1" else 6
-        attr = torch.randn(n_edges, k, generator=gen)
-        We = (torch.randn(32, k, generator=gen) * 0.5).requires_grad_()
-        be = torch.randn(32, generator=gen).requires_grad_()
-        edge_vec = F.linear(attr, We, be)
-        a_used = alpha
-        coef = ops.edge_coef_fwd(We.detach().cuda(), be.detach().cuda(), k, alpha.detach().cuda(), stride, off_e)
-        attr_sorted = ops.gather_rows(attr.cuda(), graph.eid, n_edges)
-        kw = dict(edge_attr=attr_sorted, coef=coef)
-    else:
-        feat = torch.randn(n_edges, 128, generator=gen).requires_grad_()
-        edge_vec = feat
-        a_used = alpha
-        se = (feat.detach() @ alpha.detach()[:, 32:160].t()).contiguous()
-        kw = dict(edge_attr=se.cuda())
-    # oracle
-    out_ref, w_ref = O.attention_block(h.view(n_nodes, 4, 32), dst, src, edge_vec, a_used)
-    (out_ref * gout).sum().backward()
-    # cuda
-    hc, ac = h.detach().cuda(), alpha.detach().cuda()
-    S = ops.node_scalars(hc, ac, stride, off_t, off_s)
-    mode_id = dict(none=ops.EDGE_NONE, affine1=ops.EDGE_AFFINE1, affine6=ops.EDGE_AFFINE6, table=ops.EDGE_TABLE)[mode]
-    out, p, _ = ops.gat_fwd(graph, hc, S, mode_id, **kw)
-    assert rel_err(out, out_ref) <= FP32_REL_TOL
-    assert rel_err(ops.attn_by_source(graph, p), w_ref) <= FP32_REL_TOL
-    go = gout.cuda()
-    dz, dSt, d_coef = ops.gat_bwd_dst(graph, hc, go, p, mode_id if mode.startswith("affine") else ops.EDGE_NONE,
-                                      kw.get("edge_attr") if mode.startswith("affine") else None,
-                                      mode.startswith("affine"))
-    d_alpha = torch.zeros(4, stride, device="cuda")
-    dh, dbias = ops.gat_bwd_src(graph, hc, go, p, dz, dSt, ac, stride, off_t, off_s, d_alpha, want_bias_grad=True)
-    assert rel_err(dbias, h.grad.sum(0)) <= 2e-4
-    gtol = 2e-5      # gradients: sums of O(100) fp32 products, two independent summation orders
-    assert rel_err(dh, h.grad) <= gtol
-    if mode.startswith("affine"):
-        k = 1 if mode == "affine1" else 6
-        dWe, dbe = ops.edge_coef_bwd(We.detach().cuda(), be.detach().cuda(), k, ac, stride, off_e, d_coef, d_alpha)
-        assert rel_err(dWe, We.grad) <= gtol and rel_err(dbe, be.grad) <= gtol
-    if mode == "table":
-        gbase = torch.randn(n_edges, 128, generator=gen)
-        g_feat = ops.edge_table_bwd(graph, dz, feat.detach().cuda(), ac, stride, off_e, gbase.cuda(), d_alpha)
-        assert rel_err(g_feat - gbase.cuda(), feat.grad) <= gtol
-    if mode == "none":
-        want = alpha.grad.clone()
-        assert rel_err(d_alpha[:, 0:32], want[:, 0:32]) <= gtol and rel_err(d_alpha[:, 64:96], want[:, 64:96]) <= gtol
-    else:
-        assert rel_err(d_alpha, alpha.grad) <= gtol
-
-
-def test_attention_masks_and_fused_next_edge_term():
-    from fragnet_b200 import ops
-    dst, src = _random_graph(100, 700, 3)
-    gen = torch.Generator().manual_seed(1)
-    h = torch.randn(100, 128, generator=gen).cuda()
-    alpha = torch.randn(4, 96, generator=gen).cuda()
-    nxt = torch.randn(4, 192, generator=gen).cuda()
-    graph = ops.csr_build(dst.cuda(), src.cuda(), 100)
-    S = ops.node_scalars(h, alpha, 96, 0, 64)
-    out0, _, _ = ops.gat_fwd(graph, h, S, ops.EDGE_NONE, save_p=False)
-    out1, _, se = ops.gat_fwd(graph, h, S, ops.EDGE_NONE, save_p=False, mask=(10, 12), next_alpha=nxt[:, 32:],
-                              next_alpha_stride=192)
-    want = out0.clone()
-    want[10:12] = 0
-    assert torch.equal(out1, want)
-    assert rel_err(se, want @ nxt[:, 32:160].t()) <= FP32_REL_TOL
-
-
 def test_segment_sum_and_gather():
     from fragnet_b200 import ops
     gen = torch.Generator().manual_seed(4)
