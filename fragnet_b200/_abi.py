@@ -107,7 +107,7 @@ class CWidenJob(C.Structure):
 WIDEN_U8_F32, WIDEN_I32_I64, WIDEN_MAX_JOBS = 0, 1, 16
 ARENA_COPY32, ARENA_INDEX, ARENA_FILL = 0, 1, 2
 ARENA_MAX_KINDS, ARENA_MAX_JOBS = 24, 32
-ABI_VERSION = 11
+ABI_VERSION = 12
 EDGE_NONE, EDGE_AFFINE1, EDGE_AFFINE6, EDGE_TABLE = 0, 1, 2, 3
 PRECISION_FP32, PRECISION_TF32, PRECISION_TF32X3 = 0, 1, 2
 
@@ -179,7 +179,7 @@ class CBatchInputs(C.Structure):
 class CEncoderOpts(C.Structure):
     _fields_ = [("n_layers", _i32), ("post_act", _i32), ("drop_p", _f32), ("training", _i32), ("seed", _u64),
                 ("offset", _u64), ("precision", _i32), ("save_for_backward", _i32), ("need_dx_atoms", _i32),
-                ("need_dx_bond", _i32), ("need_dx_fbond", _i32)]
+                ("need_dx_bond", _i32), ("need_dx_fbond", _i32), ("first_trained_layer", _i32)]
 
 
 class CEncoderIO(C.Structure):
@@ -237,4 +237,4 @@ class CFinetuneStepArgs(C.Structure):
                [("n_layers", _i32), ("layers", _vp), ("layer_grads", _vp), ("n_head_layers", _i32), ("head", _vp),
                 ("loss_kind", _i32), ("drop_p", _f32), ("training", _i32), ("seed", _u64), ("offset", _u64),
                 ("precision", _i32), ("backward", _i32)] + \
-               [(n, _vp) for n in ("loss", "predictions", "plan_arena")]
+               [(n, _vp) for n in ("loss", "predictions", "plan_arena")] + [("first_trained_layer", _i32)]

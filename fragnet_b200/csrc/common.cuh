@@ -269,15 +269,20 @@ struct FnbMlpRun {
   uint64_t in_base[FNB_MLP_MAX_LAYERS], out_base[FNB_MLP_MAX_LAYERS];   // fnb_mlp_rng
   float *x0;                        // [G, L[0].in_dim] head input
   float *xd[FNB_MLP_MAX_LAYERS];    // [G, L[l].in_dim] what layer l multiplies; xd[0] == x0 when nothing drops there
-  float *u[FNB_MLP_MAX_LAYERS];     // [G, L[l].out_dim] pre-activation of the hidden layers (NULL: not kept)
+  float *u[FNB_MLP_MAX_LAYERS];     // [G, L[l].out_dim] pre-activation of the hidden layers (NULL: not kept; the
+                                    // backward reads u[l] where layer l + 1's input gradient runs)
   float *out;                       // [G, L[n-1].out_dim] predictions
   float *dz[FNB_MLP_MAX_LAYERS];    // backward: [G, L[l].out_dim] gradient of layer l's pre-dropout output; dz[n-1] is input
-  float *dx0;                       // backward: [G, L[0].in_dim] gradient of x0
+  float *dx0;                       // backward: [G, L[0].in_dim] gradient of x0 (NULL: not wanted)
   float *rec;                       // backward: fnb_mlp_dw_record_floats() floats
 };
 int fnb_mlp_check(const fnb_mlp_layer *L, int n, int64_t G, int in0, int backward);
 uint64_t fnb_mlp_rng(const fnb_mlp_layer *L, int n, int64_t G, uint64_t offset, uint64_t *in_base, uint64_t *out_base);
+// Weight-gradient records of the trained layers (dW != NULL).
 size_t fnb_mlp_dw_record_floats(const fnb_mlp_layer *L, int n, int64_t G);
+// Whether the backward runs layer l's input-gradient GEMM: a trained layer lies below l, or (want_dx0) the caller wants
+// the gradient of the head input.
+bool fnb_mlp_needs_dx(const fnb_mlp_layer *L, int l, bool want_dx0);
 int fnb_mlp_forward(const FnbMlpRun *r, cudaStream_t stream);
 int fnb_mlp_backward(const FnbMlpRun *r, cudaStream_t stream);
 // loss[0] = mean of BCE-with-logits over the labels > -0.5 (NaN if none); grad (may be NULL) = its logit gradient.

@@ -71,7 +71,7 @@ size_t layout(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fnb_l
   for (int l = 0; l < o->n_layers; ++l) {
     LayerBufs b{};
     const bool last = l == o->n_layers - 1;
-    const bool keep = o->save_for_backward != 0;
+    const bool keep = o->save_for_backward != 0 && l >= o->first_trained_layer;   // frozen layers: nothing to save
     const bool want_p = keep || L[l].want_attention;
     const bool frag = L[l].run_frag_block != 0;
     if (l == 0 && input_dropout(o)) b.xa0 = a.take<float>(z.Na * L[0].K_atom);
@@ -149,7 +149,7 @@ size_t bwd_layout(const fnb_batch_plan *plan, const fnb_encoder_opts *o, char *b
   b.dh_fb = a.take<float>(z.Nfb * kD); b.dx_fbond = a.take<float>(z.Nfb * kD);
   b.g_frag = a.take<float>(z.Nf * kD); b.dz_f = a.take<float>(z.Ef * 4); b.dSt_f = a.take<float>(z.Nf * 4);
   b.d_hf = a.take<float>(z.Nf * kD);
-  b.Wt = a.take<float>((size_t)o->n_layers * 3 * kD * kD);
+  b.Wt = a.take<float>((size_t)(o->n_layers - o->first_trained_layer) * 3 * kD * kD);   // trained layers only
   b.scratch2 = a.take<float>(kScratchFloats);
   b.scratch3 = a.take<float>(kScratchFloats);
   b.scratch4 = a.take<float>(kScratchFloats);
@@ -268,6 +268,7 @@ int check_common(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fn
                  const fnb_encoder_io *io) {
   if (!plan || !o || !L || !io) return FNB_ERR_NULL;
   if (o->n_layers < 1 || o->n_layers > 16) return FNB_ERR_SIZE;
+  if (o->first_trained_layer < 0 || o->first_trained_layer > o->n_layers) return FNB_ERR_SIZE;
   if (!o->post_act && o->n_layers != 1) return FNB_ERR_MODE;
   if (!(o->drop_p >= 0.f && o->drop_p < 1.f)) return FNB_ERR_SIZE;
   const Sizes z = sizes_of(plan);
@@ -290,6 +291,7 @@ int check_common(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fn
 extern "C" size_t fnb_encoder_workspace_bytes(const fnb_batch_plan *plan, const fnb_encoder_opts *opts,
                                               const fnb_layer_params *layers) {
   if (!plan || !opts || !layers || opts->n_layers < 1 || opts->n_layers > 16) return 0;
+  if (opts->first_trained_layer < 0 || opts->first_trained_layer > opts->n_layers) return 0;
   return layout(plan, opts, layers, nullptr, nullptr);
 }
 
@@ -297,6 +299,7 @@ extern "C" size_t fnb_encoder_bwd_workspace_bytes(const fnb_batch_plan *plan, co
                                                   const fnb_layer_params *layers) {
   (void)layers;
   if (!plan || !opts || opts->n_layers < 1 || opts->n_layers > 16) return 0;
+  if (opts->first_trained_layer < 0 || opts->first_trained_layer > opts->n_layers) return 0;
   return bwd_layout(plan, opts, nullptr, nullptr);
 }
 
@@ -326,7 +329,6 @@ int fnb_encoder_forward_impl(const fnb_batch_plan *plan, const fnb_encoder_opts 
   const Sizes z = sizes_of(plan);
   const RngPlan ph = rng_plan(plan, o, L);
   cudaStream_t stream = (cudaStream_t)stream_;
-  const bool keep = o->save_for_backward != 0;
 
   const float *xa = io->x_atoms, *xb = io->x_bond, *xfb = io->x_fbond;
   // nn.Dropout on the raw atom features (gat2.py:396).  When layer 0 takes the padded operands anyway and nobody asks
@@ -400,7 +402,7 @@ int fnb_encoder_forward_impl(const fnb_batch_plan *plan, const fnb_encoder_opts 
     LayerBufs &b = B[l];
     const bool last = l == o->n_layers - 1;
     const bool frag = P.run_frag_block != 0;
-    const bool want_p = keep || P.want_attention;
+    const bool want_p = (o->save_for_backward != 0 && l >= o->first_trained_layer) || P.want_attention;
     // layer-0 operands may be the zero-padded copies (TF32 path)
     const bool pb = l == 0 && b.k_pad[0], pa = l == 0 && b.k_pad[1], pf = l == 0 && b.k_pad[2];
     const float *xb_in = pb ? b.x_pad[0] : xb, *Wb_in = pb ? b.W_pad[0] : P.Wb;
@@ -526,18 +528,21 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
   bool counters_cleared = false;
   const bool tf32 = fnb_tc_precision(o->precision);
   const int x3 = o->precision == FNB_PRECISION_TF32X3;
+  // layers below first_trained_layer are frozen: the pass ends at that layer, which needs no input gradient
+  const int first = o->first_trained_layer;
 
   // W^T of every K = 128 projection in one launch per 16 matrices (used by the tensor-core dX GEMMs)
   int wt_slot[16][3];
   {
     const float *mats[48];
     int nm = 0;
-    for (int l = 0; l < o->n_layers; ++l) {
+    for (int l = first; l < o->n_layers; ++l) {
       const float *ws[3] = {L[l].Wb, L[l].Wa, L[l].Wfb};
       const int ks[3] = {L[l].K_bond, L[l].K_atom, L[l].K_fbond};
       for (int j = 0; j < 3; ++j) {
         wt_slot[l][j] = -1;
-        if (tf32 && ks[j] == kD && (l > 0 || (j == 0 ? o->need_dx_bond : (j == 1 ? o->need_dx_atoms : o->need_dx_fbond)))) {
+        if (tf32 && ks[j] == kD &&
+            (l > first || (l == 0 && (j == 0 ? o->need_dx_bond : (j == 1 ? o->need_dx_atoms : o->need_dx_fbond))))) {
           wt_slot[l][j] = nm;
           mats[nm++] = ws[j];
         }
@@ -620,7 +625,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
 
   // gradients arriving at the four outputs of the current layer (post-activation copies in post_act mode)
   const float *dy_atom = io->g_atoms, *dy_bond = io->g_bond, *dy_fbond = io->g_fbond, *dy_frag = io->g_frags;
-  for (int l = o->n_layers - 1; l >= 0; --l) {
+  for (int l = o->n_layers - 1; l >= first; --l) {
     const fnb_layer_params &P = L[l];
     const fnb_layer_grads &D = G[l];
     LayerBufs &b = B[l];
@@ -635,7 +640,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
     const float *y_frag = o->post_act ? (last ? io->out_frags : b.y_frag) : nullptr;
     const float *pre_bond = o->post_act ? b.pre_bond : io->out_bond;
     const float *pre_fbond = o->post_act ? b.pre_fbond : io->out_fbond;
-    const bool need_dx = l > 0;
+    const bool need_dx = l > first;
     const int par = l & 1;
     float *dh_a = par ? W.dh_a2 : W.dh_a, *dh_b = par ? W.dh_b2 : W.dh_b;
     // dz of the atom graph is double-buffered by layer parity like dh: its last reader, the edge-term kernel that forms
@@ -688,7 +693,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
         fz.dz_up = frag_feeds_fbond ? W.dz_f : nullptr; fz.slot_of_eid = plan->frag.slot_of_eid; fz.alpha_up = P.f + A_E;
         fz.alpha_up_stride = A_STRIDE; fz.dy = dy_fbond; fz.y = dy_fbond ? y_fbond : nullptr; fz.scale = scale;
         RC(fnb_gat_bwd_tiled_fused(&plan->fbond, &a, &fz, nullptr, nullptr, sB_));
-        float *dx = need_dx ? W.dx_fbond : (o->need_dx_fbond ? io->dx_fbond : nullptr);
+        float *dx = need_dx ? W.dx_fbond : (l == 0 && o->need_dx_fbond ? io->dx_fbond : nullptr);
         if (l == 0 && b.k_pad[2] && !dx)
           RC(fnb_tc_dw_launch(W.dh_fb, b.x_pad[2], z.Nfb, b.k_pad[2], P.K_fbond, D.Wfb, scratch_body(scratchB), sB, x3));
         else
@@ -736,7 +741,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
         RC(fnb_gat_bwd_tiled_fused(&plan->atom, &a, &fza, two ? aux.a_dz : nullptr, nullptr, sA_));
         if (two) RC((int)cudaStreamWaitEvent(stream, aux.a_dz, 0));
         RC(w_begin(0, sA));
-        float *dx = need_dx ? W.dx_atom : (o->need_dx_atoms ? io->dx_atoms : nullptr);
+        float *dx = need_dx ? W.dx_atom : (l == 0 && o->need_dx_atoms ? io->dx_atoms : nullptr);
         // layer 0 with padded operands: d Wa always from the padded copy, which holds exactly what the forward
         // multiplied (dropped or not).  The unpadded dropped copy xa0 exists only if the forward call already had
         // need_dx_atoms set; with input dropout applied inside the padding kernel it was never written.
@@ -793,7 +798,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
                                    wait_w ? done_ev(1, par) : nullptr, stream_));
         if (two && have) a_table_pending = true;
         RC(w_begin(1, stream));
-        float *dx = need_dx ? W.dx_bond : (o->need_dx_bond ? io->dx_bond : nullptr);
+        float *dx = need_dx ? W.dx_bond : (l == 0 && o->need_dx_bond ? io->dx_bond : nullptr);
         if (l == 0 && b.k_pad[0] && !dx) {
           RC(fnb_tc_dw_launch(dh_b, b.x_pad[0], z.Nb, b.k_pad[0], P.K_bond, D.Wb, scratch_body(scratchWs[1]), sWs[1], x3));
         } else {
@@ -829,7 +834,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
     RC((int)cudaStreamWaitEvent(stream, aux.e_join, 0));
   }
   // input dropout backward (gat2.py:396) when the caller wants d x_atoms: same RNG stream as the forward
-  if (o->need_dx_atoms && io->dx_atoms && input_dropout(o)) {
+  if (first == 0 && o->need_dx_atoms && io->dx_atoms && input_dropout(o)) {
     const RngPlan ph = rng_plan(plan, o, L);
     RC(fnb_dropout_relu_fwd(io->dx_atoms, io->dx_atoms, z.Na * (int64_t)L[0].K_atom, o->drop_p, 1, 0, o->seed, ph.input,
                             stream_));

@@ -16,7 +16,9 @@
 // row chunks, summed in a fixed order by k_reduce_partials: deterministic, no floating-point atomics), and one GEMM
 // dz_l W_l whose epilogue folds what lies between xd[l] and u[l-1] -- the replayed input mask of layer l, the derivative
 // of layer l-1's activation at u[l-1] and layer l-1's output mask -- so it writes dz_{l-1} directly (for l = 0: the
-// gradient of the head input).  Each of these factors is evaluated once per element.
+// gradient of the head input).  Each of these factors is evaluated once per element.  A frozen layer (dW = db = NULL)
+// skips its weight-gradient GEMM and reduction; the input-gradient GEMMs stop where no trained layer lies below and the
+// caller wants no gradient of the head input (dx0 = NULL).
 #include <cmath>
 
 #include "common.cuh"
@@ -293,7 +295,7 @@ int fnb_mlp_check(const fnb_mlp_layer *L, int n, int64_t G, int in0, int backwar
   for (int l = 0; l < n; ++l) {
     const fnb_mlp_layer &y = L[l];
     if (!y.W || !y.b) return FNB_ERR_NULL;
-    if (backward && (!y.dW || !y.db)) return FNB_ERR_NULL;
+    if (backward && (!y.dW != !y.db)) return FNB_ERR_NULL;          // both NULL: a frozen layer
     if (y.in_dim < 1 || y.out_dim < 1 || y.in_dim != (l == 0 ? in0 : L[l - 1].out_dim)) return FNB_ERR_SIZE;
     if ((int64_t)y.in_dim * y.out_dim + y.out_dim >= INT32_MAX || G * y.in_dim >= INT32_MAX || G * y.out_dim >= INT32_MAX)
       return FNB_ERR_SIZE;
@@ -317,9 +319,16 @@ uint64_t fnb_mlp_rng(const fnb_mlp_layer *L, int n, int64_t G, uint64_t offset, 
   return c - offset;
 }
 
+bool fnb_mlp_needs_dx(const fnb_mlp_layer *L, int l, bool want_dx0) {
+  for (int j = 0; j < l; ++j)
+    if (L[j].dW) return true;
+  return want_dx0;
+}
+
 size_t fnb_mlp_dw_record_floats(const fnb_mlp_layer *L, int n, int64_t G) {
   size_t most = 0;
   for (int l = 0; l < n; ++l) {
+    if (!L[l].dW) continue;
     const int chunk = dw_chunk(G, L[l].out_dim, L[l].in_dim);
     const size_t splits = (size_t)((G + chunk - 1) / chunk);
     const size_t f = splits * ((size_t)L[l].in_dim * L[l].out_dim + L[l].out_dim);
@@ -351,22 +360,26 @@ int fnb_mlp_forward(const FnbMlpRun *r, cudaStream_t stream) {
 int fnb_mlp_backward(const FnbMlpRun *r, cudaStream_t stream) {
   const fnb_mlp_layer *L = r->L;
   for (int l = r->n - 1; l >= 0; --l) {
-    // weight and bias gradients: per-chunk records, then a fixed-order sum
-    GemmArgs w{};
-    w.A = r->dz[l]; w.B = r->xd[l]; w.M = L[l].out_dim; w.N = L[l].in_dim; w.K = (int)r->G;
-    w.k_chunk = dw_chunk(r->G, L[l].out_dim, L[l].in_dim);
-    w.rec = r->rec;
-    w.rec_stride = (int64_t)L[l].in_dim * L[l].out_dim + L[l].out_dim;
-    const int splits = (int)((r->G + w.k_chunk - 1) / w.k_chunk);
-    RC_INLINE(launch_gemm<MODE_DW>(w, splits, stream));
-    ReduceSegments segs{};
-    segs.n = 2;
-    segs.rec_off[0] = 0; segs.width[0] = L[l].in_dim * L[l].out_dim; segs.out[0] = L[l].dW;
-    segs.row_len[0] = segs.width[0]; segs.out_stride[0] = segs.width[0];
-    segs.rec_off[1] = L[l].in_dim * L[l].out_dim; segs.width[1] = L[l].out_dim; segs.out[1] = L[l].db;
-    segs.row_len[1] = L[l].out_dim; segs.out_stride[1] = L[l].out_dim;
-    RC_INLINE(fnb_launch_reduce_segments(r->rec, splits, (int)w.rec_stride, segs, stream));
-    // input gradient, folded down to dz of the layer below (or the gradient of the head input)
+    // weight and bias gradients: per-chunk records, then a fixed-order sum (not for a frozen layer)
+    if (L[l].dW) {
+      GemmArgs w{};
+      w.A = r->dz[l]; w.B = r->xd[l]; w.M = L[l].out_dim; w.N = L[l].in_dim; w.K = (int)r->G;
+      w.k_chunk = dw_chunk(r->G, L[l].out_dim, L[l].in_dim);
+      w.rec = r->rec;
+      w.rec_stride = (int64_t)L[l].in_dim * L[l].out_dim + L[l].out_dim;
+      const int splits = (int)((r->G + w.k_chunk - 1) / w.k_chunk);
+      RC_INLINE(launch_gemm<MODE_DW>(w, splits, stream));
+      ReduceSegments segs{};
+      segs.n = 2;
+      segs.rec_off[0] = 0; segs.width[0] = L[l].in_dim * L[l].out_dim; segs.out[0] = L[l].dW;
+      segs.row_len[0] = segs.width[0]; segs.out_stride[0] = segs.width[0];
+      segs.rec_off[1] = L[l].in_dim * L[l].out_dim; segs.width[1] = L[l].out_dim; segs.out[1] = L[l].db;
+      segs.row_len[1] = L[l].out_dim; segs.out_stride[1] = L[l].out_dim;
+      RC_INLINE(fnb_launch_reduce_segments(r->rec, splits, (int)w.rec_stride, segs, stream));
+    }
+    // input gradient, folded down to dz of the layer below (or the gradient of the head input): only while a trained
+    // layer lies below, or the caller wants the head input's gradient
+    if (!fnb_mlp_needs_dx(L, l, r->dx0 != nullptr)) break;
     GemmArgs d{};
     d.A = r->dz[l]; d.B = L[l].W; d.M = (int)r->G; d.N = L[l].in_dim; d.K = L[l].out_dim; d.seed = r->seed;
     d.drop1 = drop_of(L[l].p_in, r->training, r->in_base[l]);

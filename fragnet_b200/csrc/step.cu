@@ -225,8 +225,19 @@ namespace {
 
 bool ft_args_ok(const fnb_finetune_step_args *a) {
   return a && a->n_layers >= 1 && a->n_layers <= 16 && a->layers && a->batch.n_atoms >= 0 && a->batch.n_frags >= 0 &&
-         a->batch.n_bonds >= 0 && a->batch.n_graphs >= 1 &&
-         fnb_mlp_check(a->head, a->n_head_layers, a->batch.n_graphs, 2 * kD, 0) == 0;
+         a->batch.n_bonds >= 0 && a->batch.n_graphs >= 1 && a->first_trained_layer >= 0 &&
+         a->first_trained_layer <= a->n_layers && fnb_mlp_check(a->head, a->n_head_layers, a->batch.n_graphs, 2 * kD, 0) == 0;
+}
+
+// Layers 0 .. first_trained_layer - 1 of the encoder are frozen; first_trained_layer == n_layers freezes all of it: the
+// forward then saves nothing and the backward ends in the head.
+bool encoder_trained(const fnb_finetune_step_args *a) { return a->first_trained_layer < a->n_layers; }
+
+fnb_encoder_opts ft_opts_of(const fnb_finetune_step_args *a) {
+  fnb_encoder_opts o = opts_of(a);
+  o.first_trained_layer = a->first_trained_layer;
+  o.save_for_backward = a->backward && encoder_trained(a);
+  return o;
 }
 
 struct FtBufs {
@@ -242,7 +253,8 @@ struct FtBufs {
 size_t ft_layout(const fnb_finetune_step_args *a, char *base, FtBufs *out) {
   const fnb_batch_inputs *in = &a->batch;
   const fnb_batch_plan sp = sizes_plan(in);
-  const fnb_encoder_opts o = opts_of(a);
+  const fnb_encoder_opts o = ft_opts_of(a);
+  const bool enc = a->backward && encoder_trained(a);
   const int64_t Na = in->n_atoms, Nf = in->n_frags, Nb = in->n_bonds, Nfb = in->n_fbond_nodes, G = in->n_graphs;
   const fnb_mlp_layer *L = a->head;
   const int n = a->n_head_layers;
@@ -257,14 +269,18 @@ size_t ft_layout(const fnb_finetune_step_args *a, char *base, FtBufs *out) {
   b.readout = ar.take<float>(G * 2 * kD);
   if (L[0].p_in > 0.f) b.xd0 = ar.take<float>(G * 2 * kD);
   b.pred = ar.take<float>(G * L[n - 1].out_dim);
+  // backward: u[l] and dz[l] where layer l + 1's input gradient runs (dz[n-1]: the loss gradient)
   for (int l = 0; l + 1 < n; ++l) {
     b.xd[l + 1] = ar.take<float>(G * L[l].out_dim);
-    if (a->backward) b.u[l] = ar.take<float>(G * L[l].out_dim);
+    if (a->backward && fnb_mlp_needs_dx(L, l + 1, enc)) b.u[l] = ar.take<float>(G * L[l].out_dim);
   }
   if (a->backward) {
-    for (int l = 0; l < n; ++l) b.dz[l] = ar.take<float>(G * L[l].out_dim);
-    b.d_readout = ar.take<float>(G * 2 * kD);
+    for (int l = 0; l < n; ++l)
+      if (l == n - 1 || fnb_mlp_needs_dx(L, l + 1, enc)) b.dz[l] = ar.take<float>(G * L[l].out_dim);
+    if (enc) b.d_readout = ar.take<float>(G * 2 * kD);
     b.rec = ar.take<float>(fnb_mlp_dw_record_floats(L, n, G));
+  }
+  if (enc) {
     b.g_atoms = ar.take<float>(Na * kD); b.g_frags = ar.take<float>(Nf * kD);
     b.enc_bws_bytes = fnb_encoder_bwd_workspace_bytes(&sp, &o, a->layers);
     b.enc_bws = ar.bytes(b.enc_bws_bytes);
@@ -283,7 +299,7 @@ extern "C" size_t fnb_finetune_step_workspace_bytes(const fnb_finetune_step_args
 extern "C" uint64_t fnb_finetune_step_rng_span(const fnb_finetune_step_args *a) {
   if (!ft_args_ok(a)) return 0;
   const fnb_batch_plan sp = sizes_plan(&a->batch);
-  const fnb_encoder_opts o = opts_of(a);
+  const fnb_encoder_opts o = ft_opts_of(a);
   return fnb_encoder_rng_span(&sp, &o, a->layers) +
          fnb_mlp_rng(a->head, a->n_head_layers, a->batch.n_graphs, 0, nullptr, nullptr);
 }
@@ -293,13 +309,20 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
   if (!a || !workspace || !scratch) return FNB_ERR_NULL;
   if (!a->head || !a->layers) return FNB_ERR_NULL;
   if (a->n_layers < 1 || a->n_layers > 16) return FNB_ERR_SIZE;
+  if (a->first_trained_layer < 0 || a->first_trained_layer > a->n_layers) return FNB_ERR_SIZE;
   const fnb_batch_inputs *in = &a->batch;
   if (in->n_atoms < 1 || in->n_bonds < 0 || in->n_frags < 0 || in->n_graphs < 1 || !in->batch || !in->frag_batch)
     return FNB_ERR_SIZE;
   RC(fnb_mlp_check(a->head, a->n_head_layers, in->n_graphs, 2 * kD, a->backward));
   if (a->loss_kind != FNB_LOSS_MSE && a->loss_kind != FNB_LOSS_BCE_MASKED) return FNB_ERR_MODE;
   if (!a->loss || !a->target || !a->x_atoms || !a->x_bond || !a->x_fbond) return FNB_ERR_NULL;
-  if (a->backward && !a->layer_grads) return FNB_ERR_NULL;
+  const bool enc_bwd = a->backward && encoder_trained(a);
+  if (a->backward && !enc_bwd) {   // a backward that trains nothing is a caller's mistake
+    bool head_trained = false;
+    for (int l = 0; l < a->n_head_layers; ++l) head_trained |= a->head[l].dW != nullptr;
+    if (!head_trained) return FNB_ERR_MODE;
+  }
+  if (enc_bwd && !a->layer_grads) return FNB_ERR_NULL;
   if (reinterpret_cast<uintptr_t>(workspace) & 255u) return FNB_ERR_ALIGN;
   FtBufs B;
   if (ft_layout(a, (char *)workspace, &B) > workspace_bytes) return FNB_ERR_WORKSPACE;
@@ -312,7 +335,7 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
   FnbAux aux{};
   const bool two = fnb_aux_streams(&aux) == 0;
   fnb_batch_plan plan{};
-  fnb_encoder_opts o = opts_of(a);
+  fnb_encoder_opts o = ft_opts_of(a);
   fnb_encoder_io eio{};
   eio.x_atoms = a->x_atoms; eio.x_bond = a->x_bond; eio.x_fbond = a->x_fbond;
   eio.out_atoms = B.out_atoms; eio.out_frags = B.out_frags; eio.out_bond = B.out_bond; eio.out_fbond = B.out_fbond;
@@ -341,10 +364,11 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
     RC(fnb_bce_masked_loss(r.out, a->target, n_out, a->loss, d_pred, s));
   }
   if (!a->backward) return 0;
-  // ---- head backward, readout backward, encoder backward
+  // ---- head backward, readout backward, encoder backward (the last two only where the encoder trains)
   for (int l = 0; l < n; ++l) r.dz[l] = B.dz[l];
   r.dx0 = B.d_readout; r.rec = B.rec;
   RC(fnb_mlp_backward(&r, s));
+  if (!enc_bwd) return 0;
   RC(fnb_segment_gather(B.d_readout, 2 * kD, plan.batch32, in->n_atoms, nullptr, B.g_atoms, stream));
   RC(fnb_segment_gather(B.d_readout + kD, 2 * kD, plan.frag_batch32, in->n_frags, nullptr, B.g_frags, stream));
   eio.g_atoms = B.g_atoms; eio.g_frags = B.g_frags; eio.g_bond = nullptr; eio.g_fbond = nullptr;

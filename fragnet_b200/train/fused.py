@@ -14,6 +14,9 @@ into one flat buffer and their ``.grad`` are views into a second one.
 
 ``FusedFineTuneStep`` does the same for a ``FragNetFineTune`` model and the finetuning loop's body
 (fragnet/train/utils.py:330-470: ``model(batch)`` -> MSE or masked BCE -> backward -> Adam) with ``fnb_finetune_step``.
+It honours frozen parameters (``requires_grad = False``) in the layout the library supports -- the lower encoder layers
+or the whole encoder, and any of the head's linears: only the trained tensors are re-homed and updated, and the
+backward stops below the lowest trained layer.
 """
 from __future__ import annotations
 
@@ -72,6 +75,7 @@ class _FlatStep:
         self.exp_avg = torch.zeros_like(self.flat_p)
         self.exp_avg_sq = torch.zeros_like(self.flat_p)
         self.t = 0
+        self._adam_runs = [(0, self.flat_p.numel(), 0)]    # (first, end, steps behind self.t) of the flat buffer
         self._p_views = p_views
         self._ws: Optional[torch.Tensor] = None
         self._loss = torch.zeros(8, dtype=torch.float32, device=dev)      # ring of loss scalars
@@ -90,31 +94,49 @@ class _FlatStep:
 
     def attach_optimizer(self, optimizer) -> None:
         """Keep a caller-owned ``torch.optim.Adam`` truthful: its ``state`` entries of the live parameters become VIEWS
-        of this object's moment buffers plus a shared step counter, so ``optimizer.state_dict()`` checkpoints the real
-        state; moments already present in ``optimizer.state`` (a resumed run) are adopted first."""
+        of this object's moment buffers plus step counters, so ``optimizer.state_dict()`` checkpoints the real state;
+        moments already present in ``optimizer.state`` (a resumed run) are adopted first.  Step counts stay per
+        parameter, as in ``torch.optim.Adam``: when some parameters have state and others not (a layer unfrozen
+        after the others trained for a while), the new ones start from step 1."""
         from .optim import flat_views
         _, m_views = flat_views(self.live, self.dev, storage=self.exp_avg)
         _, v_views = flat_views(self.live, self.dev, storage=self.exp_avg_sq)
-        steps = [int(optimizer.state[p]["step"]) for p in self.live if p in optimizer.state and "step" in optimizer.state[p]]
+        steps = [int(optimizer.state[p]["step"]) if "step" in optimizer.state.get(p, {}) else None for p in self.live]
         with torch.no_grad():
             for p, m, v in zip(self.live, m_views, v_views):
                 st = optimizer.state.get(p)
                 if st and "exp_avg" in st:
                     m.copy_(st["exp_avg"])
                     v.copy_(st["exp_avg_sq"])
-        if steps:
-            self.t = max(steps)
-        self._opt_step = torch.tensor(float(self.t))
-        for p, m, v in zip(self.live, m_views, v_views):
-            optimizer.state[p] = {"step": self._opt_step, "exp_avg": m, "exp_avg_sq": v}
+        known = [s for s in steps if s is not None]
+        if known:
+            self.t = max(known)
+        lags = [self.t - s if s is not None else (self.t if known else 0) for s in steps]
+        # contiguous runs of the flat buffer whose parameters are equally many steps behind (one run in a plain run)
+        base = self.flat_p.data_ptr()
+        starts = [(v.data_ptr() - base) // self.flat_p.element_size() for v in self._p_views] + [self.flat_p.numel()]
+        self._adam_runs = []
+        for i, lag in enumerate(lags):
+            if self._adam_runs and self._adam_runs[-1][2] == lag:
+                self._adam_runs[-1] = (self._adam_runs[-1][0], starts[i + 1], lag)
+            else:
+                self._adam_runs.append((starts[i], starts[i + 1], lag))
+        self._opt_steps = {lag: torch.tensor(float(self.t - lag)) for lag in set(lags)}
+        for p, m, v, lag in zip(self.live, m_views, v_views, lags):
+            optimizer.state[p] = {"step": self._opt_steps[lag], "exp_avg": m, "exp_avg_sq": v}
+
+    def _sync_opt_steps(self) -> None:
+        for lag, t in getattr(self, "_opt_steps", {}).items():
+            t.fill_(float(self.t - lag))
 
     def _adam(self) -> None:
-        """``fnb_adam_step`` over the flat buffers at step ``self.t``."""
-        _abi.check(ops._lib().fnb_adam_step(ops._p(self.flat_p), ops._p(self.flat_g), ops._p(self.exp_avg),
-                                            ops._p(self.exp_avg_sq), self.flat_p.numel(), self.lr, self.betas[0],
-                                            self.betas[1], self.eps, self.weight_decay, self.t, ops._stream()), "adam_step")
-        if getattr(self, "_opt_step", None) is not None:
-            self._opt_step.fill_(float(self.t))
+        """``fnb_adam_step`` over the flat buffers at step ``self.t`` (one launch per run of equal step counts)."""
+        for lo, hi, lag in self._adam_runs:
+            _abi.check(ops._lib().fnb_adam_step(
+                ops._p(self.flat_p[lo:]), ops._p(self.flat_g[lo:]), ops._p(self.exp_avg[lo:]),
+                ops._p(self.exp_avg_sq[lo:]), hi - lo, self.lr, self.betas[0], self.betas[1], self.eps,
+                self.weight_decay, self.t - lag, ops._stream()), "adam_step")
+        self._sync_opt_steps()
 
     def _next_loss(self) -> torch.Tensor:
         self._loss_i = (self._loss_i + 1) % self._loss.numel()
@@ -390,8 +412,7 @@ class FusedPretrainStep(_FlatStep):
                 C.byref(self._peers), ops._p(self.flat_p), ops._p(self.exp_avg), ops._p(self.exp_avg_sq),
                 self.flat_p.numel(), self.lr, self.betas[0], self.betas[1], self.eps, self.weight_decay, self.t,
                 self._epoch & 0xFFFFFFFF, ops._p(self._done), ops._stream()), "allreduce_adam_step")
-            if getattr(self, "_opt_step", None) is not None:
-                self._opt_step.fill_(float(self.t))
+            self._sync_opt_steps()
             return loss
         if w > 1:
             dist.all_reduce(self.flat_g, op=dist.ReduceOp.SUM, group=self.group)
@@ -440,21 +461,57 @@ class FusedFineTuneStep(_FlatStep):
     collate, encoder, readout, head, loss and every gradient in one ``fnb_finetune_step`` call, then Adam over the flat
     buffers (hyper-parameters as ``torch.optim.Adam``).  ``loss``: ``"mse"`` (``nn.MSELoss`` over the flattened
     predictions, ``TrainerFineTune.train_regr``) or ``"bce"`` (BCE-with-logits over the labels > -0.5,
-    ``TrainerFineTune.train_clsf_bce``).  Models the library does not cover raise ``NotImplementedError``: other heads
-    or activations (PReLU and RReLU among them), the lite / edge variants, other encoder geometries, several ranks."""
+    ``TrainerFineTune.train_clsf_bce``).
+
+    Frozen parameters (``requires_grad = False``, read at construction) are honoured: the trained set is the library's
+    live tensors that require a gradient, and only those go into the flat buffers and get Adam state; frozen tensors
+    keep their storage and their ``.grad``.  The library freezes whole units: all live tensors of one encoder layer (the
+    last layer's ``f`` included), ``weight`` and ``bias`` of one head linear, and frozen encoder layers must be the
+    lowest ones (``0 .. k-1``, or all of them).  The backward then stops at the lowest trained layer.
+
+    Models the library does not cover raise ``NotImplementedError``: other heads or activations (PReLU and RReLU among
+    them), the lite / edge variants, other encoder geometries, several ranks, other freezing patterns (a frozen layer
+    above a trained one, a frozen tensor inside a trained layer or linear) and a model with nothing to train."""
 
     _NATIVE = "finetune_step"
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.0,
                  loss: str = "mse"):
+        if loss not in ("mse", "bce"):
+            raise ValueError(f"FusedFineTuneStep: loss must be 'mse' or 'bce', got {loss!r}")
+        spec, layer_params, units, live, self.first_trained_layer = self._analyse(model)
+        self.model, self.loss_kind = model, loss
+        self.lr, self.betas, self.eps, self.weight_decay = float(lr), betas, float(eps), float(weight_decay)
+        self.dev = dev = ops.require_cuda(model.pretrain.layers[0].a.device)
+        if any(p.dtype != torch.float32 or p.device != dev for u in units for p in u):
+            raise ValueError("FusedFineTuneStep needs fp32 parameters on one CUDA device")
+        self._requires = [p.requires_grad for u in units for p in u]
+        n_layers = len(layer_params)
+        g_views = self._bind_flat(live, dev)
+        grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
+        self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of)
+        self._head = (_abi.CMlpLayer * len(spec))()
+        for h, (lin, p_in, p_out, act) in zip(self._head, spec):
+            h.W, h.b = lin.weight.data_ptr(), lin.bias.data_ptr()
+            if id(lin.weight) in grad_of:                   # frozen linear: dW = db = NULL
+                h.dW, h.db = grad_of[id(lin.weight)].data_ptr(), grad_of[id(lin.bias)].data_ptr()
+            h.in_dim, h.out_dim, h.p_in, h.p_out, h.act = lin.in_features, lin.out_features, p_in, p_out, act
+        self.n_classes = self._y_width = spec[-1][0].out_features
+        self._head_drops = any(p_in > 0 or p_out > 0 for _, p_in, p_out, _ in spec)
+        self._keep = (layer_params, self._p_views, g_views)
+        self._units = units
+        self.n_layers = n_layers
+
+    @staticmethod
+    def _analyse(model):
+        """(head spec, encoder live tensors per layer, freezable units, trained tensors in flat-buffer order, first
+        trained encoder layer) of a model, or ``NotImplementedError`` for one the library does not cover."""
         from ..model.gat import gat2
         if type(model) is not gat2.FragNetFineTune:
             raise NotImplementedError("FusedFineTuneStep needs fragnet_b200's gat2 FragNetFineTune "
                                       f"(got {type(model).__module__}.{type(model).__name__})")
         if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
             raise NotImplementedError("FusedFineTuneStep runs on one GPU")
-        if loss not in ("mse", "bce"):
-            raise ValueError(f"FusedFineTuneStep: loss must be 'mse' or 'bce', got {loss!r}")
         enc = model.pretrain
         spec = _head_layers(getattr(model, "fthead", None))
         if spec is None or any(act is None for _, _, _, act in spec):
@@ -464,30 +521,36 @@ class FusedFineTuneStep(_FlatStep):
             raise NotImplementedError("FusedFineTuneStep: unsupported head shape")
         for layer in enc.layers:
             layer._check_geometry()
-        self.model, self.loss_kind = model, loss
-        self.lr, self.betas, self.eps, self.weight_decay = float(lr), betas, float(eps), float(weight_decay)
-        self.dev = dev = ops.require_cuda(enc.layers[0].a.device)
         n_layers = len(enc.layers)
         layer_params = [list(layer._live_parameters()) for layer in enc.layers]
-        live: List[torch.nn.Parameter] = []
-        for li, ps in enumerate(layer_params):
-            live += [p for j, p in enumerate(ps) if j != _F_INDEX or li == n_layers - 1]
-        for lin, _, _, _ in spec:
-            live += [lin.weight, lin.bias]
-        if any(p.dtype != torch.float32 or p.device != dev for p in live):
-            raise ValueError("FusedFineTuneStep needs fp32 parameters on one CUDA device")
-        g_views = self._bind_flat(live, dev)
-        grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
-        self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of)
-        self._head = (_abi.CMlpLayer * len(spec))()
-        for h, (lin, p_in, p_out, act) in zip(self._head, spec):
-            h.W, h.b = lin.weight.data_ptr(), lin.bias.data_ptr()
-            h.dW, h.db = grad_of[id(lin.weight)].data_ptr(), grad_of[id(lin.bias)].data_ptr()
-            h.in_dim, h.out_dim, h.p_in, h.p_out, h.act = lin.in_features, lin.out_features, p_in, p_out, act
-        self.n_classes = self._y_width = spec[-1][0].out_features
-        self._head_drops = any(p_in > 0 or p_out > 0 for _, p_in, p_out, _ in spec)
-        self._keep = (layer_params, self._p_views, g_views)
-        self.n_layers = n_layers
+        # the library's live tensors per unit it can freeze: encoder layers (the dead f of lower layers left out), then
+        # the head's linears
+        units = [[p for j, p in enumerate(ps) if j != _F_INDEX or li == n_layers - 1] for li, ps in enumerate(layer_params)]
+        units += [[lin.weight, lin.bias] for lin, _, _, _ in spec]
+        trained = []
+        for u in units:
+            if len({p.requires_grad for p in u}) > 1:
+                raise NotImplementedError("FusedFineTuneStep: every live tensor of an encoder layer, and weight and bias "
+                                          "of a head linear, must be frozen or trained together")
+            trained.append(u[0].requires_grad)
+        enc_trained = trained[:n_layers]
+        first = enc_trained.index(True) if any(enc_trained) else n_layers
+        if not all(enc_trained[first:]):
+            raise NotImplementedError("FusedFineTuneStep: frozen encoder layers must be the lowest ones (0 .. k-1)")
+        live = [p for u, t in zip(units, trained) if t for p in u]
+        if not live:
+            raise NotImplementedError("FusedFineTuneStep: the model has no parameter to train")
+        return spec, layer_params, units, live, first
+
+    @classmethod
+    def trained_parameters(cls, model) -> List[torch.nn.Parameter]:
+        """The tensors a step built for ``model`` now would train (``NotImplementedError`` as the constructor)."""
+        return cls._analyse(model)[3]
+
+    def bound_to_model(self) -> bool:
+        """As ``_FlatStep.bound_to_model, and False as well once a parameter's ``requires_grad`` has changed since
+        construction (the trained set is fixed here)."""
+        return super().bound_to_model() and [p.requires_grad for u in self._units for p in u] == self._requires
 
     def _draws(self, a) -> bool:
         return bool(a.training and (a.drop_p > 0 or self._head_drops))
@@ -512,6 +575,7 @@ class FusedFineTuneStep(_FlatStep):
         a.drop_p, a.training = float(self.model.pretrain.dropout.p), int(bool(self.model.training))
         a.seed, a.offset = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF, 0
         a.precision, a.backward = config.precision_id(), int(backward)
+        a.first_trained_layer = self.first_trained_layer
         loss = self._next_loss()
         a.loss = loss.data_ptr()
         preds = None

@@ -10,8 +10,10 @@ on the device and read back once per epoch instead of one ``loss.item()`` synchr
 
 ``TrainerFineTune(..., fused=True)`` runs each training batch of this package's ``FragNetFineTune`` as one library call
 (``FusedFineTuneStep``: collate, encoder, readout, head, loss, backward, then Adam over flat buffers) when the
-optimizer is a plain ``torch.optim.Adam`` and the model is one the library covers; anything else silently takes the
-generic loop below.  Validation and test always call ``model(batch)``.
+optimizer is a plain ``torch.optim.Adam`` holding every trained tensor in its one parameter group and the model is one
+the library covers, frozen parameters included (the lower encoder layers or the whole encoder, any head linear);
+anything else silently takes the generic loop below.  A change of ``requires_grad`` between epochs (unfreezing the
+encoder after a warm-up) rebuilds the fused step.  Validation and test always call ``model(batch)``.
 """
 from __future__ import annotations
 
@@ -90,7 +92,8 @@ class TrainerFineTune:
         self.target_pos = target_pos
         self.n_multi_task_heads = n_multi_task_heads
         self.fused = fused
-        self._fused_steps = []       # [(weakref(model), weakref(optimizer), FusedFineTuneStep | None)]
+        # [(weakref(model), weakref(optimizer), FusedFineTuneStep | None, requires_grad of the model's parameters)]
+        self._fused_steps = []
         if target_type == "regr":
             self.train, self.validate, self.test = self.train_regr, self.validate_regr, self.test_regr
             self.loss_fn = nn.MSELoss()
@@ -128,19 +131,28 @@ class TrainerFineTune:
         if not (ok and _plain_adam(optimizer) and torch.is_tensor(p0) and p0.is_cuda):
             return None
         import weakref
-        self._fused_steps = [e for e in self._fused_steps if e[0]() is not None and e[1]() is not None]
-        for wm, wo, fs in self._fused_steps:
-            if wm() is model and wo() is optimizer:
-                return fs if fs is not None and fs.bound_to_model() else None
-        from .fused import FusedFineTuneStep
+        frozen = tuple(p.requires_grad for p in model.parameters())
+        # a step is built for one set of trained tensors: after a requires_grad change it is rebuilt
+        self._fused_steps = [e for e in self._fused_steps if e[0]() is not None and e[1]() is not None and
+                             not (e[0]() is model and e[1]() is optimizer and e[3] != frozen)]
         g = optimizer.param_groups[0]
+        owned = {id(p) for p in g["params"]}
+        for wm, wo, fs, _ in self._fused_steps:
+            if wm() is model and wo() is optimizer:
+                ok = fs is not None and fs.bound_to_model() and all(id(p) in owned for p in fs.live)
+                return fs if ok else None
+        from .fused import FusedFineTuneStep
+        fs = None
         try:
-            fs = FusedFineTuneStep(model, lr=g["lr"], betas=g["betas"], eps=g["eps"], weight_decay=g["weight_decay"],
-                                   loss=loss)
-            fs.attach_optimizer(optimizer)          # optimizer.state_dict() keeps checkpointing the real moments
+            # every trained tensor must be the optimizer's: the generic loop's Adam updates nothing else (frozen or
+            # gradient-less tensors in the optimizer are skipped by both paths)
+            if all(id(p) in owned for p in FusedFineTuneStep.trained_parameters(model)):
+                fs = FusedFineTuneStep(model, lr=g["lr"], betas=g["betas"], eps=g["eps"],
+                                       weight_decay=g["weight_decay"], loss=loss)
+                fs.attach_optimizer(optimizer)      # optimizer.state_dict() keeps checkpointing the real moments
         except NotImplementedError:
             fs = None
-        self._fused_steps.append((weakref.ref(model), weakref.ref(optimizer), fs))
+        self._fused_steps.append((weakref.ref(model), weakref.ref(optimizer), fs, frozen))
         return fs
 
     @staticmethod

@@ -36,7 +36,7 @@ extern "C" {
 
 #define FNB_D 128 /* embedding width  */
 #define FNB_H 4   /* attention heads  */
-#define FNB_ABI_VERSION 11
+#define FNB_ABI_VERSION 12
 
 /* arithmetic of the dense projections */
 #define FNB_PRECISION_FP32 0 /* FP32 FFMA: bit-for-bit comparable with the reference within 1e-5            */
@@ -279,6 +279,11 @@ typedef struct fnb_encoder_opts {
                                                      need_dx_atoms only selects where input dropout runs (its own
                                                      kernel instead of the padding kernel); the backward is right
                                                      whichever values the forward call had */
+  int first_trained_layer; /* 0 .. n_layers: layers below it are frozen (finetuning a pretrained encoder).  The
+                              forward saves nothing of theirs for the backward (smaller workspaces); the backward
+                              does not visit them, and layer first_trained_layer writes its parameter gradients but
+                              no input gradient, so dx_* are written only when it is 0 (see need_dx_*).  Dropout
+                              counters are the same whatever its value.  0 = train every layer. */
 } fnb_encoder_opts;
 
 typedef struct fnb_encoder_io {
@@ -306,7 +311,8 @@ uint64_t fnb_encoder_rng_span(const fnb_batch_plan *plan, const fnb_encoder_opts
 int fnb_encoder_forward(const fnb_batch_plan *plan, const fnb_encoder_opts *opts, const fnb_layer_params *layers,
                         const fnb_encoder_io *io, void *workspace, size_t workspace_bytes, void *scratch,
                         void *stream);
-/* workspace = the forward call's workspace (unchanged since), bwd_workspace = fnb_encoder_bwd_workspace_bytes(). */
+/* workspace = the forward call's workspace (unchanged since), bwd_workspace = fnb_encoder_bwd_workspace_bytes().
+ * grads: one entry per layer; the entries of layers below first_trained_layer are not read (may be all NULL). */
 int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encoder_opts *opts, const fnb_layer_params *layers,
                          const fnb_layer_grads *grads, const fnb_encoder_io *io, void *workspace,
                          size_t workspace_bytes, void *bwd_workspace, size_t bwd_workspace_bytes, void *scratch,
@@ -487,7 +493,9 @@ int fnb_pretrain_plan_prefetch(const fnb_batch_inputs *next, void *arena, size_t
 #define FNB_MLP_MAX_LAYERS 8
 typedef struct fnb_mlp_layer {
   const float *W, *b;  /* nn.Linear weight [out,in] and bias [out] */
-  float *dW, *db;      /* their gradients (backward only; written) */
+  float *dW, *db;      /* their gradients (backward only; written).  Both NULL: the layer is frozen -- no weight
+                          gradient is formed, and its input gradient only where a trained layer lies below it or the
+                          encoder trains */
   int in_dim, out_dim; /* any positive widths; in_dim of layer 0 = 2 * FNB_D (the readout), of layer l = out_dim of l-1 */
   float p_in, p_out;   /* dropout probability on the layer's input / on its pre-activation output; 0 = none */
   int act;             /* FNB_ACT_* */
@@ -517,6 +525,11 @@ typedef struct fnb_finetune_step_args {
   float *loss;                              /* device scalar */
   float *predictions;                       /* optional [G, n_classes] output */
   const void *plan_arena;                   /* NULL, or an arena fnb_pretrain_plan_prefetch() filled for `batch` */
+  int first_trained_layer;                  /* 0 .. n_layers (else FNB_ERR_SIZE): encoder layers below it are frozen,
+                                               as fnb_encoder_opts.first_trained_layer; their layer_grads entries may
+                                               be NULL.  n_layers freezes the encoder: no encoder backward, no readout
+                                               backward, layer_grads may be NULL.  A backward that trains nothing
+                                               (this at n_layers and every head layer frozen) is FNB_ERR_MODE. */
 } fnb_finetune_step_args;
 size_t fnb_finetune_step_workspace_bytes(const fnb_finetune_step_args *args);
 uint64_t fnb_finetune_step_rng_span(const fnb_finetune_step_args *args);

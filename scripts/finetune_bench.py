@@ -7,6 +7,10 @@ model on the same batches; the autograd leg is the loop body of ``TrainerFineTun
 ``MSELoss(model(b).view(-1), y)``, backward, ``optimizer.step()``) with the per-batch losses summed on the device.
 The legs alternate, ``--rounds`` times each.
 
+``--freeze`` also times the usual finetuning set-ups with frozen parameters (``requires_grad = False``): ``lower2``
+freezes encoder layers 0 and 1, ``encoder`` the whole encoder.  Both legs then train the same tensors: the autograd leg's
+Adam holds the trainable ones, and the fused step stops its backward below the lowest trained layer.
+
 Per leg and batch size: ms per step (host clock around the timed steps, ending in a device synchronise),
 molecules/s, host enqueue ms per step (the same clock before the synchronise) and library launches per step
 (``fnb_launch_count``).  Prints one JSON line, with the card's name and power limit read in the same run."""
@@ -29,6 +33,7 @@ FT_KW = dict(n_classes=1, num_layer=4, drop_ratio=0.1, num_heads=4, emb_dim=128,
              act="relu", fthead="FTHead3")
 LR = 1e-4
 L2_BYTES = 126 * 2 ** 20
+FREEZE = {"none": 0, "lower2": 2, "encoder": FT_KW["num_layer"]}     # encoder layers frozen from the bottom
 
 
 def card():
@@ -88,7 +93,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--rounds", type=int, default=2, help="alternations of the two legs per batch size")
     ap.add_argument("--pool", type=int, default=1128, help="distinct synthetic molecules (ESOL has 1 128)")
+    ap.add_argument("--freeze", default="none", help=f"comma separated, of {', '.join(FREEZE)}")
     args = ap.parse_args()
+    modes = args.freeze.split(",")
+    if any(m not in FREEZE for m in modes):
+        raise SystemExit(f"--freeze: expected names from {sorted(FREEZE)}, got {args.freeze!r}")
     if not torch.cuda.is_available():
         raise SystemExit("finetune_bench.py needs a CUDA device")
     from fragnet.model.gat.gat2 import FragNetFineTune
@@ -96,13 +105,16 @@ def main():
     result = {"workload": "FragNetFineTune exps/ft/esol/e1pt4.yaml training step (fwd + MSE + bwd + Adam), "
                           "ESOL-shaped synthetic batches resident in HBM", "card": card(), "steps": args.steps,
               "warmup": args.warmup, "rounds": args.rounds, "legs": {}}
-    for batch in (int(x) for x in args.batches.split(",")):
+    for batch, mode in ((int(x), m) for x in args.batches.split(",") for m in modes):
         batches, nbytes = make_batches(batch, args.pool, seed=7)
         torch.manual_seed(0)
         m_fused = FragNetFineTune(**FT_KW).cuda().train()
+        for layer in m_fused.pretrain.layers[:FREEZE[mode]]:
+            for p in layer.parameters():
+                p.requires_grad_(False)
         m_auto = copy.deepcopy(m_fused)
         fused = FusedFineTuneStep(m_fused, lr=LR)
-        opt = torch.optim.Adam(m_auto.parameters(), lr=LR)
+        opt = torch.optim.Adam([p for p in m_auto.parameters() if p.requires_grad], lr=LR)
         loss_fn = torch.nn.MSELoss()
         nb = len(batches)
 
@@ -128,7 +140,7 @@ def main():
                          "host_enqueue_ms_per_step": round(enq, 3), "fnb_launches_per_step": round(launches, 1),
                          "ms_per_step_all_rounds": [round(r[0], 3) for r in runs]}
         out["speedup"] = round(out["autograd"]["ms_per_step"] / out["fused"]["ms_per_step"], 2)
-        result["legs"][f"batch_{batch}"] = out
+        result["legs"][f"batch_{batch}" + ("" if mode == "none" else f"_freeze_{mode}")] = out
         del batches, fused, m_fused, m_auto, opt
         torch.cuda.empty_cache()
     result["card_after"] = card()
