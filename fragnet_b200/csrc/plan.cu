@@ -4,11 +4,13 @@
 // What this replaces in the reference: torch_scatter groups edges implicitly on EVERY scatter_softmax / scatter_add
 // call (fragnet/model/gat/gat2.py:153-165, 210-219, 234, 257-268, 303-312, 820-821), torch_geometric's add_self_loops
 // (gat2.py:179) re-concatenates the edge list in every layer.  Here the grouping is done once per batch and shared
-// by all layers, forward and backward.  csr.cu builds one graph per call (~9 launches each); this file runs the same
-// counting sort over the CONCATENATION of the five edge lists, so a batch costs 9 launches in total:
+// by all layers, forward and backward.  One counting sort runs over the CONCATENATION of the five edge lists, so a
+// batch costs 9 launches in total:
 //   memset, histogram, 3-launch exclusive scan, slot claim, rank (forward), rank (reverse), aux (narrowing, offsets).
+// fnb_csr_build runs the same sort (counting_sort below) over one caller's graph, with the other four graphs empty.
 // Bit-exactness contract (tested against torch.sort(stable=True)): slots of one destination (source) are ordered by
 // edge id; the only non-deterministic step (the atomic slot claim) is followed by a rank-by-counting pass.
+// Also here: the small standalone index helpers fnb_gather_rows, fnb_segment_offsets and fnb_narrow_index.
 #include "common.cuh"
 
 namespace {
@@ -244,10 +246,12 @@ struct AuxArgs {
   int *a2f32, *batch32, *frag_batch32, *atom_ptr, *frag_ptr;
   int n_atoms, n_frags, n_graphs;
 };
-__device__ __forceinline__ int lower_bound64(const int64_t *ids, int n, int64_t key) {
-  int lo = 0, hi = n;
+// First position i in [0, n) with ids[i] >= key (ids sorted ascending); I is the index type of the caller's loop.
+template <class I>
+__device__ __forceinline__ I lower_bound64(const int64_t *ids, I n, int64_t key) {
+  I lo = 0, hi = n;
   while (lo < hi) {
-    const int mid = (lo + hi) >> 1;
+    const I mid = (lo + hi) >> 1;
     if (ids[mid] < key) lo = mid + 1; else hi = mid;
   }
   return lo;
@@ -270,18 +274,70 @@ __global__ void k_plan_aux(AuxArgs a) {
     }
 }
 
+// ---- standalone index helpers (fnb_gather_rows, fnb_segment_offsets, fnb_narrow_index)
+__global__ void k_gather_rows(const float *__restrict__ in, const int *__restrict__ index, int64_t n_rows, int width,
+                              float *__restrict__ out) {
+  const int64_t total = n_rows * width;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / width;
+    const int c = (int)(i - r * width);
+    out[i] = in[(int64_t)index[r] * width + c];
+  }
+}
+
+__global__ void k_segment_offsets(const int64_t *__restrict__ ids, int64_t n, int64_t n_segments,
+                                  int *__restrict__ offsets) {
+  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g <= n_segments;
+       g += (int64_t)gridDim.x * blockDim.x)
+    offsets[g] = (int)lower_bound64(ids, n, g);
+}
+
+__global__ void k_narrow(const int64_t *__restrict__ in, int64_t n, int *__restrict__ out) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    out[i] = (int)in[i];
+}
+
+template <class T>
+T *take(char *base, size_t &off, size_t n) {
+  off = (off + 255) & ~(size_t)255;
+  T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
+  off += n * sizeof(T);
+  return p;
+}
+
+// Temporaries of one counting sort over n_nodes counters and n_edges edges (all graphs of a PlanArgs together).
+struct SortTemps {
+  int *cnt_dst, *cnt_src, *x_dst, *x_src, *tmp_eid, *tmp_reid, *tiles0, *tiles1;
+  size_t cnt_bytes;   // cnt_dst and cnt_src are adjacent: one memset
+};
+
+SortTemps take_sort_temps(char *base, size_t &off, int64_t n_nodes, int64_t n_edges) {
+  SortTemps t;
+  t.cnt_dst = take<int>(base, off, n_nodes);
+  t.cnt_src = take<int>(base, off, n_nodes);
+  t.cnt_bytes = base ? (size_t)(reinterpret_cast<char *>(t.cnt_src) - reinterpret_cast<char *>(t.cnt_dst)) +
+                           (size_t)n_nodes * 4
+                     : 0;
+  t.x_dst = take<int>(base, off, n_nodes + 1);
+  t.x_src = take<int>(base, off, n_nodes + 1);
+  t.tmp_eid = take<int>(base, off, n_edges);
+  t.tmp_reid = take<int>(base, off, n_edges);
+  const int64_t n_tiles = (n_nodes + kScanTile - 1) / kScanTile;
+  t.tiles0 = take<int>(base, off, n_tiles + 1);
+  t.tiles1 = take<int>(base, off, n_tiles + 1);
+  return t;
+}
+
 struct PlanLayout {
   // outputs
   int *rowptr[PG], *col[PG], *row[PG], *eid[PG], *slot_of_eid[PG], *rrowptr[PG], *rslot[PG], *rdst[PG];
   float *attr_bond, *attr_fbond;
   int *a2f32, *batch32, *frag_batch32, *atom_ptr, *frag_ptr, *status;
-  // temporaries
-  int *cnt_dst, *cnt_src, *x_dst, *x_src, *tmp_eid, *tmp_reid, *tiles0, *tiles1;
-  size_t cnt_bytes;   // cnt_dst and cnt_src are adjacent: one memset
+  SortTemps t;
   size_t total;
 };
 
-struct Sz { int n_nodes[PG], n_total[PG], reverse[PG]; int e_total, n_total_nodes, n_tiles; };
+struct Sz { int n_nodes[PG], n_total[PG], reverse[PG]; int e_total, n_total_nodes; };
 
 Sz sizes(const fnb_batch_inputs *in) {
   Sz z;
@@ -293,16 +349,7 @@ Sz sizes(const fnb_batch_inputs *in) {
     z.n_nodes[i] = (int)nn[i]; z.n_total[i] = (int)ne[i]; z.reverse[i] = rev[i];
     z.e_total += (int)ne[i]; z.n_total_nodes += (int)nn[i];
   }
-  z.n_tiles = (z.n_total_nodes + kScanTile - 1) / kScanTile;
   return z;
-}
-
-template <class T>
-T *take(char *base, size_t &off, size_t n) {
-  off = (off + 255) & ~(size_t)255;
-  T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
-  off += n * sizeof(T);
-  return p;
 }
 
 PlanLayout plan_layout(const fnb_batch_inputs *in, char *base) {
@@ -329,19 +376,25 @@ PlanLayout plan_layout(const fnb_batch_inputs *in, char *base) {
   L.atom_ptr = take<int>(base, off, (size_t)in->n_graphs + 1);
   L.frag_ptr = take<int>(base, off, (size_t)in->n_graphs + 1);
   L.status = take<int>(base, off, 1);    // index error
-  L.cnt_dst = take<int>(base, off, (size_t)z.n_total_nodes);
-  {
-    char *before = reinterpret_cast<char *>(L.cnt_dst);
-    L.cnt_src = take<int>(base, off, (size_t)z.n_total_nodes);
-    L.cnt_bytes = base ? (size_t)(reinterpret_cast<char *>(L.cnt_src) - before) + (size_t)z.n_total_nodes * 4 : 0;
-  }
-  L.x_dst = take<int>(base, off, (size_t)z.n_total_nodes + 1);
-  L.x_src = take<int>(base, off, (size_t)z.n_total_nodes + 1);
-  L.tmp_eid = take<int>(base, off, z.e_total);
-  L.tmp_reid = take<int>(base, off, z.e_total);
-  L.tiles0 = take<int>(base, off, (size_t)z.n_tiles + 1);
-  L.tiles1 = take<int>(base, off, (size_t)z.n_tiles + 1);
+  L.t = take_sort_temps(base, off, z.n_total_nodes, z.e_total);
   L.total = (off + 255) & ~(size_t)255;
+  return L;
+}
+
+// fnb_csr_build's workspace: the sort temporaries and two spare words -- rowptr[0] of the four empty graphs, and the
+// status word when the caller passes none.
+struct CsrLayout {
+  SortTemps t;
+  int *spare;
+  size_t total;
+};
+
+CsrLayout csr_layout(int64_t n_nodes, int64_t n_edges_total, char *base) {
+  CsrLayout L;
+  size_t off = 0;
+  L.t = take_sort_temps(base, off, n_nodes, n_edges_total);
+  L.spare = take<int>(base, off, 2);
+  L.total = off;
   return L;
 }
 
@@ -364,6 +417,10 @@ inline int grid_for(int64_t n) {
   return (int)g;
 }
 
+// The k_plan_* kernels index edges and nodes with int and stride by up to one grid_for() grid (kNumSMs * 16 blocks of
+// 256 threads): a sort of at most this many edges or nodes keeps every index plus one stride inside int32.
+constexpr int64_t kMaxSortItems = (int64_t)INT32_MAX - (int64_t)kNumSMs * 16 * 256;
+
 // The plan struct over a laid-out arena (pure function of the inputs' sizes).
 void fill_plan(const fnb_batch_inputs *in, const PlanLayout &L, const Sz &z, fnb_batch_plan *out) {
   const int n_real[PG] = {(int)in->n_bond_edges, (int)in->n_bonds, (int)in->n_fbond_edges, (int)in->n_fbond_nodes,
@@ -383,6 +440,54 @@ void fill_plan(const fnb_batch_inputs *in, const PlanLayout &L, const Sz &z, fnb
   out->batch32 = in->batch ? L.batch32 : nullptr; out->frag_batch32 = in->batch ? L.frag_batch32 : nullptr;
   out->n_graphs = in->batch ? in->n_graphs : 0;
   out->status = L.status;
+}
+
+// The counting sort of the graphs described by `a` (its graphs, e_total, n_total and status), with the temporaries `t`:
+// zero the counters, histogram, 3-launch exclusive scan, slot claim, forward rank, forward_ready (optional), reverse
+// rank.  Every launch is in stream order on `stream`.
+int counting_sort(PlanArgs a, const SortTemps &t, cudaStream_t stream, cudaEvent_t forward_ready) {
+  a.cnt_dst = t.cnt_dst; a.cnt_src = t.cnt_src; a.x_dst = t.x_dst; a.x_src = t.x_src;
+  a.tmp_eid = t.tmp_eid; a.tmp_reid = t.tmp_reid;
+  const int n_tiles = (a.n_total + kScanTile - 1) / kScanTile;
+  if (a.n_total > 0) {
+    const cudaError_t err = cudaMemsetAsync(t.cnt_dst, 0, t.cnt_bytes, stream);
+    if (err != cudaSuccess) return (int)err;
+  }
+  if (a.e_total > 0) {
+    if (cudaError_t le = fnb_launch(k_plan_histogram, dim3(grid_for(a.e_total)), dim3(256), 0, stream, a)) return (int)le;
+    FNB_CHECK_LAUNCH();
+  }
+  ScanArrays2 sc;
+  sc.in[0] = t.cnt_dst; sc.out[0] = t.x_dst; sc.tile_sums[0] = t.tiles0;
+  sc.in[1] = t.cnt_src; sc.out[1] = t.x_src; sc.tile_sums[1] = t.tiles1;
+  sc.n = a.n_total;
+  if (n_tiles > 0) {
+    if (cudaError_t le = fnb_launch(k_plan_scan_tiles, dim3(n_tiles, 2), dim3(kScanBlock), 0, stream, sc)) return (int)le;
+    FNB_CHECK_LAUNCH();
+  }
+  if (cudaError_t le = fnb_launch(k_plan_scan_sums, dim3(2), dim3(kScanBlock), 0, stream, sc, n_tiles)) return (int)le;
+  FNB_CHECK_LAUNCH();
+  if (n_tiles > 0) {
+    if (cudaError_t le = fnb_launch(k_plan_scan_apply, dim3(n_tiles, 2), dim3(kScanBlock), 0, stream, sc)) return (int)le;
+    FNB_CHECK_LAUNCH();
+  }
+  if (a.e_total > 0) {
+    if (cudaError_t le = fnb_launch(k_plan_claim, dim3(grid_for(a.e_total)), dim3(256), 0, stream, a)) return (int)le;
+    FNB_CHECK_LAUNCH();
+  }
+  if (cudaError_t le = fnb_launch(k_plan_rank_forward, dim3(grid_for(a.e_total > a.n_total ? a.e_total : a.n_total)),
+                                  dim3(256), 0, stream, a))
+    return (int)le;
+  FNB_CHECK_LAUNCH();
+  if (forward_ready) {
+    const cudaError_t err = cudaEventRecord(forward_ready, stream);
+    if (err != cudaSuccess) return (int)err;
+  }
+  if (a.e_total > 0) {
+    if (cudaError_t le = fnb_launch(k_plan_rank_reverse, dim3(grid_for(a.e_total)), dim3(256), 0, stream, a)) return (int)le;
+    FNB_CHECK_LAUNCH();
+  }
+  return 0;
 }
 
 }  // namespace
@@ -453,50 +558,11 @@ int fnb_batch_plan_build_impl(const fnb_batch_inputs *in, void *arena, size_t ar
   }
   a.g[0].attr_in = in->edge_attr_bonds; a.g[0].attr_out = L.attr_bond; a.g[0].attr_w = 1;
   a.g[2].attr_in = in->edge_attr_fbonds; a.g[2].attr_out = L.attr_fbond; a.g[2].attr_w = 6;
-  a.e_total = z.e_total; a.n_total = z.n_total_nodes;
-  a.cnt_dst = L.cnt_dst; a.cnt_src = L.cnt_src; a.x_dst = L.x_dst; a.x_src = L.x_src;
-  a.tmp_eid = L.tmp_eid; a.tmp_reid = L.tmp_reid; a.status = L.status;
+  a.e_total = z.e_total; a.n_total = z.n_total_nodes; a.status = L.status;
 
-  cudaError_t err = cudaMemsetAsync(L.status, 0, sizeof(int), stream);
+  const cudaError_t err = cudaMemsetAsync(L.status, 0, sizeof(int), stream);
   if (err != cudaSuccess) return (int)err;
-  if (z.n_total_nodes > 0) {
-    err = cudaMemsetAsync(L.cnt_dst, 0, L.cnt_bytes, stream);
-    if (err != cudaSuccess) return (int)err;
-  }
-  if (z.e_total > 0) {
-    if (cudaError_t le = fnb_launch(k_plan_histogram, dim3(grid_for(z.e_total)), dim3(256), 0, stream, a)) return (int)le;
-    FNB_CHECK_LAUNCH();
-  }
-  ScanArrays2 sc;
-  sc.in[0] = L.cnt_dst; sc.out[0] = L.x_dst; sc.tile_sums[0] = L.tiles0;
-  sc.in[1] = L.cnt_src; sc.out[1] = L.x_src; sc.tile_sums[1] = L.tiles1;
-  sc.n = z.n_total_nodes;
-  if (z.n_tiles > 0) {
-    if (cudaError_t le = fnb_launch(k_plan_scan_tiles, dim3(z.n_tiles, 2), dim3(kScanBlock), 0, stream, sc)) return (int)le;
-    FNB_CHECK_LAUNCH();
-  }
-  if (cudaError_t le = fnb_launch(k_plan_scan_sums, dim3(2), dim3(kScanBlock), 0, stream, sc, z.n_tiles)) return (int)le;
-  FNB_CHECK_LAUNCH();
-  if (z.n_tiles > 0) {
-    if (cudaError_t le = fnb_launch(k_plan_scan_apply, dim3(z.n_tiles, 2), dim3(kScanBlock), 0, stream, sc)) return (int)le;
-    FNB_CHECK_LAUNCH();
-  }
-  if (z.e_total > 0) {
-    if (cudaError_t le = fnb_launch(k_plan_claim, dim3(grid_for(z.e_total)), dim3(256), 0, stream, a)) return (int)le;
-    FNB_CHECK_LAUNCH();
-  }
-  if (cudaError_t le = fnb_launch(k_plan_rank_forward, dim3(grid_for(z.e_total > z.n_total_nodes ? z.e_total : z.n_total_nodes)), dim3(256), 0,
-                                  stream, a))
-    return (int)le;
-  FNB_CHECK_LAUNCH();
-  if (forward_ready) {
-    err = cudaEventRecord(forward_ready, stream);
-    if (err != cudaSuccess) return (int)err;
-  }
-  if (z.e_total > 0) {
-    if (cudaError_t le = fnb_launch(k_plan_rank_reverse, dim3(grid_for(z.e_total)), dim3(256), 0, stream, a)) return (int)le;
-    FNB_CHECK_LAUNCH();
-  }
+  if (int rc = counting_sort(a, L.t, stream, forward_ready)) return rc;
   AuxArgs x;
   x.a2f = in->atom_to_frag_ids; x.batch = in->batch; x.frag_batch = in->frag_batch; x.a2f32 = L.a2f32;
   x.batch32 = L.batch32; x.frag_batch32 = L.frag_batch32; x.atom_ptr = L.atom_ptr; x.frag_ptr = L.frag_ptr;
@@ -506,5 +572,72 @@ int fnb_batch_plan_build_impl(const fnb_batch_inputs *in, void *arena, size_t ar
   FNB_CHECK_LAUNCH();
 
   fill_plan(in, L, z, out);
+  return 0;
+}
+
+extern "C" size_t fnb_csr_workspace_bytes(int64_t n_nodes, int64_t n_edges_total) {
+  if (n_nodes < 0 || n_edges_total < 0) return 0;
+  return csr_layout(n_nodes, n_edges_total, nullptr).total;
+}
+
+// One graph through the batch plan's counting sort: graph 0 of the PlanArgs is the caller's, graphs 1..4 are empty.
+extern "C" int fnb_csr_build(const int64_t *dst, const int64_t *src, int64_t n_edges, int64_t n_nodes,
+                             int append_self_loops, int32_t *rowptr, int32_t *col, int32_t *row, int32_t *eid,
+                             int32_t *slot_of_eid, int32_t *rrowptr, int32_t *rslot, int32_t *rdst, void *workspace,
+                             size_t workspace_bytes, int32_t *status, void *stream) {
+  if (n_edges < 0 || n_nodes < 0) return FNB_ERR_SIZE;
+  const int64_t n_total = n_edges + (append_self_loops ? n_nodes : 0);
+  if (n_total > kMaxSortItems || n_nodes > kMaxSortItems) return FNB_ERR_SIZE;
+  if (!rowptr || !workspace || (n_edges > 0 && !dst)) return FNB_ERR_NULL;
+  const bool reverse = rrowptr != nullptr;
+  if (reverse && n_total > 0 && (!rslot || !rdst || !slot_of_eid)) return FNB_ERR_NULL;
+  if (workspace_bytes < fnb_csr_workspace_bytes(n_nodes, n_total)) return FNB_ERR_WORKSPACE;
+  // With src == NULL the "source" index space is the edge list itself (membership lists); a reverse
+  // CSR makes no sense there.
+  if (!src && reverse && n_edges > 0) return FNB_ERR_MODE;
+
+  const CsrLayout L = csr_layout(n_nodes, n_total, (char *)workspace);
+  PlanArgs a{};
+  GDesc &G = a.g[0];
+  G.dst = dst; G.src = src; G.n_real = (int)n_edges; G.n_total = (int)n_total; G.n_nodes = (int)n_nodes;
+  G.n_src_nodes = src ? (int)n_nodes : (int)n_total;
+  G.reverse = reverse;
+  G.rowptr = rowptr; G.col = col; G.row = row; G.eid = eid; G.slot_of_eid = slot_of_eid;
+  G.rrowptr = rrowptr; G.rslot = rslot; G.rdst = rdst;
+  for (int i = 1; i < PG; ++i) {     // empty graphs after the caller's; k_plan_rank_forward writes their rowptr[0]
+    a.g[i].node_base = (int)n_nodes;
+    a.g[i].edge_base = (int)n_total;
+    a.g[i].rowptr = L.spare;
+  }
+  a.e_total = (int)n_total; a.n_total = (int)n_nodes;
+  a.status = status ? status : L.spare + 1;    // the caller's status word is not zeroed here
+  return counting_sort(a, L.t, (cudaStream_t)stream, nullptr);
+}
+
+extern "C" int fnb_gather_rows(const float *in, const int32_t *index, int64_t n_rows, int width, float *out,
+                               void *stream) {
+  if (n_rows < 0 || width <= 0) return FNB_ERR_SIZE;
+  if (n_rows == 0) return 0;
+  if (!in || !index || !out) return FNB_ERR_NULL;
+  k_gather_rows<<<grid_for(n_rows * width), 256, 0, (cudaStream_t)stream>>>(in, index, n_rows, width, out);
+  FNB_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fnb_segment_offsets(const int64_t *sorted_ids, int64_t n, int64_t n_segments, int32_t *offsets,
+                                   void *stream) {
+  if (n < 0 || n_segments < 0 || n >= (int64_t)INT32_MAX) return FNB_ERR_SIZE;
+  if (!offsets || (n > 0 && !sorted_ids)) return FNB_ERR_NULL;
+  k_segment_offsets<<<grid_for(n_segments + 1), 256, 0, (cudaStream_t)stream>>>(sorted_ids, n, n_segments, offsets);
+  FNB_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fnb_narrow_index(const int64_t *in, int64_t n, int32_t *out, void *stream) {
+  if (n < 0) return FNB_ERR_SIZE;
+  if (n == 0) return 0;
+  if (!in || !out) return FNB_ERR_NULL;
+  k_narrow<<<grid_for(n), 256, 0, (cudaStream_t)stream>>>(in, n, out);
+  FNB_CHECK_LAUNCH();
   return 0;
 }

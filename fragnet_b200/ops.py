@@ -251,6 +251,33 @@ def _idx(t: torch.Tensor, dev) -> torch.Tensor:
     return t if t.is_contiguous() else t.contiguous()
 
 
+def batch_inputs(edge_index, frag_index, atom_to_frag_ids, edge_index_bonds_graph, edge_attr_bonds, edge_index_fbonds,
+                 edge_attr_fbonds, batch_vec, frag_batch_vec, n_atoms: int, n_frags: int, n_bond_nodes: int,
+                 n_fbond_nodes: int, n_graphs: int, device, convert: bool = True):
+    """``fnb_batch_inputs`` of one batch and the tensors it points into (keep them alive until the library has read
+    them).  The library reads (``device``, contiguous) int64 indices and float32 edge attributes: ``convert`` converts a
+    tensor that is not; without it the result is None instead (nothing is copied).  The batch vectors may be None."""
+    if edge_index.shape[1] != n_bond_nodes or frag_index.shape[1] != n_fbond_nodes:
+        raise ValueError("fragnet_b200: the bond graph needs one node per column of edge_index and the "
+                         "fragment-connection graph one node per column of frag_index (gat2.py:179-185, 293-295); got "
+                         f"{n_bond_nodes} vs {edge_index.shape[1]} and {n_fbond_nodes} vs {frag_index.shape[1]}")
+    i64, f32 = torch.int64, torch.float32
+    t = dict(edge_index=(edge_index, i64), frag_index=(frag_index, i64), atom_to_frag_ids=(atom_to_frag_ids, i64),
+             edge_index_bonds_graph=(edge_index_bonds_graph, i64), edge_index_fbonds=(edge_index_fbonds, i64),
+             batch=(batch_vec, i64), frag_batch=(frag_batch_vec, i64), edge_attr_bonds=(edge_attr_bonds, f32),
+             edge_attr_fbonds=(edge_attr_fbonds, f32))
+    for name, (x, dtype) in t.items():
+        if x is not None and (x.device != device or x.dtype != dtype or not x.is_contiguous()):
+            if not convert:
+                return None
+            x = x.to(device=device, dtype=dtype).contiguous()
+        t[name] = x
+    inp = _abi.CBatchInputs(**{name: _ptr(x) for name, x in t.items()}, n_atoms=n_atoms, n_frags=n_frags,
+                            n_bonds=n_bond_nodes, n_bond_edges=t["edge_index_bonds_graph"].shape[1],
+                            n_fbond_nodes=n_fbond_nodes, n_fbond_edges=t["edge_index_fbonds"].shape[1], n_graphs=n_graphs)
+    return inp, tuple(t.values())
+
+
 def build_layer_plan(edge_index, frag_index, atom_to_frag_ids, edge_index_bonds_graph, edge_attr_bonds,
                      edge_index_fbonds, edge_attr_fbonds, n_atoms: int, n_frags: int, n_bond_nodes: int,
                      n_fbond_nodes: int, device, batch_vec=None, frag_batch_vec=None) -> LayerPlan:
@@ -260,26 +287,15 @@ def build_layer_plan(edge_index, frag_index, atom_to_frag_ids, edge_index_bonds_
     segment (reference gat2.py:138, :239); atom / fragment graphs use row 1 (gat2.py:187, :283), and
     the atom graph gets its self loops appended (gat2.py:179)."""
     dev = require_cuda(device)
-    if edge_index.shape[1] != n_bond_nodes or frag_index.shape[1] != n_fbond_nodes:
-        raise ValueError("fragnet_b200: the bond graph needs one node per column of edge_index and the "
-                         "fragment-connection graph one node per column of frag_index (gat2.py:179-185, 293-295); got "
-                         f"{n_bond_nodes} vs {edge_index.shape[1]} and {n_fbond_nodes} vs {frag_index.shape[1]}")
     # molecule count: read back lazily (MoleculeCount); the offset arrays are sized by the upper bound n_frags
     # (every molecule owns at least one fragment, fragments.py:230-234)
     have_batch = batch_vec is not None and frag_batch_vec is not None
     count = MoleculeCount(batch_vec, frag_batch_vec) if have_batch else None
-    n_graphs = n_frags if have_batch else 0
-    ei, fi = _idx(edge_index, dev), _idx(frag_index, dev)
-    eb, efb = _idx(edge_index_bonds_graph, dev), _idx(edge_index_fbonds, dev)
-    a2f = _idx(atom_to_frag_ids, dev)
-    cos = _f32c(edge_attr_bonds.to(dev)).reshape(-1)
-    a6 = _f32c(edge_attr_fbonds.to(dev))
-    bv = fbv = None
-    if have_batch:
-        bv, fbv = _idx(batch_vec, dev), _idx(frag_batch_vec, dev)
-    keep = (ei, fi, eb, efb, a2f, cos, a6, bv, fbv)
-    inp = _abi.CBatchInputs(_ptr(ei), _ptr(fi), _ptr(a2f), _ptr(eb), _ptr(efb), _ptr(bv), _ptr(fbv), _ptr(cos), _ptr(a6),
-                            n_atoms, n_frags, n_bond_nodes, eb.shape[1], n_fbond_nodes, efb.shape[1], n_graphs)
+    if not have_batch:
+        batch_vec = frag_batch_vec = None
+    inp, keep = batch_inputs(edge_index, frag_index, atom_to_frag_ids, edge_index_bonds_graph, edge_attr_bonds,
+                             edge_index_fbonds, edge_attr_fbonds, batch_vec, frag_batch_vec, n_atoms, n_frags,
+                             n_bond_nodes, n_fbond_nodes, n_frags if have_batch else 0, dev)
     lib = _lib()
     nbytes = lib.fnb_batch_plan_bytes(C.byref(inp))
     arena = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=dev)

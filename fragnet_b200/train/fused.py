@@ -142,24 +142,20 @@ class _FlatStep:
         self._loss_i = (self._loss_i + 1) % self._loss.numel()
         return self._loss[self._loss_i]
 
+    def _plan_inputs(self, b, g: int, convert: bool = True):
+        """``ops.batch_inputs`` of a batch dict with ``g`` molecules (``prefetch_plan`` and the step build the same)."""
+        return ops.batch_inputs(b["edge_index"], b["frag_index"], b["atom_to_frag_ids"], b["edge_index_bonds_graph"],
+                                b["edge_attr_bonds"], b["edge_index_fbonds"], b["edge_attr_fbonds"], b["batch"],
+                                b["frag_batch"], b["x_atoms"].shape[0], b["x_frags"].shape[0],
+                                b["node_features_bonds"].shape[0], b["node_features_fbonds"].shape[0], g, self.dev,
+                                convert)
+
     def _batch_inputs(self, batch, g: int):
         """``fnb_batch_inputs`` of a batch dict with ``g`` molecules, the tensors it points into, and the raw features."""
-        dev = self.dev
-        idx = lambda k: _on(batch, k, dev, torch.int64)
-        f32 = lambda k: _on(batch, k, dev, torch.float32)
-        ei, fi, a2f = idx("edge_index"), idx("frag_index"), idx("atom_to_frag_ids")
-        eb, efb = idx("edge_index_bonds_graph"), idx("edge_index_fbonds")
-        bv, fbv = idx("batch"), idx("frag_batch")
-        cos, a6 = f32("edge_attr_bonds"), f32("edge_attr_fbonds")
-        xa, xb, xfb = f32("x_atoms"), f32("node_features_bonds"), f32("node_features_fbonds")
-        na, nf, nb, nfb = xa.shape[0], batch["x_frags"].shape[0], xb.shape[0], xfb.shape[0]
-        if ei.shape[1] != nb or fi.shape[1] != nfb:
-            raise ValueError("fragnet_b200: the bond graph needs one node per column of edge_index and the "
-                             "fragment-connection graph one node per column of frag_index")
-        pt = ops._ptr
-        inp = _abi.CBatchInputs(pt(ei), pt(fi), pt(a2f), pt(eb), pt(efb), pt(bv), pt(fbv), pt(cos), pt(a6),
-                                na, nf, nb, eb.shape[1], nfb, efb.shape[1], g)
-        return inp, (ei, fi, a2f, eb, efb, bv, fbv, cos, a6, xa, xb, xfb), (xa, xb, xfb)
+        inp, keep = self._plan_inputs(batch, g)
+        feats = tuple(_on(batch, k, self.dev, torch.float32) for k in ("x_atoms", "node_features_bonds",
+                                                                        "node_features_fbonds"))
+        return inp, keep + feats, feats
 
     def _take_prefetched(self, inp) -> Optional[int]:
         """Arena address of the plan ``prefetch_plan`` built for exactly these batch inputs, or None."""
@@ -172,9 +168,6 @@ class _FlatStep:
         return None
 
     # ---- collate of the next batch underneath the running step -------------------------------------------------------
-    _PLAN_TENSORS = ("edge_index", "frag_index", "atom_to_frag_ids", "edge_index_bonds_graph", "edge_index_fbonds",
-                     "batch", "frag_batch")
-
     @staticmethod
     def _plan_key(inp: "_abi.CBatchInputs"):
         return tuple(getattr(inp, n) for n, _ in _abi.CBatchInputs._fields_)
@@ -189,22 +182,10 @@ class _FlatStep:
         must not be modified until that step has been launched."""
         self._prefetched = None
         dev = self.dev
-        for k in self._PLAN_TENSORS:
-            t = next_batch.get(k)
-            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.int64 or not t.is_contiguous():
-                return False
-        for k in ("edge_attr_bonds", "edge_attr_fbonds"):
-            t = next_batch.get(k)
-            if not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != torch.float32 or not t.is_contiguous():
-                return False
-        b = next_batch
-        na, nf = b["x_atoms"].shape[0], b["x_frags"].shape[0]
-        nb, nfb, g = b["edge_index"].shape[1], b["frag_index"].shape[1], b["y"].numel() // self._y_width
-        pt = ops._ptr
-        inp = _abi.CBatchInputs(pt(b["edge_index"]), pt(b["frag_index"]), pt(b["atom_to_frag_ids"]),
-                                pt(b["edge_index_bonds_graph"]), pt(b["edge_index_fbonds"]), pt(b["batch"]),
-                                pt(b["frag_batch"]), pt(b["edge_attr_bonds"]), pt(b["edge_attr_fbonds"]),
-                                na, nf, nb, b["edge_index_bonds_graph"].shape[1], nfb, b["edge_index_fbonds"].shape[1], g)
+        got = self._plan_inputs(next_batch, next_batch["y"].numel() // self._y_width, convert=False)
+        if got is None:
+            return False
+        inp, keep = got
         lib = ops._lib()
         need = lib.fnb_batch_plan_bytes(C.byref(inp))
         if need == 0:
@@ -223,7 +204,6 @@ class _FlatStep:
         rc = lib.fnb_pretrain_plan_prefetch(C.byref(inp), ops._ptr(arena), arena.numel(), ev)
         if rc != 0:
             return False                 # single-stream mode: the step collates by itself
-        keep = tuple(b[k] for k in self._PLAN_TENSORS) + (b["edge_attr_bonds"], b["edge_attr_fbonds"])
         self._prefetched = (self._plan_key(inp), arena, keep, parity)
         return True
 

@@ -67,8 +67,12 @@ size_t fnb_scratch_bytes(void);
  *   eid[slot] = edge id, slot_of_eid[e] = slot
  * Reverse CSR groups the same edges by source, again ordered by edge id:
  *   rrowptr[n_nodes+1], rslot[r] = forward slot of that edge, rdst[r] = its destination node.
+ * With rrowptr != NULL and at least one edge, rslot, rdst and slot_of_eid are required.
  * src == NULL means src[e] = e (membership lists such as atom_to_frag_ids, gat2.py:234).
- * status[0] is set non-zero on the device if an index is out of [0, n_nodes).
+ * status[0] is set non-zero on the device if an index is out of [0, n_nodes); it is not zeroed here (may be NULL).
+ * This is the counting sort of fnb_batch_plan_build run over one graph.  Its kernels index with int32 and stride by
+ * up to 148*16*256 = 606208 threads, so n_nodes and the edge count (with self loops) must each be at most
+ * 2^31 - 1 - 606208 (FNB_ERR_SIZE otherwise).
  */
 size_t fnb_csr_workspace_bytes(int64_t n_nodes, int64_t n_edges_total);
 int fnb_csr_build(const int64_t *dst, const int64_t *src, int64_t n_edges, int64_t n_nodes,

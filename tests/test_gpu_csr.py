@@ -33,12 +33,13 @@ def _check(dst, src, n_nodes, self_loops):
         assert torch.equal(got, w), k
 
 
-@pytest.mark.parametrize("n_nodes,n_edges,self_loops", [(1, 1, False), (7, 0, True), (50, 400, False), (50, 400, True),
-                                                        (5000, 40000, True), (3, 5000, False), (100000, 650000, False)])
+@pytest.mark.parametrize("n_nodes,n_edges,self_loops", [(0, 0, False), (1, 1, False), (7, 0, True), (50, 400, False),
+                                                        (50, 400, True), (5000, 40000, True), (3, 5000, False),
+                                                        (100000, 650000, False)])
 def test_csr_equals_stable_sort(n_nodes, n_edges, self_loops):
     g = torch.Generator().manual_seed(n_nodes + n_edges)
-    dst = torch.randint(0, n_nodes, (n_edges,), generator=g)
-    src = torch.randint(0, n_nodes, (n_edges,), generator=g)
+    dst = torch.randint(0, max(n_nodes, 1), (n_edges,), generator=g)
+    src = torch.randint(0, max(n_nodes, 1), (n_edges,), generator=g)
     _check(dst, src, n_nodes, self_loops)
 
 
