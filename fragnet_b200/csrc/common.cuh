@@ -259,6 +259,45 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
                                     void *workspace, size_t workspace_bytes, void *scratch, void *stream,
                                     int skip_tails);
 
+// Exact FP32 GEMM (proj.cu: k_mlp_gemm, FFMA, one k-ascending chain per output), for the projections' SIMT path and
+// the finetuning head.  C[M,N] = sum_k A(m,k) B(k,n):
+//   GEMM_FWD: A = x [M, K], B = W [N, K] (nn.Linear weight); epilogue z = acc (+ bias); z *= drop1; u = z;
+//             C = act(z) * drop2, and optionally S (below).
+//   GEMM_DX:  A = dz [M, K], B = W [K, N]; epilogue C = acc * drop1 * act'(u) * drop2 (u == NULL: no activation).
+//   GEMM_DW:  through fnb_gemm_dw.
+struct Drop {                       // one dropout site: element i of a [rows, width] tensor draws from base + i / 4
+  float p, scale;
+  uint64_t base;
+  int on;
+};
+Drop fnb_drop(float p, int training, uint64_t base);
+enum { GEMM_FWD = 0, GEMM_DX = 1, GEMM_DW = 2 };
+struct GemmArgs {
+  const float *A, *B;
+  int M, N, K;
+  float *C;
+  uint64_t seed;
+  const float *bias;        // FWD: [N] or NULL
+  Drop drop1, drop2;
+  int act;
+  float *u;                 // FWD: written (may be NULL); DX: read (NULL = no activation between the layers)
+  // FWD, N = 128 and no dropout or activation: S[m, h] = <C[m, 32h:32h+32], alpha[h, off_t:off_t+32]>, S[m, 4+h]
+  // likewise at off_s (the per-node logit halves of the projections); NULL: not written
+  const float *alpha;
+  int alpha_stride, off_t, off_s;
+  float *S;
+  // DW (set by fnb_gemm_dw): per-chunk records [M*N dW | M db], record z at rec + z * rec_stride
+  int k_chunk;
+  float *rec;
+  int64_t rec_stride;
+};
+int fnb_gemm(int mode, const GemmArgs &a, cudaStream_t stream);
+// dW[out, in] = dz^T x and db[out] = column sums of dz (db may be NULL) over `rows` rows of dz [rows, out] and
+// x [rows, in]: per-chunk records in `rec` (fnb_gemm_dw_record_floats), summed in a fixed order.
+int fnb_gemm_dw(const float *dz, const float *x, int64_t rows, int out, int in, float *dW, float *db, float *rec,
+                cudaStream_t stream);
+size_t fnb_gemm_dw_record_floats(int64_t rows, int out, int in);
+
 // Finetuning head (finetune.cu).  One run of an fnb_mlp_layer list over G rows; every buffer is caller-provided.
 struct FnbMlpRun {
   const fnb_mlp_layer *L;

@@ -7,183 +7,218 @@
 // epilogue while the output tile is still in registers, so the attention kernels never re-read
 // 128-wide rows to form a logit (SURVEY.md App. A.5).
 //
-// This file is the fp32 SIMT implementation used for exact (<=1e-5) parity with the reference;
-// FFMA-bound, not HBM-bound -- see DESIGN.md "projection" for the tensor-core plan.
+// This file holds every FP32 SIMT kernel of the projections, used for exact (<=1e-5) parity with the reference
+// (FFMA-bound, not HBM-bound -- see DESIGN.md "projection" for the tensor-core kernels): the FFMA GEMM k_mlp_gemm, which
+// also runs the finetuning head (finetune.cu), the row-sparse kernel for raw input features, k_linear_rows for few
+// rows, and k_node_scalars.
 #include "common.cuh"
 
 namespace {
 
-constexpr int BM = 64, BN = 128, BK = 32;
-constexpr int kGemmThreads = 256;
+// ---- k_mlp_gemm: the register-tiled FP32 FFMA GEMM (GemmArgs, common.cuh) ---------------------------------------------
+// 64 x 64 output tile per CTA, 4 x 4 outputs per thread, K in slabs of 16 whose global loads are in flight (in
+// registers) while the previous slab's FMAs run.  Rows are on gridDim.x (no limit but INT32_MAX), columns on gridDim.y,
+// weight-gradient row chunks on gridDim.z.
+constexpr int BM = 64, BN = 64, BK = 16, kThreads = 256;
+constexpr int SA = BM + 4;          // shared-memory row stride (floats): float4 aligned
+constexpr int kDwTargetCtas = 2 * kNumSMs;
 
-struct GemmArgs {
-  const float *A; int lda;      // [M, Kd]
-  const float *B; int ldb;      // TRANS_B: [Nc, Kd] (nn.Linear weight), else [Kd, Nc]
-  float *C; int ldc;            // [M, Nc]
-  int64_t M; int Kd; int Nc;
-  const float *bias;            // [Nc] or NULL
-  const float *alpha; int alpha_stride, off_t, off_s;  // epilogue scalars (EPI only)
-  float *S;                     // [M, 8] or NULL
-};
+__device__ __forceinline__ float drop_factor(const Drop &d, uint64_t seed, int64_t i) {
+  if (!d.on) return 1.f;
+  const uint2 r = dropout_bits(seed, d.base + (uint64_t)(i >> 2));
+  const int pos = (int)(i & 3);
+  const uint32_t w = pos < 2 ? r.x : r.y;
+  const uint32_t r16 = (pos & 1) ? (w >> 16) : (w & 0xffffu);
+  return r16 >= dropout_threshold(d.p) ? d.scale : 0.f;
+}
 
-template <bool TRANS_B, bool EPI>
-__global__ void __launch_bounds__(kGemmThreads) k_gemm(GemmArgs g) {
+constexpr float kSeluAlpha = 1.6732632423543772f, kSeluScale = 1.0507009873554805f;
+
+__device__ __forceinline__ float act_fwd(int act, float z) {
+  switch (act) {
+    case FNB_ACT_RELU: return fmaxf(z, 0.f);
+    case FNB_ACT_CELU: return z > 0.f ? z : expm1f(z);
+    case FNB_ACT_SILU: return z / (1.f + expf(-z));
+    case FNB_ACT_GELU: return 0.5f * z * (1.f + erff(z * 0.70710678118654752f));
+    case FNB_ACT_SELU: return kSeluScale * (z > 0.f ? z : kSeluAlpha * expm1f(z));
+    case FNB_ACT_RELU6: return fminf(fmaxf(z, 0.f), 6.f);
+    case FNB_ACT_LEAKYRELU: return z > 0.f ? z : 0.01f * z;
+    default: return z;
+  }
+}
+
+// d act / d z at z, with torch's choices at the kinks (relu: 0 at 0, relu6: 0 at 0 and 6, celu / selu: the exp branch
+// at 0, leaky relu: the slope at 0).
+__device__ __forceinline__ float act_grad(int act, float z) {
+  switch (act) {
+    case FNB_ACT_RELU: return z > 0.f ? 1.f : 0.f;
+    case FNB_ACT_CELU: return z > 0.f ? 1.f : expf(z);
+    case FNB_ACT_SILU: {
+      const float s = 1.f / (1.f + expf(-z));
+      return s * (1.f + z * (1.f - s));
+    }
+    case FNB_ACT_GELU:
+      return 0.5f * (1.f + erff(z * 0.70710678118654752f)) + z * 0.39894228040143268f * expf(-0.5f * z * z);
+    case FNB_ACT_SELU: return z > 0.f ? kSeluScale : kSeluScale * kSeluAlpha * expf(z);
+    case FNB_ACT_RELU6: return (z > 0.f && z < 6.f) ? 1.f : 0.f;
+    case FNB_ACT_LEAKYRELU: return z > 0.f ? 1.f : 0.01f;
+    default: return 1.f;
+  }
+}
+
+// Loads one BK-deep slab of a 64-row operand tile into registers.  KC: the operand is K-contiguous (element (r, k) at
+// p[r * ld + k]), else R-contiguous (p[k * ld + r]).  Thread t holds 4 elements; out-of-range elements are 0.
+template <bool KC>
+__device__ __forceinline__ void load_slab(const float *__restrict__ p, int ld, int r0, int nr, int k0, int k1,
+                                          float v[4]) {
+  const int t = threadIdx.x;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int kk = KC ? (t & 15) : (t >> 6) + 4 * i;
+    const int r = KC ? (t >> 4) + 16 * i : (t & 63);
+    const int k = k0 + kk, row = r0 + r;
+    v[i] = (row < nr && k < k1) ? __ldg(KC ? p + (int64_t)row * ld + k : p + (int64_t)k * ld + row) : 0.f;
+  }
+}
+
+template <bool KC>
+__device__ __forceinline__ void store_slab(float (*s)[SA], const float v[4]) {
+  const int t = threadIdx.x;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int kk = KC ? (t & 15) : (t >> 6) + 4 * i;
+    const int r = KC ? (t >> 4) + 16 * i : (t & 63);
+    s[kk][r] = v[i];
+  }
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(kThreads) k_mlp_gemm(GemmArgs a) {
+  constexpr bool A_KC = MODE != GEMM_DW;      // FWD / DX: A rows are molecules, K contiguous; DW: A = dz, M contiguous
+  constexpr bool B_KC = MODE == GEMM_FWD;     // FWD: B = W [N, K]; DX: W [K, N]; DW: xd [K, N]
+  __shared__ __align__(16) float As[BK][SA];
+  __shared__ __align__(16) float Bs[BK][SA];
   pdl_wait();
-  __shared__ float As[BM][BK + 1];
-  __shared__ __align__(16) float Bs[BK][BN];
-  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  const int64_t m0 = (int64_t)blockIdx.x * BM;
-  const int n0 = blockIdx.y * BN;
-  float acc[4][8];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-
-  for (int k0 = 0; k0 < g.Kd; k0 += BK) {
-#pragma unroll
-    for (int i = 0; i < (BM * BK) / kGemmThreads; ++i) {
-      const int idx = tid + i * kGemmThreads;
-      const int k = idx & (BK - 1), r = idx / BK;
-      const int64_t row = m0 + r;
-      As[r][k] = (row < g.M && k0 + k < g.Kd) ? __ldg(g.A + row * g.lda + k0 + k) : 0.f;
-    }
-#pragma unroll
-    for (int i = 0; i < (BK * BN) / kGemmThreads; ++i) {
-      const int idx = tid + i * kGemmThreads;
-      const int n = idx & (BN - 1), k = idx / BN;
-      float v = 0.f;
-      if (n0 + n < g.Nc && k0 + k < g.Kd)
-        v = TRANS_B ? __ldg(g.B + (int64_t)(n0 + n) * g.ldb + k0 + k) : __ldg(g.B + (int64_t)(k0 + k) * g.ldb + n0 + n);
-      Bs[k][n] = v;
-    }
+  const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
+  const int m0 = blockIdx.x * BM, n0 = blockIdx.y * BN;
+  int k0 = 0, k1 = a.K;
+  if (MODE == GEMM_DW) {
+    k0 = blockIdx.z * a.k_chunk;
+    k1 = min(a.K, k0 + a.k_chunk);
+  }
+  // leading dimensions: FWD A = xd [G, K], B = W [N, K]; DX A = dz [G, K], B = W [K, N]; DW A = dz [K, M], B = xd [K, N]
+  const int lda = MODE == GEMM_DW ? a.M : a.K;
+  const int ldb = MODE == GEMM_FWD ? a.K : a.N;
+  const bool want_db = MODE == GEMM_DW && blockIdx.y == 0;
+  float acc[4][4] = {};
+  float db_acc = 0.f;
+  float ra[4], rb[4];
+  load_slab<A_KC>(a.A, lda, m0, a.M, k0, k1, ra);
+  load_slab<B_KC>(a.B, ldb, n0, a.N, k0, k1, rb);
+  for (int kt = k0; kt < k1; kt += BK) {
+    store_slab<A_KC>(As, ra);
+    store_slab<B_KC>(Bs, rb);
     __syncthreads();
+    if (kt + BK < k1) {                    // next slab's global loads are in flight during this slab's FMAs
+      load_slab<A_KC>(a.A, lda, m0, a.M, kt + BK, k1, ra);
+      load_slab<B_KC>(a.B, ldb, n0, a.N, kt + BK, k1, rb);
+    }
 #pragma unroll
-    for (int k = 0; k < BK; ++k) {
-      float a[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) a[i] = As[ty * 4 + i][k];
-      const float4 b0 = *reinterpret_cast<const float4 *>(&Bs[k][tx * 8]);
-      const float4 b1 = *reinterpret_cast<const float4 *>(&Bs[k][tx * 8 + 4]);
-      const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+    for (int kk = 0; kk < BK; ++kk) {
+      const float4 av = *reinterpret_cast<const float4 *>(&As[kk][ty * 4]);
+      const float4 bv = *reinterpret_cast<const float4 *>(&Bs[kk][tx * 4]);
+      const float ar[4] = {av.x, av.y, av.z, av.w}, br[4] = {bv.x, bv.y, bv.z, bv.w};
 #pragma unroll
       for (int i = 0; i < 4; ++i)
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
+        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(ar[i], br[j], acc[i][j]);
+    }
+    if (want_db && t < BM) {
+#pragma unroll
+      for (int kk = 0; kk < BK; ++kk) db_acc += As[kk][t];
     }
     __syncthreads();
   }
-
-  const int c0 = n0 + tx * 8;
-  if (g.bias) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const float bj = (c0 + j < g.Nc) ? __ldg(g.bias + c0 + j) : 0.f;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) acc[i][j] += bj;
-    }
-  }
-  const bool vec_ok = ((g.ldc & 3) == 0) && (c0 + 8 <= g.Nc) && fnb_is_aligned16_dev(g.C);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int64_t row = m0 + ty * 4 + i;
-    if (row >= g.M) continue;
-    float *cp = g.C + row * g.ldc + c0;
-    if (vec_ok) {
-      st4(cp, make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]));
-      st4(cp + 4, make_float4(acc[i][4], acc[i][5], acc[i][6], acc[i][7]));
-    } else {
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        if (c0 + j < g.Nc) cp[j] = acc[i][j];
-    }
-  }
-  if (EPI && g.S) {
-    // columns c0..c0+7 lie in head c0/32; the 4 threads tx&~3 .. tx|3 cover that head's 32 columns
-    const int head = tx >> 2, within = (tx & 3) * 8;
-    float at[8], as[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      at[j] = __ldg(g.alpha + head * g.alpha_stride + g.off_t + within + j);
-      as[j] = __ldg(g.alpha + head * g.alpha_stride + g.off_s + within + j);
-    }
+  pdl_launch_dependents();
+  if constexpr (MODE == GEMM_DW) {
+    float *rec = a.rec + (int64_t)blockIdx.z * a.rec_stride;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      float st = 0.f, ss = 0.f;
+      const int m = m0 + ty * 4 + i;
+      if (m >= a.M) continue;
 #pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        st = fmaf(acc[i][j], at[j], st);
-        ss = fmaf(acc[i][j], as[j], ss);
+      for (int j = 0; j < 4; ++j) {
+        const int n = n0 + tx * 4 + j;
+        if (n < a.N) rec[(int64_t)m * a.N + n] = acc[i][j];
       }
-      st += __shfl_xor_sync(kFull, st, 1); st += __shfl_xor_sync(kFull, st, 2);
-      ss += __shfl_xor_sync(kFull, ss, 1); ss += __shfl_xor_sync(kFull, ss, 2);
-      const int64_t row = m0 + ty * 4 + i;
-      if ((tx & 3) == 0 && row < g.M) {
-        g.S[row * 8 + head] = st;
-        g.S[row * 8 + 4 + head] = ss;
+    }
+    if (want_db && t < BM && m0 + t < a.M) rec[(int64_t)a.M * a.N + m0 + t] = db_acc;
+  } else {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int m = m0 + ty * 4 + i;
+      if (m >= a.M) continue;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int n = n0 + tx * 4 + j;
+        if (n >= a.N) continue;
+        const int64_t idx = (int64_t)m * a.N + n;
+        float v = acc[i][j];
+        if (MODE == GEMM_FWD) {
+          if (a.bias) v += __ldg(a.bias + n);
+          v *= drop_factor(a.drop1, a.seed, idx);
+          if (a.u) a.u[idx] = v;
+          v = act_fwd(a.act, v) * drop_factor(a.drop2, a.seed, idx);
+          acc[i][j] = v;
+        } else {
+          v *= drop_factor(a.drop1, a.seed, idx);
+          if (a.u) v *= act_grad(a.act, __ldg(a.u + idx));
+          v *= drop_factor(a.drop2, a.seed, idx);
+        }
+        a.C[idx] = v;
+      }
+    }
+    if (MODE == GEMM_FWD && a.S) {
+      // the thread's 4 columns lie in head c / 32, whose 32 columns the 8 threads tx & ~7 .. tx | 7 of this row group own
+      const int c = n0 + tx * 4, head = c >> 5;
+      const float *pt = a.alpha + head * a.alpha_stride + a.off_t + (c & 31);
+      const float *ps = a.alpha + head * a.alpha_stride + a.off_s + (c & 31);
+      const float4 at = make_float4(__ldg(pt), __ldg(pt + 1), __ldg(pt + 2), __ldg(pt + 3));
+      const float4 as = make_float4(__ldg(ps), __ldg(ps + 1), __ldg(ps + 2), __ldg(ps + 3));
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const float4 v = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
+        const float st = head_sum(dot4(v, at)), ss = head_sum(dot4(v, as));
+        const int m = m0 + ty * 4 + i;
+        if ((tx & 7) == 0 && m < a.M) {
+          a.S[(int64_t)m * 8 + head] = st;
+          a.S[(int64_t)m * 8 + 4 + head] = ss;
+        }
       }
     }
   }
 }
 
-// dW[o,k] = sum_n dh[n,o] x[n,k], db[o] = sum_n dh[n,o]; per-CTA partial over a contiguous row range.
-constexpr int kDwRows = 32;
-__global__ void __launch_bounds__(256) k_proj_dw(const float *__restrict__ dh, const float *__restrict__ x, int64_t n_rows,
-                                                 int K, int64_t rows_per_block, float *__restrict__ partials,
-                                                 int64_t rec_stride) {
-  pdl_wait();
-  __shared__ __align__(16) float dhs[kDwRows][128];
-  __shared__ __align__(16) float xs[kDwRows][128];
-  const int tid = threadIdx.x, tk = tid & 15, to = tid >> 4;
-  const int kt0 = blockIdx.y * 128;
-  const int64_t r_begin = (int64_t)blockIdx.x * rows_per_block;
-  const int64_t r_end = min(n_rows, r_begin + rows_per_block);
-  float acc[8][8], dbacc[8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    dbacc[i] = 0.f;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-  }
-  for (int64_t r0 = r_begin; r0 < r_end; r0 += kDwRows) {
-#pragma unroll
-    for (int i = 0; i < (kDwRows * 128) / 256; ++i) {
-      const int idx = tid + i * 256;
-      const int c = idx & 127, r = idx >> 7;
-      const int64_t row = r0 + r;
-      const bool in = row < r_end;
-      dhs[r][c] = in ? __ldg(dh + row * 128 + c) : 0.f;
-      xs[r][c] = (in && kt0 + c < K) ? __ldg(x + row * K + kt0 + c) : 0.f;
-    }
-    __syncthreads();
-#pragma unroll 4
-    for (int r = 0; r < kDwRows; ++r) {
-      const float4 a0 = *reinterpret_cast<const float4 *>(&dhs[r][to * 8]);
-      const float4 a1 = *reinterpret_cast<const float4 *>(&dhs[r][to * 8 + 4]);
-      const float4 b0 = *reinterpret_cast<const float4 *>(&xs[r][tk * 8]);
-      const float4 b1 = *reinterpret_cast<const float4 *>(&xs[r][tk * 8 + 4]);
-      const float a[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-      const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        dbacc[i] += a[i];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
-      }
-    }
-    __syncthreads();
-  }
-  float *rec = partials + (int64_t)blockIdx.x * rec_stride;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int o = to * 8 + i;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int k = kt0 + tk * 8 + j;
-      if (k < K) rec[(int64_t)o * K + k] = acc[i][j];
-    }
-    if (tk == 0 && blockIdx.y == 0) rec[(int64_t)128 * K + o] = dbacc[i];
-  }
+// Row chunk of the weight-gradient GEMM: enough chunks to give ~2 CTAs per SM, each at least 64 rows.  With out = 128
+// (two row tiles) that is at most kNumSMs chunks, which is what kScratchFloats holds for the projections.
+int dw_chunk(int64_t G, int out, int in) {
+  const int64_t tiles = (int64_t)((out + BM - 1) / BM) * ((in + BN - 1) / BN);
+  int64_t splits = (kDwTargetCtas + tiles - 1) / tiles;
+  const int64_t max_splits = (G + 63) / 64;
+  if (splits > max_splits) splits = max_splits;
+  if (splits < 1) splits = 1;
+  int64_t chunk = (G + splits - 1) / splits;
+  chunk = (chunk + BK - 1) / BK * BK;
+  return (int)chunk;
+}
+
+template <int MODE>
+int launch_gemm(const GemmArgs &a, int splits, cudaStream_t stream) {
+  const dim3 grid((a.M + BM - 1) / BM, (a.N + BN - 1) / BN, splits);
+  if (grid.y > 65535u || a.M > INT32_MAX - BM) return FNB_ERR_SIZE;
+  if (cudaError_t le = fnb_launch(k_mlp_gemm<MODE>, grid, dim3(kThreads), 0, stream, a)) return (int)le;
+  FNB_CHECK_LAUNCH();
+  return 0;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -281,7 +316,7 @@ __global__ void __launch_bounds__(256) k_node_scalars(const float *__restrict__ 
 }
 
 // Small-M linear layer: C[M, Nc] = A[M, Kd] @ op(B) (+ bias) for a few thousand rows at most (the energy head:
-// one row per molecule, [G, 256] x [256 -> 128] forward and [G, 128] x [128 -> 256] input gradient).  k_gemm tiles 64
+// one row per molecule, [G, 256] x [256 -> 128] forward and [G, 128] x [128 -> 256] input gradient).  The GEMM tiles 64
 // rows per CTA: 16 CTAs at G = 1024 and 45 us of pure latency on the critical path between the encoder's forward and
 // backward (gpurun_out/r4j_device_profile.log).  Here a CTA owns LR_ROWS = 8 rows (128 CTAs at G = 1024), a thread owns
 // output columns t, t + 128, ... for all 8 rows: the A rows sit in shared memory (broadcast reads), every thread
@@ -292,11 +327,12 @@ template <bool TRANS_B>
 __global__ void __launch_bounds__(LR_THREADS) k_linear_rows(GemmArgs g) {
   pdl_wait();
   __shared__ __align__(16) float sA[LR_ROWS][LR_MAXK];
+  const int Kd = g.K, Nc = g.N, ldb = TRANS_B ? Kd : Nc;   // A [M, Kd], C [M, Nc]
   const int tid = threadIdx.x;
   const int64_t m0 = (int64_t)blockIdx.x * LR_ROWS;
-  for (int i = tid; i < LR_ROWS * g.Kd; i += LR_THREADS) {
-    const int r = i / g.Kd, k = i - r * g.Kd;
-    sA[r][k] = (m0 + r < g.M) ? __ldg(g.A + (m0 + r) * g.lda + k) : 0.f;
+  for (int i = tid; i < LR_ROWS * Kd; i += LR_THREADS) {
+    const int r = i / Kd, k = i - r * Kd;
+    sA[r][k] = (m0 + r < g.M) ? __ldg(g.A + (m0 + r) * Kd + k) : 0.f;
   }
   __syncthreads();
   float acc[LR_MAXC][LR_ROWS];
@@ -308,16 +344,16 @@ __global__ void __launch_bounds__(LR_THREADS) k_linear_rows(GemmArgs g) {
 #pragma unroll
     for (int c = 0; c < LR_MAXC; ++c) {
       const int n = tid + c * LR_THREADS;
-      if (n >= g.Nc) break;
-      const float *brow = g.B + (int64_t)n * g.ldb;
-      for (int k0 = 0; k0 < g.Kd; k0 += 32) {        // 8 independent 16-byte loads in flight (Kd is a multiple of 32 here)
+      if (n >= Nc) break;
+      const float *brow = g.B + (int64_t)n * ldb;
+      for (int k0 = 0; k0 < Kd; k0 += 32) {        // 8 independent 16-byte loads in flight (Kd is a multiple of 32 here)
         float4 w[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) w[u] = (k0 + 4 * u < g.Kd) ? ldg4(brow + k0 + 4 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int u = 0; u < 8; ++u) w[u] = (k0 + 4 * u < Kd) ? ldg4(brow + k0 + 4 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
           const int k = k0 + 4 * u;
-          if (k >= g.Kd) break;
+          if (k >= Kd) break;
 #pragma unroll
           for (int r = 0; r < LR_ROWS; ++r) {
             const float4 a = ld4(&sA[r][k]);
@@ -330,14 +366,14 @@ __global__ void __launch_bounds__(LR_THREADS) k_linear_rows(GemmArgs g) {
       }
     }
   } else {                  // B [Kd, Nc]: coalesced reads of B's rows
-    for (int k0 = 0; k0 < g.Kd; k0 += 8) {             // 16 independent loads in flight per thread
+    for (int k0 = 0; k0 < Kd; k0 += 8) {             // 16 independent loads in flight per thread
       float w[8][LR_MAXC];
 #pragma unroll
       for (int u = 0; u < 8; ++u)
 #pragma unroll
         for (int c = 0; c < LR_MAXC; ++c) {
           const int n = tid + c * LR_THREADS;
-          w[u][c] = (n < g.Nc && k0 + u < g.Kd) ? __ldg(g.B + (int64_t)(k0 + u) * g.ldb + n) : 0.f;
+          w[u][c] = (n < Nc && k0 + u < Kd) ? __ldg(g.B + (int64_t)(k0 + u) * ldb + n) : 0.f;
         }
 #pragma unroll
       for (int u = 0; u < 8; ++u)
@@ -352,21 +388,76 @@ __global__ void __launch_bounds__(LR_THREADS) k_linear_rows(GemmArgs g) {
 #pragma unroll
   for (int c = 0; c < LR_MAXC; ++c) {
     const int n = tid + c * LR_THREADS;
-    if (n >= g.Nc) break;
+    if (n >= Nc) break;
     const float b = g.bias ? __ldg(g.bias + n) : 0.f;
 #pragma unroll
     for (int r = 0; r < LR_ROWS; ++r)
-      if (m0 + r < g.M) g.C[(m0 + r) * g.ldc + n] = acc[c][r] + b;
+      if (m0 + r < g.M) g.C[(m0 + r) * Nc + n] = acc[c][r] + b;
   }
 }
 
 // Shapes k_linear_rows takes: few rows, K a multiple of 32 up to 256, at most 256 output columns, 16-byte aligned rows.
-bool linear_rows_shape(int64_t M, int Kd, int Nc, const float *A, int lda, const float *B, int ldb, bool trans_b) {
-  return M > 0 && M <= 8192 && Kd <= LR_MAXK && (Kd & 31) == 0 && Nc <= LR_MAXC * LR_THREADS && fnb_aligned16(A) &&
-         (lda & 3) == 0 && (!trans_b || (fnb_aligned16(B) && (ldb & 3) == 0));
+bool linear_rows_shape(const GemmArgs &g, bool trans_b) {
+  return g.M > 0 && g.M <= 8192 && g.K <= LR_MAXK && (g.K & 31) == 0 && g.N <= LR_MAXC * LR_THREADS &&
+         fnb_aligned16(g.A) && (!trans_b || fnb_aligned16(g.B));
 }
 
+template <bool TRANS_B>
+int launch_linear_rows(const GemmArgs &g, cudaStream_t stream) {
+  if (cudaError_t le = fnb_launch(k_linear_rows<TRANS_B>, dim3((unsigned)((g.M + LR_ROWS - 1) / LR_ROWS)), dim3(LR_THREADS), 0,
+                                  stream, g))
+    return (int)le;
+  FNB_CHECK_LAUNCH();
+  return 0;
+}
+
+// The FFMA GEMM indexes rows with int32.
+inline bool gemm_rows_ok(int64_t n_rows) { return n_rows <= INT32_MAX - BM; }
+
 }  // namespace
+
+Drop fnb_drop(float p, int training, uint64_t base) {
+  Drop d{};
+  d.on = training && p > 0.f;
+  d.p = p;
+  d.scale = d.on ? 1.f / (1.f - p) : 1.f;
+  d.base = base;
+  return d;
+}
+
+int fnb_gemm(int mode, const GemmArgs &a, cudaStream_t stream) {
+  if (mode == GEMM_FWD) return launch_gemm<GEMM_FWD>(a, 1, stream);
+  if (mode == GEMM_DX) return launch_gemm<GEMM_DX>(a, 1, stream);
+  return FNB_ERR_MODE;
+}
+
+size_t fnb_gemm_dw_record_floats(int64_t rows, int out, int in) {
+  if (rows <= 0) return 0;
+  const int chunk = dw_chunk(rows, out, in);
+  return (size_t)((rows + chunk - 1) / chunk) * ((size_t)in * out + out);
+}
+
+int fnb_gemm_dw(const float *dz, const float *x, int64_t rows, int out, int in, float *dW, float *db, float *rec,
+                cudaStream_t stream) {
+  if (rows == 0) {
+    if (cudaError_t e = cudaMemsetAsync(dW, 0, (size_t)out * in * sizeof(float), stream)) return (int)e;
+    if (db)
+      if (cudaError_t e = cudaMemsetAsync(db, 0, (size_t)out * sizeof(float), stream)) return (int)e;
+    return 0;
+  }
+  GemmArgs w{};
+  w.A = dz; w.B = x; w.M = out; w.N = in; w.K = (int)rows;
+  w.k_chunk = dw_chunk(rows, out, in);
+  w.rec = rec;
+  w.rec_stride = (int64_t)in * out + out;
+  const int splits = (int)((rows + w.k_chunk - 1) / w.k_chunk);
+  if (const int rc = launch_gemm<GEMM_DW>(w, splits, stream)) return rc;
+  ReduceSegments segs{};
+  segs.n = db ? 2 : 1;
+  segs.rec_off[0] = 0; segs.width[0] = in * out; segs.out[0] = dW; segs.row_len[0] = in * out; segs.out_stride[0] = in * out;
+  segs.rec_off[1] = in * out; segs.width[1] = out; segs.out[1] = db; segs.row_len[1] = out; segs.out_stride[1] = out;
+  return fnb_launch_reduce_segments(rec, splits, (int)w.rec_stride, segs, stream);
+}
 
 extern "C" int fnb_proj_fwd(const float *x, const float *W, const float *b, int64_t n_rows, int K, const float *alpha,
                             int alpha_stride, int off_t, int off_s, float *h, float *S, int precision, void *stream) {
@@ -405,20 +496,12 @@ extern "C" int fnb_proj_fwd(const float *x, const float *W, const float *b, int6
     FNB_CHECK_LAUNCH();
     return 0;
   }
-  GemmArgs g;
-  g.A = x; g.lda = K; g.B = W; g.ldb = K; g.C = h; g.ldc = kD; g.M = n_rows; g.Kd = K; g.Nc = kD; g.bias = b;
+  if (!gemm_rows_ok(n_rows)) return FNB_ERR_SIZE;
+  GemmArgs g{};
+  g.A = x; g.B = W; g.M = (int)n_rows; g.N = kD; g.K = K; g.C = h; g.bias = b;
+  if (!S && K > kD && linear_rows_shape(g, true)) return launch_linear_rows<true>(g, (cudaStream_t)stream);
   g.alpha = alpha; g.alpha_stride = alpha_stride; g.off_t = off_t; g.off_s = off_s; g.S = S;
-  if (!S && K > kD && linear_rows_shape(n_rows, K, kD, x, K, W, K, true)) {
-    if (cudaError_t le = fnb_launch(k_linear_rows<true>, dim3((unsigned)((n_rows + LR_ROWS - 1) / LR_ROWS)), dim3(LR_THREADS), 0,
-                                    (cudaStream_t)stream, g))
-      return (int)le;
-    FNB_CHECK_LAUNCH();
-    return 0;
-  }
-  dim3 grid((unsigned)((n_rows + BM - 1) / BM), 1);
-  if (cudaError_t le = fnb_launch(k_gemm<true, true>, grid, dim3(kGemmThreads), 0, (cudaStream_t)stream, g)) return (int)le;
-  FNB_CHECK_LAUNCH();
-  return 0;
+  return launch_gemm<GEMM_FWD>(g, 1, (cudaStream_t)stream);
 }
 
 extern "C" int fnb_proj_bwd(const float *x, const float *W, const float *dh, int64_t n_rows, int K, float *dx,
@@ -450,20 +533,11 @@ int fnb_proj_bwd_dx(const float *W, const float *Wt_pre, const float *dh, int64_
                             precision == FNB_PRECISION_TF32X3);
     if (rc != FNB_ERR_MODE) return rc;
   }
-  GemmArgs g;
-  g.A = dh; g.lda = kD; g.B = W; g.ldb = K; g.C = dx; g.ldc = K; g.M = n_rows; g.Kd = kD; g.Nc = K; g.bias = nullptr;
-  g.alpha = nullptr; g.alpha_stride = 0; g.off_t = 0; g.off_s = 0; g.S = nullptr;
-  if (linear_rows_shape(n_rows, kD, K, dh, kD, W, K, false)) {
-    if (cudaError_t le = fnb_launch(k_linear_rows<false>, dim3((unsigned)((n_rows + LR_ROWS - 1) / LR_ROWS)), dim3(LR_THREADS), 0,
-                                    stream, g))
-      return (int)le;
-    FNB_CHECK_LAUNCH();
-    return 0;
-  }
-  dim3 grid((unsigned)((n_rows + BM - 1) / BM), (unsigned)((K + BN - 1) / BN));
-  if (cudaError_t le = fnb_launch(k_gemm<false, false>, grid, dim3(kGemmThreads), 0, stream, g)) return (int)le;
-  FNB_CHECK_LAUNCH();
-  return 0;
+  if (!gemm_rows_ok(n_rows)) return FNB_ERR_SIZE;
+  GemmArgs g{};
+  g.A = dh; g.B = W; g.M = (int)n_rows; g.N = K; g.K = kD; g.C = dx;
+  if (linear_rows_shape(g, false)) return launch_linear_rows<false>(g, stream);
+  return launch_gemm<GEMM_DX>(g, 1, stream);
 }
 
 int fnb_proj_bwd_dw(const float *x, const float *dh, int64_t n_rows, int K, float *dW, float *db, int precision,
@@ -477,23 +551,8 @@ int fnb_proj_bwd_dw(const float *x, const float *dh, int64_t n_rows, int K, floa
                                     precision == FNB_PRECISION_TF32X3);
     if (rc != FNB_ERR_MODE) return rc;
   }
-  int64_t nb = (n_rows + 255) / 256;
-  if (nb > kNumSMs) nb = kNumSMs;
-  if (nb < 1) nb = 1;
-  int64_t rows_per_block = (n_rows + nb - 1) / nb;
-  rows_per_block = ((rows_per_block + kDwRows - 1) / kDwRows) * kDwRows;
-  if (rows_per_block < kDwRows) rows_per_block = kDwRows;
-  const int64_t rec_stride = (int64_t)128 * K + 128;
-  dim3 grid((unsigned)nb, (unsigned)((K + 127) / 128));
-  if (cudaError_t le = fnb_launch(k_proj_dw, grid, dim3(256), 0, stream, dh, x, n_rows, K, rows_per_block, scratch_body(scratch),
-                                  rec_stride))
-    return (int)le;
-  FNB_CHECK_LAUNCH();
-  ReduceSegments segs{};
-  segs.n = db ? 2 : 1;
-  segs.rec_off[0] = 0;       segs.width[0] = 128 * K; segs.out[0] = dW; segs.row_len[0] = 128 * K; segs.out_stride[0] = 128 * K;
-  segs.rec_off[1] = 128 * K; segs.width[1] = 128;     segs.out[1] = db; segs.row_len[1] = 128;     segs.out_stride[1] = 128;
-  return fnb_launch_reduce_segments(scratch_body(scratch), (int)nb, (int)rec_stride, segs, stream);
+  if (!gemm_rows_ok(n_rows)) return FNB_ERR_SIZE;
+  return fnb_gemm_dw(dh, x, n_rows, kD, K, dW, db, scratch_body(scratch), stream);
 }
 
 int fnb_proj_bwd_impl(const float *x, const float *W, const float *Wt_pre, const float *dh, int64_t n_rows, int K,

@@ -1,8 +1,10 @@
 #!/usr/bin/env python
 """Projection GEMMs alone, per precision mode (0 FFMA, 1 TF32, 2 3xTF32): cold (L2 flushed) and back-to-back timings
-with CUDA events; algorithmic GB/s = (N*K + N*128 + N*8)*4 bytes (forward), 4*N*128*4 (dX + dW).
+with CUDA events; algorithmic GB/s = (N*K + N*128 + N*8)*4 bytes (forward), (2*N*128 + 2*N*K)*4 (dX + dW).  K is the
+weight's input width: 128 for the attention projections, 167 / 17 / 6 for the raw input features of layer 0, 256 for
+the energy head's readout.
 
-usage (GPU box): python scripts/gemm_bench.py [--rows 53940,26000,10000] [--iters 20]
+usage (GPU box): python scripts/gemm_bench.py [--rows 53940,26000,10000] [--k 128] [--iters 20]
 """
 import argparse
 import os
@@ -18,6 +20,7 @@ sys.path.insert(0, ROOT)
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rows", default="53940,26000,10000,215000")
+    ap.add_argument("--k", type=int, default=128, help="input width K of the [128, K] weight")
     ap.add_argument("--iters", type=int, default=20)
     args = ap.parse_args()
     from fragnet_b200 import ops
@@ -39,16 +42,17 @@ def main():
         return statistics.median(ts)
 
     a96 = torch.randn(4, 96, device=dev) * 0.1
+    K = args.k
     for N in [int(r) for r in args.rows.split(",")]:
-        x, W, b, dh = (torch.randn(N, 128, device=dev), torch.randn(128, 128, device=dev) * 0.1,
+        x, W, b, dh = (torch.randn(N, K, device=dev), torch.randn(128, K, device=dev) * 0.1,
                        torch.randn(128, device=dev), torch.randn(N, 128, device=dev))
-        fb, bb = (N * 128 + N * 128 + N * 8) * 4, 4 * N * 128 * 4
+        fb, bb = (N * K + N * 128 + N * 8) * 4, (2 * N * 128 + 2 * N * K) * 4
         for prec, name in ((0, "ffma"), (1, "tf32"), (2, "3xtf32")):
             f = lambda: ops.proj_fwd(x, W, b, a96, 96, 0, 64, precision=prec)
             g = lambda: ops.proj_bwd(x, W, dh, True, prec, want_db=False)
             w = lambda: ops.proj_bwd(x, W, dh, False, prec, want_db=False)
             fc, fw, gc, gw, wc = timeit(f, True), timeit(f, False), timeit(g, True), timeit(g, False), timeit(w, True)
-            print(f"N={N:7d} {name:7s} fwd cold {fc:7.2f} us ({fb / fc / 1e3:6.0f} GB/s) warm {fw:7.2f} us | "
+            print(f"N={N:7d} K={K:3d} {name:7s} fwd cold {fc:7.2f} us ({fb / fc / 1e3:6.0f} GB/s) warm {fw:7.2f} us | "
                   f"dX+dW cold {gc:7.2f} us ({bb / gc / 1e3:6.0f} GB/s) warm {gw:7.2f} us | dW only cold {wc:7.2f} us",
                   flush=True)
 

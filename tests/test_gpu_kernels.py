@@ -8,7 +8,8 @@ from conftest import FP32_REL_TOL, rel_err
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("n,K", [(1, 128), (77, 128), (1000, 167), (333, 17), (65, 6), (4097, 128)])
+@pytest.mark.parametrize("n,K", [(1, 128), (77, 128), (1000, 167), (333, 17), (65, 6), (4097, 128), (9000, 128),
+                                 (9000, 167)])
 def test_projection_forward_backward(n, K):
     from fragnet_b200 import ops
     g = torch.Generator().manual_seed(n * 1000 + K)
@@ -28,6 +29,25 @@ def test_projection_forward_backward(n, K):
     assert rel_err(dW, dh.t() @ x) <= FP32_REL_TOL
     assert rel_err(db, dh.sum(0)) <= FP32_REL_TOL
     assert rel_err(ops.node_scalars(h, alpha.cuda(), 96, 0, 64), Sref) <= FP32_REL_TOL
+
+
+def test_projection_forward_beyond_65535_row_tiles():
+    # 65 538 tiles of 64 rows: more than a grid's y dimension holds, so the GEMM's row tiles must be on x
+    from fragnet_b200 import ops
+    n, K, m = 4_194_400, 128, 3000
+    g = torch.Generator(device="cuda").manual_seed(11)
+    x = torch.randn(n, K, device="cuda", generator=g)
+    W = torch.randn(128, K, device="cuda", generator=g) * 0.2
+    b = torch.randn(128, device="cuda", generator=g)
+    alpha = torch.randn(4, 96, device="cuda", generator=g)
+    h, S = ops.proj_fwd(x, W, b, alpha, 96, 0, 64)
+    for rows in (slice(0, m), slice(n - m, n)):
+        href = F.linear(x[rows].double(), W.double(), b.double())
+        assert rel_err(h[rows], href) <= FP32_REL_TOL
+        hv = href.view(m, 4, 32)
+        ad = alpha.double()
+        Sref = torch.cat([(hv * ad[:, 0:32]).sum(-1), (hv * ad[:, 64:96]).sum(-1)], dim=1)
+        assert rel_err(S[rows], Sref) <= FP32_REL_TOL
 
 
 def test_segment_sum_and_gather():

@@ -12,7 +12,7 @@ X3_TOL = 4e-6        # 3xTF32: hi*hi + hi*lo + lo*hi, FP32 accumulate (measured 
 
 
 @pytest.mark.parametrize("n,K", [(1, 128), (127, 128), (129, 128), (1000, 128), (54001, 128), (300, 32), (300, 64),
-                                 (300, 256), (40000, 128), (9473, 128)])
+                                 (300, 256), (40000, 128), (9473, 128), (9473, 256)])
 def test_x3_projection_forward_is_fp32_grade(n, K):
     from fragnet_b200 import ops
     g = torch.Generator().manual_seed(1000 + n + K)
