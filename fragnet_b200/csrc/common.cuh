@@ -35,8 +35,29 @@ extern unsigned long long g_fnb_launches;
     if (e__ != cudaSuccess) return (int)e__;            \
     __atomic_fetch_add(&g_fnb_launches, 1ull, __ATOMIC_RELAXED); \
   } while (0)
+// Returns a non-zero status (FNB_ERR_* or a cudaError_t) to the caller.
+#define RC(expr)             \
+  do {                       \
+    const int rc__ = (expr); \
+    if (rc__) return rc__;   \
+  } while (0)
 static inline bool fnb_aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 __device__ __forceinline__ bool fnb_is_aligned16_dev(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// Workspace carving: every buffer starts on a 256-byte boundary.  base == NULL only measures (take() returns NULL).
+struct Arena {
+  char *base;
+  size_t off;
+  template <class T>
+  T *take(size_t n) {
+    off = (off + 255) & ~(size_t)255;
+    T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
+    off += n * sizeof(T);
+    return p;
+  }
+  char *bytes(size_t n) { return take<char>(n); }
+  size_t total() const { return (off + 255) & ~(size_t)255; }   // bytes of the layout, a multiple of 256
+};
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

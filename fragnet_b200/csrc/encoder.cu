@@ -20,18 +20,6 @@ namespace {
 constexpr int AB_STRIDE = 96, AB_T = 0, AB_E = 32, AB_S = 64;    // a_b / f_a_b = [target 32 | edge 32 | source 32]
 constexpr int A_STRIDE = 192, A_T = 0, A_E = 32, A_S = 160;      // a / f     = [target 32 | edge 128 | source 32]
 
-struct Arena {
-  char *base;
-  size_t off;
-  template <class T>
-  T *take(size_t n) {
-    off = (off + 255) & ~(size_t)255;
-    T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
-    off += n * sizeof(T);
-    return p;
-  }
-};
-
 struct LayerBufs {
   float *xa0;                                                   // layer 0: Dropout(x_atoms) (training only)
   float *x_pad[3], *W_pad[3];                                   // layer 0, TF32: inputs / weights zero-padded to k_pad columns
@@ -120,7 +108,7 @@ size_t layout(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fnb_l
     }
     if (bufs) bufs[l] = b;
   }
-  return (a.off + 255) & ~(size_t)255;
+  return a.total();
 }
 
 struct BwdBufs {
@@ -156,7 +144,7 @@ size_t bwd_layout(const fnb_batch_plan *plan, const fnb_encoder_opts *o, char *b
   b.scratch5 = a.take<float>(kScratchFloats);
   b.scratch6 = a.take<float>(kScratchFloats);
   if (out) *out = b;
-  return (a.off + 255) & ~(size_t)255;
+  return a.total();
 }
 
 // RNG counters consumed by one dropout site over n elements.
@@ -257,12 +245,6 @@ __global__ void __launch_bounds__(256) k_gather_rows4(const float *__restrict__ 
   const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (e < n) st4(out + e * 4, ldg4(src + (int64_t)__ldg(index + e) * 4));
 }
-
-#define RC(expr)            \
-  do {                      \
-    const int rc__ = (expr); \
-    if (rc__) return rc__;   \
-  } while (0)
 
 int check_common(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fnb_layer_params *L,
                  const fnb_encoder_io *io) {

@@ -4,7 +4,7 @@
 // A head is a list of linear layers (fnb_mlp_layer), each  y = act(drop_out(drop_in(x) W^T + b)).  Every layer is one
 // launch of the library's FP32 FFMA GEMM (k_mlp_gemm, proj.cu: 64 x 64 tile, 4 x 4 outputs per thread) whose epilogue
 // applies the bias, the dropout masks and the activation; the heads stay exact FP32 in every precision mode (as
-// k_linear_rows does for the energy head): rows are molecules (128 to a few thousand) and widths are whatever a hyper-parameter search picks,
+// k_energy_head does for the energy head): rows are molecules (128 to a few thousand) and widths are whatever a hyper-parameter search picks,
 // shapes the N = 128 tensor-core kernels do not cover.
 //
 // Buffers of a run (FnbMlpRun): xd[l] is what layer l multiplies (its input after its input dropout), u[l] its output
@@ -22,12 +22,6 @@
 #include <algorithm>
 
 #include "common.cuh"
-
-#define RC_INLINE(expr)      \
-  do {                       \
-    const int rc__ = (expr); \
-    if (rc__) return rc__;   \
-  } while (0)
 
 namespace {
 
@@ -121,8 +115,8 @@ int fnb_mlp_forward(const FnbMlpRun *r, cudaStream_t stream) {
   const fnb_mlp_layer *L = r->L;
   const fnb_mlp_layer &first = L[0];
   if (r->xd[0] != r->x0)
-    RC_INLINE(fnb_dropout_relu_fwd(r->x0, r->xd[0], r->G * first.in_dim, first.p_in, r->training, 0, r->seed, r->in_base[0],
-                                   stream));
+    RC(fnb_dropout_relu_fwd(r->x0, r->xd[0], r->G * first.in_dim, first.p_in, r->training, 0, r->seed, r->in_base[0],
+                            stream));
   for (int l = 0; l < r->n; ++l) {
     GemmArgs a{};
     a.A = r->xd[l]; a.B = L[l].W; a.M = (int)r->G; a.N = L[l].out_dim; a.K = L[l].in_dim;
@@ -132,7 +126,7 @@ int fnb_mlp_forward(const FnbMlpRun *r, cudaStream_t stream) {
     a.drop2 = last ? fnb_drop(0.f, 0, 0) : fnb_drop(L[l + 1].p_in, r->training, r->in_base[l + 1]);
     a.u = last ? nullptr : r->u[l];
     a.C = last ? r->out : r->xd[l + 1];
-    RC_INLINE(fnb_gemm(GEMM_FWD, a, stream));
+    RC(fnb_gemm(GEMM_FWD, a, stream));
   }
   return 0;
 }
@@ -142,7 +136,7 @@ int fnb_mlp_backward(const FnbMlpRun *r, cudaStream_t stream) {
   for (int l = r->n - 1; l >= 0; --l) {
     // weight and bias gradients: per-chunk records, then a fixed-order sum (not for a frozen layer)
     if (L[l].dW)
-      RC_INLINE(fnb_gemm_dw(r->dz[l], r->xd[l], r->G, L[l].out_dim, L[l].in_dim, L[l].dW, L[l].db, r->rec, stream));
+      RC(fnb_gemm_dw(r->dz[l], r->xd[l], r->G, L[l].out_dim, L[l].in_dim, L[l].dW, L[l].db, r->rec, stream));
     // input gradient, folded down to dz of the layer below (or the gradient of the head input): only while a trained
     // layer lies below, or the caller wants the head input's gradient
     if (!fnb_mlp_needs_dx(L, l, r->dx0 != nullptr)) break;
@@ -157,7 +151,7 @@ int fnb_mlp_backward(const FnbMlpRun *r, cudaStream_t stream) {
       d.drop2 = fnb_drop(0.f, 0, 0);
       d.C = r->dx0;
     }
-    RC_INLINE(fnb_gemm(GEMM_DX, d, stream));
+    RC(fnb_gemm(GEMM_DX, d, stream));
   }
   return 0;
 }

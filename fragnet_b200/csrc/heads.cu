@@ -11,31 +11,23 @@
 // (profiles/r1n_device_profile.log: ~700 us of library kernels, ~2 ms of host time per step at batch 1024).
 //
 // Decomposition.  Every head is "wide first layer + narrow tail":
-//   * the first layers are dense [N,128]x[128,64|128] contractions over tens of thousands of rows: they run on the
-//     projection kernels of this library (tcgen05 TF32 or FP32 FFMA, tc_gemm.cu / proj.cu) with the 64-row weights
-//     zero-padded to 128 rows, so forward, dX and dW reuse three tested kernels;
+//   * the first layers of the per-atom / per-bond heads are dense [N,128]x[128,64] contractions over tens of
+//     thousands of rows: they run on the projection kernels of this library (tcgen05 TF32 or FP32 FFMA, tc_gemm.cu /
+//     proj.cu) with the 64-row weights zero-padded to 128 rows, so forward, dX and dW reuse three tested kernels;
 //   * the 384-wide bond-length reduce layer never materialises the [Ea,384] concatenation: Linear(cat(a,b,e)) =
 //     a W_a^T + b W_b^T + e W_e^T + bias, i.e. two [Na,128] and one [Ea,128] projections followed by a gather-add;
-//   * the tails (64-32-1 or 128-64-1 per row, ~2-8 kFMA) are FP32 thread-per-row kernels with the weights broadcast
-//     from shared memory; the backward tail recomputes the hidden layer, and reduces the parameter gradients of the
-//     tail (dW1 [MID,IN], db1, dW2, db2, db0) over the rows of its tile out of shared memory into per-CTA records.
+//   * their tails (64-32-1 per row, ~2 kFMA) are register-tiled FP32 kernels out of shared memory; the backward tail
+//     recomputes the hidden layer, and reduces the parameter gradients of the tail (dW1 [MID,IN], db1, dW2, db2, db0)
+//     over the rows of its tile into per-CTA records;
+//   * the energy head (~1e3 molecules) is one kernel, k_energy_head, in the forward and in the backward program:
+//     readout, first layer and tail (128-64-1), and in the backward the tail's gradients, the input gradient and the
+//     fragments' readout backward; exact FP32 in every precision mode.  Only the weight gradient of its first layer
+//     ([128,256], summed over the molecules) runs on the projection kernels.
 // Parameter-gradient sums are fixed-order two-stage reductions: run-to-run deterministic, no atomics.
 
 #include "common.cuh"
 
 namespace {
-
-struct Arena {
-  char *base;
-  size_t off;
-  template <class T>
-  T *take(size_t n) {
-    off = (off + 255) & ~(size_t)255;
-    T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
-    off += n * sizeof(T);
-    return p;
-  }
-};
 
 constexpr int kPadMat = kD * kD;
 
@@ -43,7 +35,7 @@ constexpr int kPadMat = kD * kD;
 struct FwdBufs {
   // saved for backward
   float *h0_ba, *h0_da;          // [Na,128], [Ea,128] first-layer pre-activations (columns 64.. are zero)
-  float *readout, *h0_fc;        // [G,256], [G,128]
+  float *readout;                // [G,256] (read by the weight gradient of the energy head's first layer)
   float *W0pad_ba, *W0pad_da;    // [128,128] rows 64.. zero
   float *W0padT_ba, *W0padT_da;  // transposes (B operand of the dX GEMM)
   // transient (bond-length head and padded operands)
@@ -57,7 +49,6 @@ size_t fwd_layout(int64_t Na, int64_t Ea, int64_t G, char *base, FwdBufs *out) {
   b.h0_ba = a.take<float>(Na * kD);
   b.h0_da = a.take<float>(Ea * kD);
   b.readout = a.take<float>(G * 2 * kD);
-  b.h0_fc = a.take<float>(G * kD);
   b.W0pad_ba = a.take<float>(kPadMat); b.W0pad_da = a.take<float>(kPadMat);
   b.W0padT_ba = a.take<float>(kPadMat); b.W0padT_da = a.take<float>(kPadMat);
   b.b0pad_ba = a.take<float>(kD); b.b0pad_da = a.take<float>(kD); b.b0pad_bl = a.take<float>(kD);
@@ -66,7 +57,7 @@ size_t fwd_layout(int64_t Na, int64_t Ea, int64_t G, char *base, FwdBufs *out) {
   b.U = a.take<float>(Na * kD); b.V = a.take<float>(Na * kD);
   b.T = a.take<float>(Ea * kD); b.h0_bl = a.take<float>(Ea * kD);
   if (out) *out = b;
-  return (a.off + 255) & ~(size_t)255;
+  return a.total();
 }
 
 // ---- backward workspace -----------------------------------------------------------------------------------------------
@@ -103,7 +94,7 @@ size_t bwd_layout(int64_t Na, int64_t Ea, int64_t G, char *base, BwdBufs *out) {
   b.scratch3 = a.take<float>(kScratchFloats);
   b.loss_parts = a.take<float>(4);
   if (out) *out = b;
-  return (a.off + 255) & ~(size_t)255;
+  return a.total();
 }
 
 // ---- operand packing --------------------------------------------------------------------------------------------------
@@ -180,220 +171,6 @@ __device__ __forceinline__ void load_tail_weights(const TailJob &job, float *sW1
     sW2[i] = __ldg(job.W2 + i);
   }
   if (threadIdx.x == 0) sb2[0] = __ldg(job.b2);
-}
-
-// acc[j] = b1[j] + sum_k W1[j,k] ReLU(h0[k]) for the row at `rp`.
-template <int IN, int MID>
-__device__ __forceinline__ void tail_hidden(const float *rp, const float *sW1t, const float *sb1, float (&acc)[MID]) {
-#pragma unroll
-  for (int j = 0; j < MID; ++j) acc[j] = sb1[j];
-#pragma unroll 2
-  for (int k4 = 0; k4 < IN / 4; ++k4) {
-    const float4 a = ldg4(rp + k4 * 4);
-    const float av[4] = {fmaxf(a.x, 0.f), fmaxf(a.y, 0.f), fmaxf(a.z, 0.f), fmaxf(a.w, 0.f)};
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const float *w = sW1t + (k4 * 4 + u) * MID;
-#pragma unroll
-      for (int j4 = 0; j4 < MID / 4; ++j4) {
-        const float4 wv = ld4(w + j4 * 4);
-        acc[j4 * 4 + 0] = fmaf(av[u], wv.x, acc[j4 * 4 + 0]);
-        acc[j4 * 4 + 1] = fmaf(av[u], wv.y, acc[j4 * 4 + 1]);
-        acc[j4 * 4 + 2] = fmaf(av[u], wv.z, acc[j4 * 4 + 2]);
-        acc[j4 * 4 + 3] = fmaf(av[u], wv.w, acc[j4 * 4 + 3]);
-      }
-    }
-  }
-}
-
-template <int IN, int MID>
-__global__ void __launch_bounds__(128) k_mlp_tail_fwd(TailJobs J) {
-  pdl_wait();
-  const TailJob &job = J.j[blockIdx.y];
-  __shared__ __align__(16) float sW1t[IN * MID];
-  __shared__ float sb1[MID], sW2[MID], sb2[1];
-  if ((int64_t)blockIdx.x * 128 >= job.n) return;
-  load_tail_weights<IN, MID>(job, sW1t, sb1, sW2, sb2);
-  __syncthreads();
-  for (int64_t row = (int64_t)blockIdx.x * 128 + threadIdx.x; row < job.n; row += (int64_t)gridDim.x * 128) {
-    float acc[MID];
-    tail_hidden<IN, MID>(job.h0 + row * kD, sW1t, sb1, acc);
-    float o = sb2[0];
-#pragma unroll
-    for (int j = 0; j < MID; ++j) o = fmaf(fmaxf(acc[j], 0.f), sW2[j], o);
-    job.out[row] = o;
-  }
-}
-
-// Backward tail.  THREADS threads, ROWS <= THREADS rows per tile (thread-per-row phase), then the cross-row sums of
-// the tile: thread t owns row j = t / 4 of dW1 and, of every 16-column group, the 4 columns 4 (t % 4) .. +3 (the four
-// threads of a row read one contiguous 64-byte chunk of shared memory per step), plus one of the vector sums.
-template <int IN, int MID, int THREADS, int ROWS>
-__global__ void __launch_bounds__(THREADS) k_mlp_tail_bwd(TailJobs J) {
-  pdl_wait();
-  constexpr int KPT = MID * IN / THREADS;      // k per thread in the dW1 phase
-  static_assert(MID * 4 == THREADS && KPT * 4 == IN, "dW1 ownership needs THREADS = 4 * MID");
-  constexpr int SA = IN + 4, SD = MID + 1;     // shared-memory row strides
-  constexpr int REC = rec_floats(IN, MID);
-  const TailJob &job = J.j[blockIdx.y];
-  extern __shared__ __align__(16) float smem[];
-  float *sW1t = smem;                          // [IN][MID]
-  float *s_a = sW1t + IN * MID;                // [ROWS][SA]   ReLU(h0)
-  float *s_dh0 = s_a + ROWS * SA;              // [ROWS][SA]
-  float *s_d1 = s_dh0 + ROWS * SA;             // [ROWS][SD]   gradient of the hidden pre-activation
-  float *s_h1g = s_d1 + ROWS * SD;             // [ROWS][SD]   gout * ReLU(hidden)
-  float *s_g = s_h1g + ROWS * SD;              // [ROWS]
-  __shared__ float sb1[MID], sW2[MID], sb2[1];
-  __shared__ float s_part[ROWS * 8], s_loss[ROWS];
-  const int tid = threadIdx.x;
-  const int64_t n_tiles = (job.n + ROWS - 1) / ROWS;
-  if (blockIdx.x >= n_tiles && blockIdx.x > 0) return;   // CTA 0 always runs: it writes a (possibly zero) record
-  load_tail_weights<IN, MID>(job, sW1t, sb1, sW2, sb2);
-  float lossacc = 0.f;   // tid == 0
-  const int oj = tid >> 2, ok0 = (tid & 3) * 4;
-  float wacc[KPT];
-#pragma unroll
-  for (int q = 0; q < KPT; ++q) wacc[q] = 0.f;
-  float vacc = 0.f;    // tid & 3 == 0: db1[oj];  == 1: dW2[oj]
-  float b0acc = 0.f;   // tid < IN: db0[tid]
-  float b2acc = 0.f;   // tid == 0: db2
-  __syncthreads();
-
-  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const int64_t r0 = tile * ROWS;
-    const int rows = (int)min((int64_t)ROWS, job.n - r0);
-    // ---- phase 1: SPLIT = THREADS / ROWS threads per row (row = tid % ROWS, part q = tid / ROWS): a thread computes
-    // MID / SPLIT hidden units, then IN / SPLIT columns of dh0 -- 1/SPLIT of the serial chain of the thread-per-row
-    // form, which at ~1e3 rows (the energy head) is pure latency
-    {
-      constexpr int SPLIT = THREADS / ROWS, JQ = MID / SPLIT, KQ = IN / SPLIT;
-      static_assert(THREADS == SPLIT * ROWS && (JQ % 4) == 0 && (KQ % 4) == 0 && SPLIT <= 8, "phase 1 row split");
-      const int r = tid % ROWS, q = tid / ROWS;
-      const bool live = r < rows;
-      const int64_t row = r0 + r;
-      const float *rp = job.h0 + (live ? row : 0) * kD;
-      const bool fused = job.target != nullptr;
-      float g = 0.f;
-      float acc[JQ];
-#pragma unroll
-      for (int j = 0; j < JQ; ++j) acc[j] = 0.f;
-      if (live) {
-        g = __ldg((fused ? job.target : job.gout) + row);
-#pragma unroll
-        for (int j = 0; j < JQ; ++j) acc[j] = sb1[q * JQ + j];
-#pragma unroll 2
-        for (int k4 = 0; k4 < IN / 4; ++k4) {
-          const float4 a = ldg4(rp + k4 * 4);
-          const float av[4] = {fmaxf(a.x, 0.f), fmaxf(a.y, 0.f), fmaxf(a.z, 0.f), fmaxf(a.w, 0.f)};
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const float *w = sW1t + (k4 * 4 + u) * MID + q * JQ;
-#pragma unroll
-            for (int j4 = 0; j4 < JQ / 4; ++j4) {
-              const float4 wv = ld4(w + j4 * 4);
-              acc[j4 * 4 + 0] = fmaf(av[u], wv.x, acc[j4 * 4 + 0]);
-              acc[j4 * 4 + 1] = fmaf(av[u], wv.y, acc[j4 * 4 + 1]);
-              acc[j4 * 4 + 2] = fmaf(av[u], wv.z, acc[j4 * 4 + 2]);
-              acc[j4 * 4 + 3] = fmaf(av[u], wv.w, acc[j4 * 4 + 3]);
-            }
-          }
-        }
-      }
-      if (fused) {   // the row's prediction = sum of the SPLIT partial dots with W2 (+ b2); g held the target
-        float o = 0.f;
-#pragma unroll
-        for (int j = 0; j < JQ; ++j) o = fmaf(fmaxf(acc[j], 0.f), sW2[q * JQ + j], o);
-        s_part[r * 8 + q] = o;
-        __syncthreads();
-        float pred = sb2[0];
-#pragma unroll
-        for (int qq = 0; qq < SPLIT; ++qq) pred += s_part[r * 8 + qq];
-        const float diff = live ? pred - g : 0.f;
-        g = 2.f * job.loss_coef * diff;
-        if (q == 0) s_loss[r] = job.loss_coef * diff * diff;
-      } else if (q == 0) {
-        s_loss[r] = 0.f;
-      }
-      if (live) {
-#pragma unroll
-        for (int j = 0; j < JQ; ++j) {
-          const int jj = q * JQ + j;
-          s_h1g[r * SD + jj] = g * fmaxf(acc[j], 0.f);
-          s_d1[r * SD + jj] = acc[j] > 0.f ? g * sW2[jj] : 0.f;
-        }
-      }
-      if (q == 0) s_g[r] = g;
-      __syncthreads();   // the row's four quarters of d1 are in shared memory
-      if (live) {
-        float d1[MID];
-#pragma unroll
-        for (int j = 0; j < MID; ++j) d1[j] = s_d1[r * SD + j];
-        float *dp = job.dh0 + row * kD;
-        float *a_row = s_a + r * SA, *d_row = s_dh0 + r * SA;
-#pragma unroll 1
-        for (int k4 = q * (KQ / 4); k4 < (q + 1) * (KQ / 4); ++k4) {
-          const float4 a = ldg4(rp + k4 * 4);
-          const float av[4] = {a.x, a.y, a.z, a.w};
-          float dv[4];
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const float *w = sW1t + (k4 * 4 + u) * MID;
-            float s_ = 0.f;
-#pragma unroll
-            for (int j4 = 0; j4 < MID / 4; ++j4) {
-              const float4 wv = ld4(w + j4 * 4);
-              s_ = fmaf(d1[j4 * 4 + 0], wv.x, s_);
-              s_ = fmaf(d1[j4 * 4 + 1], wv.y, s_);
-              s_ = fmaf(d1[j4 * 4 + 2], wv.z, s_);
-              s_ = fmaf(d1[j4 * 4 + 3], wv.w, s_);
-            }
-            dv[u] = av[u] > 0.f ? s_ : 0.f;
-          }
-          st4(dp + k4 * 4, make_float4(dv[0], dv[1], dv[2], dv[3]));
-          st4(d_row + k4 * 4, make_float4(dv[0], dv[1], dv[2], dv[3]));
-          st4(a_row + k4 * 4, make_float4(fmaxf(av[0], 0.f), fmaxf(av[1], 0.f), fmaxf(av[2], 0.f), fmaxf(av[3], 0.f)));
-        }
-        if (IN < kD && q == 0) {
-#pragma unroll
-          for (int k4 = IN / 4; k4 < kD / 4; ++k4) st4(dp + k4 * 4, make_float4(0.f, 0.f, 0.f, 0.f));
-        }
-      }
-    }
-    __syncthreads();
-    // ---- phase 2: sums over the rows of the tile
-    for (int r = 0; r < rows; ++r) {
-      const float d = s_d1[r * SD + oj];
-      const float *ap = s_a + r * SA + ok0;
-#pragma unroll
-      for (int q4 = 0; q4 < KPT / 4; ++q4) {
-        const float4 av = ld4(ap + q4 * 16);
-        wacc[q4 * 4 + 0] = fmaf(d, av.x, wacc[q4 * 4 + 0]);
-        wacc[q4 * 4 + 1] = fmaf(d, av.y, wacc[q4 * 4 + 1]);
-        wacc[q4 * 4 + 2] = fmaf(d, av.z, wacc[q4 * 4 + 2]);
-        wacc[q4 * 4 + 3] = fmaf(d, av.w, wacc[q4 * 4 + 3]);
-      }
-      if ((tid & 3) == 0) vacc += d;
-      else if ((tid & 3) == 1) vacc += s_h1g[r * SD + oj];
-      if (tid < IN) b0acc += s_dh0[r * SA + tid];
-      if (tid == 0) {
-        b2acc += s_g[r];
-        lossacc += s_loss[r];
-      }
-    }
-    __syncthreads();
-  }
-  // ---- CTA record: [dW1 MID*IN][db1 MID][dW2 MID][db2 1][db0 IN]
-  float *rec = job.rec + (size_t)blockIdx.x * REC;
-#pragma unroll
-  for (int q4 = 0; q4 < KPT / 4; ++q4)
-    st4(rec + oj * IN + ok0 + q4 * 16, make_float4(wacc[q4 * 4], wacc[q4 * 4 + 1], wacc[q4 * 4 + 2], wacc[q4 * 4 + 3]));
-  if ((tid & 3) == 0) rec[MID * IN + oj] = vacc;
-  if ((tid & 3) == 1) rec[MID * IN + MID + oj] = vacc;
-  if (tid == 0) {
-    rec[MID * IN + 2 * MID] = b2acc;
-    rec[MID * IN + 2 * MID + 1 + IN] = lossacc;   // spare slot of the record (rec_floats rounds up to 4)
-  }
-  if (tid < IN) rec[MID * IN + 2 * MID + 1 + tid] = b0acc;
 }
 
 // Forward tail of the big heads (IN = 64, MID = 32), register-tiled like k_mlp_tail_bwd2's first GEMM: the ReLU(h0) tile
@@ -677,29 +454,33 @@ __global__ void __launch_bounds__(128, 3) k_mlp_tail_bwd2(TailJobs J) {
   }
 }
 
-// ---- the energy head of a training step as ONE kernel -------------------------------------------------------------
+// ---- the energy head as ONE kernel ----------------------------------------------------------------------------------
 // pretrain_heads.py:93-102 for G ~ 1e3 molecules is six latency-bound launches in a chain (two readout sums, first
 // layer, tail forward+backward, input gradient, readout backward) that the encoder backward has to wait for: 165 us in
 // the step (gpurun_out/r5k_device_profile.log) for 70 MFLOP.  Here a CTA takes 8 molecules through the whole chain in
 // shared memory: readout (written out for the weight-gradient GEMM of the first layer) -> h0 = W0 readout + b0 ->
 // tail forward, loss share, tail backward -> dh0 (written out, same GEMM) -> d_readout = dh0 W0 (atom half written out
 // for the caller's gather, fragment half scattered to the molecule's fragment rows here) and the per-CTA record of the
-// tail's parameter gradients in k_mlp_tail_bwd's layout.  Exact FP32, fixed summation order.
+// tail's parameter gradients (SumBuilder::add_tail's layout).  Exact FP32, fixed summation order.
+// The pointers that are set select the mode:
+//   target : fused loss (training step): g = 2 loss_coef (pred - target), the loss share goes into the record;
+//   gout   : the caller's gradient of the prediction, g = gout; the loss share is 0;
+//   neither: forward only: readout and pred; the tail's backward is skipped and no record is written.
 struct EnergyArgs {
   const int *atom_ptr, *frag_ptr;             // [G + 1] molecule boundaries
   const float *x_atoms, *x_frags;             // [Na,128], [Nf,128]
   const float *W0, *b0, *W1, *b1, *W2, *b2;   // fc head: [128,256] [128] [64,128] [64] [64] [1]
-  const float *target;                        // [G]
+  const float *target, *gout;                 // [G]
   float loss_coef;
   int G;
-  float *readout, *dh0, *d_readout, *g_frags, *rec;
+  float *readout, *pred, *dh0, *d_readout, *g_frags, *rec;
 };
 constexpr int EH_ROWS = 8, EH_THREADS = 256, EH_IN0 = 2 * kD, EH_H = kD, EH_MID = 64;
 constexpr size_t kEnergySmem =
     sizeof(float) * ((size_t)2 * EH_H * EH_MID + EH_ROWS * EH_IN0 + 2 * EH_ROWS * EH_H + 2 * EH_ROWS * EH_H +
                      3 * EH_ROWS * EH_MID + 2 * EH_MID + 4 * EH_ROWS);
 
-__global__ void __launch_bounds__(EH_THREADS) k_energy_head_fused(EnergyArgs a) {
+__global__ void __launch_bounds__(EH_THREADS) k_energy_head(EnergyArgs a) {
   constexpr int REC = rec_floats(EH_H, EH_MID);
   extern __shared__ __align__(16) float smem[];
   float *sW1 = smem;                          // [MID][H]   W1[i][k]
@@ -725,7 +506,8 @@ __global__ void __launch_bounds__(EH_THREADS) k_energy_head_fused(EnergyArgs a) 
   }
   const float b2 = __ldg(a.b2);
   pdl_wait();
-  const int oj = tid >> 2, ok0 = (tid & 3) * 4;   // dW1 ownership as in k_mlp_tail_bwd: row oj, columns ok0 + 16 q .. +3
+  const bool fwd_only = !a.target && !a.gout;
+  const int oj = tid >> 2, ok0 = (tid & 3) * 4;   // dW1 ownership: row oj, columns ok0 + 16 q .. +3
   float wacc[32];
 #pragma unroll
   for (int q = 0; q < 32; ++q) wacc[q] = 0.f;
@@ -815,10 +597,18 @@ __global__ void __launch_bounds__(EH_THREADS) k_energy_head_fused(EnergyArgs a) 
     if (tid < EH_ROWS) {
       float o = b2;
       for (int i = 0; i < EH_MID; ++i) o = fmaf(fmaxf(sH1[tid * EH_MID + i], 0.f), sb1[EH_MID + i], o);
-      const float diff = tid < rows ? o - __ldg(a.target + g0 + tid) : 0.f;
-      sG[tid] = 2.f * a.loss_coef * diff;
-      sG[EH_ROWS + tid] = a.loss_coef * diff * diff;
+      if (a.target) {
+        const float diff = tid < rows ? o - __ldg(a.target + g0 + tid) : 0.f;
+        sG[tid] = 2.f * a.loss_coef * diff;
+        sG[EH_ROWS + tid] = a.loss_coef * diff * diff;
+      } else if (fwd_only) {
+        if (tid < rows) a.pred[g0 + tid] = o;
+      } else {
+        sG[tid] = tid < rows ? __ldg(a.gout + g0 + tid) : 0.f;
+        sG[EH_ROWS + tid] = 0.f;
+      }
     }
+    if (fwd_only) continue;   // the same for every thread of the CTA: the next tile's barriers stay matched
     __syncthreads();
     {
       const int i = tid & 63, mp = tid >> 6;
@@ -902,8 +692,9 @@ __global__ void __launch_bounds__(EH_THREADS) k_energy_head_fused(EnergyArgs a) 
       }
     }
   }
-  // ---- CTA record: [dW1 MID*H][db1 MID][dW2 MID][db2 1][db0 H][loss]  (k_mlp_tail_bwd<128, 64>'s layout)
+  // ---- CTA record: [dW1 MID*H][db1 MID][dW2 MID][db2 1][db0 H][loss]
   pdl_launch_dependents();
+  if (fwd_only) return;
   float *rec = a.rec + (size_t)blockIdx.x * REC;
 #pragma unroll
   for (int q4 = 0; q4 < 8; ++q4)
@@ -915,11 +706,6 @@ __global__ void __launch_bounds__(EH_THREADS) k_energy_head_fused(EnergyArgs a) 
     rec[EH_MID * EH_H + 2 * EH_MID + 1 + EH_H] = lossacc;
   }
   if (tid < EH_H) rec[EH_MID * EH_H + 2 * EH_MID + 1 + tid] = b0acc;
-}
-
-template <int IN, int MID, int ROWS>
-constexpr size_t tail_bwd_smem() {
-  return sizeof(float) * ((size_t)IN * MID + 2 * (size_t)ROWS * (IN + 4) + 2 * (size_t)ROWS * (MID + 1) + ROWS);
 }
 
 // Fixed-order sum of per-CTA records (or a plain copy with n_blocks = 1) into the gradient tensors: one launch for all
@@ -990,11 +776,28 @@ int tail_grid(int64_t n, int rows) {
   return (int)t;
 }
 
-#define RC(expr)             \
-  do {                       \
-    const int rc__ = (expr); \
-    if (rc__) return rc__;   \
-  } while (0)
+// The kernels that use more than 48 KB of dynamic shared memory opt in once per device, before their first launch.
+int opt_in_smem() {
+  static bool done[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 64) return FNB_ERR_SIZE;
+  if (!done[dev]) {
+    RC((int)cudaFuncSetAttribute(k_mlp_tail_bwd2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTailBwd2Smem));
+    RC((int)cudaFuncSetAttribute(k_energy_head, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEnergySmem));
+    done[dev] = true;
+  }
+  return 0;
+}
+
+// The energy head's inputs, parameters and readout buffer; the caller sets the pointers of the mode (EnergyArgs).
+EnergyArgs energy_args(const fnb_pretrain_head_params *P, const fnb_pretrain_head_io *io, float *readout) {
+  EnergyArgs e{};
+  e.atom_ptr = io->mol_atom_ptr; e.frag_ptr = io->mol_frag_ptr; e.x_atoms = io->x_atoms; e.x_frags = io->x_frags;
+  e.W0 = P->fc.W0; e.b0 = P->fc.b0; e.W1 = P->fc.W1; e.b1 = P->fc.b1; e.W2 = P->fc.W2; e.b2 = P->fc.b2;
+  e.G = (int)io->n_graphs; e.readout = readout;
+  return e;
+}
 
 int check_io(const fnb_pretrain_head_params *P, const fnb_pretrain_head_io *io) {
   if (!P || !io) return FNB_ERR_NULL;
@@ -1029,26 +832,25 @@ extern "C" int fnb_pretrain_heads_forward(const fnb_pretrain_head_params *P, con
   return fnb_pretrain_heads_forward_impl(P, io, precision, workspace, workspace_bytes, scratch, stream_, 0);
 }
 
-// skip_tails != 0: only the first layers and the readout (what the backward needs); the training step forms the
-// predictions inside the backward tails (fused loss) and never materialises them.
+// skip_tails != 0: only the first layers of the per-atom / per-bond heads (what the backward needs); the training step
+// forms the predictions inside the backward tails and the energy kernel (fused loss) and never materialises them.
 int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb_pretrain_head_io *io, int precision,
                                     void *workspace, size_t workspace_bytes, void *scratch, void *stream_,
                                     int skip_tails) {
   RC(check_io(P, io));
   if (!workspace || !scratch) return FNB_ERR_NULL;
   if (!skip_tails && (!io->bond_angle || !io->dihedral || !io->energy)) return FNB_ERR_NULL;
-  const int64_t Na = io->n_atoms, Ea = io->n_edges, G = io->n_graphs, Nf = io->n_frags;
+  const int64_t Na = io->n_atoms, Ea = io->n_edges, G = io->n_graphs;
   FwdBufs B;
   if (fwd_layout(Na, Ea, G, (char *)workspace, &B) > workspace_bytes) return FNB_ERR_WORKSPACE;
   cudaStream_t stream = (cudaStream_t)stream_;
   const bool want_bl = io->bond_length != nullptr && Ea > 0 && !skip_tails;
 
-  // ---- energy head: ~1e3 rows, latency-bound kernels on an auxiliary stream underneath the per-atom / per-bond heads.
-  // Training step (skip_tails): the fused energy kernel is launched by the backward program.
+  // ---- energy head: ~1e3 rows, one latency-bound kernel on an auxiliary stream underneath the per-atom / per-bond
+  // heads.  Training step (skip_tails): the backward program runs it, forward included.
   FnbAux aux{};
   const bool two = fnb_aux_streams(&aux) == 0;
   cudaStream_t sB = two ? aux.hstream : stream;
-  void *sB_ = (void *)sB;
   {  // padded / split operands (one launch)
     PackJobs p{};
     p.W0[0] = P->ba.W0; p.b0[0] = P->ba.b0; p.Wpad[0] = B.W0pad_ba; p.WpadT[0] = B.W0padT_ba; p.bpad[0] = B.b0pad_ba;
@@ -1062,21 +864,17 @@ int fnb_pretrain_heads_forward_impl(const fnb_pretrain_head_params *P, const fnb
   }
   // ---- energy head (graph readout pretrain_heads.py:93-96, first layer, tail)
   if (G > 0 && !skip_tails) {
+    RC(opt_in_smem());
     if (two) {
       RC((int)cudaEventRecord(aux.fork, stream));
       RC((int)cudaStreamWaitEvent(sB, aux.fork, 0));
     }
-    RC(fnb_segment_sum(io->mol_atom_ptr, nullptr, G, io->x_atoms, B.readout, 2 * kD, nullptr, 0, 0, 0, nullptr, sB_));
-    RC(fnb_segment_sum(io->mol_frag_ptr, nullptr, G, io->x_frags, B.readout + kD, 2 * kD, nullptr, 0, 0, 0, nullptr, sB_));
-    RC(fnb_proj_fwd(B.readout, P->fc.W0, P->fc.b0, G, 2 * kD, nullptr, 0, 0, 0, B.h0_fc, nullptr, precision, sB_));
-    TailJobs F{};
-    F.n = 1;
-    TailJob &t = F.j[0];
-    t.h0 = B.h0_fc; t.n = G; t.W1 = P->fc.W1; t.b1 = P->fc.b1; t.W2 = P->fc.W2; t.b2 = P->fc.b2; t.out = io->energy;
-    if (cudaError_t le = fnb_launch(k_mlp_tail_fwd<128, 64>, dim3((unsigned)((G + 127) / 128), 1), dim3(128), 0, sB, F)) return (int)le;
+    EnergyArgs e = energy_args(P, io, B.readout);
+    e.pred = io->energy;
+    if (cudaError_t le = fnb_launch(k_energy_head, dim3(tail_grid(G, EH_ROWS)), dim3(EH_THREADS), kEnergySmem, sB, e))
+      return (int)le;
     FNB_CHECK_LAUNCH();
   }
-  (void)Nf;
   // ---- first layers on the projection kernels
   RC(fnb_proj_fwd(io->x_atoms, B.W0pad_ba, B.b0pad_ba, Na, kD, nullptr, 0, 0, 0, B.h0_ba, nullptr, precision, stream_));
   RC(fnb_proj_fwd(io->edge_feat, B.W0pad_da, B.b0pad_da, Ea, kD, nullptr, 0, 0, 0, B.h0_da, nullptr, precision, stream_));
@@ -1139,7 +937,7 @@ int fnb_pretrain_heads_backward_impl(const fnb_pretrain_head_params *P, const fn
   const fnb_mlp3_grads *gm[3] = {&D->ba, &D->da, &D->fc};
   for (int i = 0; i < 3; ++i)
     if (!gm[i]->W0 || !gm[i]->b0 || !gm[i]->W1 || !gm[i]->b1 || !gm[i]->W2 || !gm[i]->b2) return FNB_ERR_NULL;
-  const int64_t Na = io->n_atoms, Ea = io->n_edges, G = io->n_graphs, Nf = io->n_frags;
+  const int64_t Na = io->n_atoms, Ea = io->n_edges, G = io->n_graphs;
   FwdBufs B;
   BwdBufs W;
   if (fwd_layout(Na, Ea, G, (char *)workspace, &B) > workspace_bytes) return FNB_ERR_WORKSPACE;
@@ -1152,56 +950,27 @@ int fnb_pretrain_heads_backward_impl(const fnb_pretrain_head_params *P, const fn
   void *sB_ = (void *)sB;
   void *scratchB = two ? (void *)W.scratch2 : scratch;
   int ctas_ba = 0, ctas_da = 0, ctas_fc = 0;
-  {
-    static bool done[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) return FNB_ERR_SIZE;
-    if (!done[dev]) {
-      cudaError_t e = cudaFuncSetAttribute(k_mlp_tail_bwd2, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)kTailBwd2Smem);
-      if (e != cudaSuccess) return (int)e;
-      e = cudaFuncSetAttribute(k_mlp_tail_bwd<128, 64, 256, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)tail_bwd_smem<128, 64, 32>());
-      if (e != cudaSuccess) return (int)e;
-      e = cudaFuncSetAttribute(k_energy_head_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEnergySmem);
-      if (e != cudaSuccess) return (int)e;
-      done[dev] = true;
-    }
-  }
-  // ---- energy head on the auxiliary stream (its ~1e3-row kernels are latency-bound and hide under the other heads):
-  // tail, dX / dW of its first layer, readout backward of the fragments
+  RC(opt_in_smem());
+  // ---- energy head on the auxiliary stream (latency-bound ~1e3-row work that hides under the other heads): readout,
+  // first layer, tail forward and backward (with the loss in the training step), input gradient and the fragments'
+  // readout backward in one kernel, then the weight gradient of the first layer
   if (G > 0) {
     if (two) {
       RC((int)cudaEventRecord(aux.fork, stream));
       RC((int)cudaStreamWaitEvent(sB, aux.fork, 0));
       RC((int)cudaMemsetAsync(W.scratch2, 0, kScratchCounters * sizeof(float), sB));
     }
+    EnergyArgs e = energy_args(P, io, B.readout);
     if (fused) {
-      // training step: readout, first layer, tail forward + loss + backward, input gradient and the fragments' readout
-      // backward in one kernel (the forward program skipped the energy head)
-      EnergyArgs e{};
-      e.atom_ptr = io->mol_atom_ptr; e.frag_ptr = io->mol_frag_ptr; e.x_atoms = io->x_atoms; e.x_frags = io->x_frags;
-      e.W0 = P->fc.W0; e.b0 = P->fc.b0; e.W1 = P->fc.W1; e.b1 = P->fc.b1; e.W2 = P->fc.W2; e.b2 = P->fc.b2;
-      e.target = fused[2].target; e.loss_coef = fused[2].weight / (float)G; e.G = (int)G;
-      e.readout = B.readout; e.dh0 = W.dh0_fc; e.d_readout = W.d_readout; e.g_frags = io->g_frags; e.rec = W.rec_fc;
-      ctas_fc = tail_grid(G, EH_ROWS);
-      if (cudaError_t le = fnb_launch(k_energy_head_fused, dim3(ctas_fc), dim3(EH_THREADS), kEnergySmem, sB, e)) return (int)le;
-      FNB_CHECK_LAUNCH();
+      e.target = fused[2].target;
+      e.loss_coef = fused[2].weight / (float)G;
     } else {
-    TailJobs F{};
-    F.n = 1;
-    ctas_fc = tail_grid(G, 32);
-    TailJob &t = F.j[0];
-    t.h0 = B.h0_fc; t.n = G; t.W1 = P->fc.W1; t.b1 = P->fc.b1; t.W2 = P->fc.W2; t.b2 = P->fc.b2; t.gout = io->g_energy;
-    t.dh0 = W.dh0_fc; t.rec = W.rec_fc;
-    if (cudaError_t le = fnb_launch(k_mlp_tail_bwd<128, 64, 256, 32>, dim3(ctas_fc, 1), dim3(256), tail_bwd_smem<128, 64, 32>(), sB, F))
-      return (int)le;
-    FNB_CHECK_LAUNCH();
-    // input gradient first: the atoms' gradient on the caller's stream waits for d_readout, nothing waits for dW
-    RC(fnb_proj_bwd_dx(P->fc.W0, nullptr, W.dh0_fc, G, 2 * kD, W.d_readout, precision, scratchB, sB_));
-    RC(fnb_segment_gather(W.d_readout + kD, 2 * kD, io->frag_batch32, Nf, nullptr, io->g_frags, sB_));
+      e.gout = io->g_energy;
     }
+    e.dh0 = W.dh0_fc; e.d_readout = W.d_readout; e.g_frags = io->g_frags; e.rec = W.rec_fc;
+    ctas_fc = tail_grid(G, EH_ROWS);
+    if (cudaError_t le = fnb_launch(k_energy_head, dim3(ctas_fc), dim3(EH_THREADS), kEnergySmem, sB, e)) return (int)le;
+    FNB_CHECK_LAUNCH();
     if (two) RC((int)cudaEventRecord(aux.join, sB));
     RC(fnb_proj_bwd_dw(B.readout, W.dh0_fc, G, 2 * kD, D->fc.W0, nullptr, precision, scratchB, sB_));
     if (two) RC((int)cudaEventRecord(defer_join ? aux.h_done : aux.wjoin, sB));

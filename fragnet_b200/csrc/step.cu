@@ -11,19 +11,6 @@
 
 namespace {
 
-struct Arena {
-  char *base;
-  size_t off;
-  template <class T>
-  T *take(size_t n) {
-    off = (off + 255) & ~(size_t)255;
-    T *p = base ? reinterpret_cast<T *>(base + off) : nullptr;
-    off += n * sizeof(T);
-    return p;
-  }
-  char *bytes(size_t n) { return take<char>(n); }
-};
-
 // Sizes-only view of the plan a batch will get (what the workspace-size functions of the sub-programs read).
 fnb_batch_plan sizes_plan(const fnb_batch_inputs *in) {
   fnb_batch_plan p{};
@@ -86,14 +73,8 @@ size_t step_layout(const fnb_pretrain_step_args *a, char *base, StepBufs *out) {
     b.enc_bws = ar.bytes(b.enc_bws_bytes);
   }
   if (out) *out = b;
-  return (ar.off + 255) & ~(size_t)255;
+  return ar.total();
 }
-
-#define RC(expr)             \
-  do {                       \
-    const int rc__ = (expr); \
-    if (rc__) return rc__;   \
-  } while (0)
 
 // The first half of both step programs: the on-device collate of the batch (north-star kernel a) and the encoder
 // forward (FragNet.forward, gat2.py:381-442).  The collate runs on an auxiliary stream, underneath the plan-independent
@@ -286,7 +267,7 @@ size_t ft_layout(const fnb_finetune_step_args *a, char *base, FtBufs *out) {
     b.enc_bws = ar.bytes(b.enc_bws_bytes);
   }
   if (out) *out = b;
-  return (ar.off + 255) & ~(size_t)255;
+  return ar.total();
 }
 
 }  // namespace
