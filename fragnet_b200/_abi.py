@@ -179,7 +179,8 @@ class CBatchInputs(C.Structure):
 class CEncoderOpts(C.Structure):
     _fields_ = [("n_layers", _i32), ("post_act", _i32), ("drop_p", _f32), ("training", _i32), ("seed", _u64),
                 ("offset", _u64), ("precision", _i32), ("save_for_backward", _i32), ("need_dx_atoms", _i32),
-                ("need_dx_bond", _i32), ("need_dx_fbond", _i32), ("first_trained_layer", _i32)]
+                ("need_dx_bond", _i32), ("need_dx_fbond", _i32), ("first_trained_layer", _i32), ("pool_frags", _i32),
+                ("skip_fbond", _i32)]
 
 
 class CEncoderIO(C.Structure):
@@ -224,6 +225,7 @@ class CPretrainStepArgs(C.Structure):
 ACT_NONE, ACT_RELU, ACT_CELU, ACT_SILU, ACT_GELU, ACT_SELU, ACT_RELU6, ACT_LEAKYRELU = range(8)
 MLP_MAX_LAYERS = 8
 LOSS_MSE, LOSS_BCE_MASKED = 0, 1
+VARIANT_GAT2, VARIANT_LITE, VARIANT_EDGE = 0, 1, 2
 
 
 class CMlpLayer(C.Structure):
@@ -237,4 +239,5 @@ class CFinetuneStepArgs(C.Structure):
                [("n_layers", _i32), ("layers", _vp), ("layer_grads", _vp), ("n_head_layers", _i32), ("head", _vp),
                 ("loss_kind", _i32), ("drop_p", _f32), ("training", _i32), ("seed", _u64), ("offset", _u64),
                 ("precision", _i32), ("backward", _i32)] + \
-               [(n, _vp) for n in ("loss", "predictions", "plan_arena")] + [("first_trained_layer", _i32)]
+               [(n, _vp) for n in ("loss", "predictions", "plan_arena")] + [("first_trained_layer", _i32)] + \
+               [("variant", _i32)] + [(n, _vp) for n in ("cnx_attr", "W_cnx", "b_cnx", "dW_cnx", "db_cnx")]

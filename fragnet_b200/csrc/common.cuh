@@ -348,6 +348,15 @@ int fnb_mlp_backward(const FnbMlpRun *r, cudaStream_t stream);
 // loss[0] = mean of BCE-with-logits over the labels > -0.5 (NaN if none); grad (may be NULL) = its logit gradient.
 int fnb_bce_masked_loss(const float *logits, const float *labels, int64_t n, float *loss, float *grad,
                         cudaStream_t stream);
+// gat2_edge's fragment edge table (gat2_edge.py:152-158) and its gradient, exact FP32 (finetune.cu).  cnx: [n,8]
+// connection attributes, W8 / b8: cnx_attr_transform [128,8] / [128], f: the last layer's head vectors [4,192].
+//   table[e,h] = sum_k cnx[e,k] coef[k,h] + bias[h],  coef = W8^T f_e^T [8,4],  bias = b8 f_e^T [4],  f_e = f[:, 32:160]
+// The backward writes dW8, db8 and the edge slice df[:, 32:160] (the rest of df is left alone); scratch: a step
+// scratch whose arrival counters are zero (cta_finish).
+int fnb_cnx_table_fwd(const float *cnx, int64_t n, const float *W8, const float *b8, const float *f, float *table,
+                      cudaStream_t stream);
+int fnb_cnx_table_bwd(const float *cnx, const float *d_table, int64_t n, const float *W8, const float *b8,
+                      const float *f, float *dW8, float *db8, float *df, void *scratch, cudaStream_t stream);
 
 // Tensor-core (tcgen05, TF32) projection path, tc_gemm.cu.  Returns FNB_ERR_MODE when the shape cannot use TMA.
 // x3 != 0: 3xTF32 (error-compensated, FP32-grade) instead of one TF32 product.

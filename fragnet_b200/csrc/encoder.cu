@@ -62,12 +62,13 @@ size_t layout(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fnb_l
     const bool keep = o->save_for_backward != 0 && l >= o->first_trained_layer;   // frozen layers: nothing to save
     const bool want_p = keep || L[l].want_attention;
     const bool frag = L[l].run_frag_block != 0;
+    const bool pool_out = last && o->pool_frags;   // gat2_lite: the pooled pre-activation atoms are the fragment output
     if (l == 0 && input_dropout(o)) b.xa0 = a.take<float>(z.Na * L[0].K_atom);
     if (l == 0) {
       const int ks[3] = {L[0].K_bond, L[0].K_atom, L[0].K_fbond};
       const int64_t ns[3] = {z.Nb, z.Na, z.Nfb};
       for (int j = 0; j < 3; ++j) {
-        b.k_pad[j] = pad_width(o, ks[j]);
+        b.k_pad[j] = j == 2 && o->skip_fbond ? 0 : pad_width(o, ks[j]);
         if (b.k_pad[j]) {
           b.x_pad[j] = a.take<float>(ns[j] * b.k_pad[j]);
           b.W_pad[j] = a.take<float>((size_t)kD * b.k_pad[j]);
@@ -91,7 +92,7 @@ size_t layout(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fnb_l
       // block's backward; the atom features feed the pooling; the fragment-connection features feed d alpha_e of
       // the fragment block.  Post-activations of the last layer go straight to the caller's outputs.
       if (keep) b.pre_bond = a.take<float>(z.Nb * kD);
-      if (frag) b.pre_atom = a.take<float>(z.Na * kD);
+      if (frag || pool_out) b.pre_atom = a.take<float>(z.Na * kD);
       if (frag && keep) b.pre_fbond = a.take<float>(z.Nfb * kD);
       if (!last) {
         b.y_bond = a.take<float>(z.Nb * kD);
@@ -256,14 +257,17 @@ int check_common(const fnb_batch_plan *plan, const fnb_encoder_opts *o, const fn
   const Sizes z = sizes_of(plan);
   // a graph without nodes (gat2_lite runs with empty fragment-side graphs) has no feature rows to point at
   if ((z.Na > 0 && (!io->x_atoms || !io->out_atoms)) || (z.Nb > 0 && (!io->x_bond || !io->out_bond)) ||
-      (z.Nfb > 0 && (!io->x_fbond || !io->out_fbond)))
+      (z.Nfb > 0 && !o->skip_fbond && (!io->x_fbond || !io->out_fbond)))
     return FNB_ERR_NULL;
+  if (o->pool_frags && (!o->post_act || (z.Nf > 0 && !io->out_frags))) return FNB_ERR_MODE;
   if (z.Na != plan->n_atoms || z.Nf != plan->n_frags) return FNB_ERR_SIZE;
   // the atom graph's edges are the bond graph's nodes, the fragment graph's edges the fragment-connection nodes
   if (plan->atom.n_real_edges != z.Nb || plan->frag.n_real_edges != z.Nfb) return FNB_ERR_SIZE;
   for (int l = 0; l < o->n_layers; ++l) {
     if (l > 0 && (L[l].K_atom != kD || L[l].K_bond != kD || L[l].K_fbond != kD)) return FNB_ERR_SIZE;
     if (L[l].run_frag_block && !io->out_frags && l == o->n_layers - 1) return FNB_ERR_NULL;
+    // the pooled output replaces the fragment block; a skipped fragment-connection chain emits no fragment edge term
+    if (L[l].run_frag_block && (o->pool_frags || (o->skip_fbond && !io->frag_table))) return FNB_ERR_MODE;
   }
   return 0;
 }
@@ -448,10 +452,10 @@ int fnb_encoder_forward_impl(const fnb_batch_plan *plan, const fnb_encoder_opts 
       a_pending = true;
     }
     // ---- fragment-connection graph (gat2.py:239-278); epilogue emits the fragment graph's edge term
-    RC(fnb_proj_fwd(xfb_in, Wfb_in, P.bfb, z.Nfb, Kfb_in, P.f_a_b, AB_STRIDE, AB_T, AB_S, b.hfb, b.Sfb, o->precision,
-                    sB_));
-    pending = true;
-    {
+    if (!o->skip_fbond) {
+      RC(fnb_proj_fwd(xfb_in, Wfb_in, P.bfb, z.Nfb, Kfb_in, P.f_a_b, AB_STRIDE, AB_T, AB_S, b.hfb, b.Sfb, o->precision,
+                      sB_));
+      pending = true;
       fnb_gat_fwd_args f{};
       f.h = b.hfb; f.S = b.Sfb; f.edge_mode = FNB_EDGE_AFFINE6; f.We = P.We_fb; f.be = P.be_fb;
       f.alpha_e = P.f_a_b + AB_E; f.alpha_stride = AB_STRIDE; f.out = pre_fbond; f.y = y_fbond;
@@ -468,7 +472,16 @@ int fnb_encoder_forward_impl(const fnb_batch_plan *plan, const fnb_encoder_opts 
         FNB_CHECK_LAUNCH();
       }
     }
-    if (frag || P.want_attention) RC(join());
+    const bool pool_out = last && o->pool_frags;
+    if (frag || pool_out || P.want_attention) RC(join());
+    // ---- gat2_lite's fragment output (gat2_lite.py:140, 205-212): ReLU(Dropout(pooled pre-activation atoms)) at the
+    // last layer's fragment site, pooled into out_frags and activated in place
+    if (pool_out) {
+      RC(fnb_segment_sum(plan->pool_rowptr, plan->pool_col, z.Nf, pre_atom, io->out_frags, kD, nullptr, 0, 0, 0, nullptr,
+                         stream_));
+      RC(fnb_dropout_relu_fwd(io->out_frags, io->out_frags, z.Nf * kD, o->drop_p, o->training, 1, o->seed, ph.frag[l],
+                              stream_));
+    }
     // ---- atom -> fragment pooling (gat2.py:234) and the fragment graph (gat2.py:283-316): only where its output lives
     if (frag) {
       RC(fnb_segment_sum(plan->pool_rowptr, plan->pool_col, z.Nf, pre_atom, b.hf, kD, P.f, A_STRIDE, A_T, A_S, b.Sf,
@@ -523,7 +536,7 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
       const int ks[3] = {L[l].K_bond, L[l].K_atom, L[l].K_fbond};
       for (int j = 0; j < 3; ++j) {
         wt_slot[l][j] = -1;
-        if (tf32 && ks[j] == kD &&
+        if (tf32 && ks[j] == kD && !(j == 2 && o->skip_fbond) &&
             (l > first || (l == 0 && (j == 0 ? o->need_dx_bond : (j == 1 ? o->need_dx_atoms : o->need_dx_fbond))))) {
           wt_slot[l][j] = nm;
           mats[nm++] = ws[j];
@@ -655,9 +668,13 @@ extern "C" int fnb_encoder_backward(const fnb_batch_plan *plan, const fnb_encode
       }
       d_hf = W.d_hf;
     }
+    if (last && o->pool_frags && dy_frag) {   // gat2_lite: the gradient of the pooled rows, dy (y > 0) / (1 - p)
+      RC(fnb_dropout_relu_bwd(dy_frag, y_frag, W.d_hf, z.Nf * kD, o->drop_p, o->training, stream_));
+      d_hf = W.d_hf;     // the atom graph's destination pass hands it to the member atoms
+    }
     const bool frag_feeds_fbond = frag_bwd && !io->frag_table;   // gat2: the fragment graph's edges ARE the fbond rows
     // ---- fragment-connection graph block
-    {
+    if (!o->skip_fbond) {
       RC(fork());
       // incoming gradient = ReLU(Dropout) backward of dy_fbond + (last layer) the fragment graph's edge term
       // sum_h dz_f alpha_e, assembled inside the destination pass; d f[:, edge slice] by the edge-table kernel

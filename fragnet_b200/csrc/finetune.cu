@@ -66,7 +66,153 @@ __global__ void __launch_bounds__(kBceThreads) k_bce_masked(const float *__restr
   }
 }
 
+// ---- gat2_edge's fragment edge table --------------------------------------------------------------------------------
+// <cnx_attr_transform(cnx[e]), f_e[h]> = cnx[e] . (W8^T f_e[h]) + <b8, f_e[h]>: the 36 folded constants (coef[k,h] at
+// k * 4 + h, bias[h] at 32 + h) are formed per CTA in a fixed order, one warp per constant.
+constexpr int kCnxIn = 8, kCnxThreads = 256, kCnxConst = kCnxIn * kH + kH;
+constexpr int kFStride = 192, kFEdge = 32;      // f = [target 32 | edge 128 | source 32] per head
+
+__device__ __forceinline__ void cnx_fold(const float *__restrict__ W8, const float *__restrict__ b8,
+                                         const float *__restrict__ f, float *s_c) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int o = warp; o < kCnxConst; o += kCnxThreads / 32) {
+    const int k = o >> 2, h = o & 3;              // k == kCnxIn: the bias term
+    float s = 0.f;
+    for (int j = lane; j < kD; j += 32)
+      s += (k < kCnxIn ? __ldg(W8 + j * kCnxIn + k) : __ldg(b8 + j)) * __ldg(f + h * kFStride + kFEdge + j);
+    s = warp_sum(s);
+    if (lane == 0) s_c[o] = s;
+  }
+  __syncthreads();
+}
+
+__device__ __forceinline__ void cnx_row(const float *__restrict__ cnx, int64_t e, float x[kCnxIn]) {
+  const float4 lo = ldg4(cnx + e * kCnxIn), hi = ldg4(cnx + e * kCnxIn + 4);
+  x[0] = lo.x; x[1] = lo.y; x[2] = lo.z; x[3] = lo.w; x[4] = hi.x; x[5] = hi.y; x[6] = hi.z; x[7] = hi.w;
+}
+
+__global__ void __launch_bounds__(kCnxThreads) k_cnx_table(const float *__restrict__ cnx, int64_t n,
+                                                           const float *__restrict__ W8, const float *__restrict__ b8,
+                                                           const float *__restrict__ f, float *__restrict__ table) {
+  __shared__ float s_c[kCnxConst];
+  pdl_wait();
+  cnx_fold(W8, b8, f, s_c);
+  for (int64_t e = blockIdx.x * (int64_t)kCnxThreads + threadIdx.x; e < n; e += (int64_t)gridDim.x * kCnxThreads) {
+    float x[kCnxIn];
+    cnx_row(cnx, e, x);
+    float t[kH];
+#pragma unroll
+    for (int h = 0; h < kH; ++h) {
+      float s = s_c[kCnxIn * kH + h];
+#pragma unroll
+      for (int k = 0; k < kCnxIn; ++k) s += x[k] * s_c[k * kH + h];
+      t[h] = s;
+    }
+    st4(table + e * 4, make_float4(t[0], t[1], t[2], t[3]));
+  }
+}
+
+// Backward: per-CTA records of dcoef = cnx^T d_table and dbias = column sums of d_table, summed in a fixed order by
+// the last CTA (cta_finish), which then folds them through f_e and W8 / b8.
+__global__ void __launch_bounds__(kCnxThreads) k_cnx_table_bwd(const float *__restrict__ cnx,
+                                                               const float *__restrict__ d_table, int64_t n,
+                                                               const float *__restrict__ W8, const float *__restrict__ b8,
+                                                               const float *__restrict__ f, float *__restrict__ dW8,
+                                                               float *__restrict__ db8, float *__restrict__ df,
+                                                               float *scratch) {
+  __shared__ float s_part[kCnxThreads / 32][kCnxConst];
+  __shared__ float s_rec[kCnxConst], s_fin[kCnxConst];
+  pdl_wait();
+  float acc[kCnxConst];
+#pragma unroll
+  for (int o = 0; o < kCnxConst; ++o) acc[o] = 0.f;
+  for (int64_t e = blockIdx.x * (int64_t)kCnxThreads + threadIdx.x; e < n; e += (int64_t)gridDim.x * kCnxThreads) {
+    float x[kCnxIn];
+    cnx_row(cnx, e, x);
+    const float4 d = ldg4(d_table + e * 4);
+    const float dv[kH] = {d.x, d.y, d.z, d.w};
+#pragma unroll
+    for (int h = 0; h < kH; ++h) {
+#pragma unroll
+      for (int k = 0; k < kCnxIn; ++k) acc[k * kH + h] += x[k] * dv[h];
+      acc[kCnxIn * kH + h] += dv[h];
+    }
+  }
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int o = 0; o < kCnxConst; ++o) {
+    const float v = warp_sum(acc[o]);
+    if (lane == 0) s_part[warp][o] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < kCnxConst) {
+    float s = 0.f;
+    for (int w = 0; w < kCnxThreads / 32; ++w) s += s_part[w][threadIdx.x];
+    s_rec[threadIdx.x] = s;
+  }
+  __syncthreads();
+  if (!cta_finish<kCnxConst>(s_rec, s_fin, scratch)) return;
+  // dW8[j,k] = sum_h dcoef[k,h] f_e[h,j];  db8[j] = sum_h dbias[h] f_e[h,j];
+  // df[h, 32 + j] = sum_k W8[j,k] dcoef[k,h] + b8[j] dbias[h]
+  for (int j = threadIdx.x; j < kD; j += kCnxThreads) {
+    float fe[kH];
+#pragma unroll
+    for (int h = 0; h < kH; ++h) fe[h] = __ldg(f + h * kFStride + kFEdge + j);
+    float w[kCnxIn];
+#pragma unroll
+    for (int k = 0; k < kCnxIn; ++k) {
+      w[k] = __ldg(W8 + j * kCnxIn + k);
+      float s = 0.f;
+#pragma unroll
+      for (int h = 0; h < kH; ++h) s += s_fin[k * kH + h] * fe[h];
+      dW8[j * kCnxIn + k] = s;
+    }
+    float sb = 0.f;
+#pragma unroll
+    for (int h = 0; h < kH; ++h) sb += s_fin[kCnxIn * kH + h] * fe[h];
+    db8[j] = sb;
+    const float bj = __ldg(b8 + j);
+#pragma unroll
+    for (int h = 0; h < kH; ++h) {
+      float s = bj * s_fin[kCnxIn * kH + h];
+#pragma unroll
+      for (int k = 0; k < kCnxIn; ++k) s += w[k] * s_fin[k * kH + h];
+      df[h * kFStride + kFEdge + j] = s;
+    }
+  }
+}
+
+int cnx_grid(int64_t n) {
+  const int64_t blocks = (n + kCnxThreads - 1) / kCnxThreads;
+  return (int)(blocks < 1 ? 1 : (blocks > kNumSMs ? kNumSMs : blocks));
+}
+
 }  // namespace
+
+int fnb_cnx_table_fwd(const float *cnx, int64_t n, const float *W8, const float *b8, const float *f, float *table,
+                      cudaStream_t stream) {
+  if (n < 0) return FNB_ERR_SIZE;
+  if (n == 0) return 0;
+  if (!cnx || !W8 || !b8 || !f || !table) return FNB_ERR_NULL;
+  if (!fnb_aligned16(cnx) || !fnb_aligned16(table)) return FNB_ERR_ALIGN;
+  if (cudaError_t le = fnb_launch(k_cnx_table, dim3(cnx_grid(n)), dim3(kCnxThreads), 0, stream, cnx, n, W8, b8, f, table))
+    return (int)le;
+  FNB_CHECK_LAUNCH();
+  return 0;
+}
+
+int fnb_cnx_table_bwd(const float *cnx, const float *d_table, int64_t n, const float *W8, const float *b8,
+                      const float *f, float *dW8, float *db8, float *df, void *scratch, cudaStream_t stream) {
+  if (n < 0) return FNB_ERR_SIZE;
+  if (!W8 || !b8 || !f || !dW8 || !db8 || !df || !scratch || (n > 0 && (!cnx || !d_table))) return FNB_ERR_NULL;
+  if (!fnb_aligned16(cnx) || !fnb_aligned16(d_table)) return FNB_ERR_ALIGN;
+  // (n == 0: one CTA writes zero gradients)
+  if (cudaError_t le = fnb_launch(k_cnx_table_bwd, dim3(cnx_grid(n)), dim3(kCnxThreads), 0, stream, cnx, d_table, n, W8,
+                                  b8, f, dW8, db8, df, reinterpret_cast<float *>(scratch)))
+    return (int)le;
+  FNB_CHECK_LAUNCH();
+  return 0;
+}
 
 int fnb_mlp_check(const fnb_mlp_layer *L, int n, int64_t G, int in0, int backward) {
   if (!L) return FNB_ERR_NULL;

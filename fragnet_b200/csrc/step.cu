@@ -205,7 +205,7 @@ extern "C" int fnb_pretrain_plan_prefetch(const fnb_batch_inputs *next, void *ar
 namespace {
 
 bool ft_args_ok(const fnb_finetune_step_args *a) {
-  return a && a->n_layers >= 1 && a->n_layers <= 16 && a->layers && a->batch.n_atoms >= 0 && a->batch.n_frags >= 0 &&
+  return a && a->variant >= FNB_VARIANT_GAT2 && a->variant <= FNB_VARIANT_EDGE && a->n_layers >= 1 && a->n_layers <= 16 && a->layers && a->batch.n_atoms >= 0 && a->batch.n_frags >= 0 &&
          a->batch.n_bonds >= 0 && a->batch.n_graphs >= 1 && a->first_trained_layer >= 0 &&
          a->first_trained_layer <= a->n_layers && fnb_mlp_check(a->head, a->n_head_layers, a->batch.n_graphs, 2 * kD, 0) == 0;
 }
@@ -218,7 +218,17 @@ fnb_encoder_opts ft_opts_of(const fnb_finetune_step_args *a) {
   fnb_encoder_opts o = opts_of(a);
   o.first_trained_layer = a->first_trained_layer;
   o.save_for_backward = a->backward && encoder_trained(a);
+  o.pool_frags = a->variant == FNB_VARIANT_LITE;
+  o.skip_fbond = a->variant != FNB_VARIANT_GAT2;
   return o;
+}
+
+// The batch as the variant sees it (fnb_finetune_step_args.variant): the graphs it lacks are emptied.
+fnb_batch_inputs ft_inputs(const fnb_finetune_step_args *a) {
+  fnb_batch_inputs in = a->batch;
+  if (a->variant != FNB_VARIANT_GAT2) in.n_fbond_edges = 0;
+  if (a->variant == FNB_VARIANT_LITE) in.n_fbond_nodes = 0;
+  return in;
 }
 
 struct FtBufs {
@@ -229,10 +239,11 @@ struct FtBufs {
   float *readout, *xd0, *pred;
   float *xd[FNB_MLP_MAX_LAYERS], *u[FNB_MLP_MAX_LAYERS], *dz[FNB_MLP_MAX_LAYERS];
   float *d_readout, *g_atoms, *g_frags, *rec;
+  float *cnx_table, *d_cnx_table;   // EDGE: the fragment graph's edge term [Ef,4] and its gradient
 };
 
 size_t ft_layout(const fnb_finetune_step_args *a, char *base, FtBufs *out) {
-  const fnb_batch_inputs *in = &a->batch;
+  const fnb_batch_inputs in_v = ft_inputs(a), *in = &in_v;
   const fnb_batch_plan sp = sizes_plan(in);
   const fnb_encoder_opts o = ft_opts_of(a);
   const bool enc = a->backward && encoder_trained(a);
@@ -266,6 +277,10 @@ size_t ft_layout(const fnb_finetune_step_args *a, char *base, FtBufs *out) {
     b.enc_bws_bytes = fnb_encoder_bwd_workspace_bytes(&sp, &o, a->layers);
     b.enc_bws = ar.bytes(b.enc_bws_bytes);
   }
+  if (a->variant == FNB_VARIANT_EDGE) {
+    b.cnx_table = ar.take<float>(Nfb * 4);
+    if (enc) b.d_cnx_table = ar.take<float>(Nfb * 4);
+  }
   if (out) *out = b;
   return ar.total();
 }
@@ -279,7 +294,8 @@ extern "C" size_t fnb_finetune_step_workspace_bytes(const fnb_finetune_step_args
 
 extern "C" uint64_t fnb_finetune_step_rng_span(const fnb_finetune_step_args *a) {
   if (!ft_args_ok(a)) return 0;
-  const fnb_batch_plan sp = sizes_plan(&a->batch);
+  const fnb_batch_inputs in = ft_inputs(a);
+  const fnb_batch_plan sp = sizes_plan(&in);
   const fnb_encoder_opts o = ft_opts_of(a);
   return fnb_encoder_rng_span(&sp, &o, a->layers) +
          fnb_mlp_rng(a->head, a->n_head_layers, a->batch.n_graphs, 0, nullptr, nullptr);
@@ -291,12 +307,16 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
   if (!a->head || !a->layers) return FNB_ERR_NULL;
   if (a->n_layers < 1 || a->n_layers > 16) return FNB_ERR_SIZE;
   if (a->first_trained_layer < 0 || a->first_trained_layer > a->n_layers) return FNB_ERR_SIZE;
-  const fnb_batch_inputs *in = &a->batch;
+  if (a->variant < FNB_VARIANT_GAT2 || a->variant > FNB_VARIANT_EDGE) return FNB_ERR_MODE;
+  const bool edge = a->variant == FNB_VARIANT_EDGE;
+  if (edge && (!a->cnx_attr || !a->W_cnx || !a->b_cnx)) return FNB_ERR_NULL;
+  const fnb_batch_inputs in_v = ft_inputs(a), *in = &in_v;
   if (in->n_atoms < 1 || in->n_bonds < 0 || in->n_frags < 0 || in->n_graphs < 1 || !in->batch || !in->frag_batch)
     return FNB_ERR_SIZE;
   RC(fnb_mlp_check(a->head, a->n_head_layers, in->n_graphs, 2 * kD, a->backward));
   if (a->loss_kind != FNB_LOSS_MSE && a->loss_kind != FNB_LOSS_BCE_MASKED) return FNB_ERR_MODE;
-  if (!a->loss || !a->target || !a->x_atoms || !a->x_bond || !a->x_fbond) return FNB_ERR_NULL;
+  if (!a->loss || !a->target || !a->x_atoms || !a->x_bond) return FNB_ERR_NULL;
+  if (!a->x_fbond && a->variant == FNB_VARIANT_GAT2) return FNB_ERR_NULL;
   const bool enc_bwd = a->backward && encoder_trained(a);
   if (a->backward && !enc_bwd) {   // a backward that trains nothing is a caller's mistake
     bool head_trained = false;
@@ -304,6 +324,7 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
     if (!head_trained) return FNB_ERR_MODE;
   }
   if (enc_bwd && !a->layer_grads) return FNB_ERR_NULL;
+  if (enc_bwd && edge && (!a->dW_cnx || !a->db_cnx || !a->layer_grads[a->n_layers - 1].f)) return FNB_ERR_NULL;
   if (reinterpret_cast<uintptr_t>(workspace) & 255u) return FNB_ERR_ALIGN;
   FtBufs B;
   if (ft_layout(a, (char *)workspace, &B) > workspace_bytes) return FNB_ERR_WORKSPACE;
@@ -320,6 +341,11 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
   fnb_encoder_io eio{};
   eio.x_atoms = a->x_atoms; eio.x_bond = a->x_bond; eio.x_fbond = a->x_fbond;
   eio.out_atoms = B.out_atoms; eio.out_frags = B.out_frags; eio.out_bond = B.out_bond; eio.out_fbond = B.out_fbond;
+  const fnb_layer_params &top = a->layers[a->n_layers - 1];
+  if (edge) {   // gat2_edge: the fragment graph's edge term from the connection attributes (gat2_edge.py:152-158)
+    RC(fnb_cnx_table_fwd(a->cnx_attr, in->n_fbond_nodes, a->W_cnx, a->b_cnx, top.f, B.cnx_table, s));
+    eio.frag_table = B.cnx_table;
+  }
   RC(collate_and_encode(in, a->plan_arena, B.plan_arena, B.plan_bytes, &o, a->layers, &eio, B.enc_ws, B.enc_bytes,
                         scratch, stream, aux, two, &plan));
   // ---- readout: [G,256] = cat(sum over each molecule's atoms, sum over its fragments)
@@ -353,7 +379,13 @@ extern "C" int fnb_finetune_step(const fnb_finetune_step_args *a, void *workspac
   RC(fnb_segment_gather(B.d_readout, 2 * kD, plan.batch32, in->n_atoms, nullptr, B.g_atoms, stream));
   RC(fnb_segment_gather(B.d_readout + kD, 2 * kD, plan.frag_batch32, in->n_frags, nullptr, B.g_frags, stream));
   eio.g_atoms = B.g_atoms; eio.g_frags = B.g_frags; eio.g_bond = nullptr; eio.g_fbond = nullptr;
+  eio.d_frag_table = B.d_cnx_table;
   RC(fnb_encoder_backward(&plan, &o, a->layers, a->layer_grads, &eio, B.enc_ws, B.enc_bytes, B.enc_bws, B.enc_bws_bytes,
                           scratch, stream));
+  // gat2_edge: the edge term's gradient to cnx_attr_transform and to the edge slice of f, which the encoder left zero;
+  // behind the encoder backward on this stream (it ends by joining its side streams)
+  if (edge)
+    RC(fnb_cnx_table_bwd(a->cnx_attr, B.d_cnx_table, in->n_fbond_nodes, a->W_cnx, a->b_cnx, top.f, a->dW_cnx, a->db_cnx,
+                         a->layer_grads[a->n_layers - 1].f, scratch, s));
   return 0;
 }

@@ -121,13 +121,16 @@ class DevicePrefetcher:
     batches have been requested.  Host tensors that are not pinned are pinned first (``DataLoader(pin_memory=True)``
     does that in the loader's workers)."""
 
-    def __init__(self, batches: Iterable[Dict[str, torch.Tensor]], device, depth: int = 2, hot_path_only: bool = False):
+    def __init__(self, batches: Iterable[Dict[str, torch.Tensor]], device, depth: int = 2, hot_path_only: bool = False,
+                 keep: Iterable[str] = ()):
         """``hot_path_only=True`` moves only what the GAT2 path reads: ``edge_attr`` and ``cnx_attr`` are dropped
         (``FragNet.forward`` never reads them: gat2.py:381-442 takes ``node_features_bonds`` / ``edge_attr_fbonds``),
         and ``x_frags`` -- whose VALUES are overwritten unread by the atom->fragment pooling (gat2.py:234), only its
-        row count matters -- arrives as a ``meta`` tensor of the same shape.  ~20 % fewer PCIe bytes per batch."""
+        row count matters -- arrives as a ``meta`` tensor of the same shape.  ~20 % fewer PCIe bytes per batch.
+        ``keep``: entries of those two that are moved all the same (``cnx_attr`` for gat2_edge, gat2_edge.py:167)."""
         self.batches, self.device, self.depth = batches, torch.device(device), max(1, int(depth))
         self.hot_path_only = bool(hot_path_only)
+        self._unread = tuple(k for k in _UNREAD if k not in set(keep))
         if self.device.type != "cuda":
             raise ValueError("DevicePrefetcher stages batches onto a CUDA device")
         # copy stream and staging slots are recycled across prefetchers of a device (a training loop makes one per
@@ -164,7 +167,7 @@ class DevicePrefetcher:
             return host, getattr(host, "ready_event", None), None, None
         shape_only = None
         if self.hot_path_only:
-            kept = {k: v for k, v in host.items() if k not in _UNREAD}
+            kept = {k: v for k, v in host.items() if k not in self._unread}
             if getattr(host, "blob", None) is not None:      # a PackedBatch stays one (its buffer holds the hot path only)
                 kept = type(host)(kept)
                 kept.blob, kept.layout = host.blob, host.layout

@@ -39,18 +39,21 @@ def _on(batch, k, dev, dtype):
     return t
 
 
-def _encoder_structs(layer_params, grad_of):
-    """``fnb_layer_params`` / ``fnb_layer_grads`` arrays of an encoder's layers (fragment block in the last one only)."""
+def _encoder_structs(layer_params, grad_of, frag_block=True):
+    """``fnb_layer_params`` / ``fnb_layer_grads`` arrays of an encoder's layers (fragment block in the last one only,
+    or with ``frag_block=False`` in none).  A ``None`` tensor is one the program does not read (a fragment-connection
+    tensor of gat2_lite / gat2_edge)."""
     n_layers = len(layer_params)
     layers, grads = (_abi.CLayerParams * n_layers)(), (_abi.CLayerGrads * n_layers)()
     for li, ps in enumerate(layer_params):
         L, G = layers[li], grads[li]
         for name, p in zip(_abi.PARAM_FIELDS, ps):
-            setattr(L, name, p.data_ptr())
-            g = grad_of.get(id(p))
+            setattr(L, name, None if p is None else p.data_ptr())
+            g = None if p is None else grad_of.get(id(p))
             setattr(G, name, None if g is None else g.data_ptr())
-        L.K_bond, L.K_fbond, L.K_atom = ps[0].shape[1], ps[2].shape[1], ps[8].shape[1]
-        L.run_frag_block, L.want_attention = int(li == n_layers - 1), 0
+        L.K_bond, L.K_atom = ps[0].shape[1], ps[8].shape[1]
+        L.K_fbond = ops.D if ps[2] is None else ps[2].shape[1]
+        L.run_frag_block, L.want_attention = int(frag_block and li == n_layers - 1), 0
         L.bond_mask = L.frag_bond_mask = L.atom_mask = -1
         L.atom_mask_list, L.n_atom_mask = None, 0
     assert len(layer_params[0]) == N_PARAMS
@@ -436,6 +439,44 @@ def _head_layers(head):
     return None
 
 
+def _check_model(model, module, who: str):
+    """The head spec of a ``module.FragNetFineTune`` the one-call step covers, or ``NotImplementedError``."""
+    if type(model) is not module.FragNetFineTune:
+        raise NotImplementedError(f"{who} needs {module.__name__}.FragNetFineTune "
+                                  f"(got {type(model).__module__}.{type(model).__name__})")
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        raise NotImplementedError(f"{who} runs on one GPU")
+    spec = _head_layers(getattr(model, "fthead", None))
+    if spec is None or any(act is None for _, _, _, act in spec):
+        raise NotImplementedError(f"{who} needs an FTHead1-4 head with a relu, celu, silu, gelu, selu, relu6 or "
+                                  "leakyrelu activation")
+    if len(spec) > _abi.MLP_MAX_LAYERS or spec[0][0].in_features != 2 * ops.D:
+        raise NotImplementedError(f"{who}: unsupported head shape")
+    for layer in model.pretrain.layers:
+        layer._check_geometry()
+    return spec
+
+
+def _trained_set(spec, layer_params, units):
+    """``_analyse``'s result from the encoder's freezable units (one per layer); the head's linears are appended."""
+    n_layers = len(layer_params)
+    units = units + [[lin.weight, lin.bias] for lin, _, _, _ in spec]
+    trained = []
+    for u in units:
+        if len({p.requires_grad for p in u}) > 1:
+            raise NotImplementedError("FusedFineTuneStep: every live tensor of an encoder layer, and weight and bias "
+                                      "of a head linear, must be frozen or trained together")
+        trained.append(u[0].requires_grad)
+    enc_trained = trained[:n_layers]
+    first = enc_trained.index(True) if any(enc_trained) else n_layers
+    if not all(enc_trained[first:]):
+        raise NotImplementedError("FusedFineTuneStep: frozen encoder layers must be the lowest ones (0 .. k-1)")
+    live = [p for u, t in zip(units, trained) if t for p in u]
+    if not live:
+        raise NotImplementedError("FusedFineTuneStep: the model has no parameter to train")
+    return spec, layer_params, units, live, first
+
+
 class FusedFineTuneStep(_FlatStep):
     """``step(batch) -> loss`` (0-dim CUDA tensor) for this package's gat2 ``FragNetFineTune`` with an FTHead1-4 head:
     collate, encoder, readout, head, loss and every gradient in one ``fnb_finetune_step`` call, then Adam over the flat
@@ -449,11 +490,17 @@ class FusedFineTuneStep(_FlatStep):
     last layer's ``f`` included), ``weight`` and ``bias`` of one head linear, and frozen encoder layers must be the
     lowest ones (``0 .. k-1``, or all of them).  The backward then stops at the lowest trained layer.
 
+    ``FusedLiteFineTuneStep`` and ``FusedEdgeFineTuneStep`` do the same for the ``gat2_lite`` and ``gat2_edge``
+    versions of ``FragNetFineTune``; ``finetune_step_class(model)`` picks the class of a model.
+
     Models the library does not cover raise ``NotImplementedError``: other heads or activations (PReLU and RReLU among
-    them), the lite / edge variants, other encoder geometries, several ranks, other freezing patterns (a frozen layer
-    above a trained one, a frozen tensor inside a trained layer or linear) and a model with nothing to train."""
+    them), another model version than the class's, other encoder geometries, several ranks, other freezing patterns (a
+    frozen layer above a trained one, a frozen tensor inside a trained layer or linear) and a model with nothing to
+    train."""
 
     _NATIVE = "finetune_step"
+    _VARIANT = _abi.VARIANT_GAT2
+    _EXTRA_KEYS = ()          # batch entries the step reads beyond the gat2 hot path (DevicePrefetcher's ``keep``)
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.0,
                  loss: str = "mse"):
@@ -469,7 +516,8 @@ class FusedFineTuneStep(_FlatStep):
         n_layers = len(layer_params)
         g_views = self._bind_flat(live, dev)
         grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
-        self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of)
+        self._grad_of = grad_of
+        self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of, self._VARIANT != _abi.VARIANT_LITE)
         self._head = (_abi.CMlpLayer * len(spec))()
         for h, (lin, p_in, p_out, act) in zip(self._head, spec):
             h.W, h.b = lin.weight.data_ptr(), lin.bias.data_ptr()
@@ -487,40 +535,14 @@ class FusedFineTuneStep(_FlatStep):
         """(head spec, encoder live tensors per layer, freezable units, trained tensors in flat-buffer order, first
         trained encoder layer) of a model, or ``NotImplementedError`` for one the library does not cover."""
         from ..model.gat import gat2
-        if type(model) is not gat2.FragNetFineTune:
-            raise NotImplementedError("FusedFineTuneStep needs fragnet_b200's gat2 FragNetFineTune "
-                                      f"(got {type(model).__module__}.{type(model).__name__})")
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-            raise NotImplementedError("FusedFineTuneStep runs on one GPU")
+        spec = _check_model(model, gat2, "FusedFineTuneStep")
         enc = model.pretrain
-        spec = _head_layers(getattr(model, "fthead", None))
-        if spec is None or any(act is None for _, _, _, act in spec):
-            raise NotImplementedError("FusedFineTuneStep needs an FTHead1-4 head with a relu, celu, silu, gelu, selu, "
-                                      "relu6 or leakyrelu activation")
-        if len(spec) > _abi.MLP_MAX_LAYERS or spec[0][0].in_features != 2 * ops.D:
-            raise NotImplementedError("FusedFineTuneStep: unsupported head shape")
-        for layer in enc.layers:
-            layer._check_geometry()
         n_layers = len(enc.layers)
         layer_params = [list(layer._live_parameters()) for layer in enc.layers]
         # the library's live tensors per unit it can freeze: encoder layers (the dead f of lower layers left out), then
         # the head's linears
         units = [[p for j, p in enumerate(ps) if j != _F_INDEX or li == n_layers - 1] for li, ps in enumerate(layer_params)]
-        units += [[lin.weight, lin.bias] for lin, _, _, _ in spec]
-        trained = []
-        for u in units:
-            if len({p.requires_grad for p in u}) > 1:
-                raise NotImplementedError("FusedFineTuneStep: every live tensor of an encoder layer, and weight and bias "
-                                          "of a head linear, must be frozen or trained together")
-            trained.append(u[0].requires_grad)
-        enc_trained = trained[:n_layers]
-        first = enc_trained.index(True) if any(enc_trained) else n_layers
-        if not all(enc_trained[first:]):
-            raise NotImplementedError("FusedFineTuneStep: frozen encoder layers must be the lowest ones (0 .. k-1)")
-        live = [p for u, t in zip(units, trained) if t for p in u]
-        if not live:
-            raise NotImplementedError("FusedFineTuneStep: the model has no parameter to train")
-        return spec, layer_params, units, live, first
+        return _trained_set(spec, layer_params, units)
 
     @classmethod
     def trained_parameters(cls, model) -> List[torch.nn.Parameter]:
@@ -556,6 +578,7 @@ class FusedFineTuneStep(_FlatStep):
         a.seed, a.offset = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF, 0
         a.precision, a.backward = config.precision_id(), int(backward)
         a.first_trained_layer = self.first_trained_layer
+        a.variant = self._VARIANT
         loss = self._next_loss()
         a.loss = loss.data_ptr()
         preds = None
@@ -564,6 +587,112 @@ class FusedFineTuneStep(_FlatStep):
             a.predictions = pt(preds)
         a.plan_arena = self._take_prefetched(a.batch)
         return a, loss, preds, tensors + (y,)
+
+
+_EMPTY_GRAPH = {}
+
+
+def _empty_graph(dev):
+    """An empty edge list and its empty 6-wide attributes; persistent, so that the plan key of a batch is stable."""
+    key = str(dev)
+    if key not in _EMPTY_GRAPH:
+        _EMPTY_GRAPH[key] = (torch.zeros((2, 0), dtype=torch.int64, device=dev),
+                             torch.zeros((0, 6), dtype=torch.float32, device=dev))
+    return _EMPTY_GRAPH[key]
+
+
+class _VariantStep(FusedFineTuneStep):
+    """What the gat2_lite and gat2_edge steps share: a batch without the fragment-connection graph (its features are
+    never read) and, for gat2_lite, without fragment edges."""
+
+    def _plan_inputs(self, b, g: int, convert: bool = True):
+        e_idx, e_attr = _empty_graph(self.dev)
+        frag_index = e_idx if self._VARIANT == _abi.VARIANT_LITE else b["frag_index"]
+        return ops.batch_inputs(b["edge_index"], frag_index, b["atom_to_frag_ids"], b["edge_index_bonds_graph"],
+                                b["edge_attr_bonds"], e_idx, e_attr, b["batch"], b["frag_batch"], b["x_atoms"].shape[0],
+                                b["x_frags"].shape[0], b["node_features_bonds"].shape[0], frag_index.shape[1], g,
+                                self.dev, convert)
+
+    def _batch_inputs(self, batch, g: int):
+        inp, keep = self._plan_inputs(batch, g)
+        feats = tuple(_on(batch, k, self.dev, torch.float32) for k in ("x_atoms", "node_features_bonds"))
+        return inp, keep + feats, feats + (None,)
+
+    @staticmethod
+    def _layer_units(model, extra_last=()):
+        """Per encoder layer: the 14 program tensors (None where the variant has none or never reads them) and the
+        freezable unit of live tensors; ``extra_last``: live tensors of the last layer that the program does not take."""
+        layer_params, units = [], []
+        n_layers = len(model.pretrain.layers)
+        for li, layer in enumerate(model.pretrain.layers):
+            top = li == n_layers - 1
+            t = dict(Wb=layer.projection_b.weight, bb=layer.projection_b.bias, We_b=layer.edge_attr_bond_embed.weight,
+                     be_b=layer.edge_attr_bond_embed.bias, Wa=layer.projection_a.weight, ba=layer.projection_a.bias,
+                     a_b=layer.a_b, a=layer.a)
+            unit = list(t.values())
+            if extra_last and top:
+                t["f"] = layer.f
+                unit += [layer.f, *extra_last]
+            layer_params.append([t.get(n) for n in _abi.PARAM_FIELDS])
+            units.append(unit)
+        return layer_params, units
+
+
+class FusedLiteFineTuneStep(_VariantStep):
+    """``FusedFineTuneStep`` for this package's ``gat2_lite.FragNetFineTune``: bond graph, atom graph and the pooled
+    fragments ``ReLU(Dropout(pool(atoms)))`` of the last layer.  A layer's live tensors are ``projection_b``,
+    ``edge_attr_bond_embed``, ``projection_a``, ``a_b`` and ``a``; the fragment-side tensors never get a gradient.
+    Dropout counters: those of a gat2 encoder without fragment-connection nodes (``fnb_finetune_step_args``), which
+    is not the layout of the autograd ``gat2_lite`` path."""
+
+    _VARIANT = _abi.VARIANT_LITE
+
+    @staticmethod
+    def _analyse(model):
+        from ..model.gat import gat2_lite
+        spec = _check_model(model, gat2_lite, "FusedLiteFineTuneStep")
+        return _trained_set(spec, *_VariantStep._layer_units(model))
+
+
+class FusedEdgeFineTuneStep(_VariantStep):
+    """``FusedFineTuneStep`` for this package's ``gat2_edge.FragNetFineTune``.  The fragment graph's edge term
+    ``<cnx_attr_transform(cnx_attr[e]), f_e[h]>`` of the last layer is formed and differentiated on the device; the
+    batch needs 8-wide ``cnx_attr`` (``ValueError`` otherwise, as ``Linear(8, 128)`` upstream).  Live tensors: those of
+    ``FusedLiteFineTuneStep`` per layer, plus ``f`` and ``cnx_attr_transform`` in the last layer (frozen with it)."""
+
+    _VARIANT = _abi.VARIANT_EDGE
+    _EXTRA_KEYS = ("cnx_attr",)
+
+    def __init__(self, model, *args, **kw):
+        super().__init__(model, *args, **kw)
+        self._cnx = model.pretrain.layers[-1].cnx_attr_transform
+
+    @staticmethod
+    def _analyse(model):
+        from ..model.gat import gat2_edge
+        spec = _check_model(model, gat2_edge, "FusedEdgeFineTuneStep")
+        cnx = model.pretrain.layers[-1].cnx_attr_transform
+        return _trained_set(spec, *_VariantStep._layer_units(model, (cnx.weight, cnx.bias)))
+
+    def _args(self, batch, backward: bool, want_preds: bool):
+        from ..model.gat.gat2_edge import CNX_IN
+        cnx = _on(batch, "cnx_attr", self.dev, torch.float32)
+        if cnx.dim() != 2 or cnx.shape[1] != CNX_IN or cnx.shape[0] != batch["frag_index"].shape[1]:
+            raise ValueError(f"FusedEdgeFineTuneStep: cnx_attr must be [n_frag_edges, {CNX_IN}] "
+                             f"(cnx_attr_transform = Linear({CNX_IN}, 128)); got {tuple(cnx.shape)}")
+        a, loss, preds, keep = super()._args(batch, backward, want_preds)
+        pt = ops._ptr
+        a.cnx_attr, a.W_cnx, a.b_cnx = pt(cnx), pt(self._cnx.weight), pt(self._cnx.bias)
+        a.dW_cnx, a.db_cnx = pt(self._grad_of.get(id(self._cnx.weight))), pt(self._grad_of.get(id(self._cnx.bias)))
+        return a, loss, preds, keep + (cnx,)
+
+
+def finetune_step_class(model):
+    """The one-call finetuning step class for a ``FragNetFineTune`` of this package's model versions (gat2 for any
+    other model, whose constructor then raises ``NotImplementedError``)."""
+    from ..model.gat import gat2_edge, gat2_lite
+    return {gat2_lite.FragNetFineTune: FusedLiteFineTuneStep,
+            gat2_edge.FragNetFineTune: FusedEdgeFineTuneStep}.get(type(model), FusedFineTuneStep)
 
 
 class LaggedScalars:

@@ -8,8 +8,9 @@ staged by ``DevicePrefetcher`` (pinned, double-buffered copies on a side stream,
 instead of 16 blocking ``batch[k].to(device)`` calls per step (utils.py:335-336), and the per-batch losses are summed
 on the device and read back once per epoch instead of one ``loss.item()`` synchronisation per step (utils.py:344).
 
-``TrainerFineTune(..., fused=True)`` runs each training batch of this package's ``FragNetFineTune`` as one library call
-(``FusedFineTuneStep``: collate, encoder, readout, head, loss, backward, then Adam over flat buffers) when the
+``TrainerFineTune(..., fused=True)`` runs each training batch of this package's ``FragNetFineTune`` (gat2, gat2_lite or
+gat2_edge) as one library call (``FusedFineTuneStep`` and its ``FusedLiteFineTuneStep`` / ``FusedEdgeFineTuneStep``:
+collate, encoder, readout, head, loss, backward, then Adam over flat buffers) when the
 optimizer is a plain ``torch.optim.Adam`` holding every trained tensor in its one parameter group and the model is one
 the library covers, frozen parameters included (the lower encoder layers or the whole encoder, any head linear);
 anything else silently takes the generic loop below.  A change of ``requires_grad`` between epochs (unfreezing the
@@ -48,14 +49,21 @@ class EarlyStopping:
         self.val_loss_min = val_loss
 
 
+def _extra_keys(model):
+    """Batch entries a model of this package reads beyond the GAT2 hot path: gat2_edge reads ``cnx_attr``."""
+    from ..model.gat import gat2_edge
+    return ("cnx_attr",) if isinstance(model, (gat2_edge.FragNetFineTune, gat2_edge.FragNet)) else ()
+
+
 def _batches(loader, device, model=None):
     """Device-resident batch dicts of ``loader``: prefetched for CUDA devices, moved key by key otherwise.  For this
-    package's own models only the tensors the GAT2 path reads are moved."""
+    package's own models only the tensors their path reads are moved."""
     device = torch.device(device)
     if device.type == "cuda":
         from ..dataset.prefetch import DevicePrefetcher
         ours = model is not None and type(model).__module__.startswith("fragnet_b200.")
-        yield from DevicePrefetcher(loader, device, depth=2, hot_path_only=ours)
+        keep = _extra_keys(model) if ours else ()
+        yield from DevicePrefetcher(loader, device, depth=2, hot_path_only=ours, keep=keep)
     else:
         for batch in loader:
             yield {k: v.to(device) for k, v in batch.items()}
@@ -141,13 +149,14 @@ class TrainerFineTune:
             if wm() is model and wo() is optimizer:
                 ok = fs is not None and fs.bound_to_model() and all(id(p) in owned for p in fs.live)
                 return fs if ok else None
-        from .fused import FusedFineTuneStep
+        from .fused import finetune_step_class
+        step_class = finetune_step_class(model)
         fs = None
         try:
             # every trained tensor must be the optimizer's: the generic loop's Adam updates nothing else (frozen or
             # gradient-less tensors in the optimizer are skipped by both paths)
-            if all(id(p) in owned for p in FusedFineTuneStep.trained_parameters(model)):
-                fs = FusedFineTuneStep(model, lr=g["lr"], betas=g["betas"], eps=g["eps"],
+            if all(id(p) in owned for p in step_class.trained_parameters(model)):
+                fs = step_class(model, lr=g["lr"], betas=g["betas"], eps=g["eps"],
                                        weight_decay=g["weight_decay"], loss=loss)
                 fs.attach_optimizer(optimizer)      # optimizer.state_dict() keeps checkpointing the real moments
         except NotImplementedError:
@@ -159,7 +168,7 @@ class TrainerFineTune:
     def _fused_epoch(fs, loader, device, optimizer):
         """One training epoch through ``fs``; the next batch's collate is queued underneath every step."""
         from ..dataset.prefetch import DevicePrefetcher
-        staged = DevicePrefetcher(loader, device, depth=2, hot_path_only=True)
+        staged = DevicePrefetcher(loader, device, depth=2, hot_path_only=True, keep=fs._EXTRA_KEYS)
         feed = iter(staged)
         total = torch.zeros((), dtype=torch.float64, device=device)
         batch = next(feed, None)

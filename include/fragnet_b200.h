@@ -288,6 +288,14 @@ typedef struct fnb_encoder_opts {
                               does not visit them, and layer first_trained_layer writes its parameter gradients but
                               no input gradient, so dx_* are written only when it is 0 (see need_dx_*).  Dropout
                               counters are the same whatever its value.  0 = train every layer. */
+  int pool_frags;          /* gat2_lite (gat2_lite.py:140): no layer runs the fragment block; the last layer writes
+                              out_frags = ReLU(Dropout(pool(pre-activation atoms))) at its fragment dropout site, and the
+                              backward passes the gradient of out_frags back through the atom graph's pooling.  Needs
+                              post_act = 1 and out_frags.  0 = off. */
+  int skip_fbond;          /* skip the fragment-connection chain (projection_fb and its attention block) in the forward
+                              and the backward: its outputs and parameter gradients are not written, x_fbond is not
+                              read.  For variants without that graph (gat2_edge with frag_table, gat2_lite); a layer that
+                              runs the fragment block then needs frag_table.  Its dropout counters stay reserved. */
 } fnb_encoder_opts;
 
 typedef struct fnb_encoder_io {
@@ -510,7 +518,25 @@ typedef struct fnb_mlp_layer {
 
 /* Dropout counters: the encoder's sites as fnb_encoder_rng_span lays them out from `offset`, then the head's, in layer
  * order (a layer's input site, then its output site; a site exists where its p is non-zero), each a contiguous block
- * of ceil(G * width / 4) counters over the row-major [G, width] tensor. */
+ * of ceil(G * width / 4) counters over the row-major [G, width] tensor.
+ *
+ * Model versions (`variant`).  The step builds the batch plan from `batch` with the graphs the variant lacks emptied,
+ * and the encoder sites follow from those sizes (input; then per layer bond, atom, fragment-connection, fragment):
+ *   FNB_VARIANT_GAT2  gat2.  Sites over (Na, Nb, n_fbond_nodes, Nf) rows.
+ *   FNB_VARIANT_LITE  gat2_lite (bond graph, atom graph, pooling).  No fragment-connection graph (n_fbond_nodes and
+ *                     n_fbond_edges are taken as 0, so the fragment graph has no edges) and no fragment block: the
+ *                     last layer's fragment site covers ReLU(Dropout(pool(atoms))).  Sites over (Na, Nb, 0, Nf) rows.
+ *                     (The autograd gat2_lite path draws its last layer's three sites in separate blocks.)
+ *   FNB_VARIANT_EDGE  gat2_edge.  The fragment graph's edge term is <cnx_attr_transform(cnx_attr[e]), f_e[h]> of the
+ *                     last layer (formed on the device); the fragment-connection graph keeps its n_fbond_nodes nodes
+ *                     (one per fragment edge) but has no edges (n_fbond_edges is taken as 0) and its chain is skipped;
+ *                     its sites stay reserved, exactly as in the autograd gat2_edge call.  Sites over (Na, Nb,
+ *                     n_fbond_nodes, Nf) rows.
+ * In every variant the layers' fragment-connection tensors (Wfb, bfb, We_fb, be_fb, f_a_b) are read only by GAT2, and
+ * x_fbond may be NULL for LITE and EDGE. */
+#define FNB_VARIANT_GAT2 0
+#define FNB_VARIANT_LITE 1
+#define FNB_VARIANT_EDGE 2
 typedef struct fnb_finetune_step_args {
   fnb_batch_inputs batch;                   /* as fnb_pretrain_step_args.batch; n_graphs = G molecules */
   const float *x_atoms, *x_bond, *x_fbond;  /* [Na,K_atom] [Nb,K_bond] [Nfb,K_fbond] raw features */
@@ -534,6 +560,13 @@ typedef struct fnb_finetune_step_args {
                                                be NULL.  n_layers freezes the encoder: no encoder backward, no readout
                                                backward, layer_grads may be NULL.  A backward that trains nothing
                                                (this at n_layers and every head layer frozen) is FNB_ERR_MODE. */
+  /* zero = gat2, exactly as without these fields */
+  int variant;                              /* FNB_VARIANT_* (else FNB_ERR_MODE); run_frag_block: 0 in every layer for
+                                               LITE, the last layer only otherwise */
+  const float *cnx_attr;                    /* EDGE: [n_fbond_nodes, 8] connection attributes, frag_index edge order */
+  const float *W_cnx, *b_cnx;               /* EDGE: cnx_attr_transform of the LAST layer, [128, 8], [128] */
+  float *dW_cnx, *db_cnx;                   /* EDGE: their gradients (written, with the edge slice f[:, 32:160] of the
+                                               last layer's f gradient); NULL when the last encoder layer is frozen */
 } fnb_finetune_step_args;
 size_t fnb_finetune_step_workspace_bytes(const fnb_finetune_step_args *args);
 uint64_t fnb_finetune_step_rng_span(const fnb_finetune_step_args *args);

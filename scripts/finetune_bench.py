@@ -7,6 +7,11 @@ model on the same batches; the autograd leg is the loop body of ``TrainerFineTun
 ``MSELoss(model(b).view(-1), y)``, backward, ``optimizer.step()``) with the per-batch losses summed on the device.
 The legs alternate, ``--rounds`` times each.
 
+``--variant`` picks the model versions: ``gat2`` (default), ``lite`` (``gat2_lite``) and ``edge`` (``gat2_edge``), each
+with the same FTHead3 and the one-call step of its version (``FusedLiteFineTuneStep`` / ``FusedEdgeFineTuneStep``).
+The edge batches' connection attributes get two random columns: ``cnx_attr_transform`` is ``Linear(8, 128)`` and the
+featuriser emits 6.
+
 ``--freeze`` also times the usual finetuning set-ups with frozen parameters (``requires_grad = False``): ``lower2``
 freezes encoder layers 0 and 1, ``encoder`` the whole encoder.  Both legs then train the same tensors: the autograd leg's
 Adam holds the trainable ones, and the fused step stops its backward below the lowest trained layer.
@@ -47,7 +52,15 @@ def card():
     return info
 
 
-def make_batches(batch, pool, seed):
+VARIANTS = ("gat2", "lite", "edge")
+
+
+def model_class(variant):
+    from fragnet_b200.model.gat import gat2, gat2_edge, gat2_lite
+    return {"gat2": gat2, "lite": gat2_lite, "edge": gat2_edge}[variant].FragNetFineTune
+
+
+def make_batches(batch, pool, seed, variant="gat2"):
     """Collated ESOL-shaped batches on the device, as many as it takes for one pass to exceed L2 (at least 4)."""
     import random
 
@@ -58,7 +71,10 @@ def make_batches(batch, pool, seed):
     out, total = [], 0
     while len(out) < 4 or total < 2 * L2_BYTES:
         b = collate_fn([mols[rng.randrange(len(mols))] for _ in range(batch)])
-        b["y"] = torch.randn(b["y"].shape, generator=torch.Generator().manual_seed(seed + len(out)))
+        gen = torch.Generator().manual_seed(seed + len(out))
+        b["y"] = torch.randn(b["y"].shape, generator=gen)
+        if variant == "edge":
+            b["cnx_attr"] = torch.cat((b["cnx_attr"], torch.rand(b["cnx_attr"].shape[0], 2, generator=gen)), dim=1)
         b = {k: v.cuda() for k, v in b.items()}
         out.append(b)
         total += sum(v.numel() * v.element_size() for v in b.values())
@@ -94,26 +110,30 @@ def main():
     ap.add_argument("--rounds", type=int, default=2, help="alternations of the two legs per batch size")
     ap.add_argument("--pool", type=int, default=1128, help="distinct synthetic molecules (ESOL has 1 128)")
     ap.add_argument("--freeze", default="none", help=f"comma separated, of {', '.join(FREEZE)}")
+    ap.add_argument("--variant", default="gat2", help=f"comma separated, of {', '.join(VARIANTS)}")
     args = ap.parse_args()
     modes = args.freeze.split(",")
     if any(m not in FREEZE for m in modes):
         raise SystemExit(f"--freeze: expected names from {sorted(FREEZE)}, got {args.freeze!r}")
+    variants = args.variant.split(",")
+    if any(v not in VARIANTS for v in variants):
+        raise SystemExit(f"--variant: expected names from {list(VARIANTS)}, got {args.variant!r}")
     if not torch.cuda.is_available():
         raise SystemExit("finetune_bench.py needs a CUDA device")
-    from fragnet.model.gat.gat2 import FragNetFineTune
-    from fragnet_b200.train.fused import FusedFineTuneStep
+    from fragnet_b200.train.fused import finetune_step_class
     result = {"workload": "FragNetFineTune exps/ft/esol/e1pt4.yaml training step (fwd + MSE + bwd + Adam), "
                           "ESOL-shaped synthetic batches resident in HBM", "card": card(), "steps": args.steps,
               "warmup": args.warmup, "rounds": args.rounds, "legs": {}}
-    for batch, mode in ((int(x), m) for x in args.batches.split(",") for m in modes):
-        batches, nbytes = make_batches(batch, args.pool, seed=7)
+    for variant, batch, mode in ((v, int(x), m) for v in variants for x in args.batches.split(",") for m in modes):
+        batches, nbytes = make_batches(batch, args.pool, seed=7, variant=variant)
         torch.manual_seed(0)
-        m_fused = FragNetFineTune(**FT_KW).cuda().train()
+        kw = dict(FT_KW, edge_features=batches[0]["node_features_bonds"].shape[1])
+        m_fused = model_class(variant)(**kw).cuda().train()
         for layer in m_fused.pretrain.layers[:FREEZE[mode]]:
             for p in layer.parameters():
                 p.requires_grad_(False)
         m_auto = copy.deepcopy(m_fused)
-        fused = FusedFineTuneStep(m_fused, lr=LR)
+        fused = finetune_step_class(m_fused)(m_fused, lr=LR)
         opt = torch.optim.Adam([p for p in m_auto.parameters() if p.requires_grad], lr=LR)
         loss_fn = torch.nn.MSELoss()
         nb = len(batches)
@@ -140,7 +160,8 @@ def main():
                          "host_enqueue_ms_per_step": round(enq, 3), "fnb_launches_per_step": round(launches, 1),
                          "ms_per_step_all_rounds": [round(r[0], 3) for r in runs]}
         out["speedup"] = round(out["autograd"]["ms_per_step"] / out["fused"]["ms_per_step"], 2)
-        result["legs"][f"batch_{batch}" + ("" if mode == "none" else f"_freeze_{mode}")] = out
+        prefix = "" if variant == "gat2" else f"{variant}_"
+        result["legs"][f"{prefix}batch_{batch}" + ("" if mode == "none" else f"_freeze_{mode}")] = out
         del batches, fused, m_fused, m_auto, opt
         torch.cuda.empty_cache()
     result["card_after"] = card()
