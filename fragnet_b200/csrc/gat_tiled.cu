@@ -928,20 +928,23 @@ extern "C" int fnb_gat_fwd_tiled(const fnb_graph *g, const fnb_gat_fwd_args *f, 
   a.npc = pick_npc(g->n_nodes);
   a.deep = deep_graph(g) ? 1 : 0;
   cudaStream_t stream = (cudaStream_t)stream_;
+  // slot-ordered inputs are read only at slots: a graph without edges (or, for the table, without real edges) may
+  // pass NULL for them, as empty buffers are
+  const bool slots = g->n_edges > 0;
   switch (f->edge_mode) {
     case FNB_EDGE_NONE:
       return launch_fwd<FNB_EDGE_NONE>(a, stream);
     case FNB_EDGE_AFFINE1:
-      if (!g->edge_attr || !f->We || !f->be || !f->alpha_e) return FNB_ERR_NULL;
+      if ((slots && !g->edge_attr) || !f->We || !f->be || !f->alpha_e) return FNB_ERR_NULL;
       a.edge_attr = g->edge_attr;
       return launch_fwd<FNB_EDGE_AFFINE1>(a, stream);
     case FNB_EDGE_AFFINE6:
-      if (!g->edge_attr || !f->We || !f->be || !f->alpha_e) return FNB_ERR_NULL;
+      if ((slots && !g->edge_attr) || !f->We || !f->be || !f->alpha_e) return FNB_ERR_NULL;
       if (reinterpret_cast<uintptr_t>(g->edge_attr) & 7u) return FNB_ERR_ALIGN;
       a.edge_attr = g->edge_attr;
       return launch_fwd<FNB_EDGE_AFFINE6>(a, stream);
     case FNB_EDGE_TABLE:
-      if (!f->edge_table || !g->eid) return FNB_ERR_NULL;
+      if ((g->n_real_edges > 0 && !f->edge_table) || (slots && !g->eid)) return FNB_ERR_NULL;
       if (!fnb_aligned16(f->edge_table)) return FNB_ERR_ALIGN;
       a.edge_attr = f->edge_table;
       return launch_fwd<FNB_EDGE_TABLE>(a, stream);
@@ -962,8 +965,8 @@ int fnb_gat_bwd_tiled_fused(const fnb_graph *g, const fnb_gat_bwd_args *b, const
                             cudaEvent_t before_src, void *stream_) {
   if (!graph_ok(g) || !b) return g && b ? FNB_ERR_SIZE : FNB_ERR_NULL;
   if (g->n_nodes == 0) return 0;
-  if (!g->rowptr || !g->rrowptr || !g->rslot || !g->rdst || !b->h || !b->dout || !b->dSt || !b->dh || !b->alpha ||
-      !b->d_alpha || !b->scratch || (g->n_edges > 0 && (!g->col || !b->p_saved || !b->dz)))
+  if (!g->rowptr || !g->rrowptr || !b->h || !b->dout || !b->dSt || !b->dh || !b->alpha || !b->d_alpha || !b->scratch ||
+      (g->n_edges > 0 && (!g->col || !g->rslot || !g->rdst || !b->p_saved || !b->dz)))
     return FNB_ERR_NULL;
   if (fz) {
     if ((fz->dz_up && (!fz->slot_of_eid || !fz->alpha_up)) || (fz->y && !fz->dy) || (fz->pool && !fz->seg_of))
@@ -993,7 +996,7 @@ int fnb_gat_bwd_tiled_fused(const fnb_graph *g, const fnb_gat_bwd_args *b, const
   }
   const int grid = tile_grid(g->n_nodes, d.npc, 6);
   const bool affine = b->edge_mode == FNB_EDGE_AFFINE1 || b->edge_mode == FNB_EDGE_AFFINE6;
-  if (affine && (!g->edge_attr || !b->We || !b->be || !b->dWe || !b->dbe)) return FNB_ERR_NULL;
+  if (affine && ((g->n_edges > 0 && !g->edge_attr) || !b->We || !b->be || !b->dWe || !b->dbe)) return FNB_ERR_NULL;
   const bool fuse = fz != nullptr, deep = deep_graph(g);
   if (b->edge_mode != FNB_EDGE_AFFINE1 && b->edge_mode != FNB_EDGE_AFFINE6 && b->edge_mode != FNB_EDGE_NONE &&
       b->edge_mode != FNB_EDGE_TABLE)
@@ -1069,7 +1072,7 @@ extern "C" int fnb_attn_by_source(const int32_t *rrowptr, const int32_t *rslot, 
                                   float *w, void *stream) {
   if (n_nodes < 0) return FNB_ERR_SIZE;
   if (n_nodes == 0) return 0;
-  if (!rrowptr || !rslot || !p_saved || !w) return FNB_ERR_NULL;
+  if (!rrowptr || !w) return FNB_ERR_NULL;   // rslot, p_saved: read only at the slots rrowptr lists (none: may be NULL)
   int64_t blocks = (n_nodes + 255) / 256;
   if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
   k_attn_by_source<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(rrowptr, rslot, p_saved, n_nodes, w);

@@ -110,7 +110,7 @@ int fnb_node_scalars(const float *h, int64_t n_rows, const float *alpha, int alp
                      int off_t, int off_s, float *S, void *stream);
 
 /* w[n,h] = sum of p over the edges whose SOURCE is n (gat2.py:165,219,268,312), atomics-free over
- * the reverse CSR. */
+ * the reverse CSR.  rslot and p_saved may be NULL for a graph without edges. */
 int fnb_attn_by_source(const int32_t *rrowptr, const int32_t *rslot, const float *p_saved,
                        int64_t n_nodes, float *w, void *stream);
 
@@ -147,7 +147,8 @@ typedef struct fnb_graph {
   int64_t n_nodes, n_edges, n_real_edges; /* n_edges includes appended self loops */
   const int32_t *rowptr, *col, *row, *eid, *slot_of_eid; /* destination-sorted CSR (fnb_csr_build) */
   const int32_t *rrowptr, *rslot, *rdst;                 /* reverse (source-sorted) CSR             */
-  const float *edge_attr; /* slot-ordered attributes: [E] (bond graph), [E,6] (fragment-connection graph), else NULL */
+  const float *edge_attr; /* slot-ordered attributes: [E] (bond graph), [E,6] (fragment-connection graph), else NULL;
+                           * like every slot-ordered buffer, may be NULL when E = 0 */
 } fnb_graph;
 
 typedef struct fnb_post_act { /* y = ReLU(Dropout_p(out)); RNG counter of element i is offset + i/4 */
@@ -159,7 +160,7 @@ typedef struct fnb_post_act { /* y = ReLU(Dropout_p(out)); RNG counter of elemen
 typedef struct fnb_gat_fwd_args {
   const float *h, *S;      /* [N,128] projected features, [N,8] logit scalars */
   int edge_mode;           /* FNB_EDGE_* */
-  const float *edge_table; /* TABLE: [n_real_edges,4] */
+  const float *edge_table; /* TABLE: [n_real_edges,4] (may be NULL when n_real_edges = 0) */
   const float *We, *be;    /* AFFINE1/6: edge_attr_{bond,fbond}_embed weight [32,in] and bias [32] (gat2.py:91-92) */
   const float *alpha_e;    /* AFFINE1/6: head vector at its edge slice, rows alpha_stride apart */
   int alpha_stride;

@@ -121,3 +121,67 @@ def test_rowsparse_projection_on_one_hot_features(n, K):
     assert rel_err(dW, dh.t() @ x) <= 2e-5
     _, dW2, _ = ops.proj_bwd(x.cuda(), W.cuda(), dh.cuda(), False, want_db=False)
     assert torch.equal(dW, dW2)                      # deterministic
+
+
+def test_segment_sum_and_gather_with_empty_segments_over_several_grid_sweeps():
+    """Readouts have segments without members (leading, interior runs, trailing), and batches have more segments than
+    one grid sweep covers: k_segment_sum runs one warp per segment on at most 148 x 8 CTAs of 8 warps (9 472 segments
+    per sweep), k_segment_gather one thread per float4 on at most 148 x 16 CTAs (18 944 rows per sweep)."""
+    from fragnet_b200 import ops
+    gen = torch.Generator().manual_seed(12)
+    n_seg, n_rows = 3 * 9472 + 17, 2 * 18944 + 9
+    empty = torch.zeros(n_seg, dtype=torch.bool)
+    empty[:5] = True
+    empty[1000:1100] = True
+    empty[::7] = True
+    empty[-20:] = True
+    members = (~empty).nonzero().flatten()
+    ids = members[torch.randint(0, members.numel(), (n_rows,), generator=gen)]
+    x = torch.randn(n_rows, 128, generator=gen)
+    alpha = torch.randn(4, 192, generator=gen)
+    ref = torch.zeros(n_seg, 128, dtype=torch.float64).index_add_(0, ids, x.double())
+    assert torch.equal(ref[empty].abs().sum(1) == 0, torch.ones(int(empty.sum()), dtype=torch.bool))
+    rv = ref.view(n_seg, 4, 32)
+    a64 = alpha.double()
+    Sref = torch.cat([(rv * a64[:, 0:32]).sum(-1), (rv * a64[:, 160:192]).sum(-1)], 1)
+
+    pool = ops.csr_build(ids.cuda(), None, n_seg, reverse=False)
+    out, S = ops.segment_sum(pool.rowptr, pool.col, n_seg, x.cuda(), alpha=alpha.cuda(), alpha_stride=192, off_t=0,
+                             off_s=160)
+    assert rel_err(out, ref) <= FP32_REL_TOL and rel_err(S, Sref) <= FP32_REL_TOL
+    assert float(out[empty.cuda()].abs().max()) == 0.0 and float(S[empty.cuda()].abs().max()) == 0.0
+    base = torch.randn(n_rows, 128, generator=gen)
+    got = ops.segment_gather(out, 128, ops.narrow_index(ids.cuda()), n_rows, base.cuda())
+    assert torch.equal(got, base.cuda() + out[ids.cuda()])
+    assert rel_err(got, base.double() + ref[ids]) <= FP32_REL_TOL
+    # contiguous (readout) form, offsets built over the gaps
+    sorted_ids = torch.sort(ids).values
+    ptr = ops.segment_offsets(sorted_ids.cuda(), n_seg)
+    assert torch.equal(ptr.cpu().long(), torch.cat([torch.zeros(1, dtype=torch.long),
+                                                    torch.bincount(ids, minlength=n_seg).cumsum(0)]))
+    out2, _ = ops.segment_sum(ptr, None, n_seg, x[torch.sort(ids).indices].cuda())
+    assert rel_err(out2, ref) <= FP32_REL_TOL and float(out2[empty.cuda()].abs().max()) == 0.0
+
+
+@pytest.mark.parametrize("n,K", [(2 * 9472 + 5, 167), (2 * 18944 + 3, 17)])
+def test_rowsparse_projection_over_several_grid_sweeps(n, K):
+    """k_proj_rowsparse_fwd covers 4 rows per warp and at most 148 x 2 CTAs of 8 warps at K = 167 (86 KB of staged
+    weights: 9 472 rows per sweep), 148 x 4 at K = 17 (18 944 rows per sweep): these row counts make every warp loop."""
+    from fragnet_b200 import ops
+    g = torch.Generator().manual_seed(n + K)
+    x = torch.zeros(n, K)
+    for _ in range(9):
+        x[torch.arange(n), torch.randint(0, K, (n,), generator=g)] = 1.0
+    x[:, K - 1] = torch.randint(0, 5, (n,), generator=g).float()
+    x[n // 3] = 0.0                                  # a row without non-zeros: the bias alone
+    W = torch.randn(128, K, generator=g) * 0.2
+    b = torch.randn(128, generator=g)
+    alpha = torch.randn(4, 192, generator=g)
+    h, S = ops.proj_fwd(x.cuda(), W.cuda(), b.cuda(), alpha.cuda(), 192, 0, 160)
+    href = F.linear(x.double(), W.double(), b.double())
+    assert rel_err(h, href) <= FP32_REL_TOL
+    assert torch.equal(h[n // 3].cpu(), b)
+    hv = href.view(n, 4, 32)
+    a64 = alpha.double()
+    Sref = torch.cat([(hv * a64[:, 0:32]).sum(-1), (hv * a64[:, 160:192]).sum(-1)], dim=1)
+    assert rel_err(S, Sref) <= FP32_REL_TOL
