@@ -35,6 +35,8 @@ SIGNATURES = {
     "fnb_widen_batch": (C.c_int, [_vp, _i32, _vp]),
     "fnb_allreduce_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _f32, _f32, _f32, _f32, _f32, _i64, C.c_uint32, _vp,
                                           _vp]),
+    "fnb_allreduce_adam_runs": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _vp, _i32, _f32, _f32, _f32, _f32, _f32, C.c_uint32,
+                                          _vp, _vp]),
     "fnb_gat_fwd_tiled": (C.c_int, [_vp, _vp, _vp]),
     "fnb_gat_bwd_tiled": (C.c_int, [_vp, _vp, _vp]),
     "fnb_gat_bwd_tiled_marked": (C.c_int, [_vp, _vp, _vp, _vp]),
@@ -100,6 +102,13 @@ class CPeerSet(C.Structure):
     _fields_ = [("grads", _vp * 8), ("flags", _vp * 8), ("world", C.c_int32), ("rank", C.c_int32)]
 
 
+class CAdamRun(C.Structure):
+    _fields_ = [("first", _i64), ("end", _i64), ("step", _i64)]
+
+
+MAX_ADAM_RUNS = 16
+
+
 class CWidenJob(C.Structure):
     _fields_ = [("src", _vp), ("dst", _vp), ("n", C.c_int64), ("mode", C.c_int32)]
 
@@ -107,7 +116,7 @@ class CWidenJob(C.Structure):
 WIDEN_U8_F32, WIDEN_I32_I64, WIDEN_MAX_JOBS = 0, 1, 16
 ARENA_COPY32, ARENA_INDEX, ARENA_FILL = 0, 1, 2
 ARENA_MAX_KINDS, ARENA_MAX_JOBS = 24, 32
-ABI_VERSION = 12
+ABI_VERSION = 13
 EDGE_NONE, EDGE_AFFINE1, EDGE_AFFINE6, EDGE_TABLE = 0, 1, 2, 3
 PRECISION_FP32, PRECISION_TF32, PRECISION_TF32X3 = 0, 1, 2
 

@@ -16,7 +16,8 @@ into one flat buffer and their ``.grad`` are views into a second one.
 (fragnet/train/utils.py:330-470: ``model(batch)`` -> MSE or masked BCE -> backward -> Adam) with ``fnb_finetune_step``.
 It honours frozen parameters (``requires_grad = False``) in the layout the library supports -- the lower encoder layers
 or the whole encoder, and any of the head's linears: only the trained tensors are re-homed and updated, and the
-backward stops below the lowest trained layer.
+backward stops below the lowest trained layer.  Both steps train data-parallel over a process group: the mean of the
+ranks' gradients and Adam in one kernel over NVLink peer memory (``fnb_allreduce_adam_runs``), or NCCL.
 """
 from __future__ import annotations
 
@@ -60,13 +61,27 @@ def _encoder_structs(layer_params, grad_of, frag_block=True):
     return layers, grads
 
 
+def _same_on_every_rank(value, group, what: str) -> None:
+    """Collective: ``ValueError`` on every rank of ``group`` unless ``value`` (picklable) is equal on all of them.  A
+    step whose ranks disagree on its layout would otherwise wait forever in the first exchange, or read past a buffer."""
+    got = [None] * dist.get_world_size(group)
+    dist.all_gather_object(got, value, group=group)
+    if any(v != got[0] for v in got):
+        raise ValueError(f"fragnet_b200: {what} differ between the ranks of the process group")
+
+
 class _FlatStep:
     """What the one-call steps share: the live parameters re-homed as views of one flat buffer (their ``.grad`` views
-    of a second one), the flat Adam update, a caller's ``torch.optim.Adam`` kept truthful, and the collate of the next
-    batch underneath the running step."""
+    of a second one), the flat Adam update, a caller's ``torch.optim.Adam`` kept truthful, the gradient exchange of
+    data-parallel training, and the collate of the next batch underneath the running step."""
 
-    def _bind_flat(self, live, dev, g_store=None):
-        """Re-homes ``live`` into the flat buffers; returns the gradient views."""
+    def _bind_flat(self, live, dev, group=None, also=()):
+        """Re-homes ``live`` into the flat buffers; returns the gradient views.  ``group``: the ``torch.distributed``
+        process group of data-parallel training (``None``: the default group if one is initialised); with more than one
+        rank the gradient buffer is set up for the exchange, and the flat parameters and the tensors ``also`` are
+        broadcast from the group's rank 0.  Collective in that case: every rank of the group has to call it."""
+        self.group, self._peers = group, None
+        g_store = self._symmetric_gradient_buffer(live, dev, group)
         self.live = live
         self.flat_p, p_views = _flat_views(live, dev)
         self.flat_g, g_views = _flat_views(live, dev, storage=g_store)
@@ -75,6 +90,12 @@ class _FlatStep:
             for p, v, g in zip(live, p_views, g_views):
                 p.data = v
                 p.grad = g
+            if self.world_size > 1:
+                # DDP / Fabric broadcast rank 0's parameters at wrap time (finetune_gat2_pl.py:230): differently seeded
+                # ranks, or a checkpoint loaded on one rank only, must not diverge silently
+                src = dist.get_global_rank(group, 0) if group is not None else 0
+                for t in (self.flat_p, *(p.data for p in also)):
+                    dist.broadcast(t, src=src, group=group)
         self.exp_avg = torch.zeros_like(self.flat_p)
         self.exp_avg_sq = torch.zeros_like(self.flat_p)
         self.t = 0
@@ -100,7 +121,9 @@ class _FlatStep:
         of this object's moment buffers plus step counters, so ``optimizer.state_dict()`` checkpoints the real state;
         moments already present in ``optimizer.state`` (a resumed run) are adopted first.  Step counts stay per
         parameter, as in ``torch.optim.Adam``: when some parameters have state and others not (a layer unfrozen
-        after the others trained for a while), the new ones start from step 1."""
+        after the others trained for a while), the new ones start from step 1.  With several ranks this is collective,
+        and the ranks' step counts must agree (``ValueError`` on every rank otherwise): each rank updates its own
+        moments, as DDP's optimizers do, so a rank resumed from another checkpoint would diverge."""
         from .optim import flat_views
         _, m_views = flat_views(self.live, self.dev, storage=self.exp_avg)
         _, v_views = flat_views(self.live, self.dev, storage=self.exp_avg_sq)
@@ -124,6 +147,8 @@ class _FlatStep:
                 self._adam_runs[-1] = (self._adam_runs[-1][0], starts[i + 1], lag)
             else:
                 self._adam_runs.append((starts[i], starts[i + 1], lag))
+        if self.world_size > 1:
+            _same_on_every_rank((self.t, self._adam_runs), self.group, "the optimizer's step counts")
         self._opt_steps = {lag: torch.tensor(float(self.t - lag)) for lag in set(lags)}
         for p, m, v, lag in zip(self.live, m_views, v_views, lags):
             optimizer.state[p] = {"step": self._opt_steps[lag], "exp_avg": m, "exp_avg_sq": v}
@@ -140,6 +165,69 @@ class _FlatStep:
                 ops._p(self.exp_avg_sq[lo:]), hi - lo, self.lr, self.betas[0], self.betas[1], self.eps,
                 self.weight_decay, self.t - lag, ops._stream()), "adam_step")
         self._sync_opt_steps()
+
+    def _exchange_adam(self) -> None:
+        """Mean of the ranks' gradients + Adam at step ``self.t``, per run of equal step counts: one
+        ``fnb_allreduce_adam_runs`` kernel over NVLink peer memory (csrc/dist.cu) when the exchange buffer is set up,
+        else ``dist.all_reduce`` + scale + ``_adam()`` (a single rank: ``_adam()`` alone)."""
+        if self._peers is not None and len(self._adam_runs) <= _abi.MAX_ADAM_RUNS:
+            self._epoch += 1
+            runs = (_abi.CAdamRun * len(self._adam_runs))(*((lo, hi, self.t - lag) for lo, hi, lag in self._adam_runs))
+            _abi.check(ops._lib().fnb_allreduce_adam_runs(
+                C.byref(self._peers), ops._p(self.flat_p), ops._p(self.exp_avg), ops._p(self.exp_avg_sq),
+                self.flat_p.numel(), runs, len(runs), self.lr, self.betas[0], self.betas[1], self.eps,
+                self.weight_decay, self._epoch & 0xFFFFFFFF, ops._p(self._done), ops._stream()), "allreduce_adam_runs")
+            self._sync_opt_steps()
+            return
+        w = self.world_size
+        if w > 1:
+            dist.all_reduce(self.flat_g, op=dist.ReduceOp.SUM, group=self.group)
+            self.flat_g.mul_(1.0 / w)
+        self._adam()
+
+    def _symmetric_gradient_buffer(self, live, dev, group):
+        """World > 1: the flat gradient buffer is allocated in symmetric memory (peer-mapped over NVLink at rendezvous)
+        so that ``fnb_allreduce_adam_runs`` can read every rank's gradients directly -- exchange, mean and Adam are then
+        one kernel instead of ncclAllReduce + scale + Adam.  Returns the storage tensor, or None (single rank, no NVLink
+        peer access, a backend other than NCCL, ``FNB_FUSED_ALLREDUCE=0``): ``step`` then uses ``dist.all_reduce`` +
+        ``fnb_adam_step``."""
+        import os
+        if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) < 2:
+            return None
+        w = dist.get_world_size(group)
+        if os.environ.get("FNB_FUSED_ALLREDUCE", "1") == "0" or w > 8 or dist.get_backend(group) != "nccl":
+            return None
+        from .optim import ALIGN
+        total = sum((p.numel() + ALIGN - 1) // ALIGN * ALIGN for p in live)
+        try:
+            import torch.distributed._symmetric_memory as symm
+            pg = group if group is not None else dist.group.WORLD
+            g = symm.empty(total, dtype=torch.float32, device=dev)
+            flags = symm.empty(2 * w, dtype=torch.int32, device=dev)
+            g.zero_()
+            flags.zero_()
+            hg, hf = symm.rendezvous(g, pg), symm.rendezvous(flags, pg)
+            ps = _abi.CPeerSet()
+            for r in range(w):
+                ps.grads[r], ps.flags[r] = hg.buffer_ptrs[r], hf.buffer_ptrs[r]
+            ps.world, ps.rank = w, hg.rank
+            ok = torch.ones(1, device=dev)
+        except Exception as ex:          # no P2P between these devices, or an older torch: NCCL path
+            import warnings
+            warnings.warn(f"fragnet_b200: symmetric-memory gradient exchange unavailable ({type(ex).__name__}: {ex}); "
+                          "using ncclAllReduce", RuntimeWarning)
+            g, ok = None, torch.zeros(1, device=dev)
+        dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=group)       # all ranks take the same path (zeroed flags visible)
+        if float(ok) < 1.0 or g is None:
+            return None
+        self._peers, self._flags, self._epoch = ps, flags, 0
+        self._done = torch.zeros(1, dtype=torch.int32, device=dev)
+        self._symm_keep = (hg, hf)
+        return g
+
+    @property
+    def world_size(self) -> int:
+        return dist.get_world_size(self.group) if dist.is_available() and dist.is_initialized() else 1
 
     def _next_loss(self) -> torch.Tensor:
         self._loss_i = (self._loss_i + 1) % self._loss.numel()
@@ -238,7 +326,7 @@ class _FlatStep:
     def _step(self, batch) -> torch.Tensor:
         loss, _ = self._run(batch, backward=True)
         self.t += 1
-        self._adam()
+        self._exchange_adam()
         return loss
 
     def forward_backward(self, batch) -> torch.Tensor:
@@ -263,7 +351,7 @@ class FusedPretrainStep(_FlatStep):
         enc, head = model.pretrain, model.head
         if not head._library_shapes():
             raise NotImplementedError("FusedPretrainStep needs PretrainTask(128, 1, L=2)")
-        self.model, self.group = model, group
+        self.model = model
         self.lr, self.betas, self.eps, self.weight_decay = float(lr), betas, float(eps), float(weight_decay)
         self.dev = dev = ops.require_cuda(enc.layers[0].a.device)
         for layer in enc.layers:
@@ -278,13 +366,8 @@ class FusedPretrainStep(_FlatStep):
         live += head_params[8:]                       # ba, da, FC stacks (the bond-length head is never trained)
         if any(p.dtype != torch.float32 or p.device != dev for p in live):
             raise ValueError("FusedPretrainStep needs fp32 parameters on one CUDA device")
-        self._peers = None
-        g_views = self._bind_flat(live, dev, self._symmetric_gradient_buffer(live, dev, group))
+        g_views = self._bind_flat(live, dev, group)
         p_views = self._p_views
-        if self.world_size > 1:
-            # DDP / Fabric broadcast rank 0's parameters at wrap time (finetune_gat2_pl.py:230): differently seeded
-            # ranks, or a checkpoint loaded on one rank only, must not diverge silently
-            dist.broadcast(self.flat_p, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
         grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
         # ---- C structs (built once: parameter storage never moves afterwards)
         self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of)
@@ -298,50 +381,6 @@ class FusedPretrainStep(_FlatStep):
                 setattr(getattr(self._head_grads, group_name), fname, None if g is None else g.data_ptr())
         self._keep = (layer_params, head_params, p_views, g_views)
         self.n_layers = n_layers
-
-    # ------------------------------------------------------------------------------------------
-    def _symmetric_gradient_buffer(self, live, dev, group):
-        """World > 1: the flat gradient buffer is allocated in symmetric memory (peer-mapped over NVLink at rendezvous)
-        so that ``fnb_allreduce_adam_step`` can read every rank's gradients directly -- exchange, mean and Adam are then
-        one kernel instead of ncclAllReduce + scale + Adam.  Returns the storage tensor, or None (single rank, no NVLink
-        peer access, ``FNB_FUSED_ALLREDUCE=0``): ``step`` then uses ``dist.all_reduce`` + ``fnb_adam_step``."""
-        import os
-        if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) < 2:
-            return None
-        w = dist.get_world_size(group)
-        if os.environ.get("FNB_FUSED_ALLREDUCE", "1") == "0" or w > 8 or dist.get_backend(group) != "nccl":
-            return None
-        from .optim import ALIGN
-        total = sum((p.numel() + ALIGN - 1) // ALIGN * ALIGN for p in live)
-        try:
-            import torch.distributed._symmetric_memory as symm
-            pg = group if group is not None else dist.group.WORLD
-            g = symm.empty(total, dtype=torch.float32, device=dev)
-            flags = symm.empty(2 * w, dtype=torch.int32, device=dev)
-            g.zero_()
-            flags.zero_()
-            hg, hf = symm.rendezvous(g, pg), symm.rendezvous(flags, pg)
-            ps = _abi.CPeerSet()
-            for r in range(w):
-                ps.grads[r], ps.flags[r] = hg.buffer_ptrs[r], hf.buffer_ptrs[r]
-            ps.world, ps.rank = w, hg.rank
-            ok = torch.ones(1, device=dev)
-        except Exception as ex:          # no P2P between these devices, or an older torch: NCCL path
-            import warnings
-            warnings.warn(f"fragnet_b200: symmetric-memory gradient exchange unavailable ({type(ex).__name__}: {ex}); "
-                          "using ncclAllReduce", RuntimeWarning)
-            g, ok = None, torch.zeros(1, device=dev)
-        dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=group)       # all ranks take the same path (zeroed flags visible)
-        if float(ok) < 1.0 or g is None:
-            return None
-        self._peers, self._flags, self._epoch = ps, flags, 0
-        self._done = torch.zeros(1, dtype=torch.int32, device=dev)
-        self._symm_keep = (hg, hf)
-        return g
-
-    @property
-    def world_size(self) -> int:
-        return dist.get_world_size(self.group) if dist.is_available() and dist.is_initialized() else 1
 
     def _args(self, batch, backward: bool, want_preds: bool):
         dev = self.dev
@@ -384,25 +423,6 @@ class FusedPretrainStep(_FlatStep):
     def _draws(a) -> bool:
         return bool(a.training and a.drop_p > 0)
 
-    def _step(self, batch) -> torch.Tensor:
-        loss, _ = self._run(batch, backward=True)
-        w = self.world_size
-        self.t += 1
-        if w > 1 and self._peers is not None:
-            # gradient exchange + mean + Adam in one kernel over NVLink peer memory (csrc/dist.cu)
-            self._epoch += 1
-            _abi.check(ops._lib().fnb_allreduce_adam_step(
-                C.byref(self._peers), ops._p(self.flat_p), ops._p(self.exp_avg), ops._p(self.exp_avg_sq),
-                self.flat_p.numel(), self.lr, self.betas[0], self.betas[1], self.eps, self.weight_decay, self.t,
-                self._epoch & 0xFFFFFFFF, ops._p(self._done), ops._stream()), "allreduce_adam_step")
-            self._sync_opt_steps()
-            return loss
-        if w > 1:
-            dist.all_reduce(self.flat_g, op=dist.ReduceOp.SUM, group=self.group)
-            self.flat_g.mul_(1.0 / w)
-        self._adam()
-        return loss
-
 
 def _act_id(module) -> Optional[int]:
     """The library's activation code of an FTHead activation module, or None if it has none."""
@@ -444,8 +464,6 @@ def _check_model(model, module, who: str):
     if type(model) is not module.FragNetFineTune:
         raise NotImplementedError(f"{who} needs {module.__name__}.FragNetFineTune "
                                   f"(got {type(model).__module__}.{type(model).__name__})")
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        raise NotImplementedError(f"{who} runs on one GPU")
     spec = _head_layers(getattr(model, "fthead", None))
     if spec is None or any(act is None for _, _, _, act in spec):
         raise NotImplementedError(f"{who} needs an FTHead1-4 head with a relu, celu, silu, gelu, selu, relu6 or "
@@ -493,20 +511,32 @@ class FusedFineTuneStep(_FlatStep):
     ``FusedLiteFineTuneStep`` and ``FusedEdgeFineTuneStep`` do the same for the ``gat2_lite`` and ``gat2_edge``
     versions of ``FragNetFineTune``; ``finetune_step_class(model)`` picks the class of a model.
 
+    Data-parallel training (``group``: a ``torch.distributed`` process group, ``dist.group.WORLD`` included) follows
+    DDP: every rank computes the gradient of its own batch's loss (MSE or masked BCE divided by its own count, as Fabric
+    DDP does), and Adam applies the mean of the ranks' gradients; the parameters stay bitwise identical on every rank.
+    The construction is collective: it checks that every rank built the same layout (the same trained set, shapes and
+    lowest trained layer; ``ValueError`` on every rank otherwise) and broadcasts the model's parameters, trained and
+    frozen, and buffers from the group's rank 0, as DDP does at wrap time.  The exchange is ``fnb_allreduce_adam_runs`` over NVLink peer memory on NCCL
+    groups of up to 8 ranks with peer access, else ``dist.all_reduce`` + ``fnb_adam_step``.  Dropout counters stay per
+    rank.  A ``requires_grad`` change needs a new step, built by every rank in the same step.  Without ``group``, an
+    initialised default group of more than one rank is refused (``NotImplementedError``): one model per rank is then
+    trained on its own by the generic loop, e.g. one hyper-parameter trial per rank.
+
     Models the library does not cover raise ``NotImplementedError``: other heads or activations (PReLU and RReLU among
-    them), another model version than the class's, other encoder geometries, several ranks, other freezing patterns (a
-    frozen layer above a trained one, a frozen tensor inside a trained layer or linear) and a model with nothing to
-    train."""
+    them), another model version than the class's, other encoder geometries, other freezing patterns (a frozen layer
+    above a trained one, a frozen tensor inside a trained layer or linear) and a model with nothing to train."""
 
     _NATIVE = "finetune_step"
     _VARIANT = _abi.VARIANT_GAT2
     _EXTRA_KEYS = ()          # batch entries the step reads beyond the gat2 hot path (DevicePrefetcher's ``keep``)
 
     def __init__(self, model, lr: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.0,
-                 loss: str = "mse"):
+                 loss: str = "mse", group=None):
         if loss not in ("mse", "bce"):
             raise ValueError(f"FusedFineTuneStep: loss must be 'mse' or 'bce', got {loss!r}")
         spec, layer_params, units, live, self.first_trained_layer = self._analyse(model)
+        if group is None and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise NotImplementedError(f"{type(self).__name__} runs on one GPU unless a process group is passed (group=)")
         self.model, self.loss_kind = model, loss
         self.lr, self.betas, self.eps, self.weight_decay = float(lr), betas, float(eps), float(weight_decay)
         self.dev = dev = ops.require_cuda(model.pretrain.layers[0].a.device)
@@ -514,7 +544,12 @@ class FusedFineTuneStep(_FlatStep):
             raise ValueError("FusedFineTuneStep needs fp32 parameters on one CUDA device")
         self._requires = [p.requires_grad for u in units for p in u]
         n_layers = len(layer_params)
-        g_views = self._bind_flat(live, dev)
+        if group is not None and dist.get_world_size(group) > 1:
+            _same_on_every_rank((type(self).__name__, [tuple(p.shape) for u in units for p in u], self._requires,
+                                 self.first_trained_layer), group, "the models' trained sets, shapes or frozen layers")
+        trained = {id(p) for p in live}
+        g_views = self._bind_flat(live, dev, group, also=[t for t in (*model.parameters(), *model.buffers())
+                                                          if id(t) not in trained])
         grad_of: Dict[int, torch.Tensor] = {id(p): g for p, g in zip(live, g_views)}
         self._grad_of = grad_of
         self._layers, self._layer_grads = _encoder_structs(layer_params, grad_of, self._VARIANT != _abi.VARIANT_LITE)

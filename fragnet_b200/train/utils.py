@@ -13,8 +13,11 @@ gat2_edge) as one library call (``FusedFineTuneStep`` and its ``FusedLiteFineTun
 collate, encoder, readout, head, loss, backward, then Adam over flat buffers) when the
 optimizer is a plain ``torch.optim.Adam`` holding every trained tensor in its one parameter group and the model is one
 the library covers, frozen parameters included (the lower encoder layers or the whole encoder, any head linear);
-anything else silently takes the generic loop below.  A change of ``requires_grad`` between epochs (unfreezing the
-encoder after a warm-up) rebuilds the fused step.  Validation and test always call ``model(batch)``.
+anything else silently takes the generic loop below.  A model wrapped in ``DistributedDataParallel`` trains
+data-parallel over the wrapper's process group (the step's ``group``; DDP semantics, collective construction); an
+un-wrapped model under an initialised process group keeps the generic loop.  A change of ``requires_grad`` between
+epochs (unfreezing the encoder after a warm-up) rebuilds the fused step, on every rank in the same epoch.  Validation
+and test always call ``model(batch)``, through the wrapper if there is one.
 """
 from __future__ import annotations
 
@@ -126,7 +129,9 @@ class TrainerFineTune:
 
     # ---- fused path (fused=True): one library call per training batch
     def _fused_for(self, model, optimizer, device, loss):
-        """The ``FusedFineTuneStep`` bound to (model, optimizer), or None when the fused path does not apply."""
+        """The ``FusedFineTuneStep`` bound to (model, optimizer), or None when the fused path does not apply.  ``model``
+        may be a ``DistributedDataParallel`` wrapper: the step is built for its module over its process group, and
+        cached under the wrapper."""
         if not self.fused or torch.device(device).type != "cuda" or optimizer is None:
             return None
         from .pretrain_utils import _plain_adam
@@ -149,15 +154,17 @@ class TrainerFineTune:
             if wm() is model and wo() is optimizer:
                 ok = fs is not None and fs.bound_to_model() and all(id(p) in owned for p in fs.live)
                 return fs if ok else None
+        from torch.nn.parallel import DistributedDataParallel
         from .fused import finetune_step_class
-        step_class = finetune_step_class(model)
+        inner, group = (model.module, model.process_group) if isinstance(model, DistributedDataParallel) else (model, None)
+        step_class = finetune_step_class(inner)
         fs = None
         try:
             # every trained tensor must be the optimizer's: the generic loop's Adam updates nothing else (frozen or
             # gradient-less tensors in the optimizer are skipped by both paths)
-            if all(id(p) in owned for p in step_class.trained_parameters(model)):
-                fs = step_class(model, lr=g["lr"], betas=g["betas"], eps=g["eps"],
-                                       weight_decay=g["weight_decay"], loss=loss)
+            if all(id(p) in owned for p in step_class.trained_parameters(inner)):
+                fs = step_class(inner, lr=g["lr"], betas=g["betas"], eps=g["eps"], weight_decay=g["weight_decay"],
+                                loss=loss, group=group)
                 fs.attach_optimizer(optimizer)      # optimizer.state_dict() keeps checkpointing the real moments
         except NotImplementedError:
             fs = None

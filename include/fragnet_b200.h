@@ -36,7 +36,7 @@ extern "C" {
 
 #define FNB_D 128 /* embedding width  */
 #define FNB_H 4   /* attention heads  */
-#define FNB_ABI_VERSION 12
+#define FNB_ABI_VERSION 13
 
 /* arithmetic of the dense projections */
 #define FNB_PRECISION_FP32 0 /* FP32 FFMA: bit-for-bit comparable with the reference within 1e-5            */
@@ -388,6 +388,21 @@ typedef struct fnb_peer_set {
 int fnb_allreduce_adam_step(const fnb_peer_set *peers, float *param, float *exp_avg, float *exp_avg_sq, int64_t n,
                             float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,
                             uint32_t epoch, void *done_counter, void *stream);
+/* The same exchange and update with per-run Adam step counts: runs[0 .. n_runs) tile [0, n) in ascending order
+ * (runs[0].first == 0, runs[r].first == runs[r-1].end, the last end == n), and the elements of run r take the bias
+ * corrections of runs[r].step.  This is torch.optim.Adam over parameters whose step counts differ (a resumed run whose
+ * lower layers were frozen before).  One launch per optimizer step, as fnb_allreduce_adam_step; with one run its result
+ * is bitwise that of fnb_allreduce_adam_step.  Returns FNB_ERR_NULL for runs == NULL, FNB_ERR_ALIGN for a run boundary
+ * that is not a multiple of 4, FNB_ERR_SIZE for more than FNB_MAX_ADAM_RUNS runs, an empty, overlapping, gapped or
+ * short run table or a step < 1; the other arguments as fnb_allreduce_adam_step.  Nothing is launched on an error. */
+#define FNB_MAX_ADAM_RUNS 16
+typedef struct fnb_adam_run {
+  int64_t first, end; /* floats of the flat buffer, multiples of 4 */
+  int64_t step;       /* Adam step count of this run's parameters, from 1 */
+} fnb_adam_run;
+int fnb_allreduce_adam_runs(const fnb_peer_set *peers, float *param, float *exp_avg, float *exp_avg_sq, int64_t n,
+                            const fnb_adam_run *runs, int n_runs, float lr, float beta1, float beta2, float eps,
+                            float weight_decay, uint32_t epoch, void *done_counter, void *stream);
 
 /* ---- pretraining heads + loss (heads.cu) -------------------------------------------------------------------------
  * PretrainTask.forward (fragnet/model/gat/pretrain_heads.py:64-102) behind one call per direction: bond-length,
